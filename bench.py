@@ -16,6 +16,10 @@ the body of the reference loop var_updown/scripts/train.py:163-176. A caption = 
 step does its own host->device copy (prefetched on a copy stream, inside the timed region) and a
 device->host read of the step's loss.
 After the timed region two extra instrumented steps give the per-kernel-class times for `roofline`.
+
+`--dump-outputs DIR` writes what the last timed step of the device-resident arm computed (rank 0) as
+DIR/<name>.npy, see dump_outputs(). Inputs, weights and noise are seeded, so two builds run with the same
+arguments can be compared file by file.
 """
 import argparse
 import json
@@ -201,6 +205,37 @@ def synthetic_fsm(n_images, vocab, constraint_ids):
     return fsm[None].repeat(n_images, 1, 1, 1).contiguous()
 
 
+DUMP_SAMPLE = 1 << 16          # elements kept per parameter / gradient tensor
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, out, named):
+    """What a caller of one training step receives, from the last timed step: the per-caption losses `loss` and `kld`
+    (B,), and for every trainable parameter its gradient (`grad.<name>`) and its value after the clip + SGD update
+    (`param.<name>`). Tensors larger than DUMP_SAMPLE elements are reduced to a fixed sample: the flat indices of the
+    first DUMP_SAMPLE entries of a permutation seeded with 0, in ascending order, so every run picks the same ones."""
+    import numpy as np
+    arrays = {"loss": out["loss"], "kld": out["kld"]}
+    for k, p in named:
+        if p.grad is not None:
+            arrays["grad." + k] = p.grad
+        arrays["param." + k] = p.detach()
+    torch.cuda.synchronize()
+    host = {}
+    for name, t in arrays.items():
+        t = t.detach().float().reshape(-1)
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+            t = t[idx.to(t.device)]
+        host[name] = t.cpu().numpy().astype(np.float32)
+    total = sum(a.nbytes for a in host.values())
+    assert total <= DUMP_MAX_BYTES, total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return total
+
+
 def decode_legs(sscvae, vocab, train_model, dev, world, max_over_ranks, barrier):
     """BASELINE configs[3] and [4]: decode throughput through UpDownCaptioner.forward (eval), images sharded over
     ranks with no collective. (a) diverse sampling: 100 latent samples per image, greedy decode - the reference loop
@@ -277,6 +312,8 @@ def main():
     ap.add_argument("--no-decode", action="store_true")
     ap.add_argument("--no-gpu-eager", action="store_true")
     ap.add_argument("--profile-steps", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed training step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
     # a stalled run ends itself with every thread's stack on stderr instead of waiting for the caller's timeout
     import faulthandler
@@ -289,6 +326,8 @@ def main():
     warmup = max(args.warmup, 4) if args.impl == "ours" else max(args.warmup, 1)
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of --impl ours")
         if rank != 0:
             return
         r = cpu_reference_run(args.steps, warmup)
@@ -349,9 +388,12 @@ def main():
     resident = [tuple(t.to(dev) for t in b) for b in host]
     h2d_bytes = sum(t.numel() * t.element_size() for t in host[0])
 
+    last = {}                          # outputs of the latest step (for --dump-outputs)
+
     def train_step(feats, toks, sent):
         opt.zero_grad()
         out = model(feats, None, None, toks, sent)
+        last["out"] = out
         loss = out["loss"].mean() + out["kld"].mean() / KLD_WEIGHT        # train.py:168-171
         loss.backward()
         if reducer is not None:
@@ -405,6 +447,9 @@ def main():
         comm_exposed_ms = max_over_ranks(sum(ex) / len(ex))
     launches = _lib.launch_count() - launches0
     progress(f"device-resident arm done: {ms_dev / args.steps:.3f} ms/step")
+    if args.dump_outputs and rank == 0:
+        nbytes = dump_outputs(args.dump_outputs, last["out"], named)
+        progress(f"outputs of the last timed step written to {args.dump_outputs} ({nbytes / 1e6:.1f} MB)")
 
     # ---------------------------------------------------------------- end-to-end arm (host buffers)
     copy_stream = torch.cuda.Stream()

@@ -1,12 +1,15 @@
-"""CPU, build-container only: re-runs the live comparison oracle <-> unmodified reference
-(imported in place from /root/reference through oracle/ref_harness.py). Skipped on the GPU box."""
+"""CPU: re-runs the live comparison oracle <-> unmodified reference (visinf/style-seqcvae, imported in place
+through oracle/ref_harness.py from the checkout SSCVAE_REFERENCE_ROOT names). The reference is not part of this
+repository, so these tests skip without that checkout; the same comparison runs self-contained in
+tests/test_oracle_golden.py and tests/test_sentiment_vae2.py against the reference outputs stored in tests/golden/."""
 import pytest
 import torch
 
 from oracle import ref_harness as rh
 from oracle import updown_oracle as uo
 
-pytestmark = pytest.mark.skipif(not rh.reference_available(), reason="/root/reference not present")
+pytestmark = pytest.mark.skipif(not rh.reference_available(),
+                                reason="no checkout of the reference project (set SSCVAE_REFERENCE_ROOT)")
 
 
 @pytest.mark.parametrize("E,sv,simple", [(600, 1, False), (300, 0, False), (48, 1, False)])
