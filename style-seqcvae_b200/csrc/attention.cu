@@ -49,7 +49,7 @@ attention_fwd_kernel(AttnArgs a, AttnPlan pl, float* __restrict__ alpha, float* 
 
   if (warp == ATT_CWARPS) {                          // ---- producer
     if (lane == 0) {
-      const uint64_t pol = a.l2_policy == 1 ? ptx::l2_policy_evict_first() : a.l2_policy == 2 ? ptx::l2_policy_evict_last() : 0;
+      const uint64_t pol = ptx::l2_policy_evict_first();
       for (int r = r_begin; r < r_end; ++r) {
         const int img = a.rowmap ? a.rowmap[r] : r;
         produce_block(sm, ring, reinterpret_cast<const uint8_t*>(a.proj + (size_t)img * a.N * a.Ap), a.N, a.Ap * 2, pl.nP, pl.bP, pol);
@@ -126,7 +126,7 @@ attention_fwd_grouped_kernel(AttnArgs a, int rows_per_image, int chunks_per_imag
 
   if (warp == ATT_CWARPS) {                          // ---- producer: P in one go, then the feature chunks through the ring
     if (lane == 0) {
-      const uint64_t pol = a.l2_policy == 1 ? ptx::l2_policy_evict_first() : a.l2_policy == 2 ? ptx::l2_policy_evict_last() : 0;
+      const uint64_t pol = ptx::l2_policy_evict_first();
       const uint8_t* pbase = reinterpret_cast<const uint8_t*>(a.proj + (size_t)img * N * a.Ap);
       const uint32_t pbytes = (uint32_t)N * a.Ap * 2;
       ptx::mbar_expect_tx(p_full, pbytes);
@@ -141,8 +141,7 @@ attention_fwd_grouped_kernel(AttnArgs a, int rows_per_image, int chunks_per_imag
         const uint32_t bytes = (uint32_t)nb * a.Fp * 2;
         ptx::mbar_wait(&x_empty[stage], phase ^ 1);
         ptx::mbar_expect_tx(&x_full[stage], bytes);
-        if (pol) ptx::bulk_g2s_hint(x_ring + (size_t)stage * G_XSTAGE_BYTES, fbase + (size_t)n0 * a.Fp * 2, bytes, &x_full[stage], pol);
-        else ptx::bulk_g2s(x_ring + (size_t)stage * G_XSTAGE_BYTES, fbase + (size_t)n0 * a.Fp * 2, bytes, &x_full[stage]);
+        ptx::bulk_g2s_hint(x_ring + (size_t)stage * G_XSTAGE_BYTES, fbase + (size_t)n0 * a.Fp * 2, bytes, &x_full[stage], pol);
         if (++stage == G_XSTAGES) { stage = 0; phase ^= 1; }
       }
     }
@@ -280,13 +279,7 @@ static int make_plan(const AttnArgs& a, AttnPlan& pl) {
     return SSCVAE_ERR_UNSUPPORTED;
   }
   REQUIRE((a.Ap % 8) == 0 && (a.Fp % 8) == 0, "attention: Ap/Fp must be multiples of 8");
-  auto boxes_per_chunk = [](int row_bytes) {
-    int b = 1;
-    while (b * 2 <= ATT_MAXB && b * 2 * row_bytes <= ATT_STAGE_BYTES) b *= 2;
-    return b;
-  };
-  pl.bP = boxes_per_chunk(a.Ap * 2); pl.nP = ceil_div(a.N, pl.bP);
-  pl.bF = boxes_per_chunk(a.Fp * 2); pl.nF = ceil_div(a.N, pl.bF);
+  pl = attn_chunk_plan(a);
   static int n_sm = 0;
   if (n_sm == 0) {
     int dev = 0;
@@ -297,16 +290,7 @@ static int make_plan(const AttnArgs& a, AttnPlan& pl) {
   return 0;
 }
 
-static int attn_l2_policy() {
-  // SSCVAE_ATT_POLICY: 0 = no hint, 1 = evict_first (default: the stream must not push the recurrent weights out of L2),
-  // 2 = evict_last (with SSCVAE_W_EVICT_FIRST=1: keep the features resident, let the weights stream)
-  static const int v = [] { const char* e = getenv("SSCVAE_ATT_POLICY"); return e ? atoi(e) : 1; }();
-  return v;
-}
-
-int attention_forward(cudaStream_t s, const AttnArgs& a_in, float* alpha, float* smx, bf16* xhat, int ld_x) {
-  AttnArgs a = a_in;
-  a.l2_policy = attn_l2_policy();
+int attention_forward(cudaStream_t s, const AttnArgs& a, float* alpha, float* smx, bf16* xhat, int ld_x) {
   PROF_SCOPE(s, "attention_fwd", 0, (double)a.R*((double)a.N*(a.Ap+a.Fp)*2.0 + a.A*4.0 + a.Fp*2.0 + a.N*4.0));
   REQUIRE(a.R > 0 && (ld_x % 8) == 0 && (reinterpret_cast<uintptr_t>(xhat) & 15) == 0, "attention_forward: bad xhat layout");
   AttnPlan pl;
@@ -355,7 +339,7 @@ attention_bwd_kernel(AttnArgs a, AttnPlan pl, const float* __restrict__ smx, con
 
   if (warp == ATT_CWARPS) {                          // ---- producer: region features first, then projections
     if (lane == 0) {
-      const uint64_t pol = a.l2_policy == 1 ? ptx::l2_policy_evict_first() : a.l2_policy == 2 ? ptx::l2_policy_evict_last() : 0;
+      const uint64_t pol = ptx::l2_policy_evict_first();
       for (int r = r_begin; r < r_end; ++r) {
         const int img = a.rowmap ? a.rowmap[r] : r;
         produce_block(sm, ring, reinterpret_cast<const uint8_t*>(a.feats + (size_t)img * a.N * a.Fp), a.N, a.Fp * 2, pl.nF, pl.bF, pol);
@@ -487,10 +471,8 @@ attention_bwd_kernel(AttnArgs a, AttnPlan pl, const float* __restrict__ smx, con
   }
 }
 
-int attention_backward(cudaStream_t s, const AttnArgs& a_in, const float* smx, const float* dxhat, int ld_dx, bf16* dq,
+int attention_backward(cudaStream_t s, const AttnArgs& a, const float* smx, const float* dxhat, int ld_dx, bf16* dq,
                        int ld_dq, float* du) {
-  AttnArgs a = a_in;
-  a.l2_policy = attn_l2_policy();
   PROF_SCOPE(s, "attention_bwd", 0, (double)a.R*((double)a.N*(a.Ap+a.Fp)*2.0 + a.Fp*4.0 + a.A*6.0 + a.N*8.0));
   REQUIRE(a.R > 0 && (ld_dq % 2) == 0 && (reinterpret_cast<uintptr_t>(dq) & 3) == 0, "attention_backward: bad dq layout");
   AttnPlan pl;

@@ -1,5 +1,5 @@
 // Device-side building blocks of the fused region attention (attention.py:36-97, updown_cell.py:156-158), shared by the
-// stand-alone kernels (attention.cu) and the persistent recurrent kernel (recurrent_fwd.cu).
+// stand-alone kernels (attention.cu) and the persistent recurrent kernels (persistent.cuh).
 #pragma once
 #include "kernels.cuh"
 #include "ptx.cuh"
@@ -100,12 +100,28 @@ __host__ __device__ inline size_t attn_smem_bytes(const AttnArgs& a, bool bwd, i
 struct Ring {
   int stage = 0;
   uint32_t phase = 0;
-  int n = ATT_STAGES;                              // stages in use (<= ATT_STAGES; tuning knob of the persistent kernels)
   __device__ __forceinline__ void advance() {
-    if (++stage == n) { stage = 0; phase ^= 1; }
+    if (++stage == ATT_STAGES) { stage = 0; phase ^= 1; }
   }
 };
 
+// Chunking of the two streams of a row: as many boxes per chunk as fit one ring stage, at most ATT_MAXB.
+// rows_per_cta is left at 0 for the caller to set.
+inline AttnPlan attn_chunk_plan(const AttnArgs& a) {
+  auto boxes_per_chunk = [](int row_bytes) {
+    int b = 1;
+    while (b * 2 <= ATT_MAXB && b * 2 * row_bytes <= ATT_STAGE_BYTES) b *= 2;
+    return b;
+  };
+  AttnPlan pl;
+  pl.bP = boxes_per_chunk(a.Ap * 2); pl.nP = ceil_div(a.N, pl.bP);
+  pl.bF = boxes_per_chunk(a.Fp * 2); pl.nF = ceil_div(a.N, pl.bF);
+  pl.rows_per_cta = 0;
+  return pl;
+}
+
+// policy: ptx::l2_policy_evict_first() in every caller. The 52 MB of features + projections are read once per timestep
+// and would otherwise push the recurrent weights (76 MB, re-read every step) out of the 126 MB L2.
 __device__ __forceinline__ void produce_block(const AttnSmem& sm, Ring& ring, const uint8_t* base, int N, int row_bytes,
                                               int nchunks, int bper, uint64_t policy) {
   for (int c = 0; c < nchunks; ++c) {
@@ -114,11 +130,8 @@ __device__ __forceinline__ void produce_block(const AttnSmem& sm, Ring& ring, co
     const uint32_t bytes = (uint32_t)nb * (uint32_t)row_bytes;
     ptx::mbar_wait(&sm.empty[ring.stage], ring.phase ^ 1);
     ptx::mbar_expect_tx(&sm.full[ring.stage], bytes);
-    // evict_first: the 52 MB of features + projections are read once per timestep and would otherwise push the
-    // recurrent weights (76 MB, re-read every step) out of the 126 MB L2
-    if (policy) ptx::bulk_g2s_hint(sm.stage + (size_t)ring.stage * ATT_STAGE_BYTES, base + (size_t)n0 * row_bytes, bytes,
-                                   &sm.full[ring.stage], policy);
-    else ptx::bulk_g2s(sm.stage + (size_t)ring.stage * ATT_STAGE_BYTES, base + (size_t)n0 * row_bytes, bytes, &sm.full[ring.stage]);
+    ptx::bulk_g2s_hint(sm.stage + (size_t)ring.stage * ATT_STAGE_BYTES, base + (size_t)n0 * row_bytes, bytes, &sm.full[ring.stage],
+                       policy);
     ring.advance();
   }
 }
@@ -355,7 +368,7 @@ template <typename PrefetchNext, typename AfterDalpha = NoCall, typename Stamp =
 __device__ __forceinline__ void attn_bwd_row(const AttnArgs& a, const AttnPlan& pl, const AttnSmem& sm, Ring& ring, int cur,
                                              const float* mask_g, PrefetchNext prefetch_next, bf16* __restrict__ dq_row,
                                              int ld_dq, float* __restrict__ du_row, AfterDalpha after_dalpha = AfterDalpha(),
-                                             Stamp stamp = Stamp(), int probe = 0) {
+                                             Stamp stamp = Stamp()) {
   const int tid = attn_tid();
   const int warp = tid >> 5, lane = tid & 31;
   const int nfv = a.Fp >> 3, npair = a.Ap >> 1;
@@ -389,9 +402,7 @@ __device__ __forceinline__ void attn_bwd_row(const AttnArgs& a, const AttnPlan& 
     const int n0 = c * pl.bF, nb = min(pl.bF, a.N - n0);
     ptx::mbar_wait(&sm.full[ring.stage], ring.phase);
     const bf16x8* buf = reinterpret_cast<const bf16x8*>(sm.stage + (size_t)ring.stage * ATT_STAGE_BYTES);
-    if (probe == 1) {
-      // timing experiments only: consume the chunk without computing
-    } else if (nb == ATT_CWARPS) {
+    if (nb == ATT_CWARPS) {
       const int pr = warp >> 1, half = warp & 1, hv = nfv >> 1;
       const int na = n0 + 2 * pr;
       const bool ma = mask_img[na] != 0.f, mb = mask_img[na + 1] != 0.f;

@@ -161,7 +161,6 @@ struct AttnArgs {
   const float* w_a;                    // (A)
   int rows_per_image;                  // > 0: rows img*rows_per_image + i, i < rows_per_image, belong to image img (decode: the rows of
                                        // an image share its features; 0 = use rowmap / one image per row)
-  int l2_policy;                       // set by the launchers (SSCVAE_ATT_POLICY): 0 none, 1 evict_first, 2 evict_last
   const float* dalpha_extra;           // backward only: optional (R,N) added to d alpha (the attribute-grounded prior's path)
 };
 // smx (R,N): softmax(u*m) before the mask renormalisation, saved for the backward (null in decode)

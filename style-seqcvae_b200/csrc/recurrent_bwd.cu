@@ -2,9 +2,9 @@
 // timesteps of the UpDown cell's backward (the autograd graph of var_updown/var_updown/modules/updown_cell.py:123-231):
 //   cell_dec -> d z -> latent heads -> cell_enc -> d[x_hat | h1 | h_dec_{t-1} | h_enc_{t-1}] -> region attention backward ->
 //   query projection -> cell_att -> d[h1_{t-1} | h_dec_{t-1}]
-// which the per-launch path (api_train.cu) runs as ten kernels per step. Same engine as recurrent_fwd.cu: one CTA per SM in
-// CTA pairs, tcgen05.mma.cta_group::2 with M = 256 = the whole batch, TMA-fed operand ring, accumulators in TMEM, dataflow
-// through monotonic global counters instead of grid barriers, bounded waits.
+// which the per-launch path (api_train.cu) runs as ten kernels per step. Same engine as recurrent_fwd.cu (persistent.cuh):
+// one CTA per SM in CTA pairs, tcgen05.mma.cta_group::2 with M = 256 = the whole batch, TMA-fed operand ring, accumulators
+// in TMEM, dataflow through monotonic global counters instead of grid barriers, bounded waits.
 //
 // Decomposition. The data-gradient GEMMs have a long K (the 4H gate gradients, 57 k-blocks at H = 900) and few output
 // columns, so they are split over K: every (tile, K part) is a job of one pair, and its epilogue stores the partial
@@ -23,33 +23,14 @@
 // compute warps of ALL CTAs; the attention walks the per-step list of rows that still carry gradient (rb_active_rows_kernel).
 // The saved gates / cell states are read in the row-tiled layout of the persistent forward kernel or in the row-major
 // layout of the per-launch forward (RbParams::tiled).
-#define ATT_TID0 64
-#define ATT_STAGES_N 2
-#define ATT_STAGE_BYTES_N 32768
-#include "kernels.cuh"
-#include "gemm.cuh"
-#include "prof.cuh"
-#include "ptx.cuh"
-#include "tc_ptx.cuh"
-#include "attention_dev.cuh"
-#include <cuda.h>
-#include <algorithm>
-#include <vector>
+#define PK_NAME "recurrent_bwd"
+#include "persistent.cuh"
 
 namespace sscvae {
 
-using namespace attn;
-
 namespace {
 
-constexpr int RB_CWARPS = 8;                                   // compute warps (epilogues, pointwise stages, attention consumers)
-constexpr int RB_THREADS = 32 * (2 + RB_CWARPS + 1);           // + TMA producer, MMA issuer, attention producer
-constexpr int RB_CTHREADS = 32 * RB_CWARPS;
 constexpr int RB_STAGES = 5;
-constexpr int RB_X_BYTES = 128 * 64 * 2;                       // activation tile: 128 batch rows x 64 k (bf16)
-constexpr int RB_W_BYTES = 64 * 64 * 2;                        // weight tile half: <= 64 rows x 64 k
-constexpr int RB_STAGE_BYTES = RB_X_BYTES + RB_W_BYTES;
-constexpr int RB_TMEM_COLS = 512;
 constexpr int RB_MAX_JOBS = 3;
 
 enum { F_DGDEC = 0, F_DZP, F_DML, F_DHE, F_DGENC, F_DXEA, F_DQ, F_DXEB, F_DH1Q, F_DGATT, F_DXA, F_ABORT, F_COUNT };
@@ -106,12 +87,7 @@ struct RbParams {
   float* dXEA; float* dXEB; float* dXA; float* dzp; float* dhe_fc; float* dh1q;
   AttnArgs att; AttnPlan plan;
   unsigned int* flags;
-  int w_policy;
-  int sig_mode;
-  int att_stages;                  // attention ring stages in use (<= ATT_STAGES)
-  int probe;                       // timing experiments only (SSCVAE_RB_PROBE): 1 = attention consumes the feature chunks without computing, 2 = tiny copies
-  int att_prefetch;                // 1: bulk L2 prefetch of this CTA's attention rows ahead of the attention stage
-  int stages;
+  static constexpr int ABORT_FLAG = F_ABORT;
   unsigned long long timeout_ns;
   unsigned long long* dbg;         // SSCVAE_RB_DBG=1: globaltimer stamps of step dbg_s, 32 per CTA
   int dbg_s;
@@ -122,95 +98,7 @@ struct RbParams {
     if (p.dbg && s == p.dbg_s && (cond)) p.dbg[(size_t)blockIdx.x * 32 + (i)] = globaltimer_ns(); \
   } while (0)
 
-// ---- bounded waits --------------------------------------------------------------------------------------------
-__device__ __forceinline__ unsigned long long globaltimer_ns() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-__device__ __forceinline__ unsigned int ld_acquire_u32(const unsigned int* p) {
-  unsigned int v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void red_release_add(unsigned int* p, unsigned int v) {
-  asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async_global() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
-
-__device__ __noinline__ void rb_abort(const RbParams& p, int code, int s, unsigned int have, unsigned int want) {
-  if (atomicExch(&p.flags[F_ABORT], 1u) == 0u)
-    printf("[sscvae recurrent_bwd] wait timed out: cta %d thread %d code %d step %d have %u want %u\n", (int)blockIdx.x,
-           (int)threadIdx.x, code, s, have, want);
-  __threadfence();
-  __trap();
-}
-__device__ __forceinline__ void wait_flag(const RbParams& p, int flag, unsigned int target, int code, int s) {
-  const unsigned int* f = p.flags + flag;
-  unsigned long long t0 = 0;
-  int n = 0;
-  for (;;) {
-    const unsigned int v = ld_acquire_u32(f);
-    if ((int)(v - target) >= 0) return;
-    if ((++n & 255) == 0) {
-      const unsigned long long now = globaltimer_ns();
-      if (t0 == 0) t0 = now;
-      if (now - t0 > p.timeout_ns || ld_acquire_u32(p.flags + F_ABORT)) rb_abort(p, code, s, v, target);
-    }
-  }
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait_bounded(const RbParams& p, uint64_t* bar, uint32_t parity, int code, int s) {
-  unsigned long long t0 = 0;
-  int n = 0;
-  while (!mbar_try_wait(bar, parity)) {
-    if ((++n & 1023) == 0) {
-      const unsigned long long now = globaltimer_ns();
-      if (t0 == 0) t0 = now;
-      if (now - t0 > p.timeout_ns || ld_acquire_u32(p.flags + F_ABORT)) rb_abort(p, code, s, 0, parity);
-    }
-  }
-}
-
-__device__ __forceinline__ void tma_load_3d_2sm(void* dst, const CUtensorMap* tmap, uint64_t* bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(smem_u32(bar) & 0xFEFFFFFFu), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void tma_prefetch_2d(const CUtensorMap* tmap, int c0, int c1) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];" ::"l"(reinterpret_cast<uint64_t>(tmap)), "r"(c0), "r"(c1)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_ld_x8(uint32_t taddr, float (&v)[8]) {
-  uint32_t r[8];
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "r"(taddr)
-               : "memory");
-#pragma unroll
-  for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
-}
-
-struct RbSmem {
-  uint8_t* ring;           // RB_STAGES x (X | W)
-  uint64_t* full;          // [RB_STAGES]   TMA -> MMA (leader CTA's barrier collects both CTAs' bytes)
-  uint64_t* empty;         // [RB_STAGES]   MMA -> TMA (multicast commit)
-  uint64_t* tfull;         // [RB_SLOTS]    accumulator complete -> epilogue
-  uint32_t* tmem_slot;
-  RbJob* jobs;             // [RB_MAX_JOBS]
-  int* njobs;
-};
+using RbSmem = PkSmem<RbJob, RB_STAGES, RB_SLOTS>;
 
 // row-tiled fp32 matrix with B rows: element (b, col)
 __device__ __forceinline__ size_t tl_off(int B, int b, int col) { return ((size_t)(col >> 2) * B + b) * 4 + (col & 3); }
@@ -225,19 +113,9 @@ __device__ __forceinline__ void st_bf16x4_rb(bf16* p, float a, float b, float c,
   *reinterpret_cast<uint2*>(p) = o;
 }
 
-// The compute warps signal "my part of tensor X of this step is in global memory" (every CTA, every step).
-// `tma`: the tensor is read through TMA (async proxy) by its consumers.
-// sig_mode 1: no per-thread membar.gl: the CTA barrier orders the threads' stores before thread 0's gpu-scope release
-// (cumulativity; the pattern of cooperative-groups grid sync).
-__device__ __forceinline__ void signal_done(const RbParams& p, int flag, int ctid, bool tma = true) {
-  if (tma || p.sig_mode == 0) fence_proxy_async_global();   // generic-proxy stores -> later TMA (async proxy) reads
-  if (p.sig_mode == 0) __threadfence();
-  ptx::bar_sync(2, RB_CTHREADS);
-  if (ctid == 0) red_release_add(p.flags + flag, 1u);
-}
 __device__ __forceinline__ void wait_all(const RbParams& p, int flag, unsigned int target, int code, int s, int ctid) {
   if (ctid == 0 && target) wait_flag(p, flag, target, code, s);
-  ptx::bar_sync(1, RB_CTHREADS);
+  ptx::bar_sync(1, PK_CTHREADS);
 }
 
 // ---- pointwise stages (all CTAs) ---------------------------------------------------------------------------------
@@ -539,24 +417,14 @@ __device__ void build_jobs(const RbParams& p, int pair, RbJob* jobs, int* njobs)
 
 }  // namespace
 
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(RB_THREADS, 1)
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(PK_THREADS, 1)
 recurrent_bwd_kernel(const __grid_constant__ RbParams p) {
   extern __shared__ __align__(1024) uint8_t rb_smem_raw[];
-  uint8_t* smem = rb_smem_raw;
-  if (threadIdx.x == 0 && (smem_u32(smem) & 1023u)) __trap();
-  RbSmem sm;
-  sm.ring = smem;
-  uint8_t* att_raw = smem + RB_STAGES * RB_STAGE_BYTES;
+  if (threadIdx.x == 0 && (smem_u32(rb_smem_raw) & 1023u)) __trap();
   const AttnArgs a = p.att;
   const int ndx = p.splitA;
-  const AttnSmem asm_ = carve(att_raw, a, true, ndx, 1);
-  uint8_t* tail = att_raw + ((attn_smem_bytes(a, true, ndx, 1) + 127) & ~size_t(127));
-  sm.full = reinterpret_cast<uint64_t*>(tail);
-  sm.empty = sm.full + RB_STAGES;
-  sm.tfull = sm.empty + RB_STAGES;
-  sm.tmem_slot = reinterpret_cast<uint32_t*>(sm.tfull + RB_SLOTS);
-  sm.njobs = reinterpret_cast<int*>(sm.tmem_slot + 1);
-  sm.jobs = reinterpret_cast<RbJob*>(sm.tmem_slot + 4);
+  const RbSmem sm = RbSmem::carve(rb_smem_raw, attn_smem_bytes(a, true, ndx, 1));
+  const AttnSmem asm_ = carve(sm.att, a, true, ndx, 1);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int rank = (int)cluster_ctarank();
@@ -566,12 +434,10 @@ recurrent_bwd_kernel(const __grid_constant__ RbParams p) {
   if (threadIdx.x == 0) {
     for (int i = 0; i < NUM_AMAPS; ++i) prefetch_tmap(&p.amap[i]);
     for (int i = 0; i < NUM_WMAPS; ++i) prefetch_tmap(&p.wmap[i]);
-    for (int s = 0; s < RB_STAGES; ++s) { mbar_init(&sm.full[s], 1); mbar_init(&sm.empty[s], 1); }
-    for (int s = 0; s < RB_SLOTS; ++s) mbar_init(&sm.tfull[s], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    sm.init_barriers();
     build_jobs(p, pair, sm.jobs, sm.njobs);
   }
-  if (warp == 1) tmem_alloc_2sm<RB_TMEM_COLS>(sm.tmem_slot);
+  if (warp == 1) tmem_alloc_2sm<PK_TMEM_COLS>(sm.tmem_slot);
   attn_prologue(asm_, a, true);                        // attention ring barriers, w_a, zeroed q / d xhat buffers; __syncthreads inside
   tc_fence_before();
   cluster_sync_all();                                  // the peer's barriers exist before any remote arrival
@@ -583,32 +449,21 @@ recurrent_bwd_kernel(const __grid_constant__ RbParams p) {
   if (warp == 0) {
     // ================= TMA producer of the GEMM operand ring (both CTAs of the pair) =================
     if (elect_one_sync()) {
-      int stage = 0; uint32_t phase = 0;
-      uint64_t w_pol = 0;
-      if (p.w_policy) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(w_pol));
+      RingPos<RB_STAGES> pos;
+      const uint64_t w_pol = ptx::l2_policy_evict_first();
       for (int s = 0; s < T; ++s) {
         const int t = T - 1 - s;
         for (int j = 0; j < njobs; ++j) {
           const RbJob& job = sm.jobs[j];
-          const uint32_t tx = 2u * (uint32_t)(RB_X_BYTES + job.w_box_rows * 128);
+          const uint32_t tx = 2u * (uint32_t)(PK_X_BYTES + job.w_box_rows * 128);
           for (int g = 0; g < job.nseg; ++g) {
             const RbSeg sg = job.seg[g];
-            // the weight tiles do not depend on any flag: pull them into L2 while the activations are still being produced
-            for (int kb = 0; kb < sg.kblocks; ++kb) tma_prefetch_2d(&p.wmap[sg.wmap], sg.k0 + kb * 64, job.w_row[rank]);
-            wait_flag(p, sg.flag, (unsigned int)((s + 1) * sg.count), 100 + job.kind * 10 + g, s);
-            fence_proxy_async_global();
-            RB_STAMP(true, 20 + j * 2 + g);
-            for (int kb = 0; kb < sg.kblocks; ++kb) {
-              mbar_wait_bounded(p, &sm.empty[stage], phase ^ 1, 1, s);
-              if (rank == 0) mbar_expect_tx(&sm.full[stage], tx);
-              uint8_t* xs = sm.ring + (size_t)stage * RB_STAGE_BYTES;
-              tma_load_3d_2sm(xs, &p.amap[sg.amap], &sm.full[stage], sg.k0 + kb * 64, rank * 128, t);
-              if (p.w_policy)
-                tma_load_2d_2sm_hint(xs + RB_X_BYTES, &p.wmap[sg.wmap], &sm.full[stage], sg.k0 + kb * 64, job.w_row[rank], w_pol);
-              else
-                tma_load_2d_2sm(xs + RB_X_BYTES, &p.wmap[sg.wmap], &sm.full[stage], sg.k0 + kb * 64, job.w_row[rank]);
-              if (++stage == p.stages) { stage = 0; phase ^= 1; }
-            }
+            produce_segment(p, sm, pos, s, rank, tx, w_pol, &p.amap[sg.amap], sg.k0, t, &p.wmap[sg.wmap], sg.k0, job.w_row[rank],
+                            sg.kblocks, [&] {
+              wait_flag(p, sg.flag, (unsigned int)((s + 1) * sg.count), 100 + job.kind * 10 + g, s);
+              fence_proxy_async_global();
+              RB_STAMP(true, 20 + j * 2 + g);
+            });
           }
         }
       }
@@ -617,45 +472,25 @@ recurrent_bwd_kernel(const __grid_constant__ RbParams p) {
   } else if (warp == 1) {
     // ================= MMA issuer (leader CTA of the pair) =================
     if (rank == 0 && elect_one_sync()) {
-      int stage = 0; uint32_t phase = 0;
+      RingPos<RB_STAGES> pos;
       for (int s = 0; s < T; ++s) {
         for (int j = 0; j < njobs; ++j) {
           const RbJob& job = sm.jobs[j];
-          const uint32_t idesc = make_idesc(256, job.N);
           const int slot = kind_slot(job.kind);
-          const uint32_t tacc = tmem_base + slot * RB_TMEM_STRIDE;
-          bool first = true;
-          for (int g = 0; g < job.nseg; ++g) {
-            const int kbs = job.seg[g].kblocks;
-            for (int kb = 0; kb < kbs; ++kb) {
-              mbar_wait_bounded(p, &sm.full[stage], phase, 2, s);
-              tc_fence_after();
-              const uint32_t x_base = smem_u32(sm.ring + (size_t)stage * RB_STAGE_BYTES);
-              const uint32_t w_base = x_base + RB_X_BYTES;
-#pragma unroll
-              for (int k = 0; k < 4; ++k) {
-                umma_bf16_2sm(tacc, make_smem_desc(x_base + k * 32), make_smem_desc(w_base + k * 32), idesc, first ? 0u : 1u);
-                first = false;
-              }
-              umma_commit_2sm(&sm.empty[stage]);
-              if (++stage == p.stages) { stage = 0; phase ^= 1; }
-            }
-          }
-          umma_commit_2sm(&sm.tfull[slot]);
+          mma_job(p, sm, pos, s, job, tmem_base + slot * RB_TMEM_STRIDE, slot);
           RB_STAMP(true, 28 + j);
         }
       }
     }
     __syncwarp();
-  } else if (warp < 2 + RB_CWARPS) {
+  } else if (warp < 2 + PK_CWARPS) {
     // ================= compute warps: pointwise stages, epilogues, attention consumers =================
     const int cw = warp - 2;
     const int ctid = (int)threadIdx.x - 64;
-    const int gw = cta * RB_CWARPS + cw, GW = G * RB_CWARPS;
+    const int gw = cta * PK_CWARPS + cw, GW = G * PK_CWARPS;
     // spread the (few) latent items over all CTAs: consecutive global thread ids alternate between CTAs
-    const int gtid = ctid * G + cta, GT = G * RB_CTHREADS;
+    const int gtid = ctid * G + cta, GT = G * PK_CTHREADS;
     Ring ring;
-    ring.n = p.att_stages;
     const RbJob* jk[NUM_KINDS];
     for (int k = 0; k < NUM_KINDS; ++k) jk[k] = nullptr;
     for (int j = 0; j < njobs; ++j) jk[sm.jobs[j].kind] = &sm.jobs[j];
@@ -677,7 +512,7 @@ recurrent_bwd_kernel(const __grid_constant__ RbParams p) {
         const float* src = p.dXEA + (size_t)k * B * p.KX;
         float* dst = asm_.dx(slot, k);
         // quad i of the row -> two-plane layout of attn_bwd_row
-        for (int i = ctid; i < (a.Fp >> 2); i += RB_CTHREADS)
+        for (int i = ctid; i < (a.Fp >> 2); i += PK_CTHREADS)
           ptx::cp_async16(dst + (i & 1) * (a.Fp >> 1) + (i >> 1) * 4, src + ((size_t)i * B + b) * 4);
       }
     };
@@ -685,22 +520,6 @@ recurrent_bwd_kernel(const __grid_constant__ RbParams p) {
     cell_prefetch<1>(p, T - 1, gw, GW, lane);
     cell_prefetch<0>(p, T - 1, gw, GW, lane);
     latent_prefetch(p, T - 1, gtid, GT);
-    // bulk L2 prefetch of the attention stream of this CTA's rows (features + projections are evict_first: they come from
-    // HBM at every step, and the 4 x 16 KB ring then runs at HBM latency)
-    auto att_prefetch = [&](int t) {
-      if (!p.att_prefetch) return;
-      const int nact = p.nrows[t];
-      for (int i = cta; i < nact; i += G) {
-        const int b = p.rows[(size_t)t * B + i];
-        const uint8_t* f = reinterpret_cast<const uint8_t*>(a.feats + (size_t)b * a.N * a.Fp);
-        const uint8_t* pj = reinterpret_cast<const uint8_t*>(a.proj + (size_t)b * a.N * a.Ap);
-        const int nf = a.N * a.Fp * 2, np = a.N * a.Ap * 2;          // multiples of 16
-        for (int o = ctid * 8192; o < nf; o += RB_CTHREADS * 8192)
-          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(f + o), "r"(min(8192, nf - o)) : "memory");
-        for (int o = ctid * 8192; o < np; o += RB_CTHREADS * 8192)
-          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(pj + o), "r"(min(8192, np - o)) : "memory");
-      }
-    };
     for (int s = 0; s < T; ++s) {
       const int t = T - 1 - s;
       RB_STAMP(ctid == 0, 0);
@@ -734,7 +553,6 @@ recurrent_bwd_kernel(const __grid_constant__ RbParams p) {
       RB_STAMP(ctid == 0, 9);
       signal_done(p, F_DGENC, ctid);
       cell_prefetch<1>(p, t - 1, gw, GW, lane);
-      att_prefetch(t);
       RB_STAMP(ctid == 0, 10);
       epilogue(K_S6A, s);
       RB_STAMP(ctid == 0, 11);
@@ -758,7 +576,7 @@ recurrent_bwd_kernel(const __grid_constant__ RbParams p) {
                        [&] { if (bn >= 0) { prefetch_qs(t, bn, cur ^ 1); ptx::cp_async_commit(); } },
                        p.dqb + r * p.Ap, p.Ap, p.du + r * a.N,
                        [&] { if (bn >= 0) { prefetch_dx(bn, cur ^ 1); ptx::cp_async_commit(); } },   // single d xhat buffer
-                       [&](int k) { RB_STAMP(ctid == 0 && i == cta, k == 0 ? 19 : k == 1 ? 23 : k == 2 ? 25 : k == 3 ? 26 : 27); }, p.probe);
+                       [&](int k) { RB_STAMP(ctid == 0 && i == cta, k == 0 ? 19 : k == 1 ? 23 : k == 2 ? 25 : k == 3 ? 26 : 27); });
         }
       }
       RB_STAMP(ctid == 0, 13);
@@ -782,31 +600,21 @@ recurrent_bwd_kernel(const __grid_constant__ RbParams p) {
     // ================= attention producer: streams the region features and P of this CTA's rows =================
     if (lane == 0) {
       Ring ring;
-      ring.n = p.att_stages;
-      const uint64_t pol = a.l2_policy == 1 ? ptx::l2_policy_evict_first() : a.l2_policy == 2 ? ptx::l2_policy_evict_last() : 0;
+      const uint64_t pol = ptx::l2_policy_evict_first();
       for (int s = 0; s < T; ++s) {
         const int t = T - 1 - s;
         const int nact = p.nrows[t];
         const int* act = p.rows + (size_t)t * p.B;
         for (int i = cta; i < nact; i += G) {
           const int b = act[i];
-          if (p.probe == 2) {                              // same number of chunks, 16 x fewer bytes (what the consumers read is stale)
-            produce_block(asm_, ring, reinterpret_cast<const uint8_t*>(a.feats + (size_t)b * a.N * a.Fp), a.N, a.Fp * 2 / 16, p.plan.nF, p.plan.bF, pol);
-          } else {
-            produce_block(asm_, ring, reinterpret_cast<const uint8_t*>(a.feats + (size_t)b * a.N * a.Fp), a.N, a.Fp * 2, p.plan.nF, p.plan.bF, pol);
-          }
+          produce_block(asm_, ring, reinterpret_cast<const uint8_t*>(a.feats + (size_t)b * a.N * a.Fp), a.N, a.Fp * 2, p.plan.nF, p.plan.bF, pol);
           produce_block(asm_, ring, reinterpret_cast<const uint8_t*>(a.proj + (size_t)b * a.N * a.Ap), a.N, a.Ap * 2, p.plan.nP, p.plan.bP, pol);
         }
       }
     }
     __syncwarp();
   }
-  tc_fence_before();
-  cluster_sync_all();                                  // nobody deallocates while the pair's MMAs / loads are in flight
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc_2sm<RB_TMEM_COLS>(tmem_base);
-  }
+  pk_teardown(warp, tmem_base);
 }
 
 // rows[t*B + i] = i-th batch row (ascending) that still carries gradient at step t, nrows[t] = how many: a row is live at t
@@ -828,63 +636,8 @@ __global__ void rb_active_rows_kernel(const float* __restrict__ tmask, int T, in
   if (threadIdx.x == 0) nrows[t] = total;
 }
 
-// ---------------------------------------------------------------------------------------------------------------
 // host side
-// ---------------------------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static int rb_encode_act3d(CUtensorMap* out, const bf16* base, int K, int B, int T, int ld) {
-  EncodeTiledFn fn = reinterpret_cast<EncodeTiledFn>(tma_encode_fn());
-  if (!fn) { set_error("cuTensorMapEncodeTiled not available from the driver"); return SSCVAE_ERR_DRIVER; }
-  cuuint64_t dims[3] = {(cuuint64_t)K, (cuuint64_t)B, (cuuint64_t)T};
-  cuuint64_t strides[2] = {(cuuint64_t)ld * 2, (cuuint64_t)B * ld * 2};
-  cuuint32_t box[3] = {64, 128, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<bf16*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_error("recurrent_bwd: activation tensor map failed (%d) K=%d B=%d T=%d ld=%d", (int)r, K, B, T, ld); return SSCVAE_ERR_DRIVER; }
-  return 0;
-}
-static int rb_encode_w2d(CUtensorMap* out, const bf16* base, int K, int rows, int ld, int box_rows) {
-  EncodeTiledFn fn = reinterpret_cast<EncodeTiledFn>(tma_encode_fn());
-  if (!fn) { set_error("cuTensorMapEncodeTiled not available from the driver"); return SSCVAE_ERR_DRIVER; }
-  cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
-  cuuint32_t box[2] = {64, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<bf16*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_error("recurrent_bwd: weight tensor map failed (%d) K=%d rows=%d ld=%d box=%d", (int)r, K, rows, ld, box_rows); return SSCVAE_ERR_DRIVER; }
-  return 0;
-}
-
-static size_t rb_smem_bytes(const AttnArgs& a, int ndx) {
-  return 1024 + (size_t)RB_STAGES * RB_STAGE_BYTES + ((attn_smem_bytes(a, true, ndx, 1) + 127) & ~size_t(127)) +
-         (2 * RB_STAGES + RB_SLOTS) * 8 + 16 + RB_MAX_JOBS * sizeof(RbJob) + 64;
-}
-
-static int rb_grid_pairs(size_t smem) {
-  static int cached = -1;
-  static size_t cached_smem = 0;
-  if (cached >= 0 && cached_smem == smem) return cached;
-  int dev = 0, n_sm = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
-  if (cudaFuncSetAttribute(recurrent_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
-    cudaGetLastError();
-    return 0;
-  }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * (n_sm / 2)); cfg.blockDim = dim3(RB_THREADS); cfg.dynamicSmemBytes = smem;
-  int clusters = 0;
-  if (cudaOccupancyMaxActiveClusters(&clusters, recurrent_bwd_kernel, &cfg) != cudaSuccess) { cudaGetLastError(); clusters = 0; }
-  cached = std::min(clusters, n_sm / 2);
-  cached_smem = smem;
-  return cached;
-}
+static size_t rb_smem_bytes(const AttnArgs& a, int ndx) { return RbSmem::bytes(attn_smem_bytes(a, true, ndx, 1), RB_MAX_JOBS); }
 
 // Tiling of the jobs over NP CTA pairs; false if the shape does not fit.
 struct RbTiling { int nbig, nsmall, nA, splitA, nB, splitB, nX, splitX, nZt, splitZ, n4, N4; };
@@ -931,7 +684,7 @@ bool recurrent_backward_supported(const RecBwdArgs& r) {
   // the split of S6A (<= RB_MAX_SPLIT_A) sizes the d xhat staging buffers: take the worst case for the occupancy query
   const size_t smem = rb_smem_bytes(r.att, RB_MAX_SPLIT_A);
   if (smem > 227 * 1024) return false;
-  const int NP = rb_grid_pairs(smem);
+  const int NP = pk_grid_pairs(recurrent_bwd_kernel, smem);
   RbTiling t;
   return rb_tiling(r, NP, t);
 }
@@ -939,13 +692,10 @@ bool recurrent_backward_supported(const RecBwdArgs& r) {
 int recurrent_backward(cudaStream_t s, const RecBwdArgs& r) {
   RbParams p;
   memset(&p, 0, sizeof(p));
-  AttnArgs a = r.att;
-  static const int att_pol = [] { const char* e = getenv("SSCVAE_RB_ATT_POLICY"); return e ? atoi(e) : 1; }();
-  static const int w_pol = [] { const char* e = getenv("SSCVAE_RB_W_POLICY"); return e ? atoi(e) : 1; }();
-  a.l2_policy = att_pol;
+  const AttnArgs& a = r.att;
   REQUIRE(rb_shape_ok(r), "recurrent_bwd: unsupported shape");
   const size_t smem = rb_smem_bytes(a, RB_MAX_SPLIT_A);
-  const int NP = rb_grid_pairs(smem);
+  const int NP = pk_grid_pairs(recurrent_bwd_kernel, smem);
   RbTiling tl;
   REQUIRE(NP > 0 && rb_tiling(r, NP, tl), "recurrent_bwd: the shape does not fit the co-resident CTA pairs");
   p.B = r.B; p.T = r.T; p.H = r.H; p.Hp = r.Hp; p.Fp = r.Fp; p.Zp = r.Zp; p.Z = r.Z; p.Z2p = r.Z2p; p.A = r.A; p.Ap = r.Ap;
@@ -957,18 +707,18 @@ int recurrent_backward(cudaStream_t s, const RecBwdArgs& r) {
   p.cnt[F_DGDEC] = Gr; p.cnt[F_DML] = Gr; p.cnt[F_DGENC] = Gr; p.cnt[F_DQ] = Gr; p.cnt[F_DGATT] = Gr;
   p.cnt[F_DZP] = 2 * tl.nZt * tl.splitZ; p.cnt[F_DHE] = 2 * tl.n4; p.cnt[F_DH1Q] = 2 * tl.n4;
   p.cnt[F_DXEA] = 2 * tl.nA * tl.splitA; p.cnt[F_DXEB] = 2 * tl.nB * tl.splitB; p.cnt[F_DXA] = 2 * tl.nX * tl.splitX;
-  TRY(rb_encode_act3d(&p.amap[AM_DGDEC], r.dG_dec, r.Gp, r.B, r.T, r.Gp));
-  TRY(rb_encode_act3d(&p.amap[AM_DGENC], r.dG_enc, r.Gp, r.B, r.T, r.Gp));
-  TRY(rb_encode_act3d(&p.amap[AM_DGATT], r.dG_att, r.Gp, r.B, r.T, r.Gp));
-  TRY(rb_encode_act3d(&p.amap[AM_DML], r.dml, r.Z2p, r.B, r.T, r.Z2p));
-  TRY(rb_encode_act3d(&p.amap[AM_DQ], r.dqb, r.Ap, r.B, r.T, r.Ap));
-  TRY(rb_encode_w2d(&p.wmap[WM_DECX], r.w_dec_xzT, r.Gp, r.KX, r.Gp, 64));
-  TRY(rb_encode_w2d(&p.wmap[WM_DECZ], r.w_dec_xzT + (size_t)r.KX * r.Gp, r.Gp, r.Zp, r.Gp, 48));
-  TRY(rb_encode_w2d(&p.wmap[WM_ENCX], r.w_enc_xhT, r.Gp, r.KX, r.Gp, 64));
-  TRY(rb_encode_w2d(&p.wmap[WM_ENCH], r.w_enc_xhT + (size_t)r.KX * r.Gp, r.Gp, r.Hp, r.Gp, 32));
-  TRY(rb_encode_w2d(&p.wmap[WM_ATT], r.w_att_recT, r.Gp, 2 * r.Hp, r.Gp, 64));
-  TRY(rb_encode_w2d(&p.wmap[WM_FC], r.w_fcT, r.Z2p, r.Hp, r.Z2p, tl.N4 / 2));
-  TRY(rb_encode_w2d(&p.wmap[WM_Q], r.wqT, r.Ap, r.Hp, r.Ap, tl.N4 / 2));
+  TRY(encode_act3d(&p.amap[AM_DGDEC], r.dG_dec, r.Gp, r.B, r.T, r.Gp));
+  TRY(encode_act3d(&p.amap[AM_DGENC], r.dG_enc, r.Gp, r.B, r.T, r.Gp));
+  TRY(encode_act3d(&p.amap[AM_DGATT], r.dG_att, r.Gp, r.B, r.T, r.Gp));
+  TRY(encode_act3d(&p.amap[AM_DML], r.dml, r.Z2p, r.B, r.T, r.Z2p));
+  TRY(encode_act3d(&p.amap[AM_DQ], r.dqb, r.Ap, r.B, r.T, r.Ap));
+  TRY(encode_w2d(&p.wmap[WM_DECX], r.w_dec_xzT, r.Gp, r.KX, r.Gp, 64));
+  TRY(encode_w2d(&p.wmap[WM_DECZ], r.w_dec_xzT + (size_t)r.KX * r.Gp, r.Gp, r.Zp, r.Gp, 48));
+  TRY(encode_w2d(&p.wmap[WM_ENCX], r.w_enc_xhT, r.Gp, r.KX, r.Gp, 64));
+  TRY(encode_w2d(&p.wmap[WM_ENCH], r.w_enc_xhT + (size_t)r.KX * r.Gp, r.Gp, r.Hp, r.Gp, 32));
+  TRY(encode_w2d(&p.wmap[WM_ATT], r.w_att_recT, r.Gp, 2 * r.Hp, r.Gp, 64));
+  TRY(encode_w2d(&p.wmap[WM_FC], r.w_fcT, r.Z2p, r.Hp, r.Z2p, tl.N4 / 2));
+  TRY(encode_w2d(&p.wmap[WM_Q], r.wqT, r.Ap, r.Hp, r.Ap, tl.N4 / 2));
   p.gates_att = r.gates_att; p.gates_enc = r.gates_enc; p.gates_dec = r.gates_dec;
   p.c1 = r.c1; p.c_enc = r.c_enc; p.c_dec = r.c_dec;
   p.mean = r.mean; p.logvar = r.logvar; p.eps = r.eps; p.pm_row = r.pm_row;
@@ -979,68 +729,26 @@ int recurrent_backward(cudaStream_t s, const RecBwdArgs& r) {
   p.dXEA = r.dXEA; p.dXEB = r.dXEB; p.dXA = r.dXA; p.dzp = r.dzp; p.dhe_fc = r.dhe_fc; p.dh1q = r.dh1q;
   p.att = a;
   p.flags = r.flags;
-  p.w_policy = w_pol;
-  static const int sig_mode = [] { const char* e = getenv("SSCVAE_RB_SIG_MODE"); return e ? atoi(e) : 1; }();
-  static const int att_pf = [] { const char* e = getenv("SSCVAE_RB_ATT_PREFETCH"); return e ? atoi(e) : 0; }();
-  p.sig_mode = sig_mode; p.att_prefetch = att_pf;
-  static const int probe = [] { const char* e = getenv("SSCVAE_RB_PROBE"); return e ? atoi(e) : 0; }();
-  p.probe = probe;
-  static const int att_stages = [] { const char* e = getenv("SSCVAE_RB_ATT_STAGES"); return e ? std::min(ATT_STAGES, std::max(2, atoi(e))) : ATT_STAGES; }();
-  p.att_stages = att_stages;
-  static const int n_stages = [] { const char* e = getenv("SSCVAE_RB_STAGES"); return e ? std::min(RB_STAGES, std::max(2, atoi(e))) : RB_STAGES; }();
-  p.stages = n_stages;
-  static const unsigned long long timeout_ms = [] { const char* e = getenv("SSCVAE_RF_TIMEOUT_MS"); return e ? (unsigned long long)atoll(e) : 4000ull; }();
-  p.timeout_ns = timeout_ms * 1000000ull;
-  {  // chunking of the attention streams (as attention.cu: make_plan)
-    auto boxes_per_chunk = [](int row_bytes) {
-      int b = 1;
-      while (b * 2 <= ATT_MAXB && b * 2 * row_bytes <= ATT_STAGE_BYTES) b *= 2;
-      return b;
-    };
-    p.plan.bP = boxes_per_chunk(a.Ap * 2); p.plan.nP = ceil_div(a.N, p.plan.bP);
-    p.plan.bF = boxes_per_chunk(a.Fp * 2); p.plan.nF = ceil_div(a.N, p.plan.bF);
-    p.plan.rows_per_cta = 0;
-  }
+  p.timeout_ns = pk_timeout_ns();
+  p.plan = attn_chunk_plan(a);
   // model FLOPs of the loop: the three data-gradient GEMMs, d z, latent heads, query; bytes: the attention stream
   const double G4 = 4.0 * r.H;
   const double flops = 2.0 * r.B * r.T * (G4 * (r.KX + r.Zp) + G4 * (r.KX + r.Hp) + G4 * 2.0 * r.Hp + 2.0 * r.Z * r.H + (double)r.A * r.H);
   PROF_SCOPE(s, "recurrent_bwd", flops, (double)r.B * r.T * a.N * (a.Ap + a.Fp) * 2.0);
   static const bool dbg = [] { const char* e = getenv("SSCVAE_RB_DBG"); return e && e[0] == '1'; }();
-  static unsigned long long* dbg_buf = nullptr;
   if (dbg) {
-    if (!dbg_buf) CUDA_TRY(cudaMalloc(&dbg_buf, 32 * 8 * 2 * 128));
-    CUDA_TRY(cudaMemsetAsync(dbg_buf, 0, 32 * 8 * 2 * 128, s));
-    p.dbg = dbg_buf;
+    TRY(pk_dbg_begin(s, &p.dbg));
     p.dbg_s = r.T / 2;
   }
   CUDA_TRY(cudaMemsetAsync(r.flags, 0, 64 * sizeof(unsigned int), s));
   rb_active_rows_kernel<<<r.T, round_up(r.B, 32), 0, s>>>(r.tmask, r.T, r.B, r.rows, r.rows + (size_t)r.T * r.B);
   CUDA_TRY(cudaGetLastError());
   ++g_launch_count;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * NP); cfg.blockDim = dim3(RB_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeCooperative;
-  attr[0].val.cooperative = 1;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  CUDA_TRY(cudaLaunchKernelEx(&cfg, recurrent_bwd_kernel, p));
-  ++g_launch_count;
+  TRY(pk_launch(recurrent_bwd_kernel, NP, smem, s, p));
   if (dbg) {
-    static int printed = 0;
-    CUDA_TRY(cudaStreamSynchronize(s));
-    std::vector<unsigned long long> h(32 * 2 * NP);
-    CUDA_TRY(cudaMemcpy(h.data(), dbg_buf, h.size() * 8, cudaMemcpyDeviceToHost));
-    if (printed++ < 6) {
-      unsigned long long t0 = ~0ull;
-      for (int c = 0; c < 2 * NP; ++c) if (h[c * 32] && h[c * 32] < t0) t0 = h[c * 32];
-      const int show[] = {0, 1, 2 * tl.nbig - 2, 2 * tl.nbig, 2 * NP - 2};
-      for (int c : show) {
-        if (c < 0 || c >= 2 * NP) continue;
-        fprintf(stderr, "[rbdbg] B=%d s=%d cta=%3d:", r.B, p.dbg_s, c);
-        for (int i = 0; i < 32; ++i) fprintf(stderr, " %d:%.1f", i, h[c * 32 + i] ? (double)(h[c * 32 + i] - t0) / 1e3 : -1.0);
-        fprintf(stderr, "\n");
-      }
-    }
+    char head[64];
+    snprintf(head, sizeof(head), "[rbdbg] B=%d s=%d", r.B, p.dbg_s);
+    TRY(pk_dbg_print(s, p.dbg, 2 * NP, head, {0, 1, 2 * tl.nbig - 2, 2 * tl.nbig, 2 * NP - 2}, 32));
   }
   return 0;
 }

@@ -27,41 +27,19 @@
 // Deadlock freedom: a pair's jobs are issued in a fixed order and no job depends on a later job of the same pair
 // (q / fc tiles never share a pair with LSTM tiles); the launch is cooperative (all CTAs co-resident). Every wait
 // is bounded: on a timeout the kernel raises the abort flag, prints the wait that failed and traps.
-#define ATT_TID0 64
-#define ATT_STAGES_N 2
-#define ATT_STAGE_BYTES_N 32768
-#include "kernels.cuh"
-#include "gemm.cuh"
-#include "prof.cuh"
-#include "ptx.cuh"
-#include "tc_ptx.cuh"
-#include "attention_dev.cuh"
-#include <cuda.h>
+#define PK_NAME "recurrent_fwd"
+#include "persistent.cuh"
 #include <curand_kernel.h>
-#include <mutex>
-#include <unordered_map>
-#include <vector>
 
 namespace sscvae {
 
-using namespace attn;
-
 namespace {
 
-constexpr int RF_CWARPS = 8;                                   // compute warps (epilogues + attention consumers)
-constexpr int RF_THREADS = 32 * (2 + RF_CWARPS + 1);           // + TMA producer, MMA issuer, attention producer
-constexpr int RF_CTHREADS = 32 * RF_CWARPS;
 constexpr int RF_STAGES = 6;
-constexpr int RF_X_BYTES = 128 * 64 * 2;                       // activation tile: 128 batch rows x 64 k (bf16)
-constexpr int RF_W_BYTES = 64 * 64 * 2;                        // weight tile half: <= 64 rows x 64 k
-constexpr int RF_STAGE_BYTES = RF_X_BYTES + RF_W_BYTES;
-constexpr int RF_TMEM_COLS = 512;
 
+// One counter per tensor family. The hidden states (FLAG_H1, FLAG_HDEC, FLAG_HENC) are bumped by both CTAs of every
+// LSTM tile's pair: 2 * nt signals per timestep.
 enum { FLAG_H1 = 0, FLAG_HDEC, FLAG_HENC, FLAG_XHAT, FLAG_Q, FLAG_Z, FLAG_ABORT, FLAG_COUNT };
-// The three hidden states (families FLAG_H1, FLAG_HDEC, FLAG_HENC) are produced tile by tile (32 units per LSTM tile) and
-// consumed k-block by k-block (64 units = 2 tiles): they are tracked per TILE, counter = 2 per timestep (both CTAs of the
-// owning pair), so that a consumer streams the k-blocks whose tiles are done while the other epilogues still run.
-constexpr int TILE_FLAG_BASE = 16, TILE_FLAG_STRIDE = 64, RF_FLAG_WORDS = TILE_FLAG_BASE + 3 * TILE_FLAG_STRIDE;
 enum { MAP_XA = 0, MAP_XE, MAP_HE, MAP_ZB, MAP_EMB, NUM_AMAPS };
 enum { WMAP_ATT = 0, WMAP_Q, WMAP_ENC_X, WMAP_ENC_HH, WMAP_FC, WMAP_DEC_X, WMAP_DEC_Z, WMAP_ATT_E, NUM_WMAPS };
 enum { SLOT_ATT = 0, SLOT_LSTM, SLOT_Q, SLOT_FC, NUM_SLOTS };
@@ -77,7 +55,7 @@ struct RfSeg {
   int kblocks;
   int t_off;               // the activation is read at time index t + t_off
   int flag;                // counter that must reach (t + flag_toff) * flag_mult before the segment is loaded (-1: none);
-                           // FLAG_H1 / FLAG_HDEC / FLAG_HENC: per-tile counters, k-block kb waits for tiles 2kb, 2kb+1
+                           // FLAG_H1 / FLAG_HDEC / FLAG_HENC: (t + flag_toff) * flag_mult * nt
   int flag_mult, flag_toff;
 };
 struct RfJob {
@@ -114,10 +92,7 @@ struct RfParams {
   AttnArgs att; AttnPlan plan;
   float* alpha; float* smx;
   unsigned int* flags;
-  int w_policy;
-  int tile_flags;                  // 1: per-tile counters for the hidden states (SSCVAE_RF_TILE_FLAGS=1; measured slower: 2.18 vs 1.95 ms)
-  int stages;                      // ring stages in use (<= RF_STAGES; SSCVAE_RF_STAGES, tuning knob)
-  int sig_mode;                    // 0: membar.gl by every thread in front of a signal (SSCVAE_RF_SIG_MODE=0), 1: barrier + release only
+  static constexpr int ABORT_FLAG = FLAG_ABORT;
   unsigned long long timeout_ns;
   unsigned long long* dbg;         // SSCVAE_RF_DBG=1: globaltimer stamps of step dbg_t, 32 per CTA
   int dbg_t;
@@ -128,132 +103,14 @@ struct RfParams {
     if (p.dbg && t == p.dbg_t && (cond)) p.dbg[(size_t)blockIdx.x * 32 + (i)] = globaltimer_ns(); \
   } while (0)
 
-// ---- bounded waits --------------------------------------------------------------------------------------------
-__device__ __forceinline__ unsigned long long globaltimer_ns() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-__device__ __forceinline__ unsigned int ld_acquire_u32(const unsigned int* p) {
-  unsigned int v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void red_release_add(unsigned int* p, unsigned int v) {
-  asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async_global() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
-
-__device__ __noinline__ void rf_abort(const RfParams& p, int code, int t, unsigned int have, unsigned int want) {
-  if (atomicExch(&p.flags[FLAG_ABORT], 1u) == 0u)
-    printf("[sscvae recurrent_fwd] wait timed out: cta %d thread %d code %d t %d have %u want %u\n", (int)blockIdx.x,
-           (int)threadIdx.x, code, t, have, want);
-  __threadfence();
-  __trap();
-}
-__device__ __forceinline__ void wait_flag(const RfParams& p, int flag, unsigned int target, int code, int t) {
-  const unsigned int* f = p.flags + flag;
-  unsigned long long t0 = 0;
-  int n = 0;
-  for (;;) {
-    const unsigned int v = ld_acquire_u32(f);
-    if ((int)(v - target) >= 0) return;
-    if ((++n & 255) == 0) {
-      const unsigned long long now = globaltimer_ns();
-      if (t0 == 0) t0 = now;
-      if (now - t0 > p.timeout_ns || ld_acquire_u32(p.flags + FLAG_ABORT)) rf_abort(p, code, t, v, target);
-    }
-  }
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait_bounded(const RfParams& p, uint64_t* bar, uint32_t parity, int code, int t) {
-  unsigned long long t0 = 0;
-  int n = 0;
-  while (!mbar_try_wait(bar, parity)) {
-    if ((++n & 1023) == 0) {
-      const unsigned long long now = globaltimer_ns();
-      if (t0 == 0) t0 = now;
-      if (now - t0 > p.timeout_ns || ld_acquire_u32(p.flags + FLAG_ABORT)) rf_abort(p, code, t, 0, parity);
-    }
-  }
-}
-
-// ---- TMA / TMEM wrappers not in tc_ptx.cuh ---------------------------------------------------------------------
-__device__ __forceinline__ void tma_load_3d_2sm(void* dst, const CUtensorMap* tmap, uint64_t* bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(smem_u32(bar) & 0xFEFFFFFFu), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void tma_prefetch_2d(const CUtensorMap* tmap, int c0, int c1) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];" ::"l"(reinterpret_cast<uint64_t>(tmap)), "r"(c0), "r"(c1)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_ld_x8(uint32_t taddr, float (&v)[8]) {
-  uint32_t r[8];
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "r"(taddr)
-               : "memory");
-#pragma unroll
-  for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
-}
-
 __device__ __forceinline__ float philox_normal_rf(unsigned long long seed, unsigned long long step, int r, int z, int Z) {
   curandStatePhilox4_32_10_t st;                       // the stream of pointwise.cu: latent_fwd_train_kernel
   curand_init(seed, (unsigned long long)r * Z + z, step, &st);
   return curand_normal(&st);
 }
 
-struct RfSmem {
-  uint8_t* ring;           // RF_STAGES x (X | W)
-  uint64_t* full;          // [RF_STAGES]   TMA -> MMA (leader CTA's barrier collects both CTAs' bytes)
-  uint64_t* empty;         // [RF_STAGES]   MMA -> TMA (multicast commit)
-  uint64_t* tfull;         // [NUM_SLOTS]   accumulator complete -> epilogue
-  uint32_t* tmem_slot;
-  RfJob* jobs;             // [2]
-  int* njobs;
-};
+using RfSmem = PkSmem<RfJob, RF_STAGES, NUM_SLOTS>;
 
-// The compute warps signal "my part of tensor X at step t is in global memory".
-// No per-thread membar.gl (sig_mode 1, default): the CTA barrier orders the threads' stores before thread 0's gpu-scope
-// release (cumulativity; the pattern of cooperative-groups grid sync). Measured on the BPTT kernel: -0.15 ms per step.
-__device__ __forceinline__ void signal_done(const RfParams& p, int flag, int ctid) {
-  fence_proxy_async_global();                          // generic-proxy stores -> later TMA (async proxy) reads
-  if (p.sig_mode == 0) __threadfence();
-  ptx::bar_sync(2, RF_CTHREADS);
-  if (ctid == 0) red_release_add(p.flags + flag, 1u);
-}
-
-__device__ __forceinline__ void signal_tile_done(const RfParams& p, int family, int tile, int ctid) {
-  fence_proxy_async_global();
-  if (p.sig_mode == 0) __threadfence();
-  ptx::bar_sync(2, RF_CTHREADS);
-  if (ctid == 0) red_release_add(p.tile_flags ? p.flags + TILE_FLAG_BASE + family * TILE_FLAG_STRIDE + tile : p.flags + family, 1u);
-}
-// Number of leading k-blocks of a hidden-state segment whose producer tiles have reached `target` (polled by the
-// TMA producer thread: all counters of the family are read with independent loads, one fence orders them).
-__device__ __forceinline__ int ready_kblocks(const RfParams& p, int family, int nt, int kblocks, unsigned int target) {
-  const unsigned int* f = p.flags + TILE_FLAG_BASE + family * TILE_FLAG_STRIDE;
-  int first_not_ready = nt;
-  for (int i = nt - 1; i >= 0; --i) {
-    unsigned int v;
-    asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(f + i) : "memory");
-    if ((int)(v - target) < 0) first_not_ready = i;
-  }
-  asm volatile("fence.acq_rel.gpu;" ::: "memory");
-  return first_not_ready >= nt ? kblocks : min(kblocks, first_not_ready >> 1);
-}
 __device__ __forceinline__ float4 ld4g(const float* p) { return *reinterpret_cast<const float4*>(p); }
 __device__ __forceinline__ void add4v(float* v, const float4& w) { v[0] += w.x; v[1] += w.y; v[2] += w.z; v[3] += w.w; }
 __device__ __forceinline__ void fma4v(float* v, float s, const float4& w) {
@@ -267,12 +124,6 @@ __device__ __forceinline__ void st_bf16x4_rf(bf16* p, const float* h) {
   *reinterpret_cast<uint2*>(p) = o;
 }
 
-__device__ __forceinline__ void tmem_st_x8(uint32_t taddr, const float (&v)[8]) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr),
-               "r"(__float_as_uint(v[0])), "r"(__float_as_uint(v[1])), "r"(__float_as_uint(v[2])), "r"(__float_as_uint(v[3])),
-               "r"(__float_as_uint(v[4])), "r"(__float_as_uint(v[5])), "r"(__float_as_uint(v[6])), "r"(__float_as_uint(v[7]))
-               : "memory");
-}
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 // Branch-free gate nonlinearities: the epilogue warps run two per SM sub-partition with little to hide instruction
@@ -565,23 +416,13 @@ __device__ void build_jobs(const RfParams& p, int pair, RfJob* jobs, int* njobs)
 
 }  // namespace
 
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(RF_THREADS, 1)
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(PK_THREADS, 1)
 recurrent_fwd_kernel(const __grid_constant__ RfParams p) {
   extern __shared__ __align__(1024) uint8_t rf_smem_raw[];
-  uint8_t* smem = rf_smem_raw;
-  if (threadIdx.x == 0 && (smem_u32(smem) & 1023u)) __trap();
-  RfSmem sm;
-  sm.ring = smem;
-  uint8_t* att_raw = smem + RF_STAGES * RF_STAGE_BYTES;
+  if (threadIdx.x == 0 && (smem_u32(rf_smem_raw) & 1023u)) __trap();
   const AttnArgs a = p.att;
-  const AttnSmem asm_ = carve(att_raw, a, false);
-  uint8_t* tail = att_raw + ((attn_smem_bytes(a, false) + 127) & ~size_t(127));
-  sm.full = reinterpret_cast<uint64_t*>(tail);
-  sm.empty = sm.full + RF_STAGES;
-  sm.tfull = sm.empty + RF_STAGES;
-  sm.tmem_slot = reinterpret_cast<uint32_t*>(sm.tfull + NUM_SLOTS);
-  sm.njobs = reinterpret_cast<int*>(sm.tmem_slot + 1);
-  sm.jobs = reinterpret_cast<RfJob*>(sm.tmem_slot + 4);
+  const RfSmem sm = RfSmem::carve(rf_smem_raw, attn_smem_bytes(a, false));
+  const AttnSmem asm_ = carve(sm.att, a, false);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int rank = (int)cluster_ctarank();
@@ -592,12 +433,10 @@ recurrent_fwd_kernel(const __grid_constant__ RfParams p) {
   if (threadIdx.x == 0) {
     for (int i = 0; i < NUM_AMAPS; ++i) prefetch_tmap(&p.amap[i]);
     for (int i = 0; i < NUM_WMAPS; ++i) prefetch_tmap(&p.wmap[i]);
-    for (int s = 0; s < RF_STAGES; ++s) { mbar_init(&sm.full[s], 1); mbar_init(&sm.empty[s], 1); }
-    for (int s = 0; s < NUM_SLOTS; ++s) mbar_init(&sm.tfull[s], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    sm.init_barriers();
     build_jobs(p, pair, sm.jobs, sm.njobs);
   }
-  if (warp == 1) tmem_alloc_2sm<RF_TMEM_COLS>(sm.tmem_slot);
+  if (warp == 1) tmem_alloc_2sm<PK_TMEM_COLS>(sm.tmem_slot);
   attn_prologue(asm_, a, false);                       // attention ring barriers, w_a, zeroed q buffers; __syncthreads inside
   tc_fence_before();
   cluster_sync_all();                                  // the peer's barriers exist before any remote arrival
@@ -609,52 +448,24 @@ recurrent_fwd_kernel(const __grid_constant__ RfParams p) {
   if (warp == 0) {
     // ================= TMA producer of the GEMM operand ring (both CTAs of the pair) =================
     if (elect_one_sync()) {
-      int stage = 0; uint32_t phase = 0;
-      uint64_t w_pol = 0;
-      if (p.w_policy) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(w_pol));
+      RingPos<RF_STAGES> pos;
+      const uint64_t w_pol = ptx::l2_policy_evict_first();
       for (int t = 0; t < T; ++t) {
         for (int j = 0; j < njobs; ++j) {
           const RfJob& job = sm.jobs[j];
-          const uint32_t tx = 2u * (uint32_t)(RF_X_BYTES + job.w_box_rows * 128);
+          const uint32_t tx = 2u * (uint32_t)(PK_X_BYTES + job.w_box_rows * 128);
           for (int s = 0; s < job.nseg; ++s) {
             const RfSeg sg = job.seg[s];
-            // The weight tiles of a segment do not depend on any flag: pull them into L2 while the activations they
-            // multiply are still being produced (the ring alone keeps only RF_STAGES tiles in flight, which left the
-            // weight stream HBM-latency bound: ~0.4 us per k-block).
-            for (int kb = 0; kb < sg.kblocks; ++kb) tma_prefetch_2d(&p.wmap[sg.wmap], sg.wcol0 + kb * 64, job.w_row[rank]);
-            const bool hidden = sg.flag == FLAG_H1 || sg.flag == FLAG_HDEC || sg.flag == FLAG_HENC;
-            const bool tiled = hidden && p.tile_flags;
-            // hidden states: 2 signals per tile and step (per-tile counters) or 2 * nt per step (one counter per family)
-            const unsigned int target = sg.flag >= 0 ? (unsigned int)((t + sg.flag_toff) * sg.flag_mult * (hidden && !tiled ? p.nt : 1)) : 0u;
-            int ready = sg.kblocks;
-            if (target) {
-              if (tiled) {
-                ready = 0;
-              } else {
+            produce_segment(p, sm, pos, t, rank, tx, w_pol, &p.amap[sg.amap], sg.acol0, t + sg.t_off, &p.wmap[sg.wmap], sg.wcol0,
+                            job.w_row[rank], sg.kblocks, [&] {
+              const bool hidden = sg.flag == FLAG_H1 || sg.flag == FLAG_HDEC || sg.flag == FLAG_HENC;
+              const unsigned int target = sg.flag >= 0 ? (unsigned int)((t + sg.flag_toff) * sg.flag_mult * (hidden ? p.nt : 1)) : 0u;
+              if (target) {
                 wait_flag(p, sg.flag, target, 100 + j * 10 + s, t);
                 fence_proxy_async_global();
               }
-            }
-            RF_STAMP(true, 10 + j * 4 + s);
-            unsigned long long t0 = 0;
-            for (int kb = 0; kb < sg.kblocks; ++kb) {
-              while (kb >= ready) {                    // hidden-state segment: stream the k-blocks whose tiles are done
-                ready = ready_kblocks(p, sg.flag, p.nt, sg.kblocks, target);
-                if (kb < ready) { fence_proxy_async_global(); break; }
-                const unsigned long long now = globaltimer_ns();
-                if (t0 == 0) t0 = now;
-                if (now - t0 > p.timeout_ns || ld_acquire_u32(p.flags + FLAG_ABORT)) rf_abort(p, 100 + j * 10 + s, t, (unsigned)ready, target);
-              }
-              mbar_wait_bounded(p, &sm.empty[stage], phase ^ 1, 1, t);
-              if (rank == 0) mbar_expect_tx(&sm.full[stage], tx);
-              uint8_t* xs = sm.ring + (size_t)stage * RF_STAGE_BYTES;
-              tma_load_3d_2sm(xs, &p.amap[sg.amap], &sm.full[stage], sg.acol0 + kb * 64, rank * 128, t + sg.t_off);
-              if (p.w_policy)
-                tma_load_2d_2sm_hint(xs + RF_X_BYTES, &p.wmap[sg.wmap], &sm.full[stage], sg.wcol0 + kb * 64, job.w_row[rank], w_pol);
-              else
-                tma_load_2d_2sm(xs + RF_X_BYTES, &p.wmap[sg.wmap], &sm.full[stage], sg.wcol0 + kb * 64, job.w_row[rank]);
-              if (++stage == p.stages) { stage = 0; phase ^= 1; }
-            }
+              RF_STAMP(true, 10 + j * 4 + s);
+            });
           }
         }
       }
@@ -663,36 +474,17 @@ recurrent_fwd_kernel(const __grid_constant__ RfParams p) {
   } else if (warp == 1) {
     // ================= MMA issuer (leader CTA of the pair) =================
     if (rank == 0 && elect_one_sync()) {
-      int stage = 0; uint32_t phase = 0;
+      RingPos<RF_STAGES> pos;
       for (int t = 0; t < T; ++t) {
         for (int j = 0; j < njobs; ++j) {
           const RfJob& job = sm.jobs[j];
-          const uint32_t idesc = make_idesc(256, job.N);
-          const uint32_t tacc = tmem_base + job.tmem_col;
-          bool first = true;
-          for (int s = 0; s < job.nseg; ++s) {
-            const int kbs = job.seg[s].kblocks;
-            for (int kb = 0; kb < kbs; ++kb) {
-              mbar_wait_bounded(p, &sm.full[stage], phase, 2, t);
-              tc_fence_after();
-              const uint32_t x_base = smem_u32(sm.ring + (size_t)stage * RF_STAGE_BYTES);
-              const uint32_t w_base = x_base + RF_X_BYTES;
-#pragma unroll
-              for (int k = 0; k < 4; ++k) {
-                umma_bf16_2sm(tacc, make_smem_desc(x_base + k * 32), make_smem_desc(w_base + k * 32), idesc, first ? 0u : 1u);
-                first = false;
-              }
-              umma_commit_2sm(&sm.empty[stage]);
-              if (++stage == p.stages) { stage = 0; phase ^= 1; }
-            }
-          }
-          umma_commit_2sm(&sm.tfull[job.slot]);
+          mma_job(p, sm, pos, t, job, tmem_base + job.tmem_col, job.slot);
           RF_STAMP(true, 20 + j);
         }
       }
     }
     __syncwarp();
-  } else if (warp < 2 + RF_CWARPS) {
+  } else if (warp < 2 + PK_CWARPS) {
     // ================= compute warps: epilogues + attention consumers =================
     const int cw = warp - 2;
     const int ctid = (int)threadIdx.x - 64;
@@ -716,14 +508,14 @@ recurrent_fwd_kernel(const __grid_constant__ RfParams p) {
         const int b = cta + k * G;
         if (b < p.B && ctid < a.N) asm_.msk(k)[ctid] = a.mask[(size_t)b * a.N + ctid];
       }
-      ptx::bar_sync(1, RF_CTHREADS);
+      ptx::bar_sync(1, PK_CTHREADS);
     }
     for (int t = 0; t < T; ++t) {
       RF_STAMP(ctid == 0, 0);
       if (role == ROLE_ENC) {
         epi_lstm<0>(p, sm, t, tile, tmem_base, cw, lane, rank);
         RF_STAMP(ctid == 0, 1);
-        signal_tile_done(p, FLAG_H1, tile, ctid);
+        signal_done(p, FLAG_H1, ctid);
       } else if (has_q) {
         epi_q(p, sm, t, tile, tmem_base, cw, lane, rank);
         RF_STAMP(ctid == 0, 1);
@@ -733,7 +525,7 @@ recurrent_fwd_kernel(const __grid_constant__ RfParams p) {
       if (cta < p.B) {
         if (ctid == 0) wait_flag(p, FLAG_Q, (unsigned int)((t + 1) * 2 * p.nq), 20, t);
         RF_STAMP(ctid == 0, 3);
-        ptx::bar_sync(1, RF_CTHREADS);
+        ptx::bar_sync(1, PK_CTHREADS);
         const float* q_t = p.q + (size_t)t * p.B * p.A;
         prefetch_vec(asm_.q(0), q_t + (size_t)cta * p.A, a.A);
         ptx::cp_async_commit();
@@ -750,11 +542,11 @@ recurrent_fwd_kernel(const __grid_constant__ RfParams p) {
       if (role == ROLE_ENC) {
         epi_lstm<1>(p, sm, t, tile, tmem_base, cw, lane, rank);
         RF_STAMP(ctid == 0, 6);
-        signal_tile_done(p, FLAG_HENC, tile, ctid);
+        signal_done(p, FLAG_HENC, ctid);
       } else if (role == ROLE_DEC) {
         epi_lstm<2>(p, sm, t, tile, tmem_base, cw, lane, rank);
         RF_STAMP(ctid == 0, 6);
-        signal_tile_done(p, FLAG_HDEC, tile, ctid);
+        signal_done(p, FLAG_HDEC, ctid);
       } else if (has_fc) {
         epi_latent(p, sm, t, tile, tmem_base, cw, lane, rank);
         RF_STAMP(ctid == 0, 6);
@@ -766,7 +558,7 @@ recurrent_fwd_kernel(const __grid_constant__ RfParams p) {
     // ================= attention producer: streams P and the region features of this CTA's rows =================
     if (lane == 0 && cta < p.B) {
       Ring ring;
-      const uint64_t pol = a.l2_policy == 1 ? ptx::l2_policy_evict_first() : a.l2_policy == 2 ? ptx::l2_policy_evict_last() : 0;
+      const uint64_t pol = ptx::l2_policy_evict_first();
       for (int t = 0; t < T; ++t)
         for (int b = cta; b < p.B; b += G) {
           produce_block(asm_, ring, reinterpret_cast<const uint8_t*>(a.proj + (size_t)b * a.N * a.Ap), a.N, a.Ap * 2, p.plan.nP, p.plan.bP, pol);
@@ -775,12 +567,7 @@ recurrent_fwd_kernel(const __grid_constant__ RfParams p) {
     }
     __syncwarp();
   }
-  tc_fence_before();
-  cluster_sync_all();                                  // nobody deallocates while the pair's MMAs / loads are in flight
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc_2sm<RF_TMEM_COLS>(tmem_base);
-  }
+  pk_teardown(warp, tmem_base);
 }
 
 // kl[t*B + b] = -1/2 * sum of the per-tile partial sums (updown_captioner.py:299-303)
@@ -793,63 +580,8 @@ __global__ void kl_sum_parts_kernel(const float* __restrict__ parts, int nparts,
   kl[i] = -0.5f * s;
 }
 
-// ---------------------------------------------------------------------------------------------------------------
 // host side
-// ---------------------------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static int encode_act3d(CUtensorMap* out, const bf16* base, int K, int B, int T, int ld) {
-  EncodeTiledFn fn = reinterpret_cast<EncodeTiledFn>(tma_encode_fn());
-  if (!fn) { set_error("cuTensorMapEncodeTiled not available from the driver"); return SSCVAE_ERR_DRIVER; }
-  cuuint64_t dims[3] = {(cuuint64_t)K, (cuuint64_t)B, (cuuint64_t)T};
-  cuuint64_t strides[2] = {(cuuint64_t)ld * 2, (cuuint64_t)B * ld * 2};
-  cuuint32_t box[3] = {64, 128, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<bf16*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_error("recurrent_fwd: activation tensor map failed (%d) K=%d B=%d T=%d ld=%d", (int)r, K, B, T, ld); return SSCVAE_ERR_DRIVER; }
-  return 0;
-}
-static int encode_w2d(CUtensorMap* out, const bf16* base, int K, int rows, int ld, int box_rows) {
-  EncodeTiledFn fn = reinterpret_cast<EncodeTiledFn>(tma_encode_fn());
-  if (!fn) { set_error("cuTensorMapEncodeTiled not available from the driver"); return SSCVAE_ERR_DRIVER; }
-  cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
-  cuuint32_t box[2] = {64, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<bf16*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_error("recurrent_fwd: weight tensor map failed (%d) K=%d rows=%d ld=%d box=%d", (int)r, K, rows, ld, box_rows); return SSCVAE_ERR_DRIVER; }
-  return 0;
-}
-
-static size_t rf_smem_bytes(const AttnArgs& a) {
-  return 1024 + (size_t)RF_STAGES * RF_STAGE_BYTES + ((attn_smem_bytes(a, false) + 127) & ~size_t(127)) +
-         (2 * RF_STAGES + NUM_SLOTS) * 8 + 16 + 2 * sizeof(RfJob) + 64;
-}
-
-static int rf_grid_pairs(size_t smem) {
-  static int cached = -1;
-  static size_t cached_smem = 0;
-  if (cached >= 0 && cached_smem == smem) return cached;
-  int dev = 0, n_sm = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
-  if (cudaFuncSetAttribute(recurrent_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
-    cudaGetLastError();
-    return 0;
-  }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * (n_sm / 2)); cfg.blockDim = dim3(RF_THREADS); cfg.dynamicSmemBytes = smem;
-  int clusters = 0;
-  if (cudaOccupancyMaxActiveClusters(&clusters, recurrent_fwd_kernel, &cfg) != cudaSuccess) { cudaGetLastError(); clusters = 0; }
-  cached = std::min(clusters, n_sm / 2);
-  cached_smem = smem;
-  return cached;
-}
+static size_t rf_smem_bytes(const AttnArgs& a) { return RfSmem::bytes(attn_smem_bytes(a, false), 2); }
 
 size_t recurrent_forward_kl_parts(int Z) { return 2 * (size_t)((Z + 15) / 16); }
 
@@ -863,7 +595,7 @@ bool recurrent_forward_supported(const RecFwdArgs& r) {
     return false;
   const size_t smem = rf_smem_bytes(a);
   if (smem > 227 * 1024) return false;
-  const int NP = rf_grid_pairs(smem);
+  const int NP = pk_grid_pairs(recurrent_fwd_kernel, smem);
   const int nt = r.GP / 128, spare = NP - 2 * nt;
   if (spare < 1) return false;
   const int nfc = (r.Z + 15) / 16;
@@ -875,14 +607,9 @@ bool recurrent_forward_supported(const RecFwdArgs& r) {
 int recurrent_forward(cudaStream_t s, const RecFwdArgs& r) {
   RfParams p;
   memset(&p, 0, sizeof(p));
-  AttnArgs a = r.att;
-  // measured (bench.py, ms per training step / ms of this kernel): no hint 7.06 / 2.035, evict_last 7.08 / 2.038,
-  // evict_first 6.90 / 1.950
-  static const int att_pol = [] { const char* e = getenv("SSCVAE_ATT_POLICY"); return e ? atoi(e) : 1; }();
-  static const int w_pol = [] { const char* e = getenv("SSCVAE_RF_W_POLICY"); return e ? atoi(e) : 1; }();
-  a.l2_policy = att_pol;
+  const AttnArgs& a = r.att;
   const size_t smem = rf_smem_bytes(a);
-  const int NP = rf_grid_pairs(smem);
+  const int NP = pk_grid_pairs(recurrent_fwd_kernel, smem);
   REQUIRE(NP > 0, "recurrent_fwd: no co-resident CTA pairs");
   const int nt = r.GP / 128, spare = NP - 2 * nt;
   p.B = r.B; p.T = r.T; p.H = r.H; p.Hp = r.Hp; p.Fp = r.Fp; p.Zp = r.Zp; p.Z = r.Z; p.A = r.A; p.KX = r.KX; p.GP = r.GP;
@@ -914,61 +641,22 @@ int recurrent_forward(cudaStream_t s, const RecFwdArgs& r) {
   p.mean = r.mean; p.logvar = r.logvar; p.eps_out = r.eps_out; p.kl_part = r.kl_part;
   p.att = a; p.alpha = r.alpha; p.smx = r.smx;
   p.flags = r.flags;
-  p.w_policy = w_pol;
-  static const int n_stages = [] { const char* e = getenv("SSCVAE_RF_STAGES"); return e ? std::min(RF_STAGES, std::max(2, atoi(e))) : RF_STAGES; }();
-  p.stages = n_stages;
-  static const int sig_mode = [] { const char* e = getenv("SSCVAE_RF_SIG_MODE"); return e ? atoi(e) : 1; }();
-  p.sig_mode = sig_mode;
-  static const int tile_flags = [] { const char* e = getenv("SSCVAE_RF_TILE_FLAGS"); return e && e[0] == '1' ? 1 : 0; }();
-  p.tile_flags = tile_flags;
-  static const unsigned long long timeout_ms = [] { const char* e = getenv("SSCVAE_RF_TIMEOUT_MS"); return e ? (unsigned long long)atoll(e) : 4000ull; }();
-  p.timeout_ns = timeout_ms * 1000000ull;
-  {  // chunking of the attention streams (as attention.cu: make_plan)
-    auto boxes_per_chunk = [](int row_bytes) {
-      int b = 1;
-      while (b * 2 <= ATT_MAXB && b * 2 * row_bytes <= ATT_STAGE_BYTES) b *= 2;
-      return b;
-    };
-    p.plan.bP = boxes_per_chunk(a.Ap * 2); p.plan.nP = ceil_div(a.N, p.plan.bP);
-    p.plan.bF = boxes_per_chunk(a.Fp * 2); p.plan.nF = ceil_div(a.N, p.plan.bF);
-    p.plan.rows_per_cta = 0;
-  }
+  p.timeout_ns = pk_timeout_ns();
+  p.plan = attn_chunk_plan(a);
   // model FLOPs of the loop (un-hoisted parts only): the three gate GEMMs, q, fc; bytes: the attention stream
   const double flops = 2.0 * r.B * r.T * ((double)r.GP * (r.Ep + 2 * r.Hp + r.KX + r.Hp + r.KX + r.Zp) + (double)r.A * r.Hp + 2.0 * r.Z * r.Hp);
   PROF_SCOPE(s, "recurrent_fwd", flops, (double)r.B * r.T * a.N * (a.Ap + a.Fp) * 2.0);
   static const bool dbg = [] { const char* e = getenv("SSCVAE_RF_DBG"); return e && e[0] == '1'; }();
-  static unsigned long long* dbg_buf = nullptr;
   if (dbg) {
-    if (!dbg_buf) CUDA_TRY(cudaMalloc(&dbg_buf, 32 * 8 * 2 * 128));
-    CUDA_TRY(cudaMemsetAsync(dbg_buf, 0, 32 * 8 * 2 * 128, s));
-    p.dbg = dbg_buf;
+    TRY(pk_dbg_begin(s, &p.dbg));
     p.dbg_t = r.T / 2;
   }
-  CUDA_TRY(cudaMemsetAsync(r.flags, 0, RF_FLAG_WORDS * sizeof(unsigned int), s));
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * NP); cfg.blockDim = dim3(RF_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeCooperative;
-  attr[0].val.cooperative = 1;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  CUDA_TRY(cudaLaunchKernelEx(&cfg, recurrent_fwd_kernel, p));
-  ++g_launch_count;
+  CUDA_TRY(cudaMemsetAsync(r.flags, 0, FLAG_COUNT * sizeof(unsigned int), s));
+  TRY(pk_launch(recurrent_fwd_kernel, NP, smem, s, p));
   if (dbg) {
-    static int printed = 0;
-    CUDA_TRY(cudaStreamSynchronize(s));
-    std::vector<unsigned long long> h(32 * 2 * NP);
-    CUDA_TRY(cudaMemcpy(h.data(), dbg_buf, h.size() * 8, cudaMemcpyDeviceToHost));
-    if (printed++ < 6) {
-      unsigned long long t0 = ~0ull;
-      for (int c = 0; c < 2 * NP; ++c) if (h[c * 32] && h[c * 32] < t0) t0 = h[c * 32];
-      const int show[] = {0, 1, 2 * nt - 2, 2 * nt, 4 * nt - 2, 4 * nt, 4 * nt + 2 * p.nfc, 2 * NP - 2};
-      for (int c : show) {
-        if (c < 0 || c >= 2 * NP) continue;
-        fprintf(stderr, "[rfdbg] B=%d t=%d cta=%3d:", r.B, p.dbg_t, c);
-        for (int i = 0; i < 24; ++i) fprintf(stderr, " %d:%.1f", i, h[c * 32 + i] ? (double)(h[c * 32 + i] - t0) / 1e3 : -1.0);
-        fprintf(stderr, "\n");
-      }
-    }
+    char head[64];
+    snprintf(head, sizeof(head), "[rfdbg] B=%d t=%d", r.B, p.dbg_t);
+    TRY(pk_dbg_print(s, p.dbg, 2 * NP, head, {0, 1, 2 * nt - 2, 2 * nt, 4 * nt - 2, 4 * nt, 4 * nt + 2 * p.nfc, 2 * NP - 2}, 24));
   }
   const int TB = r.T * r.B;
   kl_sum_parts_kernel<<<ceil_div(TB, 256), 256, 0, s>>>(r.kl_part, 2 * p.nfc, r.B, TB, r.kl);

@@ -1,5 +1,5 @@
 // tcgen05 / TMEM / TMA / mbarrier PTX wrappers shared by the sm_100a GEMM kernels (gemm_sm100.cu) and the persistent
-// recurrent kernels (recurrent_fwd.cu).
+// recurrent kernels (persistent.cuh, recurrent_fwd.cu, recurrent_bwd.cu).
 #pragma once
 #include <cuda.h>
 #include <cstdint>
@@ -161,6 +161,62 @@ __device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, uint32_t (&r)[32])
       : "memory");
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ void tmem_ld_x8(uint32_t taddr, float (&v)[8]) {
+  uint32_t r[8];
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+               : "r"(taddr)
+               : "memory");
+#pragma unroll
+  for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
+}
+__device__ __forceinline__ void tmem_st_x8(uint32_t taddr, const float (&v)[8]) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr),
+               "r"(__float_as_uint(v[0])), "r"(__float_as_uint(v[1])), "r"(__float_as_uint(v[2])), "r"(__float_as_uint(v[3])),
+               "r"(__float_as_uint(v[4])), "r"(__float_as_uint(v[5])), "r"(__float_as_uint(v[6])), "r"(__float_as_uint(v[7]))
+               : "memory");
+}
+
+// ---- TMA operands of the CTA-pair kernels ------------------------------------------------------------------
+// 3-D tile (k, batch row, t) into both CTAs of the pair; the transaction bytes land on the leader's barrier
+__device__ __forceinline__ void tma_load_3d_2sm(void* dst, const CUtensorMap* tmap, uint64_t* bar, int c0, int c1, int c2) {
+  asm volatile(
+      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
+      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(smem_u32(bar) & 0xFEFFFFFFu), "r"(c0), "r"(c1), "r"(c2)
+      : "memory");
+}
+__device__ __forceinline__ void tma_prefetch_2d(const CUtensorMap* tmap, int c0, int c1) {
+  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];" ::"l"(reinterpret_cast<uint64_t>(tmap)), "r"(c0), "r"(c1)
+               : "memory");
+}
+
+// ---- global-memory dataflow counters and timing ----------------------------------------------------------
+__device__ __forceinline__ unsigned long long globaltimer_ns() {
+  unsigned long long t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+  return t;
+}
+__device__ __forceinline__ unsigned int ld_acquire_u32(const unsigned int* p) {
+  unsigned int v;
+  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ void red_release_add(unsigned int* p, unsigned int v) {
+  asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+// generic-proxy global stores -> later TMA (async proxy) reads
+__device__ __forceinline__ void fence_proxy_async_global() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
+__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
+  uint32_t ok;
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
+      "selp.u32 %0, 1, 0, p;\n\t}"
+      : "=r"(ok)
+      : "r"(smem_u32(bar)), "r"(parity)
+      : "memory");
+  return ok != 0;
+}
 
 // K-major, 128B-swizzled shared-memory matrix descriptor (cf. cute::UMMA::SmemDescriptor):
 //   [0,14) start address >> 4 ; [16,30) leading byte offset >> 4 (unused for swizzled K-major, =1) ;
