@@ -281,8 +281,8 @@ int sscvae_profile_report(char* buf, size_t n);
 int sscvae_test_gemm(const void* A, int lda, const void* B, int ldb, int M, int N, int K, float* C32, int ldc,
                      const float* bias, int act_tanh, int accumulate, void* stream);
 
-/* the skinny-M (M <= 256) swapped-operand kernel with a forced cluster split of K (1, 2 or 4; 0 = the library's
- * choice), for unit tests and tools/gemm_bench.py */
+/* the skinny-M (M <= 256) swapped-operand CTA-pair kernel with a forced cluster split of K (1..4; 0 = the library's
+ * choice of kernel and split; other values return SSCVAE_ERR_BAD_ARG), for unit tests and tools/gemm_bench.py */
 int sscvae_test_gemm_splitk(const void* A, int lda, const void* B, int ldb, int M, int N, int K, float* C32, int ldc,
                             int splits, const float* bias, void* stream);
 

@@ -135,8 +135,7 @@ static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, cons
 
   // Unconstrained K = 1 search (greedy decode, diverse sampling): arg max and log-sum-exp come out of the head GEMM's
   // epilogue (RowStatsEpi) and the (rows, V) fp32 logits are never written: -2 x rows x V x 4 bytes per step.
-  static const bool no_fused_head = [] { const char* e = getenv("SSCVAE_DECODE_FUSED_HEAD"); return e && e[0] == '0'; }();
-  const bool greedy = S == 1 && K == 1 && fsm == nullptr && !no_fused_head;
+  const bool greedy = S == 1 && K == 1 && fsm == nullptr;
   RowStatsEpi rs;
   rs.mode = 1; rs.st_max = Wf("rs_max"); rs.st_sum = Wf("rs_sum"); rs.st_arg = Wi("rs_arg");
   const int nst = gemm_rowstats_tiles(d.V);
@@ -149,9 +148,11 @@ static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, cons
       l.R = rows; l.H = H; l.add2 = Wf("gavg"); l.ld2 = GP; l.rowmap = rowmap; l.bias = Pf("b_att");
       l.c_prev = first ? nullptr : c1[0]; l.c_out = c1[1];
       l.h1_dst = Wb("XE") + Fp; l.ld_h1 = KXe; l.h2_dst = XA[1]; l.ld_h2 = 2 * Hp;
+      l.acc = Wf("acc"); l.ld_acc = GP; l.perm = 1;
       GemmSeg sg[2] = {seg(Wb("embb_r"), d.Ep, Pb("w_att_e"), d.Ep, d.E), seg(XA[0], 2 * Hp, Pb("w_att_rec"), 2 * Hp, 2 * Hp)};
-      GemmEpi e; e.tag = "gemm.decode"; e.C32 = Wf("acc"); e.ldc32 = GP; e.lstm = &l;   // cell fused when rows <= 256
+      GemmEpi e; e.tag = "gemm.decode"; e.C32 = Wf("acc"); e.ldc32 = GP;
       TRY(gemm_bf16_tn(s, rows, GP, first ? 1 : 2, sg, e));
+      TRY(lstm_forward(s, l));
     }
     {
       GemmSeg sg = seg(Wb("XE") + Fp, KXe, Pb("wq"), Hp, Hp);
@@ -181,8 +182,10 @@ static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, cons
       if (csent) { l.sent = Wf("sent"); l.scol = Pf("scol_dec"); }
       l.c_prev = first ? nullptr : cd[0]; l.c_out = cd[1];
       l.h1_dst = XA[1] + Hp; l.ld_h1 = 2 * Hp;
-      GemmEpi e; e.tag = "gemm.decode"; e.C32 = Wf("acc"); e.ldc32 = GP; e.lstm = &l;
+      l.acc = Wf("acc"); l.ld_acc = GP; l.perm = 1;
+      GemmEpi e; e.tag = "gemm.decode"; e.C32 = Wf("acc"); e.ldc32 = GP;
       TRY(gemm_bf16_tn(s, rows, GP, first ? 2 : 3, sg, e));
+      TRY(lstm_forward(s, l));
     }
     if (d.tied) {
       GemmSeg sg = seg(XA[1] + Hp, 2 * Hp, Pb("w_out"), Hp, Hp);

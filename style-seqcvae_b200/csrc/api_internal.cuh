@@ -28,7 +28,6 @@ struct Dims {
   int GP;                              // rows of a packed forward LSTM weight block: gate-interleaved, lstm_gate_rows(H)
 };
 int init_dims(const SscvaeDims* in, Dims& d);
-int set_l2_window(cudaStream_t s, const void* base, size_t bytes);
 
 struct Region { const char* name; size_t off, bytes; };
 struct Plan {
@@ -38,54 +37,8 @@ struct Plan {
   const Region* find(const char* name) const;
 };
 
-// Fork / join of independent launches over a few auxiliary streams (works inside a stream capture: the auxiliary streams
-// join the capture through the fork event and are joined back before the call returns). Used for the weight-gradient
-// GEMMs of one LSTM, which share an operand but are otherwise independent: launched back to back on one stream each
-// of them ends in a partial wave on the 74 CTA pairs.
-struct StreamFork {
-  static constexpr int kAux = 3;
-  cudaStream_t aux[kAux] = {nullptr, nullptr, nullptr};
-  cudaEvent_t ev_fork = nullptr, ev_join[kAux] = {nullptr, nullptr, nullptr};
-  bool forked = false;
-  int init() {
-    if (ev_fork) return 0;
-    for (int i = 0; i < kAux; ++i) {
-      CUDA_TRY(cudaStreamCreateWithFlags(&aux[i], cudaStreamNonBlocking));
-      CUDA_TRY(cudaEventCreateWithFlags(&ev_join[i], cudaEventDisableTiming));
-    }
-    CUDA_TRY(cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming));
-    return 0;
-  }
-  int fork(cudaStream_t s) {
-    TRY(init());
-    CUDA_TRY(cudaEventRecord(ev_fork, s));
-    for (int i = 0; i < kAux; ++i) CUDA_TRY(cudaStreamWaitEvent(aux[i], ev_fork, 0));
-    forked = true;
-    return 0;
-  }
-  // stream of the i-th independent item
-  cudaStream_t pick(cudaStream_t s, int i) const { return (!forked || i % (kAux + 1) == 0) ? s : aux[i % (kAux + 1) - 1]; }
-  int join(cudaStream_t s) {
-    if (!forked) return 0;
-    for (int i = 0; i < kAux; ++i) {
-      CUDA_TRY(cudaEventRecord(ev_join[i], aux[i]));
-      CUDA_TRY(cudaStreamWaitEvent(s, ev_join[i], 0));
-    }
-    forked = false;
-    return 0;
-  }
-  ~StreamFork() {
-    for (int i = 0; i < kAux; ++i) {
-      if (aux[i]) cudaStreamDestroy(aux[i]);
-      if (ev_join[i]) cudaEventDestroy(ev_join[i]);
-    }
-    if (ev_fork) cudaEventDestroy(ev_fork);
-  }
-};
-
 struct Handle {
   Dims d;
-  StreamFork fork;
   Plan pp;                 // packed weights
   Plan tp; int tp_B = -1, tp_N = -1;   // training workspace for the last (B,N)
   Plan dp; int dp_B = -1, dp_N = -1, dp_S = -1, dp_K = -1, dp_J = -1;   // decode workspace

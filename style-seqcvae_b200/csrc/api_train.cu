@@ -344,38 +344,6 @@ static int pack_weights_impl(Handle* h, const void* const* wv, char* pk, const u
 }
 
 
-// ---- L2 residency of the per-image tensors --------------------------------------------------------
-// The bf16 region features and their W_v projection are re-read by the attention kernel at every one of
-// the 21 forward and 21 backward steps, while ~78 MB of recurrent weights stream through L2 in between.
-// A persisting access-policy window on [featsb .. projb] keeps them L2-resident (B200: 126 MB L2).
-int set_l2_window(cudaStream_t s, const void* base, size_t bytes) {
-  static int max_window = -1, max_persist = -1;
-  // Measured on B200 (bench8, round 1): the persisting carve-out takes L2 away from everything else in the step and
-  // costs 5% end to end, so the window is opt-in (SSCVAE_L2_WINDOW=1) and off by default.
-  static const bool enabled = [] { const char* e = getenv("SSCVAE_L2_WINDOW"); return e && e[0] == '1'; }();
-  if (!enabled) return 0;
-  if (max_window < 0) {
-    int dev = 0;
-    CUDA_TRY(cudaGetDevice(&dev));
-    CUDA_TRY(cudaDeviceGetAttribute(&max_window, cudaDevAttrMaxAccessPolicyWindowSize, dev));
-    CUDA_TRY(cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, dev));
-    if (max_persist > 0) CUDA_TRY(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)max_persist));
-  }
-  if (max_window <= 0 || max_persist <= 0) return 0;
-  cudaStreamAttrValue attr;
-  memset(&attr, 0, sizeof(attr));
-  if (base && bytes) {
-    const size_t win = std::min(bytes, (size_t)max_window);
-    attr.accessPolicyWindow.base_ptr = const_cast<void*>(base);
-    attr.accessPolicyWindow.num_bytes = win;
-    attr.accessPolicyWindow.hitRatio = win <= (size_t)max_persist ? 1.0f : (float)max_persist / (float)win;
-    attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-    attr.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-  }
-  CUDA_TRY(cudaStreamSetAttribute(s, cudaStreamAttributeAccessPolicyWindow, &attr));
-  return 0;
-}
-
 // ---- small helpers -----------------------------------------------------------------------------
 static inline GemmSeg seg(const bf16* A, int lda, const bf16* B, int ldb, int K) {
   GemmSeg s; s.A = A; s.lda = lda; s.B = B; s.ldb = ldb; s.K = K; return s;
@@ -432,8 +400,6 @@ static int train_forward_impl(Handle* h, int B, int N, const char* pk, const voi
   const unsigned long long* seed_dev = reinterpret_cast<const unsigned long long*>(ws + tp.find("seed")->off);
   (void)seed;                                          // copied to `seed_dev` by the caller, in front of the graph
 
-  // keep the per-timestep weights L2-resident across the 21 steps (they are re-read every step)
-  TRY(set_l2_window(s, pk + pp.find("w_att_rec")->off, pp.find("fwd_end")->off - pp.find("w_att_rec")->off));
   // operand buffers carry zero padding columns and the zero initial states (updown_cell.py:131-140)
   CUDA_TRY(zero("XA")); CUDA_TRY(zero("XE")); CUDA_TRY(zero("HE")); CUDA_TRY(zero("projb")); CUDA_TRY(zero("ZB"));
   if (d.tied) CUDA_TRY(zero("ob"));
@@ -496,15 +462,17 @@ static int train_forward_impl(Handle* h, int B, int N, const char* pk, const voi
       bf16* HE_n = HE_t + (size_t)B * Hp;
       bf16* ZB_t = Wb("ZB") + (size_t)t * B * d.ZC;
       const size_t rG = (size_t)t * B * d.G, rH = (size_t)t * B * H, rZ = (size_t)t * B * d.Z;
-      {  // attention LSTM (updown_cell.py:143-148): gate GEMM with the cell fused into its epilogue
+      {  // attention LSTM (updown_cell.py:143-148): gate GEMM, then the cell
         LstmFwdArgs l = {};
         l.R = B; l.H = H; l.add1 = Wf("gx_att") + (size_t)t * B * GP; l.ld1 = GP; l.add2 = Wf("gavg"); l.ld2 = GP;
         l.bias = Pf("b_att");
         l.c_prev = t ? Wf("c1") + rH - (size_t)B * H : nullptr; l.c_out = Wf("c1") + rH; l.gates_out = Wf("gates_att") + rG;
         l.h1_dst = XE_t + Fp; l.ld_h1 = KX; l.h2_dst = XA_n; l.ld_h2 = 2 * Hp;
+        l.acc = acc; l.ld_acc = GP; l.perm = 1;
         GemmSeg sg = seg(XA_t, 2 * Hp, Pb("w_att_rec"), 2 * Hp, 2 * Hp);
-        GemmEpi e; e.tag = "gemm.step"; e.C32 = acc; e.ldc32 = GP; e.lstm = &l;
+        GemmEpi e; e.tag = "gemm.step"; e.C32 = acc; e.ldc32 = GP;
         TRY(gemm_bf16_tn(s, B, GP, 1, &sg, e));
+        TRY(lstm_forward(s, l));
       }
       {  // query projection + fused region attention (attention.py:69-93, updown_cell.py:156)
         GemmSeg sg = seg(XE_t + Fp, KX, Pb("wq"), Hp, Hp);
@@ -526,10 +494,12 @@ static int train_forward_impl(Handle* h, int B, int N, const char* pk, const voi
         if (csent) { l.sent = sent; l.scol = Pf("scol_enc"); }
         l.c_prev = t ? Wf("c_enc") + rH - (size_t)B * H : nullptr; l.c_out = Wf("c_enc") + rH;
         l.gates_out = Wf("gates_enc") + rG; l.h1_dst = HE_n; l.ld_h1 = Hp;
+        l.acc = acc; l.ld_acc = GP; l.perm = 1;
         GemmSeg sg[3] = {seg(XE_t, KX, Pb("w_enc_x"), KX, KX), seg(HE_t, Hp, Pb("w_enc_hh"), Hp, Hp), GemmSeg()};
         if (d.cvar) sg[2] = seg(ZB_t + d.Zp, d.ZC, Pb("w_enc_c"), d.Cp, d.Cp);
-        GemmEpi e; e.tag = "gemm.step"; e.C32 = acc; e.ldc32 = GP; e.lstm = &l;
+        GemmEpi e; e.tag = "gemm.step"; e.C32 = acc; e.ldc32 = GP;
         TRY(gemm_bf16_tn(s, B, GP, d.cvar ? 3 : 2, sg, e));
+        TRY(lstm_forward(s, l));
         GemmSeg sf = seg(HE_n, Hp, Pb("w_fc"), Hp, Hp);
         GemmEpi ef; ef.tag = "gemm.step"; ef.C32 = Wf("ml"); ef.ldc32 = d.Z2;
         TRY(gemm_bf16_tn(s, B, d.Z2, 1, &sf, ef));
@@ -543,9 +513,11 @@ static int train_forward_impl(Handle* h, int B, int N, const char* pk, const voi
         l.c_prev = t ? Wf("c_dec") + rH - (size_t)B * H : nullptr; l.c_out = Wf("c_dec") + rH;
         l.gates_out = Wf("gates_dec") + rG; l.h1_dst = XA_n + Hp; l.ld_h1 = 2 * Hp;
         if (XE_n) { l.h2_dst = XE_n + Fp + Hp; l.ld_h2 = KX; }
+        l.acc = acc; l.ld_acc = GP; l.perm = 1;
         GemmSeg sg[2] = {seg(XE_t, KX, Pb("w_dec_x"), KX, KX), seg(ZB_t, d.ZC, Pb("w_dec_z"), d.ZC, d.ZC)};
-        GemmEpi e; e.tag = "gemm.step"; e.C32 = acc; e.ldc32 = GP; e.lstm = &l;
+        GemmEpi e; e.tag = "gemm.step"; e.C32 = acc; e.ldc32 = GP;
         TRY(gemm_bf16_tn(s, B, GP, 2, sg, e));
+        TRY(lstm_forward(s, l));
       }
     }
   }
@@ -572,7 +544,6 @@ static int train_forward_impl(Handle* h, int B, int N, const char* pk, const voi
   }
   TRY(ce_merge(s, rs.st_max, rs.st_sum, rs.st_arg, gemm_rowstats_tiles(d.V), TB, Wf("rs_tgt"), Wf("lse"), Wf("nll")));
   TRY(loss_reduce(s, Wf("nll"), Wf("kl"), tmask, Wf("lengths"), T, B, loss, kld));
-  TRY(set_l2_window(s, nullptr, 0));
   return 0;
 }
 
@@ -608,7 +579,6 @@ static int train_backward_impl(Handle* h, int B, int N, const char* pk, const vo
 
   const int tiled = persistent_forward(d, B, N) ? 1 : 0;
   const bool pbwd = h->opt_persistent_bwd && persistent_backward(d, B, N);
-  TRY(set_l2_window(s, pk + pp.find("w_dec_xzT")->off, pp.find("bwd_end")->off - pp.find("w_dec_xzT")->off));
   if (pbwd) {
     const char* zl[] = {"dc1", "dc_enc", "dc_dec", "dG_att", "dG_enc", "dG_dec", "dqb", "dml", "du"};
     for (const char* n : zl) CUDA_TRY(zero(n));
@@ -778,30 +748,20 @@ static int train_backward_impl(Handle* h, int B, int N, const char* pk, const vo
     }
   }
 
-  TRY(set_l2_window(s, nullptr, 0));
   // ---- weight gradients: one GEMM per weight block over all T*B rows (K = T*B). The GEMMs of one LSTM share the
-  //      transposed gate-gradient operand dGT and are otherwise independent: optionally (see below) they are spread over
-  //      auxiliary streams (StreamFork) so that the partial last wave of one overlaps the first wave of the next.
-  StreamFork& fk = h->fork;
-  // OFF by default (SSCVAE_WGRAD_FORK=1 turns it on): the first GPU run with it on hung in the test suite and in bench.py
-  // (not investigated: no GPU budget left this round); with it off every launch below goes to `s` as before.
-  static const bool want_fork = [] { const char* e = getenv("SSCVAE_WGRAD_FORK"); return e && e[0] == '1'; }();
-  const bool use_fork = want_fork && !g_prof_enabled;  // the per-launch profiler times launches on ONE stream
-  int item = 0;
-  auto next_stream = [&]() { return fk.pick(s, item++); };
+  //      transposed gate-gradient operand dGT.
   auto wgrad = [&](const bf16* AT, int M, const bf16* BT, int Ncols, int K, int ldk, float* C, int ldc) -> int {
     if (!C) return 0;
     GemmSeg sg = seg(AT, ldk, BT, ldk, K);
     GemmEpi e; e.tag = "gemm.wgrad"; e.C32 = C; e.ldc32 = ldc;
-    return gemm_bf16_tn(next_stream(), M, Ncols, 1, &sg, e);
+    return gemm_bf16_tn(s, M, Ncols, 1, &sg, e);
   };
   // b_ih and b_hh get the same gradient (both are added to the gates): one row sum, copied
   auto bias_pair = [&](const bf16* dGT_, int ib, int ih) -> int {
     float* g1 = Gr(ib); float* g2 = Gr(ih);
     if (!g1 && !g2) return 0;
-    cudaStream_t st = next_stream();
-    TRY(rowsum_bf16(st, dGT_, G, TB, TBp, g1 ? g1 : g2, 0));
-    if (g1 && g2) CUDA_TRY(cudaMemcpyAsync(g2, g1, (size_t)G * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    TRY(rowsum_bf16(s, dGT_, G, TB, TBp, g1 ? g1 : g2, 0));
+    if (g1 && g2) CUDA_TRY(cudaMemcpyAsync(g2, g1, (size_t)G * sizeof(float), cudaMemcpyDeviceToDevice, s));
     return 0;
   };
   auto any = [&](std::initializer_list<int> ids) { for (int i : ids) if (gv[i]) return true; return false; };
@@ -819,20 +779,17 @@ static int train_backward_impl(Handle* h, int B, int N, const char* pk, const vo
   // group 1: decoder LSTM. W_ih column blocks [xhat | h1 | h_dec | cond | z]; W_hh shares the h_dec operand.
   if (any({SSCVAE_W_DEC_IH, SSCVAE_W_DEC_HH, SSCVAE_W_DEC_BIH, SSCVAE_W_DEC_BHH})) {
     TRY(transpose_bf16(s, Wb("dG_dec"), TB, G, Gp, dGT, TBp));
-    if (use_fork) TRY(fk.fork(s));
-    item = 0;
     float* g = Gr(SSCVAE_W_DEC_IH);
     if (g) {
       TRY(wgrad(dGT, G, xhatT, F, TB, TBp, g, ldD));
       TRY(wgrad(dGT, G, h1T, H, TB, TBp, g + F, ldD));
       TRY(wgrad(dGT, G, hdecpT, H, TB, TBp, g + F + H, ldD));
       TRY(wgrad(dGT, G, Wb("ZBT"), Z, TB, TBp, g + F + 2 * H + c, ldD));
-      if (c && !d.cvar) TRY(rowdot_bf16(next_stream(), dGT, G, TB, TBp, sentv, B, g + F + 2 * H, ldD));
+      if (c && !d.cvar) TRY(rowdot_bf16(s, dGT, G, TB, TBp, sentv, B, g + F + 2 * H, ldD));
       if (d.cvar) TRY(wgrad(dGT, G, condT, c, TB, TBp, g + F + 2 * H, ldD));
     }
     TRY(wgrad(dGT, G, hdecpT, H, TB, TBp, Gr(SSCVAE_W_DEC_HH), H));
     TRY(bias_pair(dGT, SSCVAE_W_DEC_BIH, SSCVAE_W_DEC_BHH));
-    TRY(fk.join(s));
   }
   TRY(event(1));
 
@@ -840,32 +797,26 @@ static int train_backward_impl(Handle* h, int B, int N, const char* pk, const vo
   if (any({SSCVAE_W_ENC_IH, SSCVAE_W_ENC_HH, SSCVAE_W_ENC_BIH, SSCVAE_W_ENC_BHH})) {
     TRY(transpose_bf16(s, Wb("dG_enc"), TB, G, Gp, dGT, TBp));
     if (Gr(SSCVAE_W_ENC_HH)) TRY(transpose_bf16(s, Wb("HE"), TB, Hp, Hp, Wb("HETp"), TBp));   // h_enc_{t-1}
-    if (use_fork) TRY(fk.fork(s));
-    item = 0;
     float* g = Gr(SSCVAE_W_ENC_IH);
     if (g) {
       TRY(wgrad(dGT, G, xhatT, F, TB, TBp, g, ldE));
       TRY(wgrad(dGT, G, h1T, H, TB, TBp, g + F, ldE));
       TRY(wgrad(dGT, G, hdecpT, H, TB, TBp, g + F + H, ldE));
-      if (c && !d.cvar) TRY(rowdot_bf16(next_stream(), dGT, G, TB, TBp, sentv, B, g + F + 2 * H, ldE));
+      if (c && !d.cvar) TRY(rowdot_bf16(s, dGT, G, TB, TBp, sentv, B, g + F + 2 * H, ldE));
       if (d.cvar) TRY(wgrad(dGT, G, condT, c, TB, TBp, g + F + 2 * H, ldE));
     }
     TRY(wgrad(dGT, G, Wb("HETp"), H, TB, TBp, Gr(SSCVAE_W_ENC_HH), H));
     TRY(bias_pair(dGT, SSCVAE_W_ENC_BIH, SSCVAE_W_ENC_BHH));
-    TRY(fk.join(s));
   }
   if (any({SSCVAE_W_FC_MEAN_W, SSCVAE_W_FC_MEAN_B, SSCVAE_W_FC_LOGVAR_W, SSCVAE_W_FC_LOGVAR_B})) {
     TRY(transpose_bf16(s, Wb("dml"), TB, d.Z2p, d.Z2p, Wb("dmlT"), TBp));
     TRY(transpose_bf16(s, Wb("HE") + (size_t)B * Hp, TB, Hp, Hp, Wb("HETc"), TBp));   // h_enc_t
     const bf16* dmT = Wb("dmlT");
     const bf16* dlT = Wb("dmlT") + (size_t)Z * TBp;
-    if (use_fork) TRY(fk.fork(s));
-    item = 0;
     TRY(wgrad(dmT, Z, Wb("HETc"), H, TB, TBp, Gr(SSCVAE_W_FC_MEAN_W), H));
     TRY(wgrad(dlT, Z, Wb("HETc"), H, TB, TBp, Gr(SSCVAE_W_FC_LOGVAR_W), H));
-    if (Gr(SSCVAE_W_FC_MEAN_B)) TRY(rowsum_bf16(next_stream(), dmT, Z, TB, TBp, Gr(SSCVAE_W_FC_MEAN_B), 0));
-    if (Gr(SSCVAE_W_FC_LOGVAR_B)) TRY(rowsum_bf16(next_stream(), dlT, Z, TB, TBp, Gr(SSCVAE_W_FC_LOGVAR_B), 0));
-    TRY(fk.join(s));
+    if (Gr(SSCVAE_W_FC_MEAN_B)) TRY(rowsum_bf16(s, dmT, Z, TB, TBp, Gr(SSCVAE_W_FC_MEAN_B), 0));
+    if (Gr(SSCVAE_W_FC_LOGVAR_B)) TRY(rowsum_bf16(s, dlT, Z, TB, TBp, Gr(SSCVAE_W_FC_LOGVAR_B), 0));
   }
   TRY(event(2));
 
@@ -884,8 +835,6 @@ static int train_backward_impl(Handle* h, int B, int N, const char* pk, const vo
       TRY(transpose_bf16(s, Wb("dGsum"), B, G, Gp, Wb("dGsumT"), Bp));
       TRY(transpose_bf16(s, Wb("avgb"), B, Fp, Fp, Wb("avgT"), Bp));
     }
-    if (use_fork) TRY(fk.fork(s));
-    item = 0;
     if (g) {
       TRY(wgrad(dGT, G, Wb("embT_t"), E, TB, TBp, g, ldA));
       TRY(wgrad(Wb("dGsumT"), G, Wb("avgT"), F, B, Bp, g + E, ldA));
@@ -895,14 +844,12 @@ static int train_backward_impl(Handle* h, int B, int N, const char* pk, const vo
     TRY(wgrad(dGT, G, h1pT, H, TB, TBp, Gr(SSCVAE_W_ATT_HH), H));
     TRY(bias_pair(dGT, SSCVAE_W_ATT_BIH, SSCVAE_W_ATT_BHH));
     if (need_demb) {  // learned embedding (untied): d emb rows = dG_att W_att_ih[:, :E], scattered by token id
-      cudaStream_t st = next_stream();
       GemmSeg sg = seg(Wb("dG_att"), Gp, Pb("w_att_eT"), Gp, G);
       GemmEpi e; e.tag = "gemm.wgrad"; e.C32 = Wf("dxemb"); e.ldc32 = E;
-      TRY(gemm_bf16_tn(st, TB, E, 1, &sg, e));
-      CUDA_TRY(cudaMemsetAsync(Gr(SSCVAE_W_EMBEDDING), 0, (size_t)V * E * sizeof(float), st));
-      TRY(embed_scatter_add(st, tok, B, d.L, d.pad, Wf("dxemb"), E, E, Gr(SSCVAE_W_EMBEDDING)));
+      TRY(gemm_bf16_tn(s, TB, E, 1, &sg, e));
+      CUDA_TRY(cudaMemsetAsync(Gr(SSCVAE_W_EMBEDDING), 0, (size_t)V * E * sizeof(float), s));
+      TRY(embed_scatter_add(s, tok, B, d.L, d.pad, Wf("dxemb"), E, E, Gr(SSCVAE_W_EMBEDDING)));
     }
-    TRY(fk.join(s));
   }
   TRY(event(3));
 

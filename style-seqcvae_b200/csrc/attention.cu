@@ -40,8 +40,6 @@ attention_fwd_kernel(AttnArgs a, AttnPlan pl, float* __restrict__ alpha, float* 
   extern __shared__ __align__(128) uint8_t att_smem_raw[];
   const AttnSmem sm = carve(att_smem_raw, a, false);
   attn_prologue(sm, a, false);
-  pdl_wait();                                        // the prologue overlaps the previous kernel's tail
-  pdl_launch_dependents(2);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int r_begin = blockIdx.x * pl.rows_per_cta;
   const int r_end = min(a.R, r_begin + pl.rows_per_cta);
@@ -120,8 +118,6 @@ attention_fwd_grouped_kernel(AttnArgs a, int rows_per_image, int chunks_per_imag
   }
   for (int i = threadIdx.x; i < N4 * GR; i += blockDim.x) al_s[i] = 0.f;
   __syncthreads();
-  pdl_wait();
-  pdl_launch_dependents(2);
   for (int i = threadIdx.x; i < N4; i += blockDim.x) mask_s[i] = i < N ? a.mask[(size_t)img * N + i] : 0.f;
 
   if (warp == ATT_CWARPS) {                          // ---- producer: P in one go, then the feature chunks through the ring
@@ -296,8 +292,7 @@ int attention_forward(cudaStream_t s, const AttnArgs& a, float* alpha, float* sm
   AttnPlan pl;
   TRY(make_plan(a, pl));
   // decode: rows of an image are contiguous and share its features -> one CTA per 8 rows of an image
-  static const bool no_grouped = [] { const char* e = getenv("SSCVAE_ATT_GROUPED"); return e && e[0] == '0'; }();
-  if (!no_grouped && a.rows_per_image >= 4 && smx == nullptr && a.Fp <= 8 * ATT_CONSUMERS && a.Ap <= 256 * G_PVMAX &&
+  if (a.rows_per_image >= 4 && smx == nullptr && a.Fp <= 8 * ATT_CONSUMERS && a.Ap <= 256 * G_PVMAX &&
       (a.R % a.rows_per_image) == 0 && grouped_smem_bytes(a) <= 113 * 1024 && pl.bF * a.Fp * 2 <= G_XSTAGE_BYTES) {
     const size_t gsmem = grouped_smem_bytes(a);
     static bool gconf = false;
@@ -307,8 +302,8 @@ int attention_forward(cudaStream_t s, const AttnArgs& a, float* alpha, float* sm
     }
     const int cpi = ceil_div(a.rows_per_image, GR);
     const int images = a.R / a.rows_per_image;
-    CUDA_TRY(launch_pdl(attention_fwd_grouped_kernel, dim3(images * cpi), dim3(ATT_THREADS), gsmem, s, a, a.rows_per_image, cpi, pl.bF,
-                        pl.nF, alpha, xhat, ld_x));
+    attention_fwd_grouped_kernel<<<dim3(images * cpi), dim3(ATT_THREADS), gsmem, s>>>(a, a.rows_per_image, cpi, pl.bF, pl.nF,
+                                                                                    alpha, xhat, ld_x);
     LAUNCHED();
     return 0;
   }
@@ -318,7 +313,7 @@ int attention_forward(cudaStream_t s, const AttnArgs& a, float* alpha, float* sm
     CUDA_TRY(cudaFuncSetAttribute(attention_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024));
     configured = true;
   }
-  CUDA_TRY(launch_pdl(attention_fwd_kernel, dim3(ceil_div(a.R, pl.rows_per_cta)), dim3(ATT_THREADS), smem, s, a, pl, alpha, smx, xhat, ld_x));
+  attention_fwd_kernel<<<dim3(ceil_div(a.R, pl.rows_per_cta)), dim3(ATT_THREADS), smem, s>>>(a, pl, alpha, smx, xhat, ld_x);
   LAUNCHED();
   return 0;
 }
@@ -330,8 +325,6 @@ attention_bwd_kernel(AttnArgs a, AttnPlan pl, const float* __restrict__ smx, con
   extern __shared__ __align__(128) uint8_t att_smem_raw[];
   const AttnSmem sm = carve(att_smem_raw, a, true);
   attn_prologue(sm, a, true);
-  pdl_wait();                                        // the prologue overlaps the previous kernel's tail
-  pdl_launch_dependents(2);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int r_begin = blockIdx.x * pl.rows_per_cta;
   const int r_end = min(a.R, r_begin + pl.rows_per_cta);
@@ -483,8 +476,8 @@ int attention_backward(cudaStream_t s, const AttnArgs& a, const float* smx, cons
     CUDA_TRY(cudaFuncSetAttribute(attention_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024));
     configured = true;
   }
-  CUDA_TRY(launch_pdl(attention_bwd_kernel, dim3(ceil_div(a.R, pl.rows_per_cta)), dim3(ATT_THREADS), smem, s, a, pl, smx, dxhat, ld_dx, dq,
-                      ld_dq, du));
+  attention_bwd_kernel<<<dim3(ceil_div(a.R, pl.rows_per_cta)), dim3(ATT_THREADS), smem, s>>>(a, pl, smx, dxhat, ld_dx, dq, ld_dq,
+                                                                                             du);
   LAUNCHED();
   return 0;
 }

@@ -48,43 +48,6 @@ static inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
 static inline size_t round_up_sz(size_t x, size_t m) { return (x + m - 1) / m * m; }
 static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 
-// ---- programmatic dependent launch ----------------------------------------------------------------
-// The time loops are ~10 dependent kernels of 3-15 us per step; what separates them is the launch / drain gap.
-// Kernels of the loops are launched with cudaLaunchAttributeProgrammaticStreamSerialization (launch_pdl): the next
-// grid may be scheduled while the previous one drains, runs its prologue (barrier init, TMEM allocation, descriptor
-// prefetch, index math) and blocks in pdl_wait() until the previous grid has completed and flushed. Rule: a kernel
-// launched through launch_pdl executes pdl_wait() before its first global-memory access (reads AND writes).
-// Both instructions are no-ops in a kernel launched without the attribute.
-// The early trigger is conditional, see pdl_launch_dependents().
-// OFF by default (SSCVAE_PDL=1 turns it on): measured gain on the single-GPU training step 0.4 % (7.33 -> 7.30 ms; the
-// step is kernel-time bound, not gap bound), while a dependent grid that becomes resident early can starve CTAs the
-// primary still has to place - seen as a hang of the decode path at 1024 rows before the trigger became conditional,
-// and suspected in a hang of the 8-GPU training run, where NCCL's kernels share the SMs with the step's graph.
-inline bool pdl_enabled() {
-  static const bool on = [] { const char* e = getenv("SSCVAE_PDL"); return e && e[0] == '1'; }();
-  return on;
-}
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr; cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-// Early trigger ONLY when every CTA of this grid is resident at once (`ctas_per_sm` = how many of them one SM holds).
-// A dependent grid that starts while CTAs of the primary are still waiting for an SM takes the resources those CTAs
-// need and then blocks in pdl_wait() for a primary that can no longer finish: observed as a hang of the decode path
-// at 1024 rows (two-wave GEMMs followed by cell kernels). A multi-wave grid keeps the implicit trigger at exit.
-__device__ __forceinline__ void pdl_launch_dependents(unsigned ctas_per_sm) {
-  unsigned nsm;
-  asm volatile("mov.u32 %0, %%nsmid;" : "=r"(nsm));
-  if (gridDim.x * gridDim.y * gridDim.z <= nsm * ctas_per_sm) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-}
-
 // ---- device utilities ---------------------------------------------------------------------------
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.0f / (1.0f + __expf(-x)); }
 

@@ -7,8 +7,6 @@
 
 namespace sscvae {
 
-struct LstmFwdArgs;
-
 struct GemmSeg {
   const bf16* A; int lda;   // (M, K) row-major, lda in elements (multiple of 8, base 16B aligned)
   const bf16* B; int ldb;   // (N, K) row-major
@@ -41,22 +39,12 @@ struct GemmEpi {
   float* C32 = nullptr; int ldc32 = 0; int accumulate = 0;   // C32[m,n] (+)= v
   bf16* C16 = nullptr; int ldc16 = 0;                  // C16[m,n] = bf16(v)
   const char* tag = "gemm";                            // kernel class for the optional profiler (prof.cuh)
-  // skinny GEMMs (M <= 256) run on the swapped-operand kernels with K split over a thread-block cluster; 0 = let the
-  // library choose kernel and split count, 1/2/4 = force the single-CTA kernel with that split, -1..-4 = force the
-  // CTA-pair kernel with split 1..4 (tools/gemm_bench.py, tests)
+  // skinny GEMMs (M <= 256) run on the swapped-operand CTA-pair kernel with K split over a thread-block cluster;
+  // 0 = the library's choice of kernel and split count, 1..4 = force the CTA-pair kernel with that K split
+  // (tools/gemm_bench.py, tests)
   int splits = 0;
-  // Fused LSTM cell (forward): the N = lstm_gate_rows(H) output columns are gate pre-activations in the
-  // gate-interleaved order of the packed weights; `lstm` describes the addends, states and destinations exactly as
-  // for lstm_forward (its acc / ld_acc / perm are ignored). On the CTA-pair kernel (M <= 256) the cell runs in the
-  // GEMM epilogue and the pre-activations never leave the SM; otherwise the GEMM writes C32 (required, ldc32 >= N)
-  // and lstm_forward runs behind it.
-  const LstmFwdArgs* lstm = nullptr;
   const RowStatsEpi* rs = nullptr;                     // see RowStatsEpi (forces the 128 x 128 tile kernel)
 };
-
-// K-split (cluster size 1, 2 or 4) the swapped-operand kernel uses for a skinny GEMM (M <= 256)
-int gemm_suggest_splits(int M, int N, int K_total);
-
 
 // Launches on `stream`; returns 0 or an error code (message via get_error()).
 int gemm_bf16_tn(cudaStream_t stream, int M, int N, int nseg, const GemmSeg* segs, const GemmEpi& epi);

@@ -7,16 +7,13 @@
 //                 fused bias / addends / tanh / dtanh -> fp32 and/or bf16 global stores
 // The accumulator never touches registers or shared memory until the epilogue.
 #include "gemm.cuh"
-#include "kernels.cuh"
 #include "prof.cuh"
+#include "ptx.cuh"
 #include "tc_ptx.cuh"
 #include <cuda.h>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <unordered_map>
-#include <vector>
-#include <algorithm>
 
 namespace sscvae {
 
@@ -35,18 +32,12 @@ struct GemmParams {
   int nseg;
   int M, N;
   int vec;                                        // 1: every epilogue pointer allows 16-byte access
-  int splits;                                     // gridDim.z
-  int kb_per_split;                               // split-K: CTA z works on k-blocks [z*kb_per_split, ...) of the
-                                                  // concatenated segments and ADDS its partial tile into C32
+  int splits;                                     // pair kernel: K split = cluster z = gridDim.z
+  int kb_per_split;                               // pair kernel: CTA z works on k-blocks [z*kb_per_split, ...) of the
+                                                  // concatenated segments
   int tma_store;                                  // 1: plain fp32 tile (+bias): the epilogue leaves through TMA stores of `tc`
   CUtensorMap tc;                                 // fp32 output, box 32 columns x 32 rows, no swizzle
   GemmEpi epi;
-  int w_policy;                                   // pair kernel: 1 = weight tiles are loaded with an L2 evict_first hint
-  int fuse_lstm;                                  // pair kernel: run the LSTM cell `lstm` in the epilogue
-  int lstm_tma;                                   // ... and its outputs leave through TMA stores of `tl`
-  long long* dbg;                                 // SSCVAE_GEMM_DBG=1: per-CTA clock64 stamps of the pair kernel's phases
-  LstmFwdArgs lstm;
-  CUtensorMap tl[7];                              // gates i,f,g,o (fp32), c (fp32), h -> h1_dst, h2_dst (bf16); box 32 units x 32 rows
   RowStatsEpi rs;                                 // vocabulary head: softmax statistics / CE gradient in the epilogue
 };
 
@@ -77,10 +68,6 @@ __device__ __forceinline__ float4 lds_v4(uint32_t a) {
   return v;
 }
 
-__device__ __forceinline__ void red_add_f32x4(float* p, const float4& v) {
-  asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-}
-
 // Second half of the vector epilogue: the warp's 32x32 fp32 block sits in `stage` as [row][column] (pitch 36 floats);
 // 8 consecutive lanes own 32 consecutive columns of ONE output row (128 contiguous bytes), 4 rows per instruction,
 // for the addend loads and for the stores.
@@ -88,7 +75,7 @@ __device__ __forceinline__ void red_add_f32x4(float* p, const float4& v) {
 // parameter the compiler must assume the output stores alias the struct and re-reads every field after each store
 // (measured: ~250 cycles per store, 2-3.4k cycles per 32x32 block instead of ~300).
 __device__ __forceinline__ void epilogue_block_vec(const GemmEpi e, int M, int row0, int col0, uint32_t stage,
-                                                   int splitk, bool add1_all) {
+                                                   bool add1_all) {
   constexpr int PITCH = 36;
   const int lane = threadIdx.x & 31;
   const int c4 = (lane & 7) * 4;
@@ -98,7 +85,7 @@ __device__ __forceinline__ void epilogue_block_vec(const GemmEpi e, int M, int r
   // The epilogue warps run one per SM sub-partition, so the epilogue is bound by its own instruction count
   // (measured: 3.4k cycles per 32x32 block when the tanh / dtanh / accumulate forms were compiled into the one loop).
   // The common case - scaled accumulator + bias + addends -> fp32 and/or bf16 - gets its own lean loop.
-  if (!e.act && !e.dtanh && !e.accumulate && !splitk) {
+  if (!e.act && !e.dtanh && !e.accumulate) {
     const float alpha = e.alpha;
     const float* a1 = add1_all ? e.add1 + n : nullptr;
     const float* a2 = e.add2 ? e.add2 + n : nullptr;
@@ -155,15 +142,11 @@ __device__ __forceinline__ void epilogue_block_vec(const GemmEpi e, int M, int r
       }
       if (e.C32) {
         float* p = e.C32 + (size_t)r * e.ldc32 + n;
-        if (splitk) {
-          red_add_f32x4(p, v);
-        } else {
-          if (e.accumulate) {
-            const float4 c = *reinterpret_cast<const float4*>(p);
-            v.x += c.x; v.y += c.y; v.z += c.z; v.w += c.w;
-          }
-          *reinterpret_cast<float4*>(p) = v;
+        if (e.accumulate) {
+          const float4 c = *reinterpret_cast<const float4*>(p);
+          v.x += c.x; v.y += c.y; v.z += c.z; v.w += c.w;
         }
+        *reinterpret_cast<float4*>(p) = v;
       }
       if (e.C16) {
         __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);
@@ -203,11 +186,9 @@ __device__ __forceinline__ void epilogue_tma_row32(const GemmEpi e, const CUtens
   if (lane == 0) tma_store_2d(tc, stage, col0, row0);
 }
 
-// splitk: 0 = plain store; 1 = this CTA holds a partial sum: add it into C32 (split 0 also applies the addends)
-__device__ __forceinline__ void epilogue_row32(GemmEpi e, int vec, int M, int N, int row0, int col0, int ncols,
-                                               const uint32_t (&acc)[32], uint32_t stage, int splitk, int first_split) {
+__device__ __forceinline__ void epilogue_row32(const GemmEpi e, int vec, int M, int N, int row0, int col0, int ncols,
+                                               const uint32_t (&acc)[32], uint32_t stage) {
   const int lane = threadIdx.x & 31;
-  if (splitk && !first_split) { e.bias = nullptr; e.add1 = nullptr; e.add2 = nullptr; }
   const int row = row0 + lane;           // TMEM lane == output row of this thread's 32 accumulator columns
   // `ncols` < 32 only for the narrow (BN=16) tiles; add1 may cover just the first add1_cols columns
   const bool add1_all = e.add1 && (col0 + 32 <= e.add1_cols);
@@ -224,7 +205,7 @@ __device__ __forceinline__ void epilogue_row32(GemmEpi e, int vec, int M, int N,
              make_float4(__uint_as_float(acc[4 * j]), __uint_as_float(acc[4 * j + 1]), __uint_as_float(acc[4 * j + 2]),
                          __uint_as_float(acc[4 * j + 3])));
     __syncwarp();
-    epilogue_block_vec(e, M, row0, col0, stage, splitk, add1_all);
+    epilogue_block_vec(e, M, row0, col0, stage, add1_all);
     __syncwarp();
     return;
   }
@@ -246,8 +227,7 @@ __device__ __forceinline__ void epilogue_row32(GemmEpi e, int vec, int M, int N,
       if (e.dtanh) { float t = e.dtanh[(size_t)row * e.ldd + n]; x *= 1.0f - t * t; }
       if (e.C32) {
         float* p = e.C32 + (size_t)row * e.ldc32 + n;
-        if (splitk) atomicAdd(p, x);
-        else *p = e.accumulate ? (*p + x) : x;
+        *p = e.accumulate ? (*p + x) : x;
       }
       if (e.C16) e.C16[(size_t)row * e.ldc16 + n] = __float2bfloat16_rn(x);
     }
@@ -280,8 +260,6 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_tcgen05_kernel(const __g
   int total_kb = 0;
 #pragma unroll
   for (int s = 0; s < MAX_SEG; ++s) total_kb += (s < p.nseg) ? p.kblocks[s] : 0;
-  const int kb_begin = blockIdx.z * p.kb_per_split;
-  const int kb_end = min(total_kb, kb_begin + p.kb_per_split);
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < p.nseg; ++s) { prefetch_tmap(&p.ta[s]); prefetch_tmap(&p.tb[s]); }
@@ -294,14 +272,12 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_tcgen05_kernel(const __g
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_acc = *tmem_slot;
-  pdl_wait();                                           // everything above overlaps the previous kernel's tail
-  pdl_launch_dependents(1);
 
   if (warp == 0) {
     if (elect_one_sync()) {
       int stage = 0; uint32_t phase = 0;
       int s = 0, base = 0;                              // segment of the current k-block, its first global index
-      for (int g = kb_begin; g < kb_end; ++g) {
+      for (int g = 0; g < total_kb; ++g) {
         while (g >= base + p.kblocks[s]) { base += p.kblocks[s]; ++s; }
         const int kb = g - base;
         mbar_wait(&empty_bar[stage], phase ^ 1);
@@ -314,7 +290,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_tcgen05_kernel(const __g
   } else if (warp == 1) {
     if (elect_one_sync()) {
       int stage = 0; uint32_t phase = 0;
-      for (int kb = kb_begin; kb < kb_end; ++kb) {
+      for (int kb = 0; kb < total_kb; ++kb) {
         mbar_wait(&full_bar[stage], phase);
         tc_fence_after();
         const uint32_t a_base = smem_u32(smem_a + stage * A_STAGE_BYTES);
@@ -323,7 +299,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_tcgen05_kernel(const __g
         for (int k = 0; k < BK / 16; ++k) {
           // advance 16 elements (32 bytes) along K inside the 128B swizzle atom
           umma_bf16(tmem_acc, make_smem_desc(a_base + k * 32), make_smem_desc(b_base + k * 32), IDESC,
-                    (kb > kb_begin || k > 0) ? 1u : 0u);
+                    (kb > 0 || k > 0) ? 1u : 0u);
         }
         umma_commit(&empty_bar[stage]);          // frees the smem slot once these MMAs have read it
         if (++stage == STAGES) { stage = 0; phase ^= 1; }
@@ -412,7 +388,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_tcgen05_kernel(const __g
           GemmEpi e2 = p.epi;
           e2.alpha = 1.f; e2.bias = nullptr;
           epilogue_row32(e2, p.vec, p.M, p.N, m0 + q * 32, n0 + c0, BN - c0 < 32 ? BN - c0 : 32, acc,
-                         smem_u32(smem_a) + (warp - 2) * 32 * 36 * 4, 0, 1);
+                         smem_u32(smem_a) + (warp - 2) * 32 * 36 * 4);
           continue;
         }
       }
@@ -420,7 +396,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_tcgen05_kernel(const __g
         epilogue_tma_row32(p.epi, &p.tc, p.N, m0 + q * 32, n0 + c0, acc, smem_u32(smem_a) + (warp - 2) * 4096);
       } else {
         epilogue_row32(p.epi, p.vec, p.M, p.N, m0 + q * 32, n0 + c0, BN - c0 < 32 ? BN - c0 : 32, acc,
-                       smem_u32(smem_a) + (warp - 2) * 32 * 36 * 4, gridDim.z > 1, blockIdx.z == 0);
+                       smem_u32(smem_a) + (warp - 2) * 32 * 36 * 4);
       }
     }
     if (rs.mode == 1 && row < p.M) {             // partial statistics of (row, this 128-column tile): lanes = consecutive rows
@@ -463,7 +439,6 @@ gemm_tcgen05_2cta_kernel(const __grid_constant__ GemmParams p) {
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(accum_bar + 1);
 
   const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();
   const int m0 = blockIdx.y * (2 * BM) + (int)rank * BM;
   const int n0 = (blockIdx.x >> 1) * BN;
@@ -471,8 +446,6 @@ gemm_tcgen05_2cta_kernel(const __grid_constant__ GemmParams p) {
   int total_kb = 0;
 #pragma unroll
   for (int s = 0; s < MAX_SEG; ++s) total_kb += (s < p.nseg) ? p.kblocks[s] : 0;
-  const int kb_begin = blockIdx.z * p.kb_per_split;
-  const int kb_end = min(total_kb, kb_begin + p.kb_per_split);
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < p.nseg; ++s) { prefetch_tmap(&p.ta[s]); prefetch_tmap(&p.tb[s]); }
@@ -485,14 +458,12 @@ gemm_tcgen05_2cta_kernel(const __grid_constant__ GemmParams p) {
   cluster_sync_all();                                     // both CTAs' barriers exist before any remote arrival
   tc_fence_after();
   const uint32_t tmem_acc = *tmem_slot;
-  pdl_wait();
-  pdl_launch_dependents(1);
 
   if (warp == 0) {
     if (elect_one_sync()) {
       int stage = 0; uint32_t phase = 0;
       int s = 0, base = 0;
-      for (int g = kb_begin; g < kb_end; ++g) {
+      for (int g = 0; g < total_kb; ++g) {
         while (g >= base + p.kblocks[s]) { base += p.kblocks[s]; ++s; }
         const int kb = g - base;
         mbar_wait(&empty_bar[stage], phase ^ 1);
@@ -505,7 +476,7 @@ gemm_tcgen05_2cta_kernel(const __grid_constant__ GemmParams p) {
   } else if (warp == 1) {
     if (rank == 0 && elect_one_sync()) {
       int stage = 0; uint32_t phase = 0;
-      for (int kb = kb_begin; kb < kb_end; ++kb) {
+      for (int kb = 0; kb < total_kb; ++kb) {
         mbar_wait(&full_bar[stage], phase);
         tc_fence_after();
         const uint32_t a_base = smem_u32(smem_a + stage * A_STAGE_BYTES);
@@ -513,7 +484,7 @@ gemm_tcgen05_2cta_kernel(const __grid_constant__ GemmParams p) {
 #pragma unroll
         for (int k = 0; k < BK / 16; ++k) {
           umma_bf16_2sm(tmem_acc, make_smem_desc(a_base + k * 32), make_smem_desc(b_base + k * 32), IDESC,
-                        (kb > kb_begin || k > 0) ? 1u : 0u);
+                        (kb > 0 || k > 0) ? 1u : 0u);
         }
         umma_commit_2sm(&empty_bar[stage]);
         if (++stage == STAGES) { stage = 0; phase ^= 1; }
@@ -535,7 +506,7 @@ gemm_tcgen05_2cta_kernel(const __grid_constant__ GemmParams p) {
         epilogue_tma_row32(p.epi, &p.tc, p.N, m0 + q * 32, n0 + c0, acc, smem_u32(smem_a) + (warp - 2) * 4096);
       } else {
         epilogue_row32(p.epi, p.vec, p.M, p.N, m0 + q * 32, n0 + c0, BN - c0 < 32 ? BN - c0 : 32, acc,
-                       smem_u32(smem_a) + (warp - 2) * 32 * 36 * 4, gridDim.z > 1, blockIdx.z == 0);
+                       smem_u32(smem_a) + (warp - 2) * 32 * 36 * 4);
       }
     }
   }
@@ -549,17 +520,22 @@ gemm_tcgen05_2cta_kernel(const __grid_constant__ GemmParams p) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// Skinny-M kernel (M <= 256: the per-timestep recurrent GEMMs, M = batch): operands SWAPPED, K split over a
-// thread-block cluster, partial tiles reduced through distributed shared memory.
+// Skinny-M kernel (M <= 256: the per-timestep recurrent GEMMs, M = batch): operands SWAPPED, every 256 x 256 tile
+// driven by tcgen05.mma.cta_group::2 on a CTA pair, K split over a thread-block cluster, partial tiles reduced through
+// distributed shared memory.
 //
 // Measured on B200 (tools/gemm_bench.py, profiles/README.md): an M=128 tcgen05.mma takes ~130 cycles whatever its
-// N, and one SM ingests TMA operands at ~77 GB/s at most. A skinny GEMM therefore wants (a) the <= 256 batch rows on
-// the MMA's N side so every instruction is a full 128x256x16, and (b) as few operand bytes per SM as possible.
-// A CTA owns 128 rows of the WEIGHT matrix (UMMA M) x all batch rows (UMMA N = 256) over 1/S of K: 48 KB of
-// operands per 128x256x64 k-block (the 128x64 tiling moves 24 KB per 128x64x64). The S CTAs of a cluster (1,1,S)
-// work on the same tile; afterwards CTA r owns the batch columns [r*256/S, (r+1)*256/S): every CTA pushes the other
-// CTAs' column slices of its partial accumulator into their shared memory (st.shared::cluster, coalesced), a
-// cluster barrier makes them visible, and the owner adds them to its own TMEM slice and runs the full epilogue.
+// N, and one SM ingests TMA operands at ~77 GB/s at most (the chip-wide L2 -> SM rate, ~6300 B/clk, B300_MICROARCH.md,
+// with all SMs pulling). A skinny GEMM therefore wants (a) the <= 256 batch rows on the MMA's N side so every
+// instruction is a full-width MMA, and (b) as few operand bytes per SM as possible. CTA x of a pair loads its own 128
+// WEIGHT rows (16 KB) and HALF of the batch rows (16 KB) per k-block; the MMA (M = 256 weight rows, N = 256 batch rows)
+// reads both halves across the pair. 32 KB per SM and k-block instead of 48 KB for one CTA that loads all 256 batch
+// rows (2/3 of it the activation tile every weight-row CTA re-reads): the loads of a 128x256x64 block (~415 ns at
+// 77 GB/s) hide behind its MMAs (~440 ns at the sustained tensor rate).
+// Cluster = (2, 1, S): x = the pair, z = the K split (S = 1..4). Afterwards CTA (x, z) owns the batch columns
+// [z*CW, z*CW+CW) of its 128 weight rows: every CTA pushes the other splits' column slices of its partial accumulator
+// into their shared memory (st.shared::cluster, coalesced), a cluster barrier makes them visible, and the owner adds
+// them to its own TMEM slice and runs the full epilogue.
 // The accumulator is transposed (TMEM lane = output column n, TMEM column = batch row), so for a fixed batch row the
 // 32 lanes of an epilogue warp hold 32 consecutive n: every global access is one coalesced 128-byte line.
 // ---------------------------------------------------------------------------------------------
@@ -586,7 +562,7 @@ __device__ __forceinline__ void epilogue_swapped32(const GemmEpi e, int vec, int
   const bool add1_all = e.add1 && (n_warp0 + 32 <= e.add1_cols);
   const bool add1_none = !e.add1 || (n_warp0 >= e.add1_cols);
   if (vec && n_warp0 + 32 <= N && (add1_all || add1_none)) {
-    epilogue_block_vec(e, M, b0, n_warp0, stage, 0, add1_all);
+    epilogue_block_vec(e, M, b0, n_warp0, stage, add1_all);
   } else {
     const int n = n_warp0 + lane;
     if (n < N) {
@@ -612,258 +588,6 @@ __device__ __forceinline__ void epilogue_swapped32(const GemmEpi e, int vec, int
   __syncwarp();
 }
 
-template <int STAGES>
-__global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_kernel(const __grid_constant__ GemmParams p) {
-  constexpr int BW = 128, BX = 256;                     // weight rows per CTA (UMMA M), activation rows (UMMA N)
-  constexpr int W_STAGE_BYTES = BW * BK * 2, X_STAGE_BYTES = BX * BK * 2;
-  constexpr uint32_t IDESC = make_idesc(BW, BX);
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  uint8_t* smem = smem_raw;                             // __align__(1024): the 128B swizzle needs 1024-byte aligned tiles
-  if (threadIdx.x == 0 && (smem_u32(smem) & 1023u)) __trap();
-  uint8_t* smem_w = smem;
-  uint8_t* smem_x = smem + STAGES * W_STAGE_BYTES;
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem_x + STAGES * X_STAGE_BYTES);
-  uint64_t* empty_bar = full_bar + STAGES;
-  uint64_t* accum_bar = empty_bar + STAGES;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(accum_bar + 1);
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const int n0 = blockIdx.x * BW;
-  const int S = p.splits;                               // cluster size along z; this CTA's rank = blockIdx.z
-  const int rank = blockIdx.z;
-
-  int total_kb = 0;
-#pragma unroll
-  for (int s = 0; s < MAX_SEG; ++s) total_kb += (s < p.nseg) ? p.kblocks[s] : 0;
-  const int kb_begin = rank * p.kb_per_split;
-  const int kb_end = min(total_kb, kb_begin + p.kb_per_split);
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < p.nseg; ++s) { prefetch_tmap(&p.ta[s]); prefetch_tmap(&p.tb[s]); }
-    for (int s = 0; s < STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
-    mbar_init(accum_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) tmem_alloc<BX>(tmem_slot);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_acc = *tmem_slot;
-  pdl_wait();
-  pdl_launch_dependents(1);
-
-  if (warp == 0) {
-    if (elect_one_sync()) {
-      int stage = 0; uint32_t phase = 0;
-      int s = 0, base = 0;
-      for (int g = kb_begin; g < kb_end; ++g) {
-        while (g >= base + p.kblocks[s]) { base += p.kblocks[s]; ++s; }
-        const int kb = g - base;
-        mbar_wait(&empty_bar[stage], phase ^ 1);
-        mbar_expect_tx(&full_bar[stage], W_STAGE_BYTES + X_STAGE_BYTES);
-        tma_load_2d(smem_w + stage * W_STAGE_BYTES, &p.tb[s], &full_bar[stage], kb * BK, n0);
-        tma_load_2d(smem_x + stage * X_STAGE_BYTES, &p.ta[s], &full_bar[stage], kb * BK, 0);
-        if (++stage == STAGES) { stage = 0; phase ^= 1; }
-      }
-    }
-    __syncwarp();
-  } else if (warp == 1) {
-    if (elect_one_sync()) {
-      int stage = 0; uint32_t phase = 0;
-      for (int kb = kb_begin; kb < kb_end; ++kb) {
-        mbar_wait(&full_bar[stage], phase);
-        tc_fence_after();
-        const uint32_t w_base = smem_u32(smem_w + stage * W_STAGE_BYTES);
-        const uint32_t x_base = smem_u32(smem_x + stage * X_STAGE_BYTES);
-#pragma unroll
-        for (int k = 0; k < BK / 16; ++k)
-          umma_bf16(tmem_acc, make_smem_desc(w_base + k * 32), make_smem_desc(x_base + k * 32), IDESC,
-                    (kb > kb_begin || k > 0) ? 1u : 0u);
-        umma_commit(&empty_bar[stage]);
-        if (++stage == STAGES) { stage = 0; phase ^= 1; }
-      }
-      umma_commit(accum_bar);
-    }
-    __syncwarp();
-  } else {
-    mbar_wait(accum_bar, 0);                            // this CTA's partial tile is complete in TMEM
-    tc_fence_after();
-  }
-
-  const int q = warp & 3;                               // epilogue warps 2..5 own TMEM lanes [32q, 32q+32)
-  const int tl = q * 32 + lane;                         // TMEM lane = column n0 + tl of the output
-  const int CW = BX / S;                                // batch columns owned by each CTA of the cluster
-  float* recv = reinterpret_cast<float*>(smem);         // [(S-1) sources][CW columns][128 lanes], over the dead stages
-  if (S > 1) {
-    // every CTA of the cluster has finished its main loop (its stage buffers are dead) before anyone pushes
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-    if (warp >= 2 && kb_end > kb_begin) {
-      for (int o = 0; o < S; ++o) {
-        if (o == rank) continue;
-        const int slot = rank < o ? rank : rank - 1;
-        const uint32_t rbase = mapa_shared(smem_u32(recv), (uint32_t)o);
-        for (int c = 0; c < CW; c += 32) {
-          if (o * CW + c >= p.M) break;                 // columns beyond the batch are never read
-          uint32_t acc[32];
-          tmem_ld_32x32(tmem_acc + (static_cast<uint32_t>(q * 32) << 16) + o * CW + c, acc);
-          tmem_ld_wait();
-#pragma unroll
-          for (int j = 0; j < 32; ++j)
-            st_shared_cluster_f32(rbase + (uint32_t)(((slot * CW + c + j) * 128 + tl) * 4), __uint_as_float(acc[j]));
-        }
-      }
-    }
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-  }
-  if (warp >= 2) {
-    const GemmEpi epi = p.epi;                          // registers (see the note at epilogue_block_vec)
-    // which of the other CTAs actually had k-blocks (a trailing split can be empty when K is short)
-    for (int c = 0; c < CW; c += 32) {
-      const int b0 = rank * CW + c;
-      if (b0 >= p.M) break;
-      float v[32];
-      if (kb_end > kb_begin) {
-        uint32_t acc[32];
-        tmem_ld_32x32(tmem_acc + (static_cast<uint32_t>(q * 32) << 16) + b0, acc);
-        tmem_ld_wait();
-#pragma unroll
-        for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(acc[j]);
-      } else {
-#pragma unroll
-        for (int j = 0; j < 32; ++j) v[j] = 0.f;
-      }
-      for (int o = 0; o < S; ++o) {
-        if (o == rank || o * p.kb_per_split >= total_kb) continue;
-        const int slot = o < rank ? o : o - 1;
-#pragma unroll
-        for (int j = 0; j < 32; ++j) v[j] += lds_f32(smem_u32(recv) + (uint32_t)(((slot * CW + c + j) * 128 + tl) * 4));
-      }
-      if (p.tma_store) {
-        // dense [32 batch rows][32 columns] block per warp -> one TMA store; the async engine writes it out while the
-        // warp goes on (plain STG.128 stores cost this lone warp ~220 cycles each: 1.8k cycles per block)
-        const uint32_t st = smem_u32(smem) + 96 * 1024 + (warp - 2) * 4096;
-        const float bias = (epi.bias && n0 + tl < p.N) ? epi.bias[n0 + tl] : 0.f;
-        if (lane == 0) tma_store_wait_read();           // the previous store has finished reading this buffer
-        __syncwarp();
-#pragma unroll
-        for (int j = 0; j < 32; ++j) sts_f32(st + (j * 32 + lane) * 4, fmaf(v[j], epi.alpha, bias));
-        fence_proxy_async_smem();
-        __syncwarp();
-        if (lane == 0) tma_store_2d(&p.tc, st, n0 + q * 32, b0);
-      } else {
-        epilogue_swapped32(epi, p.vec, p.M, p.N, n0 + q * 32, b0, v,
-                           smem_u32(smem) + 96 * 1024 + (warp - 2) * 32 * 36 * 4);
-      }
-    }
-  }
-  if (p.tma_store && warp >= 2 && lane == 0) tma_store_wait_all();
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc<BX>(tmem_acc);
-  }
-}
-
-// ---------------------------------------------------------------------------------------------
-// Skinny-M kernel, CTA-PAIR form: the swapped-operand cluster split-K kernel above with every 256 x 256 tile driven
-// by tcgen05.mma.cta_group::2. The chip-wide L2 -> SM rate (~6300 B/clk, B300_MICROARCH.md; measured here as
-// ~77 GB/s per SM with all SMs pulling) bounds these GEMMs, and in the single-CTA form 2/3 of every k-block's 48 KB
-// is the ACTIVATION tile, re-read by every one of the N/128 weight-row CTAs. A pair splits that tile: CTA x of the
-// pair loads its own 128 weight rows (16 KB) and HALF of the batch rows (16 KB), the MMA (M = 256 weight rows,
-// N = 256 batch rows) reads both halves across the pair. 32 KB instead of 48 KB per SM and k-block: the loads of a
-// 128x256x64 block (~415 ns at 77 GB/s) now hide behind its MMAs (~440 ns at the sustained tensor rate).
-// Cluster = (2, 1, S): x = the pair, z = the K split (S = 1..4); CTA (x, z) ends up owning the batch columns
-// [z*CW, z*CW+CW) of its 128 weight rows, receives the other splits' partial sums for them through distributed
-// shared memory and runs the epilogue, exactly as in the single-CTA form.
-// ---------------------------------------------------------------------------------------------
-// Fused LSTM cell (updown_cell.py:143-148 etc., nn.LSTMCell gate order i,f,g,o). A thread owns hidden unit j for 8
-// batch rows [r0, r0+8) of a 32-row block. Everything the cell needs besides the GEMM result - the addends of the four
-// gate pre-activations and c_{t-1} - does not depend on the GEMM, so it is loaded into registers one block AHEAD (before
-// the accumulator is ready / while the previous block is processed): the epilogue never waits on global memory.
-struct LstmCellPre { float pre[8][4]; float cp[8]; };
-
-// Branch-free forms for the epilogue: its four warps run one per SM sub-partition with nothing to hide instruction
-// latency behind, and tanhf / IEEE division are ~4x the instructions (measured: 850 cycles per cell with them).
-// Absolute error <= 2e-7, far inside the bf16 operand rounding of the next GEMM.
-__device__ __forceinline__ float cell_sigmoid(float x) { return __fdividef(1.0f, 1.0f + __expf(-x)); }
-__device__ __forceinline__ float cell_tanh(float x) { return 1.0f - __fdividef(2.0f, 1.0f + __expf(2.0f * x)); }
-
-__device__ __forceinline__ void lstm_cell_prefetch(const LstmFwdArgs& a, int j, int r0, LstmCellPre& P) {
-  const int H = a.H;
-  if (j >= H) return;
-  float bias[4];
-#pragma unroll
-  for (int k = 0; k < 4; ++k) bias[k] = a.bias ? a.bias[k * H + j] : 0.f;
-#pragma unroll
-  for (int t = 0; t < 8; ++t) {
-    const int r = min(r0 + t, a.R - 1);                 // clamped: rows beyond R are loaded but never stored
-    const int r2 = a.rowmap ? a.rowmap[r] : r;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const int na = lstm_gate_row(k, j);
-      float v = bias[k];
-      if (a.add1) v += a.add1[(size_t)r * a.ld1 + na];
-      if (a.add2) v += a.add2[(size_t)r2 * a.ld2 + na];
-      if (a.sent) v += a.sent[r2] * a.scol[k * H + j];
-      P.pre[t][k] = v;
-    }
-    P.cp[t] = a.c_prev ? a.c_prev[(size_t)r * H + j] : 0.f;
-  }
-}
-
-// the pre-activation (GEMM part) of gate k, row r0+t sits at xch + (k*32*32 + t*32) floats.
-// stg != 0: the results are staged in shared memory as dense [32 rows][32 units] tiles (gates i,f,g,o and c in fp32 at
-// stg + o*4096, h in bf16 at stg + 20480) and leave through TMA stores issued by the caller: global stores cost a lone
-// epilogue warp ~220 cycles each (measured), and a cell has seven of them. Units beyond H stage zeros: the fp32 maps
-// clip them, the bf16 maps write them into the zero padding columns of the operand buffers.
-__device__ __forceinline__ void lstm_cell_rows(const LstmFwdArgs& a, int j, int r0, uint32_t xch, const LstmCellPre& P,
-                                               uint32_t stg, int rb0) {
-  const int H = a.H;
-  if (stg) {
-    const int lane = threadIdx.x & 31;
-    const bool valid = j < H;
-#pragma unroll
-    for (int t = 0; t < 8; ++t) {
-      float g[4];
-#pragma unroll
-      for (int k = 0; k < 4; ++k) g[k] = lds_f32(xch + (uint32_t)((k * 32 * 32 + t * 32) * 4)) + P.pre[t][k];
-      float i = cell_sigmoid(g[0]), f = cell_sigmoid(g[1]), gg = cell_tanh(g[2]), o = cell_sigmoid(g[3]);
-      float c = f * P.cp[t] + i * gg;
-      float h = o * cell_tanh(c);
-      if (!valid) { i = f = gg = o = c = h = 0.f; }
-      const uint32_t off = (uint32_t)(((rb0 + t) * 32 + lane) * 4);
-      sts_f32(stg + off, i); sts_f32(stg + 4096 + off, f); sts_f32(stg + 8192 + off, gg); sts_f32(stg + 12288 + off, o);
-      sts_f32(stg + 16384 + off, c);
-      const unsigned short hb = __bfloat16_as_ushort(__float2bfloat16_rn(h));
-      asm volatile("st.shared.u16 [%0], %1;" ::"r"(stg + 20480 + (off >> 1)), "h"(hb) : "memory");
-    }
-    return;
-  }
-  if (j >= H) return;
-#pragma unroll
-  for (int t = 0; t < 8; ++t) {
-    const int r = r0 + t;
-    if (r < a.R) {
-      float g[4];
-#pragma unroll
-      for (int k = 0; k < 4; ++k) g[k] = lds_f32(xch + (uint32_t)((k * 32 * 32 + t * 32) * 4)) + P.pre[t][k];
-      const float i = cell_sigmoid(g[0]), f = cell_sigmoid(g[1]), gg = cell_tanh(g[2]), o = cell_sigmoid(g[3]);
-      const float c = f * P.cp[t] + i * gg;
-      const float h = o * cell_tanh(c);
-      a.c_out[(size_t)r * H + j] = c;
-      if (a.gates_out) {
-        float* go = a.gates_out + (size_t)r * 4 * H;
-        go[j] = i; go[H + j] = f; go[2 * H + j] = gg; go[3 * H + j] = o;
-      }
-      const bf16 hb = __float2bfloat16_rn(h);
-      if (a.h1_dst) a.h1_dst[(size_t)r * a.ld_h1 + j] = hb;
-      if (a.h2_dst) a.h2_dst[(size_t)r * a.ld_h2 + j] = hb;
-    }
-  }
-}
-
 __device__ __forceinline__ void umma_commit_2sm_mask(uint64_t* bar, uint16_t mask) {
   asm volatile(
       "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
@@ -871,12 +595,6 @@ __device__ __forceinline__ void umma_commit_2sm_mask(uint64_t* bar, uint16_t mas
       "h"(mask)
       : "memory");
 }
-
-#define DBG_STAMP(i)                                                                                         \
-  do {                                                                                                     \
-    if (p.dbg && warp == 2 && lane == 0)                                                                   \
-      p.dbg[((size_t)blockIdx.z * gridDim.x + blockIdx.x) * 16 + (i)] = clock64();                          \
-  } while (0)
 
 template <int STAGES>
 __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_pair_kernel(const __grid_constant__ GemmParams p) {
@@ -900,7 +618,6 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_pair_ker
   const int S = p.splits;
   const int rank = blockIdx.z;                          // K split of this CTA (cluster z == grid z)
   const int n0 = (blockIdx.x >> 1) * (2 * BW) + xr * BW;   // first weight row (output column) of this CTA
-  DBG_STAMP(0);
 
   int total_kb = 0;
 #pragma unroll
@@ -919,27 +636,22 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_pair_ker
   cluster_sync_all();                                   // the peer's barriers exist before any remote arrival
   tc_fence_after();
   const uint32_t tmem_acc = *tmem_slot;
-  DBG_STAMP(1);
-  pdl_wait();                                           // everything above overlaps the previous kernel's tail
-  pdl_launch_dependents(1);
-  DBG_STAMP(2);
   const int CW = S == 1 ? 256 : S == 2 ? 128 : S == 3 ? 96 : 64;   // batch columns owned by each K split
-  LstmCellPre cell_pre;                                 // fused LSTM: addends + c_{t-1} of this thread's next 8 cells
-  const LstmFwdArgs lstm = p.lstm;                      // registers (see the note at epilogue_block_vec)
 
   if (warp == 0) {
     if (elect_one_sync()) {
       int stage = 0; uint32_t phase = 0;
       int s = 0, base = 0;
-      uint64_t w_pol = 0;
-      if (p.w_policy) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(w_pol));
+      // The weights of the skinny GEMMs (76 MB per timestep) are streamed once per launch; marking them evict_first
+      // leaves L2 to the 52 MB of region features + projections the attention kernels re-read every step (measured:
+      // step 8.21 -> 8.08 ms, attention_fwd 25.1 -> 23.1 us).
+      const uint64_t w_pol = ptx::l2_policy_evict_first();
       for (int g = kb_begin; g < kb_end; ++g) {
         while (g >= base + p.kblocks[s]) { base += p.kblocks[s]; ++s; }
         const int kb = g - base;
         mbar_wait(&empty_bar[stage], phase ^ 1);
         if (xr == 0) mbar_expect_tx(&full_bar[stage], 2 * (W_STAGE_BYTES + X_STAGE_BYTES));
-        if (p.w_policy) tma_load_2d_2sm_hint(smem_w + stage * W_STAGE_BYTES, &p.tb[s], &full_bar[stage], kb * BK, n0, w_pol);
-        else tma_load_2d_2sm(smem_w + stage * W_STAGE_BYTES, &p.tb[s], &full_bar[stage], kb * BK, n0);
+        tma_load_2d_2sm_hint(smem_w + stage * W_STAGE_BYTES, &p.tb[s], &full_bar[stage], kb * BK, n0, w_pol);
         tma_load_2d_2sm(smem_x + stage * X_STAGE_BYTES, &p.ta[s], &full_bar[stage], kb * BK, xr * BXH);
         if (++stage == STAGES) { stage = 0; phase ^= 1; }
       }
@@ -965,11 +677,8 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_pair_ker
     }
     __syncwarp();
   } else {
-    if (p.fuse_lstm) lstm_cell_prefetch(lstm, (n0 >> 2) + lane, rank * CW + (warp - 2) * 8, cell_pre);
-    DBG_STAMP(3);
     mbar_wait(accum_bar, 0);                            // this pair's partial tile is complete in both CTAs' TMEM
     tc_fence_after();
-    DBG_STAMP(4);
   }
 
   const int q = warp & 3;                               // epilogue warps 2..5 own TMEM lanes [32q, 32q+32)
@@ -977,7 +686,6 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_pair_ker
   float* recv = reinterpret_cast<float*>(smem);         // [(S-1) sources][CW columns][128 lanes], over the dead stages
   // every CTA of the cluster has finished its main loop (stage buffers dead, also the ones the PEER's MMAs read)
   cluster_sync_all();
-  DBG_STAMP(5);
   if (S > 1) {
     if (warp >= 2 && kb_end > kb_begin) {
       for (int o = 0; o < S; ++o) {
@@ -995,9 +703,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_pair_ker
         }
       }
     }
-    DBG_STAMP(6);
     cluster_sync_all();
-    DBG_STAMP(7);
   }
   if (warp >= 2) {
     const GemmEpi epi = p.epi;
@@ -1021,38 +727,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_pair_ker
 #pragma unroll
         for (int j = 0; j < 32; ++j) v[j] += lds_f32(smem_u32(recv) + (uint32_t)(((slot * CW + c + j) * 128 + tl) * 4));
       }
-      if (p.fuse_lstm) {
-        // The 128 weight rows of this CTA are 4 gates x 32 hidden units (lstm_gate_row): warp q holds gate q of unit
-        // `lane` for 32 batch rows. Exchange through shared memory, then warp w runs the cell for 8 of the 32 batch
-        // rows with lane = unit, so every global access is 32 consecutive units of one row (128 / 64 bytes).
-        const uint32_t xch = smem_u32(smem) + 96 * 1024;          // [gate][batch row][unit] fp32, 16 KB
-        const uint32_t stg = p.lstm_tma ? smem_u32(smem) + 112 * 1024 : 0u;   // output tiles for the TMA stores, 22 KB
-#pragma unroll
-        for (int j = 0; j < 32; ++j) sts_f32(xch + ((q * 32 + j) * 32 + lane) * 4, v[j]);
-        if (c == 0) DBG_STAMP(8);
-        if (stg && warp == 2 && lane == 0) tma_store_wait_read();   // the previous block's stores have read the staging tiles
-        asm volatile("bar.sync 1, 128;" ::: "memory");
-        if (c == 0) DBG_STAMP(9);
-        const LstmCellPre cur = cell_pre;
-        if (c + 32 < CW && b0 + 32 < p.M && b0 + 32 < TCOLS)      // the next block's addends fly during this block's math
-          lstm_cell_prefetch(lstm, (n0 >> 2) + lane, b0 + 32 + (warp - 2) * 8, cell_pre);
-        lstm_cell_rows(lstm, (n0 >> 2) + lane, b0 + (warp - 2) * 8, xch + (uint32_t)((warp - 2) * 8 * 32 + lane) * 4, cur, stg,
-                       (warp - 2) * 8);
-        if (c == 0) DBG_STAMP(10);
-        if (stg) fence_proxy_async_smem();
-        asm volatile("bar.sync 1, 128;" ::: "memory");
-        if (c == 0) DBG_STAMP(11);
-        if (stg && warp == 2 && lane == 0 && n0 < p.N) {
-          const int j0 = n0 >> 2;
-          if (lstm.gates_out) {
-#pragma unroll
-            for (int k = 0; k < 4; ++k) tma_store_2d(&p.tl[k], stg + k * 4096, j0, b0);
-          }
-          tma_store_2d(&p.tl[4], stg + 16384, j0, b0);
-          if (lstm.h1_dst) tma_store_2d(&p.tl[5], stg + 20480, j0, b0);
-          if (lstm.h2_dst) tma_store_2d(&p.tl[6], stg + 20480, j0, b0);
-        }
-      } else if (p.tma_store) {
+      if (p.tma_store) {
         const uint32_t st = smem_u32(smem) + 96 * 1024 + (warp - 2) * 4096;
         const float bias = (epi.bias && n0 + tl < p.N) ? epi.bias[n0 + tl] : 0.f;
         if (lane == 0) tma_store_wait_read();
@@ -1068,38 +743,13 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_pair_ker
       }
     }
   }
-  DBG_STAMP(12);
-  if ((p.tma_store || p.lstm_tma) && warp >= 2 && lane == 0) tma_store_wait_all();
-  DBG_STAMP(13);
+  if (p.tma_store && warp >= 2 && lane == 0) tma_store_wait_all();
   tc_fence_before();
   cluster_sync_all();                                   // nobody deallocates while the pair's MMAs / loads are in flight
-  DBG_STAMP(14);
   if (warp == 1) {
     tc_fence_after();
     tmem_dealloc_2sm<TCOLS>(tmem_acc);
   }
-}
-
-// Bring-up aid only (SSCVAE_GEMM_DEBUG_SIMT=1): same contract on CUDA cores, one thread per output.
-__global__ void gemm_simt_debug_kernel(int M, int N, int nseg, GemmSeg s0, GemmSeg s1, GemmSeg s2, GemmEpi e) {
-  const int n = blockIdx.x * blockDim.x + threadIdx.x;
-  const int m = blockIdx.y;
-  if (n >= N || m >= M) return;
-  GemmSeg segs[3] = {s0, s1, s2};
-  float acc = 0.f;
-  for (int s = 0; s < nseg; ++s) {
-    const bf16* a = segs[s].A + (size_t)m * segs[s].lda;
-    const bf16* b = segs[s].B + (size_t)n * segs[s].ldb;
-    for (int k = 0; k < segs[s].K; ++k) acc += __bfloat162float(a[k]) * __bfloat162float(b[k]);
-  }
-  float x = acc * e.alpha;
-  if (e.bias) x += e.bias[n];
-  if (e.add1) x += e.add1[(size_t)m * e.ld1 + n];
-  if (e.add2) x += e.add2[(size_t)m * e.ld2 + n];
-  if (e.act == 1) x = tanhf(x);
-  if (e.dtanh) { float t = e.dtanh[(size_t)m * e.ldd + n]; x *= 1.0f - t * t; }
-  if (e.C32) { float* p = e.C32 + (size_t)m * e.ldc32 + n; *p = e.accumulate ? (*p + x) : x; }
-  if (e.C16) e.C16[(size_t)m * e.ldc16 + n] = __float2bfloat16_rn(x);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1164,14 +814,9 @@ static int encode_tmap_uncached(CUtensorMap* out, const bf16* base, int rows, in
   cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
   cuuint32_t box[2] = {(cuuint32_t)BK, (cuuint32_t)box_rows};
   cuuint32_t estr[2] = {1, 1};
-  static const CUtensorMapL2promotion promo = [] {
-    const char* e = getenv("SSCVAE_TMA_L2_PROMOTION");      // tuning knob: 0 none, 64, 128, 256
-    const int v = e ? atoi(e) : 256;
-    return v == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : v == 64 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
-         : v == 128 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
-  }();
   CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<bf16*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
     set_error("cuTensorMapEncodeTiled failed (%d) rows=%d K=%d ld=%d box_rows=%d", (int)r, rows, K, ld, box_rows);
     return SSCVAE_ERR_DRIVER;
@@ -1182,9 +827,8 @@ static int encode_tmap_uncached(CUtensorMap* out, const bf16* base, int rows, in
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 static bool tma_store_eligible(const GemmParams& prm) {
-  static const bool off = [] { const char* v = getenv("SSCVAE_GEMM_NO_TMA_STORE"); return v && v[0] == '1'; }();
   const GemmEpi& e = prm.epi;
-  return !off && prm.splits == 1 && e.C32 && !e.C16 && !e.act && !e.dtanh && !e.accumulate && !e.add1 && !e.add2 &&
+  return e.C32 && !e.C16 && !e.act && !e.dtanh && !e.accumulate && !e.add1 && !e.add2 &&
          aligned16(e.C32) && (e.ldc32 % 4) == 0 && (prm.N % 4) == 0 && (!e.bias || aligned16(e.bias));
   // N % 4: the TMA unit clips stores at 16-byte granularity (measured: with N = 77 the columns 77..79 were written)
 }
@@ -1213,30 +857,6 @@ static int encode_tmap_c32(CUtensorMap* out, const float* base, int rows, int co
   return 0;
 }
 
-// bf16 output tile map for TMA stores: box = 32 columns x 32 rows (64-byte rows), dense in shared memory
-static int encode_tmap_h16(CUtensorMap* out, const bf16* base, int rows, int cols, int ld) {
-  const TmapKey key{base, rows, cols, ld, -34};
-  std::lock_guard<std::mutex> lock(g_tmap_mutex);
-  auto it = g_tmap_cache.find(key);
-  if (it != g_tmap_cache.end()) { *out = it->second; return 0; }
-  EncodeTiledFn fn = get_encode_fn();
-  if (!fn) { set_error("cuTensorMapEncodeTiled not available from the driver"); return SSCVAE_ERR_DRIVER; }
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
-  cuuint32_t box[2] = {32, 32};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<bf16*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled (bf16 output) failed (%d) rows=%d cols=%d ld=%d", (int)r, rows, cols, ld);
-    return SSCVAE_ERR_DRIVER;
-  }
-  if (g_tmap_cache.size() > 8192) g_tmap_cache.clear();
-  g_tmap_cache.emplace(key, *out);
-  return 0;
-}
-
 template <int BN, int STAGES>
 static int launch_tc(cudaStream_t stream, GemmParams& prm, const GemmSeg* segs) {
   for (int s = 0; s < prm.nseg; ++s) {
@@ -1251,8 +871,9 @@ static int launch_tc(cudaStream_t stream, GemmParams& prm, const GemmSeg* segs) 
     CUDA_TRY(cudaFuncSetAttribute(gemm_tcgen05_kernel<BN, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     configured = true;
   }
-  dim3 grid(ceil_div(prm.N, BN), ceil_div(prm.M, BM), prm.splits);
-  CUDA_TRY(launch_pdl(gemm_tcgen05_kernel<BN, STAGES>, grid, dim3(GEMM_THREADS), smem, stream, prm));
+  dim3 grid(ceil_div(prm.N, BN), ceil_div(prm.M, BM));
+  gemm_tcgen05_kernel<BN, STAGES><<<grid, GEMM_THREADS, smem, stream>>>(prm);
+  CUDA_TRY(cudaGetLastError());
   ++g_launch_count;
   return 0;
 }
@@ -1271,44 +892,9 @@ static int launch_tc2(cudaStream_t stream, GemmParams& prm, const GemmSeg* segs)
     CUDA_TRY(cudaFuncSetAttribute(gemm_tcgen05_2cta_kernel<BN, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     configured = true;
   }
-  dim3 grid(2 * ceil_div(prm.N, BN), ceil_div(prm.M, 2 * BM), prm.splits);
-  CUDA_TRY(launch_pdl(gemm_tcgen05_2cta_kernel<BN, STAGES>, grid, dim3(GEMM_THREADS), smem, stream, prm));
-  ++g_launch_count;
-  return 0;
-}
-
-template <int STAGES>
-static int launch_swapped(cudaStream_t stream, GemmParams& prm, const GemmSeg* segs) {
-  for (int s = 0; s < prm.nseg; ++s) {
-    TRY(encode_tmap(&prm.ta[s], segs[s].A, prm.M, segs[s].K, segs[s].lda, 256));
-    TRY(encode_tmap(&prm.tb[s], segs[s].B, prm.N, segs[s].K, segs[s].ldb, 128));
-  }
-  const GemmEpi& e = prm.epi;
-  static const bool no_tma_store = [] { const char* v = getenv("SSCVAE_GEMM_NO_TMA_STORE"); return v && v[0] == '1'; }();
-  prm.tma_store = !no_tma_store && e.C32 && !e.C16 && !e.act && !e.dtanh && !e.accumulate && !e.add1 && !e.add2 &&
-                  aligned16(e.C32) && (e.ldc32 % 4) == 0 && (prm.N % 4) == 0;
-  if (prm.tma_store) TRY(encode_tmap_c32(&prm.tc, e.C32, prm.M, prm.N, e.ldc32, false));
-  constexpr int smem = 1024 + STAGES * (128 + 256) * BK * 2 + 256;
-  static bool configured = false;
-  if (!configured) {
-    CUDA_TRY(cudaFuncSetAttribute(gemm_tcgen05_swapped_kernel<STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    configured = true;
-  }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(ceil_div(prm.N, 128), 1, prm.splits);
-  cfg.blockDim = dim3(GEMM_THREADS, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = prm.splits;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  if (pdl_enabled()) {
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.numAttrs = 2;
-  }
-  CUDA_TRY(cudaLaunchKernelEx(&cfg, gemm_tcgen05_swapped_kernel<STAGES>, prm));
+  dim3 grid(2 * ceil_div(prm.N, BN), ceil_div(prm.M, 2 * BM));
+  gemm_tcgen05_2cta_kernel<BN, STAGES><<<grid, GEMM_THREADS, smem, stream>>>(prm);
+  CUDA_TRY(cudaGetLastError());
   ++g_launch_count;
   return 0;
 }
@@ -1361,127 +947,27 @@ static int launch_swapped_pair(cudaStream_t stream, GemmParams& prm, const GemmS
     TRY(encode_tmap(&prm.tb[s], segs[s].B, prm.N, segs[s].K, segs[s].ldb, 128));
   }
   const GemmEpi& e = prm.epi;
-  static const bool no_tma_store = [] { const char* v = getenv("SSCVAE_GEMM_NO_TMA_STORE"); return v && v[0] == '1'; }();
-  prm.tma_store = !no_tma_store && e.C32 && !e.C16 && !e.act && !e.dtanh && !e.accumulate && !e.add1 && !e.add2 &&
+  prm.tma_store = e.C32 && !e.C16 && !e.act && !e.dtanh && !e.accumulate && !e.add1 && !e.add2 &&
                   aligned16(e.C32) && (e.ldc32 % 4) == 0 && (prm.N % 4) == 0;
-  // The weights of the skinny GEMMs (76 MB per timestep) are streamed once per launch; marking them evict_first leaves
-  // L2 to the 52 MB of region features + projections the attention kernels re-read every step (measured: step
-  // 8.21 -> 8.08 ms, attention_fwd 25.1 -> 23.1 us). SSCVAE_W_EVICT_FIRST=0 turns the hint off.
-  static const bool w_evict_first = [] { const char* v = getenv("SSCVAE_W_EVICT_FIRST"); return !(v && v[0] == '0'); }();
-  prm.w_policy = w_evict_first ? 1 : 0;
-  prm.fuse_lstm = 0;
-  prm.lstm_tma = 0;
-  if (e.lstm) {
-    prm.fuse_lstm = 1;
-    prm.lstm = *e.lstm;
-    prm.tma_store = 0;
-    // outputs through TMA stores when every destination is 16-byte tileable (true for all training / decode buffers);
-    // the bf16 h destinations must have room for round_up(H, 32) columns (their K padding: Hp = round_up(H, 64))
-    const LstmFwdArgs& l = *e.lstm;
-    const int H = l.H, Hq = round_up(H, 32);
-    static const bool no_lstm_tma = [] { const char* v = getenv("SSCVAE_LSTM_TMA"); return v && v[0] == '0'; }();
-    bool ok = !no_lstm_tma && (H % 4) == 0 && aligned16(l.c_out) && (!l.gates_out || aligned16(l.gates_out));
-    ok = ok && (!l.h1_dst || (aligned16(l.h1_dst) && (l.ld_h1 % 8) == 0 && l.ld_h1 >= Hq));
-    ok = ok && (!l.h2_dst || (aligned16(l.h2_dst) && (l.ld_h2 % 8) == 0 && l.ld_h2 >= Hq));
-    if (ok) {
-      prm.lstm_tma = 1;
-      if (l.gates_out)
-        for (int k = 0; k < 4; ++k) TRY(encode_tmap_c32(&prm.tl[k], l.gates_out + (size_t)k * H, l.R, H, 4 * H, false));
-      TRY(encode_tmap_c32(&prm.tl[4], l.c_out, l.R, H, H, false));
-      if (l.h1_dst) TRY(encode_tmap_h16(&prm.tl[5], l.h1_dst, l.R, Hq, l.ld_h1));
-      if (l.h2_dst) TRY(encode_tmap_h16(&prm.tl[6], l.h2_dst, l.R, Hq, l.ld_h2));
-    }
-  }
   if (prm.tma_store) TRY(encode_tmap_c32(&prm.tc, e.C32, prm.M, prm.N, e.ldc32, false));
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(2 * pairs, 1, S);
   cfg.blockDim = dim3(GEMM_THREADS, 1, 1);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
+  cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
   attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = S;
   cfg.attrs = attr; cfg.numAttrs = 1;
-  if (pdl_enabled()) {
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.numAttrs = 2;
-  }
-  static const bool dbg = [] { const char* v = getenv("SSCVAE_GEMM_DBG"); return v && v[0] == '1'; }();
-  static long long* dbg_buf = nullptr;
-  if (dbg) {                                            // bring-up aid: phase stamps of a few CTAs, printed per launch
-    if (!dbg_buf) CUDA_TRY(cudaMalloc(&dbg_buf, 16 * 8 * 1024));
-    CUDA_TRY(cudaMemsetAsync(dbg_buf, 0, 16 * 8 * 1024, stream));
-    prm.dbg = dbg_buf;
-  }
   CUDA_TRY(cudaLaunchKernelEx(&cfg, gemm_tcgen05_swapped_pair_kernel<STAGES>, prm));
   ++g_launch_count;
-  if (dbg) {
-    static int printed = 0;
-    CUDA_TRY(cudaStreamSynchronize(stream));
-    std::vector<long long> h(16 * 2 * pairs * S);
-    CUDA_TRY(cudaMemcpy(h.data(), dbg_buf, h.size() * 8, cudaMemcpyDeviceToHost));
-    if (printed++ < 400) {
-      for (int cta : {0, 2 * pairs * S - 2}) {
-        fprintf(stderr, "[pairdbg] M=%d N=%d kb=%d S=%d fuse=%d tma=%d cta=%d:", prm.M, prm.N, total_kb, S, prm.fuse_lstm,
-                prm.fuse_lstm ? prm.lstm_tma : prm.tma_store, cta);
-        for (int i = 1; i < 15; ++i) fprintf(stderr, " %lld", h[cta * 16 + i] ? h[cta * 16 + i] - h[cta * 16] : -1);
-        fprintf(stderr, "\n");
-      }
-    }
-  }
   return 0;
-}
-
-int gemm_suggest_splits(int M, int N, int K_total) {
-  if (M > 256) return 1;
-  static int n_sm = 0;
-  if (n_sm == 0) {
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
-      n_sm = 148;
-  }
-  const int tiles = ceil_div(N, 128), kb = ceil_div(K_total, BK);
-  int s = 1;
-  while (s < 4 && tiles * s * 2 <= n_sm && kb >= 4 * s * 2) s *= 2;   // power of two: the cluster splits 256 columns
-  return s;
-}
-
-static bool pair_kernel_disabled() {
-  static const bool off = [] {
-    const char* a = getenv("SSCVAE_GEMM_PAIR");
-    const char* b = getenv("SSCVAE_GEMM_NO_SWAPPED");
-    const char* c = getenv("SSCVAE_GEMM_DEBUG_SIMT");
-    return (a && a[0] == '0') || (b && b[0] == '1') || (c && c[0] == '1');
-  }();
-  return off || getenv("SSCVAE_GEMM_FORCE") != nullptr;
 }
 
 int gemm_bf16_tn(cudaStream_t stream, int M, int N, int nseg, const GemmSeg* segs, const GemmEpi& epi) {
   REQUIRE(M > 0 && N > 0 && nseg >= 1 && nseg <= MAX_SEG, "gemm: bad shape M=%d N=%d nseg=%d", M, N, nseg);
   REQUIRE(epi.C32 || epi.C16 || (epi.rs && epi.rs->mode == 1), "gemm: no output");
-  if (epi.lstm) {
-    REQUIRE(N == lstm_gate_rows(epi.lstm->H) && epi.lstm->R == M, "gemm: fused LSTM shape mismatch (N=%d H=%d M=%d R=%d)", N,
-            epi.lstm->H, M, epi.lstm->R);
-    REQUIRE(epi.C32 && epi.ldc32 >= N && !epi.C16 && !epi.bias && !epi.add1 && !epi.add2 && !epi.act && !epi.dtanh && !epi.accumulate,
-            "gemm: fused LSTM takes a plain fp32 accumulator buffer");
-    // SSCVAE_LSTM_FUSE: 0 (default) = cell kernel behind the GEMM, 1 = fuse cells without per-row addend matrices
-    // (encoder / decoder LSTM), 2 = fuse every cell. Measured on B200 (bench27, ms per training step): 0: 7.45,
-    // 1: 7.49, 2: 7.61. Phase stamps (SSCVAE_GEMM_DBG=1) show why: the four epilogue warps run one per SM
-    // sub-partition with nothing to hide latency behind - ~170 cycles per global load, ~400 cycles per cell even with
-    // branch-free math - while the separate cell kernel is one wave of 57 600 threads that takes 4 us. The fused
-    // form stays as an opt-in for shapes where launches, not the epilogue, dominate.
-    static const int fuse_mode = [] { const char* e = getenv("SSCVAE_LSTM_FUSE"); return e ? atoi(e) : 0; }();
-    const bool heavy = epi.lstm->add1 || epi.lstm->add2;
-    if (M > 256 || fuse_mode == 0 || (fuse_mode == 1 && heavy) || pair_kernel_disabled()) {   // unfused: cell kernel behind
-      GemmEpi e2 = epi;
-      e2.lstm = nullptr;
-      TRY(gemm_bf16_tn(stream, M, N, nseg, segs, e2));
-      LstmFwdArgs l = *epi.lstm;
-      l.acc = epi.C32; l.ld_acc = epi.ldc32; l.perm = 1;
-      return lstm_forward(stream, l);
-    }
-  }
+  REQUIRE(epi.splits >= 0 && epi.splits <= 4, "gemm: pair split count %d (0..4)", epi.splits);
   double ksum = 0;
   for (int i = 0; i < nseg; ++i) ksum += segs[i].K;
   // instrumentation class: the skinny long-K GEMMs of the recurrence (the dominant kernel of a training step) are
@@ -1491,16 +977,6 @@ int gemm_bf16_tn(cudaStream_t stream, int M, int N, int nseg, const GemmSeg* seg
   const bool recurrent = M <= 256 && N >= 1024 && kb_all >= 16;
   PROF_SCOPE(stream, recurrent ? "gemm.recurrent" : epi.tag, 2.0 * M * N * ksum,
              2.0 * (M + N) * ksum + (epi.C32 ? 4.0 : 2.0) * M * N);
-  static const bool simt = [] { const char* e = getenv("SSCVAE_GEMM_DEBUG_SIMT"); return e && e[0] == '1'; }();
-  if (simt) {
-    GemmSeg z{nullptr, 0, nullptr, 0, 0};
-    dim3 grid(ceil_div(N, 128), M);
-    gemm_simt_debug_kernel<<<grid, 128, 0, stream>>>(M, N, nseg, segs[0], nseg > 1 ? segs[1] : z,
-                                                    nseg > 2 ? segs[2] : z, epi);
-    CUDA_TRY(cudaGetLastError());
-    ++g_launch_count;
-    return 0;
-  }
   GemmParams prm;
   memset(&prm, 0, sizeof(prm));
   prm.nseg = nseg; prm.M = M; prm.N = N; prm.epi = epi;
@@ -1519,21 +995,9 @@ int gemm_bf16_tn(cudaStream_t stream, int M, int N, int nseg, const GemmSeg* seg
   prm.vec = vec ? 1 : 0;
   int total_kb = 0;
   for (int s = 0; s < nseg; ++s) total_kb += prm.kblocks[s];
-  prm.splits = 1; prm.kb_per_split = total_kb;
-  // split-K: gridDim.z CTAs share one output tile, each adds its partial sum into C32 with vector reductions
-  // (red.global.add.v4.f32). Only for linear epilogues with an fp32 output; C32 is zeroed first unless accumulating.
-  auto use_splits = [&](int n) -> int {
-    if (n <= 1 || !epi.C32 || epi.C16 || epi.act || epi.dtanh) return 0;
-    n = std::min(n, std::max(1, total_kb / 2));
-    if (n <= 1) return 0;
-    prm.kb_per_split = ceil_div(total_kb, n);
-    prm.splits = ceil_div(total_kb, prm.kb_per_split);
-    if (!epi.accumulate)
-      CUDA_TRY(cudaMemset2DAsync(epi.C32, (size_t)epi.ldc32 * 4, 0, (size_t)N * 4, (size_t)M, stream));
-    return 0;
-  };
   if (epi.rs && epi.rs->mode) {                           // vocabulary head with softmax statistics / CE gradient in the epilogue
-    REQUIRE(!epi.add1 && !epi.add2 && !epi.act && !epi.dtanh && !epi.accumulate && !epi.lstm, "gemm: row statistics take a plain (alpha, bias) epilogue");
+    REQUIRE(!epi.add1 && !epi.add2 && !epi.act && !epi.dtanh && !epi.accumulate,
+            "gemm: row statistics take a plain (alpha, bias) epilogue");
     REQUIRE(epi.rs->mode != 1 || (epi.rs->st_max && epi.rs->st_sum && epi.rs->st_arg), "gemm: row statistics need their partial buffers");
     REQUIRE(epi.rs->mode != 2 || (epi.rs->lse && epi.rs->gcoef && epi.rs->target && epi.C16), "gemm: CE gradient needs lse, gcoef, target and a bf16 output");
     prm.tma_store = 0;
@@ -1548,63 +1012,21 @@ int gemm_bf16_tn(cudaStream_t stream, int M, int N, int nseg, const GemmSeg* seg
       CUDA_TRY(cudaFuncSetAttribute(gemm_tcgen05_kernel<128, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_rs));
       configured_rs = true;
     }
-    dim3 grid(ceil_div(q.N, 128), ceil_div(q.M, BM), 1);
-    CUDA_TRY(launch_pdl(gemm_tcgen05_kernel<128, 3>, grid, dim3(GEMM_THREADS), smem_rs, stream, q));
+    dim3 grid(ceil_div(q.N, 128), ceil_div(q.M, BM));
+    gemm_tcgen05_kernel<128, 3><<<grid, GEMM_THREADS, smem_rs, stream>>>(q);
+    CUDA_TRY(cudaGetLastError());
     ++g_launch_count;
     return 0;
   }
-  if (const char* e = getenv("SSCVAE_GEMM_SPLITK")) TRY(use_splits(atoi(e)));
-  static const bool no_swapped = [] { const char* e = getenv("SSCVAE_GEMM_NO_SWAPPED"); return e && e[0] == '1'; }();
-  // skinny and long-K (the per-timestep LSTM and BPTT GEMMs): swapped-operand cluster split-K. Measured on B200
-  // (tools/gemm_bench.py, GPU time inside a CUDA graph, us): 256x3600x4928: 17.0 vs 24.9 for the 128x64 tiling;
-  // 256x4160x3648: 16.0 vs 19.4; 256x1920x3648: 13.9 vs 18.8; short K (256x3600x1920: 12.6 vs 12.4) and narrow N
-  // (256x768x960: 10.2 vs 7.9) stay on the plain kernel.
-  const bool skinny = M <= 256 && N >= 1024 && total_kb >= 48;
-  // CTA-pair form (see the kernel): every skinny GEMM with enough weight rows, short K included (the attention-LSTM
-  // recurrence, K = 2Hp). SSCVAE_GEMM_PAIR=0 falls back to the single-CTA swapped kernel; epi.splits < 0 forces the
-  // pair kernel with K split -epi.splits (tools/gemm_bench.py, tests).
-  static const bool no_pair = [] { const char* e = getenv("SSCVAE_GEMM_PAIR"); return e && e[0] == '0'; }();
-  const bool pair_shape = M <= 256 && N >= 1024 && total_kb >= 16;
-  if ((epi.lstm || epi.splits < 0 || (epi.splits == 0 && pair_shape && !no_pair && !no_swapped)) && M <= 256 &&
-      !getenv("SSCVAE_GEMM_FORCE")) {
-    REQUIRE(epi.splits >= -4, "gemm: pair split count %d (1..4)", -epi.splits);
-    return launch_swapped_pair<6>(stream, prm, segs, epi.splits < 0 ? -epi.splits : 0);
-  }
-  if ((epi.splits > 0 || (skinny && !no_swapped)) && M <= 256 && !getenv("SSCVAE_GEMM_FORCE")) {
-    int S = epi.splits > 0 ? epi.splits : gemm_suggest_splits(M, N, total_kb * BK);
-    REQUIRE(S == 1 || S == 2 || S == 4, "gemm: split count %d (1, 2 or 4)", S);
-    while (S > 1 && total_kb < S) S /= 2;
-    prm.splits = S;
-    prm.kb_per_split = ceil_div(total_kb, S);
-    return launch_swapped<4>(stream, prm, segs);
-  }
+  // Skinny GEMMs with enough weight rows (the per-timestep LSTM and BPTT GEMMs, short K included: the attention-LSTM
+  // recurrence, K = 2Hp) run on the swapped-operand CTA-pair kernel (see the kernel); narrow N (256x768x960) stays on
+  // the plain kernel. epi.splits = 1..4 forces the pair kernel with that K split (tests, tools/gemm_bench.py).
+  const bool pair_shape = N >= 1024 && total_kb >= 16;
+  if (M <= 256 && (epi.splits > 0 || pair_shape)) return launch_swapped_pair<6>(stream, prm, segs, epi.splits);
   // The recurrent GEMMs have M = batch (two 128-row tiles) and stream their weights once: they are bound by
   // bytes in flight per SM, not by the tensor pipe. So: the widest N tile that still yields >= ~100 CTAs,
   // ~100 KB of TMA stages per CTA and two CTAs resident per SM (no wave-quantisation tail at 149..296 CTAs,
   // one CTA's epilogue overlaps the other's main loop).
-  if (const char* f = getenv("SSCVAE_GEMM_FORCE")) {      // tuning knob for tools/gemm_bench.py: "BN,STAGES"
-    int bn = 0, st = 0;
-    if (sscanf(f, "%d,%d", &bn, &st) == 2) {
-      if (bn == 256 && st == 4) return launch_tc<256, 4>(stream, prm, segs);
-      if (bn == 128 && st == 6) return launch_tc<128, 6>(stream, prm, segs);
-      if (bn == 128 && st == 3) return launch_tc<128, 3>(stream, prm, segs);
-      if (bn == 64 && st == 8) return launch_tc<64, 8>(stream, prm, segs);
-      if (bn == 64 && st == 4) return launch_tc<64, 4>(stream, prm, segs);
-      if (bn == 32 && st == 5) return launch_tc<32, 5>(stream, prm, segs);
-      if (bn == 32 && st == 10) return launch_tc<32, 10>(stream, prm, segs);
-      if (bn == 16 && st == 6) return launch_tc<16, 6>(stream, prm, segs);
-      // CTA-pair kernel: "2xBN,STAGES" is spelled with a leading 2 (e.g. 2256,6 = pair tile 256x256, 6 stages)
-      if (bn == 2256 && st == 6) return launch_tc2<256, 6>(stream, prm, segs);
-      if (bn == 2256 && st == 4) return launch_tc2<256, 4>(stream, prm, segs);
-      if (bn == 2128 && st == 8) return launch_tc2<128, 8>(stream, prm, segs);
-      if (bn == 2128 && st == 4) return launch_tc2<128, 4>(stream, prm, segs);
-      if (bn == 264 && st == 10) return launch_tc2<64, 10>(stream, prm, segs);
-      if (bn == 264 && st == 5) return launch_tc2<64, 5>(stream, prm, segs);
-      if (bn == 232 && st == 10) return launch_tc2<32, 10>(stream, prm, segs);
-      set_error("SSCVAE_GEMM_FORCE=%s: no such instantiation", f);
-      return SSCVAE_ERR_BAD_ARG;
-    }
-  }
   const long mt = ceil_div(M, BM);
   // large and long-K (the batched weight-gradient GEMMs): CTA pairs, 256x128 tiles (3600x2048x5376: 68 vs 76 us)
   if (M >= 1024 && N >= 512 && total_kb >= 32) return launch_tc2<128, 4>(stream, prm, segs);

@@ -155,8 +155,6 @@ int embed_gather_rows(cudaStream_t s, const int* tokens, int R, const bf16* embb
 __global__ void lstm_fwd_kernel(LstmFwdArgs a) {
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
   const int r = blockIdx.y;
-  pdl_wait();
-  pdl_launch_dependents(8);
   if (j >= a.H) return;
   const int H = a.H;
   const int r2 = a.rowmap ? a.rowmap[r] : r;
@@ -201,8 +199,6 @@ __device__ __forceinline__ void st_bf16x4(bf16* p, float a, float b, float c, fl
 __global__ void __launch_bounds__(128) lstm_fwd_v4_kernel(LstmFwdArgs a) {
   const int H = a.H, H4 = H >> 2;
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  pdl_wait();
-  pdl_launch_dependents(8);
   if (idx >= a.R * H4) return;
   const int r = idx / H4, j = (idx - r * H4) * 4;
   const int r2 = a.rowmap ? a.rowmap[r] : r;
@@ -248,10 +244,10 @@ int lstm_forward(cudaStream_t s, const LstmFwdArgs& a) {
                   (!a.c_prev || al16(a.c_prev)) && al16(a.c_out) && (!a.gates_out || al16(a.gates_out)) &&
                   (!a.h1_dst || (al8(a.h1_dst) && (a.ld_h1 % 4) == 0)) && (!a.h2_dst || (al8(a.h2_dst) && (a.ld_h2 % 4) == 0));
   if (v4) {
-    CUDA_TRY(launch_pdl(lstm_fwd_v4_kernel, dim3(ceil_div(a.R * (a.H / 4), 128)), dim3(128), 0, s, a));
+    lstm_fwd_v4_kernel<<<dim3(ceil_div(a.R * (a.H / 4), 128)), dim3(128), 0, s>>>(a);
   } else {
     dim3 grid(ceil_div(a.H, 128), a.R);
-    CUDA_TRY(launch_pdl(lstm_fwd_kernel, grid, dim3(128), 0, s, a));
+    lstm_fwd_kernel<<<grid, dim3(128), 0, s>>>(a);
   }
   LAUNCHED();
   return 0;
@@ -261,8 +257,6 @@ __global__ void lstm_bwd_kernel(LstmBwdArgs a) {
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
   const int r = blockIdx.y;
   const int H = a.H;
-  pdl_wait();
-  pdl_launch_dependents(8);
   if (j >= H) return;
   float dh = 0.f;
 #pragma unroll
@@ -287,8 +281,6 @@ __global__ void lstm_bwd_kernel(LstmBwdArgs a) {
 __global__ void __launch_bounds__(128) lstm_bwd_v4_kernel(LstmBwdArgs a) {
   const int H = a.H, H4 = H >> 2;
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  pdl_wait();
-  pdl_launch_dependents(8);
   int r, j;
   if (a.tiled) {
     // row-tiled state: a warp covers 8 rows x 4 unit-quads, so the tiled reads (8 consecutive rows = 128 contiguous
@@ -351,10 +343,10 @@ int lstm_backward(cudaStream_t s, const LstmBwdArgs& a) {
   REQUIRE(!a.tiled || v4, "lstm_backward: the row-tiled state layout needs H %% 4 == 0 and 16-byte aligned buffers");
   if (v4) {
     const int items = a.tiled ? ceil_div(a.R, 8) * ceil_div(a.H / 4, 4) * 32 : a.R * (a.H / 4);
-    CUDA_TRY(launch_pdl(lstm_bwd_v4_kernel, dim3(ceil_div(items, 128)), dim3(128), 0, s, a));
+    lstm_bwd_v4_kernel<<<dim3(ceil_div(items, 128)), dim3(128), 0, s>>>(a);
   } else {
     dim3 grid(ceil_div(a.H, 128), a.R);
-    CUDA_TRY(launch_pdl(lstm_bwd_kernel, grid, dim3(128), 0, s, a));
+    lstm_bwd_kernel<<<grid, dim3(128), 0, s>>>(a);
   }
   LAUNCHED();
   return 0;
@@ -377,8 +369,6 @@ __global__ void latent_fwd_train_kernel(LatentArgs a, const float* __restrict__ 
   __shared__ float red[32];
   const int r = blockIdx.x;
   const int Z = a.Z;
-  pdl_wait();
-  pdl_launch_dependents(8);
   const float pm_row = a.prior_mean_row ? a.prior_mean_row[a.rowmap ? a.rowmap[r] : r] : 0.f;
   const float log_pv = logf(a.prior_var);
   float part = 0.f;
@@ -415,8 +405,8 @@ int latent_forward_train(cudaStream_t s, const LatentArgs& a, const float* ml, i
                          float* logvar_out, float* eps_out, bf16* zb, int ld_z, float* kl_out) {
   PROF_SCOPE(s, "latent_fwd", 0, (double)a.R*a.Z*24.0);
   const int threads = min(256, round_up(a.Zp, 32));
-  CUDA_TRY(launch_pdl(latent_fwd_train_kernel, dim3(a.R), dim3(threads), 0, s, a, ml, ld_ml, bias_ml, eps_in, seed_dev, step,
-                      mean_out, logvar_out, eps_out, zb, ld_z, kl_out));
+  latent_fwd_train_kernel<<<dim3(a.R), dim3(threads), 0, s>>>(a, ml, ld_ml, bias_ml, eps_in, seed_dev, step, mean_out, logvar_out,
+                                                             eps_out, zb, ld_z, kl_out);
   LAUNCHED();
   return 0;
 }
@@ -425,8 +415,6 @@ __global__ void latent_fwd_eval_kernel(LatentArgs a, const float* __restrict__ e
                                        const unsigned long long* __restrict__ seed_dev, unsigned long long step, bf16* __restrict__ zb,
                                        int ld_z) {
   const int r = blockIdx.x;
-  pdl_wait();
-  pdl_launch_dependents(8);
   const float pm_row = a.prior_mean_row ? a.prior_mean_row[a.rowmap ? a.rowmap[r] : r] : 0.f;
   const float sd = sqrtf(a.prior_var);
   for (int z = threadIdx.x; z < a.Zp; z += blockDim.x) {
@@ -444,7 +432,7 @@ int latent_forward_eval(cudaStream_t s, const LatentArgs& a, const float* eps_in
                         const unsigned long long* seed_dev, unsigned long long step, bf16* zb, int ld_z) {
   PROF_SCOPE(s, "latent_fwd", 0, (double)a.R*a.Z*6.0);
   const int threads = min(256, round_up(a.Zp, 32));
-  CUDA_TRY(launch_pdl(latent_fwd_eval_kernel, dim3(a.R), dim3(threads), 0, s, a, eps_in, eps_row_stride, seed_dev, step, zb, ld_z));
+  latent_fwd_eval_kernel<<<dim3(a.R), dim3(threads), 0, s>>>(a, eps_in, eps_row_stride, seed_dev, step, zb, ld_z);
   LAUNCHED();
   return 0;
 }
@@ -455,8 +443,6 @@ __global__ void latent_bwd_kernel(LatentArgs a, const float* __restrict__ dz, in
                                   bf16* __restrict__ dml, int ld_dml) {
   const int r = blockIdx.x;
   const int Z = a.Z;
-  pdl_wait();
-  pdl_launch_dependents(8);
   const float pm_row = a.prior_mean_row ? a.prior_mean_row[a.rowmap ? a.rowmap[r] : r] : 0.f;
   const float w = gkld[r] * tmask_t[r];
   const float inv_pv = 1.0f / (a.prior_var + 0.00001f);
@@ -484,8 +470,8 @@ __global__ void latent_bwd_kernel(LatentArgs a, const float* __restrict__ dz, in
 int latent_backward(cudaStream_t s, const LatentArgs& a, const float* dz, int ld_dz, const float* eps, const float* mean,
                     const float* logvar, const float* gkld, const float* tmask_t, bf16* dml, int ld_dml) {
   PROF_SCOPE(s, "latent_bwd", 0, (double)a.R*a.Z*24.0);
-  CUDA_TRY(launch_pdl(latent_bwd_kernel, dim3(a.R), dim3(min(256, round_up(ld_dml, 32))), 0, s, a, dz, ld_dz, eps, mean, logvar,
-                      gkld, tmask_t, dml, ld_dml));
+  latent_bwd_kernel<<<dim3(a.R), dim3(min(256, round_up(ld_dml, 32))), 0, s>>>(a, dz, ld_dz, eps, mean, logvar, gkld, tmask_t, dml,
+                                                                              ld_dml);
   LAUNCHED();
   return 0;
 }
@@ -496,8 +482,6 @@ __global__ void prior_mean_fwd_kernel(const float* __restrict__ alpha, const flo
                                       bf16* __restrict__ c_dst, int ld_c, int cond) {
   extern __shared__ float al_s[];
   const int r = blockIdx.x;
-  pdl_wait();
-  pdl_launch_dependents(8);
   const int img = rowmap ? rowmap[r] : r;
   for (int n = threadIdx.x; n < N; n += blockDim.x) al_s[n] = alpha[(size_t)r * N + n];
   __syncthreads();
@@ -514,8 +498,8 @@ int prior_mean_forward(cudaStream_t s, const float* alpha, const float* obj, con
                        float* pm, bf16* c_dst, int ld_c, int cond) {
   PROF_SCOPE(s, "prior_mean", 0, (double)R * N * Z * 4.0);
   REQUIRE(cond >= 0 && cond <= Z, "prior_mean_forward: cond=%d out of range", cond);
-  CUDA_TRY(launch_pdl(prior_mean_fwd_kernel, dim3(R), dim3(min(256, round_up(Z, 32))), (size_t)N * sizeof(float), s, alpha, obj,
-                      rowmap, N, Z, pm, c_dst, ld_c, cond));
+  prior_mean_fwd_kernel<<<dim3(R), dim3(min(256, round_up(Z, 32))), (size_t)N * sizeof(float), s>>>(alpha, obj, rowmap, N, Z, pm,
+                                                                                                     c_dst, ld_c, cond);
   LAUNCHED();
   return 0;
 }
@@ -525,8 +509,6 @@ __global__ void prior_mean_bwd_kernel(int N, int Z, int cond, const float* __res
                                       float* __restrict__ dalpha) {
   extern __shared__ float dpm_s[];
   const int r = blockIdx.x;
-  pdl_wait();
-  pdl_launch_dependents(8);
   for (int z = threadIdx.x; z < Z; z += blockDim.x) {
     float v = dpm_kl[(size_t)r * Z + z];
     if (z < cond) v += dc_dec[(size_t)r * ld_dec + z] + dc_enc[(size_t)r * ld_enc + z];
@@ -546,8 +528,8 @@ __global__ void prior_mean_bwd_kernel(int N, int Z, int cond, const float* __res
 int prior_mean_backward(cudaStream_t s, int R, int N, int Z, int cond, const float* dpm_kl, const float* dc_dec, int ld_dec,
                         const float* dc_enc, int ld_enc, const float* obj, float* dalpha) {
   PROF_SCOPE(s, "prior_mean", 0, (double)R * N * Z * 4.0);
-  CUDA_TRY(launch_pdl(prior_mean_bwd_kernel, dim3(R), dim3(256), (size_t)Z * sizeof(float), s, N, Z, cond, dpm_kl, dc_dec, ld_dec,
-                      dc_enc, ld_enc, obj, dalpha));
+  prior_mean_bwd_kernel<<<dim3(R), dim3(256), (size_t)Z * sizeof(float), s>>>(N, Z, cond, dpm_kl, dc_dec, ld_dec, dc_enc, ld_enc, obj,
+                                                                               dalpha);
   LAUNCHED();
   return 0;
 }

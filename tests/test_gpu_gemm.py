@@ -11,7 +11,7 @@ pytestmark = pytest.mark.gpu
 SHAPES = [
     (128, 64, 64), (256, 3600, 1808), (256, 768, 904), (256, 300, 904), (5376, 3600, 600), (9216, 768, 2048),
     (37, 50, 72), (1, 8, 8), (300, 129, 1000), (3600, 1808, 5376), (256, 3856, 3600), (130, 10000, 600),
-    # skinny long-K -> swapped-operand cluster split-K kernel; large long-K -> CTA-pair kernel
+    # skinny (M <= 256, N >= 1024) -> swapped-operand CTA-pair kernel, cluster split-K; large long-K -> CTA-pair tiles
     (256, 3600, 4928), (200, 4160, 3648), (8, 1920, 3648), (3600, 2048, 5376), (1100, 520, 2100),
 ]
 
@@ -67,31 +67,12 @@ def test_tma_store_epilogue_matches_staged_epilogue(M, N, K):
     assert (outs[1] - ref).abs().max().item() <= 2e-3 * (K ** 0.5)
 
 
-@pytest.mark.parametrize("splits", [1, 2, 4])
-@pytest.mark.parametrize("M,N,K", [(256, 3600, 1920), (77, 1300, 4928), (256, 300, 960)])
-def test_swapped_cluster_splitk_kernel(M, N, K, splits):
-    """The swapped-operand kernel with a forced K split over a 1/2/4-CTA cluster (DSMEM reduce-scatter)."""
-    g = torch.Generator(device="cuda").manual_seed(M * 3 + N + K + splits)
-    A = torch.randn(M, K, device="cuda", generator=g).bfloat16()
-    B = torch.randn(N, K, device="cuda", generator=g).bfloat16()
-    bias = torch.randn(N, device="cuda", generator=g)
-    s = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-    for ldc in (N + 1, N + 4):
-        Cm = torch.full((M, ldc), -5.0, device="cuda")
-        _lib.check(_lib.lib().sscvae_test_gemm_splitk(_lib.ptr(A), K, _lib.ptr(B), K, M, N, K, _lib.ptr(Cm), ldc, splits,
-                                                      _lib.ptr(bias), s))
-        torch.cuda.synchronize()
-        ref = A.float() @ B.float().t() + bias
-        assert (Cm[:, :N] - ref).abs().max().item() <= 2e-3 * (K ** 0.5)
-        assert (Cm[:, N:] == -5.0).all()
-
-
 @pytest.mark.parametrize("splits", [1, 2, 3, 4])
 @pytest.mark.parametrize("M,N,K", [(256, 3600, 1920), (77, 1300, 4928), (256, 300, 960), (8, 4160, 3648), (129, 256, 512),
                                    (256, 7200, 3968)])
-def test_swapped_pair_kernel(M, N, K, splits):
+def test_swapped_pair_kernel_forced_split(M, N, K, splits):
     """The CTA-pair form of the swapped-operand kernel (tcgen05.mma.cta_group::2, cluster (2,1,S), DSMEM reduce-scatter),
-    forced with a negative split count; ragged weight rows (second CTA of the last pair fully out of range), batch rows
+    forced with a split count; ragged weight rows (second CTA of the last pair fully out of range), batch rows
     below one half tile, TMA-store and staged epilogues give the same bits."""
     g = torch.Generator(device="cuda").manual_seed(M * 3 + N + K + splits)
     A = torch.randn(M, K, device="cuda", generator=g).bfloat16()
@@ -102,7 +83,7 @@ def test_swapped_pair_kernel(M, N, K, splits):
     outs = []
     for ldc in (N + 1, N + 4):
         Cm = torch.full((M, ldc), -5.0, device="cuda")
-        _lib.check(_lib.lib().sscvae_test_gemm_splitk(_lib.ptr(A), K, _lib.ptr(B), K, M, N, K, _lib.ptr(Cm), ldc, -splits,
+        _lib.check(_lib.lib().sscvae_test_gemm_splitk(_lib.ptr(A), K, _lib.ptr(B), K, M, N, K, _lib.ptr(Cm), ldc, splits,
                                                       _lib.ptr(bias), s))
         torch.cuda.synchronize()
         assert (Cm[:, :N] - ref).abs().max().item() <= 2e-3 * (K ** 0.5)

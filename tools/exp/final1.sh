@@ -10,4 +10,3 @@ except Exception as e: print('$name', 'FAILED', e)
 PY
 }
 run k1 X=1
-run k1nofork SSCVAE_WGRAD_FORK=0

@@ -1,5 +1,6 @@
-"""Micro-benchmark of the tcgen05 GEMM at the shapes of the training step against cuBLAS (torch.matmul),
-over tile configurations (SSCVAE_GEMM_FORCE). Usage on the GPU box: python tools/gemm_bench.py [cfg ...]
+"""Micro-benchmark of the tcgen05 GEMM at the shapes of the training step against cuBLAS (torch.matmul): the
+library's own dispatch, plus the skinny-M CTA-pair kernel forced to a K split of N for every config pkN (N = 1..4).
+Usage on the GPU box: python tools/gemm_bench.py [pk1 pk2 pk3 pk4]
 
 Timing: ITERS launches back to back between two CUDA events with no Python in between (ours: the repeat loop of
 sscvae_test_gemm; cuBLAS: a captured CUDA graph), operands L2-resident."""
@@ -77,23 +78,13 @@ def main():
         ref = time_graph(lambda: torch.matmul(A, B.t()))
         line = f"{what:10s} {M}x{N}x{K}: cublas {ref:6.1f} us |"
         for cfg in configs:
-            os.environ.pop("SSCVAE_GEMM_SPLITK", None)
-            if cfg is None:
-                os.environ.pop("SSCVAE_GEMM_FORCE", None)
-            else:
-                force = cfg
-                if "/" in cfg:               # "BN,STAGES/splits"
-                    force, sp = cfg.split("/")
-                    os.environ["SSCVAE_GEMM_SPLITK"] = sp
-                os.environ["SSCVAE_GEMM_FORCE"] = force
             def fn():
                 st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
                 _lib.check(L.sscvae_test_gemm(_lib.ptr(A), K, _lib.ptr(B), K, M, N, K, _lib.ptr(Cm), N, None, 0, 0, st))
-            if cfg is not None and (cfg.startswith("sk") or cfg.startswith("pk")):
+            if cfg is not None:
                 if M > 256 or N < 256:
                     continue
-                os.environ.pop("SSCVAE_GEMM_FORCE", None)
-                S = int(cfg[2:]) * (-1 if cfg.startswith("pk") else 1)      # pkN: CTA-pair kernel, K split N
+                S = int(cfg[2:])                 # pkN: CTA-pair kernel, K split N
 
                 def fn():
                     st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
@@ -104,7 +95,6 @@ def main():
             except Exception:
                 line += f" [{cfg}] ERR"
         print(line, flush=True)
-    os.environ.pop("SSCVAE_GEMM_FORCE", None)
 
 
 if __name__ == "__main__":

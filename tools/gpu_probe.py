@@ -73,7 +73,7 @@ def train_probe(name):
 
 
 if __name__ == "__main__":
-    print("device", torch.cuda.get_device_name(0), "simt-debug", os.environ.get("SSCVAE_GEMM_DEBUG_SIMT"))
+    print("device", torch.cuda.get_device_name(0))
     try:
         gemm_probe()
     except Exception:
