@@ -1,11 +1,15 @@
 // tcgen05 / TMEM / TMA GEMM for sm_100a (see gemm.cuh for the contract).
 //
-// One CTA computes one 128 x BN output tile:
+// Three kernels: the tile kernel (one CTA per 128 x BN output tile), the CTA-pair tile kernel (a 2-CTA cluster per
+// 256 x BN tile) and the swapped-operand CTA-pair kernel of the skinny GEMMs. All three share one pipeline
+// (GemmSmem, gemm_setup, gemm_produce, gemm_mma, gemm_teardown), single-CTA or CTA-pair by a template parameter:
 //   warp 0      : TMA producer  (cp.async.bulk.tensor.2d, 128B-swizzled K-major tiles, mbarrier ring)
 //   warp 1      : TMEM allocator + single-thread tcgen05.mma issuer (kind::f16, bf16 in, fp32 accum in TMEM)
 //   warps 2..5  : epilogue: tcgen05.ld (32 lanes x 32 columns per instruction) -> registers ->
 //                 fused bias / addends / tanh / dtanh -> fp32 and/or bf16 global stores
-// The accumulator never touches registers or shared memory until the epilogue.
+// The accumulator never touches registers or shared memory until the epilogue. The two tile kernels share their
+// epilogue column loop (epilogue_tile); the swapped-pair kernel reduces its K splits through distributed shared memory
+// and has its own epilogue.
 #include "gemm.cuh"
 #include "prof.cuh"
 #include "ptx.cuh"
@@ -235,183 +239,284 @@ __device__ __forceinline__ void epilogue_row32(const GemmEpi e, int vec, int M, 
 }
 
 // ---------------------------------------------------------------------------------------------
-// the kernel
+// the pipeline shared by the three kernels: shared-memory ring, setup, TMA producer, MMA issuer, teardown
+// ---------------------------------------------------------------------------------------------
+// Dynamic shared memory: STAGES slot-0 tiles, STAGES slot-1 tiles, the ring's full / empty barriers, the accumulator
+// barrier and the TMEM base. bytes() is what the launcher requests (1024 bytes of alignment slack, 256 for the barriers).
+template <int STAGES, int BYTES0, int BYTES1>
+struct GemmSmem {
+  static constexpr int kStages = STAGES, kBytes0 = BYTES0, kBytes1 = BYTES1;
+  static_assert((2 * STAGES + 1) * 8 + 4 <= 256, "barriers and TMEM slot exceed their 256 bytes");
+  uint8_t* s0;             // [STAGES][BYTES0]
+  uint8_t* s1;             // [STAGES][BYTES1]
+  uint64_t* full;          // [STAGES]   TMA -> MMA
+  uint64_t* empty;         // [STAGES]   MMA -> TMA
+  uint64_t* accum;         // accumulator complete -> epilogue
+  uint32_t* tmem_slot;
+
+  static constexpr int bytes() { return 1024 + STAGES * (BYTES0 + BYTES1) + 256; }
+  // `smem`: the kernel's extern __shared__ __align__(1024) array; the 128B swizzle needs 1024-byte aligned tiles
+  __device__ __forceinline__ static GemmSmem carve(uint8_t* smem) {
+    if (threadIdx.x == 0 && (smem_u32(smem) & 1023u)) __trap();
+    GemmSmem sm;
+    sm.s0 = smem;
+    sm.s1 = smem + STAGES * BYTES0;
+    sm.full = reinterpret_cast<uint64_t*>(sm.s1 + STAGES * BYTES1);
+    sm.empty = sm.full + STAGES;
+    sm.accum = sm.empty + STAGES;
+    sm.tmem_slot = reinterpret_cast<uint32_t*>(sm.accum + 1);
+    return sm;
+  }
+  __device__ __forceinline__ void init_barriers() const {
+    for (int s = 0; s < STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
+    mbar_init(accum, 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+};
+
+template <int BN, int STAGES> using TileSmem = GemmSmem<STAGES, A_STAGE_BYTES, BN * BK * 2>;
+template <int BN, int STAGES> using PairTileSmem = GemmSmem<STAGES, A_STAGE_BYTES, BN / 2 * BK * 2>;  // half the B tile per CTA
+template <int STAGES> using SwappedSmem = GemmSmem<STAGES, 128 * BK * 2, 128 * BK * 2>;              // weights | activations
+
+__device__ __forceinline__ int total_kblocks(const GemmParams& p) {
+  int total = 0;
+#pragma unroll
+  for (int s = 0; s < MAX_SEG; ++s) total += (s < p.nseg) ? p.kblocks[s] : 0;
+  return total;
+}
+
+// PAIR: the CTA pair of a 2-cluster drives one 256-row tcgen05.mma.cta_group::2; otherwise one CTA, cta_group::1.
+// Thread 0 prefetches the operand maps and initialises the barriers, warp 1 allocates the accumulator; returns its TMEM
+// address once the CTA (PAIR: both CTAs, so that no remote arrival precedes the peer's barriers) has got this far.
+template <bool PAIR, int TMEM_COLS, class Smem>
+__device__ __forceinline__ uint32_t gemm_setup(const GemmParams& p, const Smem& sm, int warp) {
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < p.nseg; ++s) { prefetch_tmap(&p.ta[s]); prefetch_tmap(&p.tb[s]); }
+    sm.init_barriers();
+  }
+  if (warp == 1) {
+    if constexpr (PAIR) tmem_alloc_2sm<TMEM_COLS>(sm.tmem_slot);
+    else tmem_alloc<TMEM_COLS>(sm.tmem_slot);
+  }
+  tc_fence_before();
+  if constexpr (PAIR) cluster_sync_all();
+  else __syncthreads();
+  tc_fence_after();
+  return *sm.tmem_slot;
+}
+
+// TMA producer (one elected thread of warp 0) for k-blocks [kb_begin, kb_end) of the concatenated K segments: per
+// k-block the slot-0 tile (map0[s], rows from row0) and the slot-1 tile (map1[s], rows from row1) of its segment s.
+// PAIR: both CTAs load and the bytes land on the leader's `full` barrier, which alone expects them.
+// EVICT_FIRST0: the slot-0 tiles are loaded with an L2 evict_first hint.
+template <bool PAIR, bool EVICT_FIRST0, class Smem>
+__device__ __forceinline__ void gemm_produce(const GemmParams& p, const Smem& sm, const CUtensorMap* map0, int row0,
+                                             const CUtensorMap* map1, int row1, int kb_begin, int kb_end, bool leader) {
+  static_assert(PAIR || !EVICT_FIRST0, "the hinted load exists in the CTA-pair form only");
+  constexpr uint32_t TX = (PAIR ? 2 : 1) * (Smem::kBytes0 + Smem::kBytes1);
+  uint64_t pol = 0;
+  if constexpr (EVICT_FIRST0) pol = ptx::l2_policy_evict_first();
+  RingPos<Smem::kStages> pos;
+  // segment of the current k-block, its first global index and its two maps. The maps are generic addresses fixed once
+  // here (the empty asm): otherwise ptxas re-derives them from the kernel-parameter address after the `empty` wait, on
+  // the critical path of every k-block (measured: +0.2 us on a 15-k-block tile GEMM).
+  int s = 0, base = 0;
+  const CUtensorMap* t0 = map0;
+  const CUtensorMap* t1 = map1;
+  asm volatile("" : "+l"(t0), "+l"(t1));
+  for (int g = kb_begin; g < kb_end; ++g) {
+    while (g >= base + p.kblocks[s]) { base += p.kblocks[s]; ++s; ++t0; ++t1; }
+    const int kc = (g - base) * BK;
+    uint64_t* bar = &sm.full[pos.stage];
+    uint8_t* d0 = sm.s0 + pos.stage * Smem::kBytes0;
+    uint8_t* d1 = sm.s1 + pos.stage * Smem::kBytes1;
+    mbar_wait(&sm.empty[pos.stage], pos.phase ^ 1);
+    if (leader) mbar_expect_tx(bar, TX);
+    if constexpr (!PAIR) {
+      tma_load_2d(d0, t0, bar, kc, row0);
+      tma_load_2d(d1, t1, bar, kc, row1);
+    } else {
+      if constexpr (EVICT_FIRST0) tma_load_2d_2sm_hint(d0, t0, bar, kc, row0, pol);
+      else tma_load_2d_2sm(d0, t0, bar, kc, row0);
+      tma_load_2d_2sm(d1, t1, bar, kc, row1);
+    }
+    pos.advance();
+  }
+}
+
+// MMA issuer (one elected thread of warp 1; PAIR: of the leader CTA) for k-blocks [kb_begin, kb_end): D = slot-0 tile x
+// slot-1 tile^T into the accumulator at tmem_acc. A commit frees each stage once its MMAs have read it, a last one
+// reports the accumulator complete. PAIR: the commits arrive on the barriers of the cluster CTAs in `mask`.
+template <bool PAIR, class Smem>
+__device__ __forceinline__ void gemm_mma(const Smem& sm, uint32_t tmem_acc, uint32_t idesc, int kb_begin, int kb_end,
+                                         uint16_t mask = 3) {
+  RingPos<Smem::kStages> pos;
+  for (int kb = kb_begin; kb < kb_end; ++kb) {
+    mbar_wait(&sm.full[pos.stage], pos.phase);
+    tc_fence_after();
+    const uint32_t a_base = smem_u32(sm.s0 + pos.stage * Smem::kBytes0);
+    const uint32_t b_base = smem_u32(sm.s1 + pos.stage * Smem::kBytes1);
+#pragma unroll
+    for (int k = 0; k < BK / 16; ++k) {
+      // advance 16 elements (32 bytes) along K inside the 128B swizzle atom
+      const uint64_t ad = make_smem_desc(a_base + k * 32), bd = make_smem_desc(b_base + k * 32);
+      const uint32_t accumulate = (kb > kb_begin || k > 0) ? 1u : 0u;
+      if constexpr (PAIR) umma_bf16_2sm(tmem_acc, ad, bd, idesc, accumulate);
+      else umma_bf16(tmem_acc, ad, bd, idesc, accumulate);
+    }
+    if constexpr (PAIR) umma_commit_2sm(&sm.empty[pos.stage], mask);
+    else umma_commit(&sm.empty[pos.stage]);
+    pos.advance();
+  }
+  if constexpr (PAIR) umma_commit_2sm(sm.accum, mask);
+  else umma_commit(sm.accum);
+}
+
+// End of the kernel: the epilogue's TMA stores are complete, and nobody deallocates while MMAs, loads or (PAIR) the
+// peer's reads of its half of the accumulator are in flight.
+template <bool PAIR, int TMEM_COLS>
+__device__ __forceinline__ void gemm_teardown(const GemmParams& p, uint32_t tmem_acc, int warp) {
+  if (p.tma_store && warp >= 2 && (threadIdx.x & 31) == 0) tma_store_wait_all();
+  tc_fence_before();
+  if constexpr (PAIR) cluster_sync_all();
+  else __syncthreads();
+  if (warp == 1) {
+    tc_fence_after();
+    if constexpr (PAIR) tmem_dealloc_2sm<TMEM_COLS>(tmem_acc);
+    else tmem_dealloc<TMEM_COLS>(tmem_acc);
+  }
+}
+
+// Epilogue warps 2..5 of the two tile kernels; a warp may only touch TMEM lanes [32*(warp%4), +32): the tile rows from
+// m0 + 32*(warp%4). It walks the tile's columns 32 at a time; each block leaves through TMA stores or epilogue_row32.
+// ROW_STATS: the tile kernel's vocabulary-head branch (RowStatsEpi). smem0: the dead stage buffers.
+template <int BN, bool ROW_STATS>
+__device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t tmem_acc, uint64_t* accum, uint32_t smem0,
+                                              int m0, int n0) {
+  const int warp = threadIdx.x >> 5;
+  const int lane = threadIdx.x & 31;
+  const int q = warp & 3;
+  mbar_wait(accum, 0);
+  tc_fence_after();
+  const int row = m0 + q * 32 + lane;
+  // vocabulary head (RowStatsEpi): running softmax statistics of this thread's row over the tile's columns
+  const RowStatsEpi rs = ROW_STATS ? p.rs : RowStatsEpi();
+  float rs_m = -INFINITY, rs_s = 0.f, rs_t = 0.f; int rs_a = 0x7fffffff;
+  int rs_target = -1; float rs_lse = 0.f, rs_g = 0.f;
+  if (rs.mode && row < p.M) {
+    if (rs.target) rs_target = rs.target[row];
+    if (rs.mode == 2) { rs_lse = rs.lse[row]; rs_g = rs.gcoef[row]; }
+  }
+#pragma unroll 1
+  for (int c0 = 0; c0 < BN; c0 += 32) {
+    if (n0 + c0 >= p.N) break;                 // warp-uniform
+    uint32_t acc[32];
+    tmem_ld_32x32(tmem_acc + (static_cast<uint32_t>(q * 32) << 16) + c0, acc);
+    tmem_ld_wait();
+    if (rs.mode) {
+      // One warp per SM sub-partition runs this with nothing to hide latency behind: everything is written as
+      // independent operations + tree reductions (a running  s += exp(..)  chain cost ~120 cycles per element).
+      const int nb = n0 + c0;
+      const bool full = nb + 32 <= p.N;                     // warp-uniform: only the last tile has a ragged edge
+      float v[32];
+#pragma unroll
+      for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(acc[j]) * p.epi.alpha;
+      if (p.epi.bias) {
+#pragma unroll
+        for (int j = 0; j < 32; ++j)
+          if (full || nb + j < p.N) v[j] += p.epi.bias[nb + j];
+      }
+      if (!full) {
+#pragma unroll
+        for (int j = 0; j < 32; ++j)
+          if (nb + j >= p.N) v[j] = -INFINITY;              // exp -> 0, never the max
+      }
+      if (rs.mode == 1) {
+        float t[16];
+#pragma unroll
+        for (int j = 0; j < 16; ++j) t[j] = fmaxf(v[j], v[j + 16]);
+#pragma unroll
+        for (int w = 8; w > 0; w >>= 1)
+#pragma unroll
+          for (int j = 0; j < w; ++j) t[j] = fmaxf(t[j], t[j + w]);
+        const float cm = t[0];
+        if (cm > rs_m) {                       // strict: an earlier column / tile keeps the arg max on ties
+#pragma unroll
+          for (int j = 31; j >= 0; --j)
+            if (v[j] == cm) rs_a = nb + j;
+          rs_s *= exp2f((rs_m - cm) * 1.4426950408889634f);
+          rs_m = cm;
+        }
+        const float mb = rs_m * 1.4426950408889634f;
+        float e[32];
+#pragma unroll
+        for (int j = 0; j < 32; ++j) e[j] = exp2f(fmaf(v[j], 1.4426950408889634f, -mb));
+#pragma unroll
+        for (int w = 16; w > 0; w >>= 1)
+#pragma unroll
+          for (int j = 0; j < w; ++j) e[j] += e[j + w];
+        rs_s += e[0];
+        if (rs_target >= nb && rs_target < nb + 32) {
+#pragma unroll
+          for (int j = 0; j < 32; ++j)
+            if (nb + j == rs_target) rs_t = v[j];
+        }
+        if (!p.epi.C32 && !p.epi.C16) continue;      // statistics only: the logits are never written
+      } else {
+        const float lb = rs_lse * 1.4426950408889634f;
+#pragma unroll
+        for (int j = 0; j < 32; ++j) acc[j] = __float_as_uint(rs_g * exp2f(fmaf(v[j], 1.4426950408889634f, -lb)));
+        if (rs_target >= nb && rs_target < nb + 32) {
+#pragma unroll
+          for (int j = 0; j < 32; ++j)
+            if (nb + j == rs_target) acc[j] = __float_as_uint(__uint_as_float(acc[j]) - rs_g);
+        }
+        GemmEpi e2 = p.epi;
+        e2.alpha = 1.f; e2.bias = nullptr;
+        epilogue_row32(e2, p.vec, p.M, p.N, m0 + q * 32, n0 + c0, BN - c0 < 32 ? BN - c0 : 32, acc,
+                       smem0 + (warp - 2) * 32 * 36 * 4);
+        continue;
+      }
+    }
+    if (BN >= 32 && p.tma_store) {
+      epilogue_tma_row32(p.epi, &p.tc, p.N, m0 + q * 32, n0 + c0, acc, smem0 + (warp - 2) * 4096);
+    } else {
+      epilogue_row32(p.epi, p.vec, p.M, p.N, m0 + q * 32, n0 + c0, BN - c0 < 32 ? BN - c0 : 32, acc,
+                     smem0 + (warp - 2) * 32 * 36 * 4);
+    }
+  }
+  if (rs.mode == 1 && row < p.M) {             // partial statistics of (row, this 128-column tile): lanes = consecutive rows
+    const size_t o = (size_t)blockIdx.x * p.M + row;
+    rs.st_max[o] = rs_m; rs.st_sum[o] = rs_s; rs.st_arg[o] = rs_a;
+    if (rs.tgt_logit && rs_target >= n0 && rs_target < n0 + BN) rs.tgt_logit[row] = rs_t;
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
+// the tile kernel
 // ---------------------------------------------------------------------------------------------
 template <int BN, int STAGES>
 __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_tcgen05_kernel(const __grid_constant__ GemmParams p) {
-  constexpr int B_STAGE_BYTES = BN * BK * 2;
-  constexpr uint32_t IDESC = make_idesc(BM, BN);
   constexpr int TMEM_COLS = BN < 32 ? 32 : BN;          // allocation granularity: power of two >= 32
   extern __shared__ __align__(1024) uint8_t smem_raw[];
-  uint8_t* smem = smem_raw;                             // __align__(1024): the 128B swizzle needs 1024-byte aligned tiles
-  if (threadIdx.x == 0 && (smem_u32(smem) & 1023u)) __trap();
-  uint8_t* smem_a = smem;
-  uint8_t* smem_b = smem + STAGES * A_STAGE_BYTES;
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem_b + STAGES * B_STAGE_BYTES);
-  uint64_t* empty_bar = full_bar + STAGES;
-  uint64_t* accum_bar = empty_bar + STAGES;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(accum_bar + 1);
+  const auto sm = TileSmem<BN, STAGES>::carve(smem_raw);
 
   const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
   const int m0 = blockIdx.y * BM;
   const int n0 = blockIdx.x * BN;
-
-  int total_kb = 0;
-#pragma unroll
-  for (int s = 0; s < MAX_SEG; ++s) total_kb += (s < p.nseg) ? p.kblocks[s] : 0;
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < p.nseg; ++s) { prefetch_tmap(&p.ta[s]); prefetch_tmap(&p.tb[s]); }
-    for (int s = 0; s < STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
-    mbar_init(accum_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) tmem_alloc<TMEM_COLS>(tmem_slot);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_acc = *tmem_slot;
+  const int total_kb = total_kblocks(p);
+  const uint32_t tmem_acc = gemm_setup<false, TMEM_COLS>(p, sm, warp);
 
   if (warp == 0) {
-    if (elect_one_sync()) {
-      int stage = 0; uint32_t phase = 0;
-      int s = 0, base = 0;                              // segment of the current k-block, its first global index
-      for (int g = 0; g < total_kb; ++g) {
-        while (g >= base + p.kblocks[s]) { base += p.kblocks[s]; ++s; }
-        const int kb = g - base;
-        mbar_wait(&empty_bar[stage], phase ^ 1);
-        mbar_expect_tx(&full_bar[stage], A_STAGE_BYTES + B_STAGE_BYTES);
-        tma_load_2d(smem_a + stage * A_STAGE_BYTES, &p.ta[s], &full_bar[stage], kb * BK, m0);
-        tma_load_2d(smem_b + stage * B_STAGE_BYTES, &p.tb[s], &full_bar[stage], kb * BK, n0);
-        if (++stage == STAGES) { stage = 0; phase ^= 1; }
-      }
-    }
+    if (elect_one_sync()) gemm_produce<false, false>(p, sm, p.ta, m0, p.tb, n0, 0, total_kb, true);
+    __syncwarp();
   } else if (warp == 1) {
-    if (elect_one_sync()) {
-      int stage = 0; uint32_t phase = 0;
-      for (int kb = 0; kb < total_kb; ++kb) {
-        mbar_wait(&full_bar[stage], phase);
-        tc_fence_after();
-        const uint32_t a_base = smem_u32(smem_a + stage * A_STAGE_BYTES);
-        const uint32_t b_base = smem_u32(smem_b + stage * B_STAGE_BYTES);
-#pragma unroll
-        for (int k = 0; k < BK / 16; ++k) {
-          // advance 16 elements (32 bytes) along K inside the 128B swizzle atom
-          umma_bf16(tmem_acc, make_smem_desc(a_base + k * 32), make_smem_desc(b_base + k * 32), IDESC,
-                    (kb > 0 || k > 0) ? 1u : 0u);
-        }
-        umma_commit(&empty_bar[stage]);          // frees the smem slot once these MMAs have read it
-        if (++stage == STAGES) { stage = 0; phase ^= 1; }
-      }
-      umma_commit(accum_bar);                    // accumulator complete -> epilogue
-    }
+    if (elect_one_sync()) gemm_mma<false>(sm, tmem_acc, make_idesc(BM, BN), 0, total_kb);
     __syncwarp();
   } else {
-    // epilogue warps 2..5; a warp may only touch TMEM lanes [32*(warp%4), +32)
-    const int q = warp & 3;
-    mbar_wait(accum_bar, 0);
-    tc_fence_after();
-    const int row = m0 + q * 32 + lane;
-    // vocabulary head (RowStatsEpi): running softmax statistics of this thread's row over the tile's columns
-    const RowStatsEpi rs = p.rs;
-    float rs_m = -INFINITY, rs_s = 0.f, rs_t = 0.f; int rs_a = 0x7fffffff;
-    int rs_target = -1; float rs_lse = 0.f, rs_g = 0.f;
-    if (rs.mode && row < p.M) {
-      if (rs.target) rs_target = rs.target[row];
-      if (rs.mode == 2) { rs_lse = rs.lse[row]; rs_g = rs.gcoef[row]; }
-    }
-#pragma unroll 1
-    for (int c0 = 0; c0 < BN; c0 += 32) {
-      if (n0 + c0 >= p.N) break;                 // warp-uniform
-      uint32_t acc[32];
-      tmem_ld_32x32(tmem_acc + (static_cast<uint32_t>(q * 32) << 16) + c0, acc);
-      tmem_ld_wait();
-      if (rs.mode) {
-        // One warp per SM sub-partition runs this with nothing to hide latency behind: everything is written as
-        // independent operations + tree reductions (a running  s += exp(..)  chain cost ~120 cycles per element).
-        const int nb = n0 + c0;
-        const bool full = nb + 32 <= p.N;                     // warp-uniform: only the last tile has a ragged edge
-        float v[32];
-#pragma unroll
-        for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(acc[j]) * p.epi.alpha;
-        if (p.epi.bias) {
-#pragma unroll
-          for (int j = 0; j < 32; ++j)
-            if (full || nb + j < p.N) v[j] += p.epi.bias[nb + j];
-        }
-        if (!full) {
-#pragma unroll
-          for (int j = 0; j < 32; ++j)
-            if (nb + j >= p.N) v[j] = -INFINITY;              // exp -> 0, never the max
-        }
-        if (rs.mode == 1) {
-          float t[16];
-#pragma unroll
-          for (int j = 0; j < 16; ++j) t[j] = fmaxf(v[j], v[j + 16]);
-#pragma unroll
-          for (int w = 8; w > 0; w >>= 1)
-#pragma unroll
-            for (int j = 0; j < w; ++j) t[j] = fmaxf(t[j], t[j + w]);
-          const float cm = t[0];
-          if (cm > rs_m) {                       // strict: an earlier column / tile keeps the arg max on ties
-#pragma unroll
-            for (int j = 31; j >= 0; --j)
-              if (v[j] == cm) rs_a = nb + j;
-            rs_s *= exp2f((rs_m - cm) * 1.4426950408889634f);
-            rs_m = cm;
-          }
-          const float mb = rs_m * 1.4426950408889634f;
-          float e[32];
-#pragma unroll
-          for (int j = 0; j < 32; ++j) e[j] = exp2f(fmaf(v[j], 1.4426950408889634f, -mb));
-#pragma unroll
-          for (int w = 16; w > 0; w >>= 1)
-#pragma unroll
-            for (int j = 0; j < w; ++j) e[j] += e[j + w];
-          rs_s += e[0];
-          if (rs_target >= nb && rs_target < nb + 32) {
-#pragma unroll
-            for (int j = 0; j < 32; ++j)
-              if (nb + j == rs_target) rs_t = v[j];
-          }
-          if (!p.epi.C32 && !p.epi.C16) continue;      // statistics only: the logits are never written
-        } else {
-          const float lb = rs_lse * 1.4426950408889634f;
-#pragma unroll
-          for (int j = 0; j < 32; ++j) acc[j] = __float_as_uint(rs_g * exp2f(fmaf(v[j], 1.4426950408889634f, -lb)));
-          if (rs_target >= nb && rs_target < nb + 32) {
-#pragma unroll
-            for (int j = 0; j < 32; ++j)
-              if (nb + j == rs_target) acc[j] = __float_as_uint(__uint_as_float(acc[j]) - rs_g);
-          }
-          GemmEpi e2 = p.epi;
-          e2.alpha = 1.f; e2.bias = nullptr;
-          epilogue_row32(e2, p.vec, p.M, p.N, m0 + q * 32, n0 + c0, BN - c0 < 32 ? BN - c0 : 32, acc,
-                         smem_u32(smem_a) + (warp - 2) * 32 * 36 * 4);
-          continue;
-        }
-      }
-      if (BN >= 32 && p.tma_store) {
-        epilogue_tma_row32(p.epi, &p.tc, p.N, m0 + q * 32, n0 + c0, acc, smem_u32(smem_a) + (warp - 2) * 4096);
-      } else {
-        epilogue_row32(p.epi, p.vec, p.M, p.N, m0 + q * 32, n0 + c0, BN - c0 < 32 ? BN - c0 : 32, acc,
-                       smem_u32(smem_a) + (warp - 2) * 32 * 36 * 4);
-      }
-    }
-    if (rs.mode == 1 && row < p.M) {             // partial statistics of (row, this 128-column tile): lanes = consecutive rows
-      const size_t o = (size_t)blockIdx.x * p.M + row;
-      rs.st_max[o] = rs_m; rs.st_sum[o] = rs_s; rs.st_arg[o] = rs_a;
-      if (rs.tgt_logit && rs_target >= n0 && rs_target < n0 + BN) rs.tgt_logit[row] = rs_t;
-    }
+    epilogue_tile<BN, true>(p, tmem_acc, sm.accum, smem_u32(smem_raw), m0, n0);
   }
-  if (p.tma_store && warp >= 2 && (threadIdx.x & 31) == 0) tma_store_wait_all();
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc<TMEM_COLS>(tmem_acc);
-  }
+  gemm_teardown<false, TMEM_COLS>(p, tmem_acc, warp);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -424,99 +529,27 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_tcgen05_kernel(const __g
 template <int BN, int STAGES>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GEMM_THREADS, 1)
 gemm_tcgen05_2cta_kernel(const __grid_constant__ GemmParams p) {
-  constexpr int BH = BN / 2;                              // B rows loaded by each CTA
-  constexpr int B_STAGE_BYTES = BH * BK * 2;
-  constexpr uint32_t IDESC = make_idesc(2 * BM, BN);
   constexpr int TMEM_COLS = BN < 32 ? 32 : BN;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
-  uint8_t* smem = smem_raw;                             // __align__(1024): the 128B swizzle needs 1024-byte aligned tiles
-  if (threadIdx.x == 0 && (smem_u32(smem) & 1023u)) __trap();
-  uint8_t* smem_a = smem;
-  uint8_t* smem_b = smem + STAGES * A_STAGE_BYTES;
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem_b + STAGES * B_STAGE_BYTES);
-  uint64_t* empty_bar = full_bar + STAGES;
-  uint64_t* accum_bar = empty_bar + STAGES;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(accum_bar + 1);
+  const auto sm = PairTileSmem<BN, STAGES>::carve(smem_raw);
 
   const int warp = threadIdx.x >> 5;
   const uint32_t rank = cluster_ctarank();
   const int m0 = blockIdx.y * (2 * BM) + (int)rank * BM;
   const int n0 = (blockIdx.x >> 1) * BN;
-
-  int total_kb = 0;
-#pragma unroll
-  for (int s = 0; s < MAX_SEG; ++s) total_kb += (s < p.nseg) ? p.kblocks[s] : 0;
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < p.nseg; ++s) { prefetch_tmap(&p.ta[s]); prefetch_tmap(&p.tb[s]); }
-    for (int s = 0; s < STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
-    mbar_init(accum_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) tmem_alloc_2sm<TMEM_COLS>(tmem_slot);
-  tc_fence_before();
-  cluster_sync_all();                                     // both CTAs' barriers exist before any remote arrival
-  tc_fence_after();
-  const uint32_t tmem_acc = *tmem_slot;
+  const int total_kb = total_kblocks(p);
+  const uint32_t tmem_acc = gemm_setup<true, TMEM_COLS>(p, sm, warp);
 
   if (warp == 0) {
-    if (elect_one_sync()) {
-      int stage = 0; uint32_t phase = 0;
-      int s = 0, base = 0;
-      for (int g = 0; g < total_kb; ++g) {
-        while (g >= base + p.kblocks[s]) { base += p.kblocks[s]; ++s; }
-        const int kb = g - base;
-        mbar_wait(&empty_bar[stage], phase ^ 1);
-        if (rank == 0) mbar_expect_tx(&full_bar[stage], 2 * (A_STAGE_BYTES + B_STAGE_BYTES));
-        tma_load_2d_2sm(smem_a + stage * A_STAGE_BYTES, &p.ta[s], &full_bar[stage], kb * BK, m0);
-        tma_load_2d_2sm(smem_b + stage * B_STAGE_BYTES, &p.tb[s], &full_bar[stage], kb * BK, n0 + (int)rank * BH);
-        if (++stage == STAGES) { stage = 0; phase ^= 1; }
-      }
-    }
+    if (elect_one_sync()) gemm_produce<true, false>(p, sm, p.ta, m0, p.tb, n0 + (int)rank * (BN / 2), 0, total_kb, rank == 0);
+    __syncwarp();
   } else if (warp == 1) {
-    if (rank == 0 && elect_one_sync()) {
-      int stage = 0; uint32_t phase = 0;
-      for (int kb = 0; kb < total_kb; ++kb) {
-        mbar_wait(&full_bar[stage], phase);
-        tc_fence_after();
-        const uint32_t a_base = smem_u32(smem_a + stage * A_STAGE_BYTES);
-        const uint32_t b_base = smem_u32(smem_b + stage * B_STAGE_BYTES);
-#pragma unroll
-        for (int k = 0; k < BK / 16; ++k) {
-          umma_bf16_2sm(tmem_acc, make_smem_desc(a_base + k * 32), make_smem_desc(b_base + k * 32), IDESC,
-                        (kb > 0 || k > 0) ? 1u : 0u);
-        }
-        umma_commit_2sm(&empty_bar[stage]);
-        if (++stage == STAGES) { stage = 0; phase ^= 1; }
-      }
-      umma_commit_2sm(accum_bar);
-    }
+    if (rank == 0 && elect_one_sync()) gemm_mma<true>(sm, tmem_acc, make_idesc(2 * BM, BN), 0, total_kb);
     __syncwarp();
   } else {
-    const int q = warp & 3;
-    mbar_wait(accum_bar, 0);
-    tc_fence_after();
-#pragma unroll 1
-    for (int c0 = 0; c0 < BN; c0 += 32) {
-      if (n0 + c0 >= p.N) break;
-      uint32_t acc[32];
-      tmem_ld_32x32(tmem_acc + (static_cast<uint32_t>(q * 32) << 16) + c0, acc);
-      tmem_ld_wait();
-      if (BN >= 32 && p.tma_store) {
-        epilogue_tma_row32(p.epi, &p.tc, p.N, m0 + q * 32, n0 + c0, acc, smem_u32(smem_a) + (warp - 2) * 4096);
-      } else {
-        epilogue_row32(p.epi, p.vec, p.M, p.N, m0 + q * 32, n0 + c0, BN - c0 < 32 ? BN - c0 : 32, acc,
-                       smem_u32(smem_a) + (warp - 2) * 32 * 36 * 4);
-      }
-    }
+    epilogue_tile<BN, false>(p, tmem_acc, sm.accum, smem_u32(smem_raw), m0, n0);
   }
-  if (p.tma_store && warp >= 2 && (threadIdx.x & 31) == 0) tma_store_wait_all();
-  tc_fence_before();
-  cluster_sync_all();                                     // the peer may still be reading its half of the accumulator
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc_2sm<TMEM_COLS>(tmem_acc);
-  }
+  gemm_teardown<true, TMEM_COLS>(p, tmem_acc, warp);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -588,29 +621,12 @@ __device__ __forceinline__ void epilogue_swapped32(const GemmEpi e, int vec, int
   __syncwarp();
 }
 
-__device__ __forceinline__ void umma_commit_2sm_mask(uint64_t* bar, uint16_t mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-          smem_u32(bar)),
-      "h"(mask)
-      : "memory");
-}
-
 template <int STAGES>
 __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_pair_kernel(const __grid_constant__ GemmParams p) {
   constexpr int BW = 128, BXH = 128;                    // weight rows per CTA (half of UMMA M), batch rows LOADED per CTA
-  constexpr int W_STAGE_BYTES = BW * BK * 2, X_STAGE_BYTES = BXH * BK * 2;
-  constexpr uint32_t IDESC = make_idesc(2 * BW, 2 * BXH);
   constexpr int TCOLS = 2 * BXH;                        // accumulator: 128 lanes (this CTA's weight rows) x 256 batch rows
   extern __shared__ __align__(1024) uint8_t smem_raw[];
-  uint8_t* smem = smem_raw;
-  if (threadIdx.x == 0 && (smem_u32(smem) & 1023u)) __trap();
-  uint8_t* smem_w = smem;
-  uint8_t* smem_x = smem + STAGES * W_STAGE_BYTES;
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem_x + STAGES * X_STAGE_BYTES);
-  uint64_t* empty_bar = full_bar + STAGES;
-  uint64_t* accum_bar = empty_bar + STAGES;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(accum_bar + 1);
+  const auto sm = SwappedSmem<STAGES>::carve(smem_raw);
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -619,71 +635,30 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_pair_ker
   const int rank = blockIdx.z;                          // K split of this CTA (cluster z == grid z)
   const int n0 = (blockIdx.x >> 1) * (2 * BW) + xr * BW;   // first weight row (output column) of this CTA
 
-  int total_kb = 0;
-#pragma unroll
-  for (int s = 0; s < MAX_SEG; ++s) total_kb += (s < p.nseg) ? p.kblocks[s] : 0;
+  const int total_kb = total_kblocks(p);
   const int kb_begin = rank * p.kb_per_split;
   const int kb_end = min(total_kb, kb_begin + p.kb_per_split);
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < p.nseg; ++s) { prefetch_tmap(&p.ta[s]); prefetch_tmap(&p.tb[s]); }
-    for (int s = 0; s < STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
-    mbar_init(accum_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) tmem_alloc_2sm<TCOLS>(tmem_slot);
-  tc_fence_before();
-  cluster_sync_all();                                   // the peer's barriers exist before any remote arrival
-  tc_fence_after();
-  const uint32_t tmem_acc = *tmem_slot;
+  const uint32_t tmem_acc = gemm_setup<true, TCOLS>(p, sm, warp);
   const int CW = S == 1 ? 256 : S == 2 ? 128 : S == 3 ? 96 : 64;   // batch columns owned by each K split
 
   if (warp == 0) {
-    if (elect_one_sync()) {
-      int stage = 0; uint32_t phase = 0;
-      int s = 0, base = 0;
-      // The weights of the skinny GEMMs (76 MB per timestep) are streamed once per launch; marking them evict_first
-      // leaves L2 to the 52 MB of region features + projections the attention kernels re-read every step (measured:
-      // step 8.21 -> 8.08 ms, attention_fwd 25.1 -> 23.1 us).
-      const uint64_t w_pol = ptx::l2_policy_evict_first();
-      for (int g = kb_begin; g < kb_end; ++g) {
-        while (g >= base + p.kblocks[s]) { base += p.kblocks[s]; ++s; }
-        const int kb = g - base;
-        mbar_wait(&empty_bar[stage], phase ^ 1);
-        if (xr == 0) mbar_expect_tx(&full_bar[stage], 2 * (W_STAGE_BYTES + X_STAGE_BYTES));
-        tma_load_2d_2sm_hint(smem_w + stage * W_STAGE_BYTES, &p.tb[s], &full_bar[stage], kb * BK, n0, w_pol);
-        tma_load_2d_2sm(smem_x + stage * X_STAGE_BYTES, &p.ta[s], &full_bar[stage], kb * BK, xr * BXH);
-        if (++stage == STAGES) { stage = 0; phase ^= 1; }
-      }
-    }
+    // The weights of the skinny GEMMs (76 MB per timestep) are streamed once per launch; marking them evict_first
+    // leaves L2 to the 52 MB of region features + projections the attention kernels re-read every step (measured:
+    // step 8.21 -> 8.08 ms, attention_fwd 25.1 -> 23.1 us).
+    if (elect_one_sync()) gemm_produce<true, true>(p, sm, p.tb, n0, p.ta, xr * BXH, kb_begin, kb_end, xr == 0);
     __syncwarp();
   } else if (warp == 1) {
-    if (xr == 0 && elect_one_sync()) {
-      const uint16_t pair_mask = static_cast<uint16_t>(3u << (2 * rank));
-      int stage = 0; uint32_t phase = 0;
-      for (int kb = kb_begin; kb < kb_end; ++kb) {
-        mbar_wait(&full_bar[stage], phase);
-        tc_fence_after();
-        const uint32_t w_base = smem_u32(smem_w + stage * W_STAGE_BYTES);
-        const uint32_t x_base = smem_u32(smem_x + stage * X_STAGE_BYTES);
-#pragma unroll
-        for (int k = 0; k < BK / 16; ++k)
-          umma_bf16_2sm(tmem_acc, make_smem_desc(w_base + k * 32), make_smem_desc(x_base + k * 32), IDESC,
-                        (kb > kb_begin || k > 0) ? 1u : 0u);
-        umma_commit_2sm_mask(&empty_bar[stage], pair_mask);
-        if (++stage == STAGES) { stage = 0; phase ^= 1; }
-      }
-      umma_commit_2sm_mask(accum_bar, pair_mask);
-    }
+    if (xr == 0 && elect_one_sync())
+      gemm_mma<true>(sm, tmem_acc, make_idesc(2 * BW, 2 * BXH), kb_begin, kb_end, static_cast<uint16_t>(3u << (2 * rank)));
     __syncwarp();
   } else {
-    mbar_wait(accum_bar, 0);                            // this pair's partial tile is complete in both CTAs' TMEM
+    mbar_wait(sm.accum, 0);                             // this pair's partial tile is complete in both CTAs' TMEM
     tc_fence_after();
   }
 
   const int q = warp & 3;                               // epilogue warps 2..5 own TMEM lanes [32q, 32q+32)
   const int tl = q * 32 + lane;                         // TMEM lane = column n0 + tl of the output
-  float* recv = reinterpret_cast<float*>(smem);         // [(S-1) sources][CW columns][128 lanes], over the dead stages
+  const uint32_t recv = smem_u32(smem_raw);             // [(S-1) sources][CW columns][128 lanes] fp32, over the dead stages
   // every CTA of the cluster has finished its main loop (stage buffers dead, also the ones the PEER's MMAs read)
   cluster_sync_all();
   if (S > 1) {
@@ -691,7 +666,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_pair_ker
       for (int o = 0; o < S; ++o) {
         if (o == rank) continue;
         const int slot = rank < o ? rank : rank - 1;
-        const uint32_t rbase = mapa_shared(smem_u32(recv), (uint32_t)(xr + 2 * o));
+        const uint32_t rbase = mapa_shared(recv, (uint32_t)(xr + 2 * o));
         for (int c = 0; c < CW; c += 32) {
           if (o * CW + c >= p.M || o * CW + c >= TCOLS) break;   // columns beyond the batch are never read
           uint32_t acc[32];
@@ -725,10 +700,10 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_pair_ker
         if (o == rank || o * p.kb_per_split >= total_kb) continue;
         const int slot = o < rank ? o : o - 1;
 #pragma unroll
-        for (int j = 0; j < 32; ++j) v[j] += lds_f32(smem_u32(recv) + (uint32_t)(((slot * CW + c + j) * 128 + tl) * 4));
+        for (int j = 0; j < 32; ++j) v[j] += lds_f32(recv + (uint32_t)(((slot * CW + c + j) * 128 + tl) * 4));
       }
       if (p.tma_store) {
-        const uint32_t st = smem_u32(smem) + 96 * 1024 + (warp - 2) * 4096;
+        const uint32_t st = smem_u32(smem_raw) + 96 * 1024 + (warp - 2) * 4096;
         const float bias = (epi.bias && n0 + tl < p.N) ? epi.bias[n0 + tl] : 0.f;
         if (lane == 0) tma_store_wait_read();
         __syncwarp();
@@ -739,26 +714,16 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_pair_ker
         if (lane == 0 && n0 + q * 32 < p.N) tma_store_2d(&p.tc, st, n0 + q * 32, b0);
       } else if (n0 + q * 32 < p.N) {
         epilogue_swapped32(epi, p.vec, p.M, p.N, n0 + q * 32, b0, v,
-                           smem_u32(smem) + 96 * 1024 + (warp - 2) * 32 * 36 * 4);
+                           smem_u32(smem_raw) + 96 * 1024 + (warp - 2) * 32 * 36 * 4);
       }
     }
   }
-  if (p.tma_store && warp >= 2 && lane == 0) tma_store_wait_all();
-  tc_fence_before();
-  cluster_sync_all();                                   // nobody deallocates while the pair's MMAs / loads are in flight
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc_2sm<TCOLS>(tmem_acc);
-  }
+  gemm_teardown<true, TCOLS>(p, tmem_acc, warp);
 }
 
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
 static EncodeTiledFn get_encode_fn() {
   static EncodeTiledFn fn = nullptr;
   static std::once_flag once;
@@ -775,35 +740,7 @@ static EncodeTiledFn get_encode_fn() {
 
 void* tma_encode_fn() { return reinterpret_cast<void*>(get_encode_fn()); }
 
-// cuTensorMapEncodeTiled costs microseconds of host time and a training step issues ~500 of them with the same
-// few hundred (pointer, shape) combinations every step: memoise the encoded descriptors.
-struct TmapKey {
-  const void* base; int rows, K, ld, box_rows;
-  bool operator==(const TmapKey& o) const { return base == o.base && rows == o.rows && K == o.K && ld == o.ld && box_rows == o.box_rows; }
-};
-struct TmapKeyHash {
-  size_t operator()(const TmapKey& k) const {
-    size_t h = reinterpret_cast<size_t>(k.base) * 0x9E3779B97F4A7C15ull;
-    h ^= ((size_t)k.rows << 40) ^ ((size_t)k.K << 20) ^ ((size_t)k.ld << 4) ^ (size_t)k.box_rows;
-    return h * 0xD6E8FEB86659FD93ull;
-  }
-};
-static std::unordered_map<TmapKey, CUtensorMap, TmapKeyHash> g_tmap_cache;
-static std::mutex g_tmap_mutex;
-
-static int encode_tmap_uncached(CUtensorMap* out, const bf16* base, int rows, int K, int ld, int box_rows);
-static int encode_tmap(CUtensorMap* out, const bf16* base, int rows, int K, int ld, int box_rows) {
-  const TmapKey key{base, rows, K, ld, box_rows};
-  std::lock_guard<std::mutex> lock(g_tmap_mutex);
-  auto it = g_tmap_cache.find(key);
-  if (it != g_tmap_cache.end()) { *out = it->second; return 0; }
-  TRY(encode_tmap_uncached(out, base, rows, K, ld, box_rows));
-  if (g_tmap_cache.size() > 8192) g_tmap_cache.clear();
-  g_tmap_cache.emplace(key, *out);
-  return 0;
-}
-
-static int encode_tmap_uncached(CUtensorMap* out, const bf16* base, int rows, int K, int ld, int box_rows) {
+int encode_tmap_2d_uncached(CUtensorMap* out, const bf16* base, int rows, int K, int ld, int box_rows) {
   EncodeTiledFn fn = get_encode_fn();
   if (!fn) { set_error("cuTensorMapEncodeTiled not available from the driver"); return SSCVAE_ERR_DRIVER; }
   if ((reinterpret_cast<uintptr_t>(base) & 15) || (ld % 8) != 0) {
@@ -824,14 +761,43 @@ static int encode_tmap_uncached(CUtensorMap* out, const bf16* base, int rows, in
   return 0;
 }
 
-static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+// cuTensorMapEncodeTiled costs microseconds of host time and a training step issues ~500 of them with the same
+// few hundred (pointer, shape) combinations every step: memoise the encoded descriptors.
+struct TmapKey {
+  const void* base; int rows, K, ld, box_rows;
+  bool operator==(const TmapKey& o) const { return base == o.base && rows == o.rows && K == o.K && ld == o.ld && box_rows == o.box_rows; }
+};
+struct TmapKeyHash {
+  size_t operator()(const TmapKey& k) const {
+    size_t h = reinterpret_cast<size_t>(k.base) * 0x9E3779B97F4A7C15ull;
+    h ^= ((size_t)k.rows << 40) ^ ((size_t)k.K << 20) ^ ((size_t)k.ld << 4) ^ (size_t)k.box_rows;
+    return h * 0xD6E8FEB86659FD93ull;
+  }
+};
+static std::unordered_map<TmapKey, CUtensorMap, TmapKeyHash> g_tmap_cache;
+static std::mutex g_tmap_mutex;
 
-static bool tma_store_eligible(const GemmParams& prm) {
-  const GemmEpi& e = prm.epi;
-  return e.C32 && !e.C16 && !e.act && !e.dtanh && !e.accumulate && !e.add1 && !e.add2 &&
-         aligned16(e.C32) && (e.ldc32 % 4) == 0 && (prm.N % 4) == 0 && (!e.bias || aligned16(e.bias));
-  // N % 4: the TMA unit clips stores at 16-byte granularity (measured: with N = 77 the columns 77..79 were written)
+static int encode_tmap(CUtensorMap* out, const bf16* base, int rows, int K, int ld, int box_rows) {
+  const TmapKey key{base, rows, K, ld, box_rows};
+  std::lock_guard<std::mutex> lock(g_tmap_mutex);
+  auto it = g_tmap_cache.find(key);
+  if (it != g_tmap_cache.end()) { *out = it->second; return 0; }
+  TRY(encode_tmap_2d_uncached(out, base, rows, K, ld, box_rows));
+  if (g_tmap_cache.size() > 8192) g_tmap_cache.clear();
+  g_tmap_cache.emplace(key, *out);
+  return 0;
 }
+
+// operand maps of every K segment: A (M rows) with boxes of box_a rows, B (N rows) with boxes of box_b rows
+static int encode_operands(GemmParams& prm, const GemmSeg* segs, int box_a, int box_b) {
+  for (int s = 0; s < prm.nseg; ++s) {
+    TRY(encode_tmap(&prm.ta[s], segs[s].A, prm.M, segs[s].K, segs[s].lda, box_a));
+    TRY(encode_tmap(&prm.tb[s], segs[s].B, prm.N, segs[s].K, segs[s].ldb, box_b));
+  }
+  return 0;
+}
+
+static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 // fp32 output tile map for TMA stores: box = 32 columns x 32 rows, dense in shared memory
 static int encode_tmap_c32(CUtensorMap* out, const float* base, int rows, int cols, int ld, bool swizzle128) {
@@ -857,61 +823,79 @@ static int encode_tmap_c32(CUtensorMap* out, const float* base, int rows, int co
   return 0;
 }
 
-template <int BN, int STAGES>
-static int launch_tc(cudaStream_t stream, GemmParams& prm, const GemmSeg* segs) {
-  for (int s = 0; s < prm.nseg; ++s) {
-    TRY(encode_tmap(&prm.ta[s], segs[s].A, prm.M, segs[s].K, segs[s].lda, BM));
-    TRY(encode_tmap(&prm.tb[s], segs[s].B, prm.N, segs[s].K, segs[s].ldb, BN));
+// Sets prm.tma_store, and encodes prm.tc when it is set: a plain fp32 tile (+ bias) leaves the epilogue through TMA
+// stores. Never with row statistics, whose epilogue writes through epilogue_row32. bias_vec4: the epilogue reads the bias
+// as float4 (the tile kernels; the swapped-pair kernel reads one bias per lane). swizzle128: the layout of the staged tile.
+static int choose_tma_store(GemmParams& prm, bool bias_vec4, bool swizzle128) {
+  const GemmEpi& e = prm.epi;
+  prm.tma_store = !prm.rs.mode && e.C32 && !e.C16 && !e.act && !e.dtanh && !e.accumulate && !e.add1 && !e.add2 &&
+                  aligned16(e.C32) && (e.ldc32 % 4) == 0 && (prm.N % 4) == 0 &&
+                  (!bias_vec4 || !e.bias || aligned16(e.bias));
+  // N % 4: the TMA unit clips stores at 16-byte granularity (measured: with N = 77 the columns 77..79 were written)
+  if (prm.tma_store) TRY(encode_tmap_c32(&prm.tc, e.C32, prm.M, prm.N, e.ldc32, swizzle128));
+  return 0;
+}
+
+// GEMM_THREADS per CTA, smem bytes of dynamic shared memory; cluster_z > 0: clusters of (2, 1, cluster_z) CTAs
+// (the swapped-pair kernel; the CTA-pair tile kernel declares its cluster shape itself)
+static cudaLaunchConfig_t gemm_config(dim3 grid, int smem, cudaStream_t stream, int cluster_z, cudaLaunchAttribute* attr) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = grid;
+  cfg.blockDim = dim3(GEMM_THREADS, 1, 1);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = stream;
+  if (cluster_z > 0) {
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = cluster_z;
+    cfg.attrs = attr; cfg.numAttrs = 1;
   }
-  prm.tma_store = BN >= 32 && tma_store_eligible(prm);
-  if (prm.tma_store) TRY(encode_tmap_c32(&prm.tc, prm.epi.C32, prm.M, prm.N, prm.epi.ldc32, true));
-  constexpr int smem = 1024 + STAGES * (A_STAGE_BYTES + BN * BK * 2) + 256;
+  return cfg;
+}
+
+// raises KERNEL's dynamic shared-memory limit to Smem::bytes(), once, before its first launch or occupancy query
+template <void (*KERNEL)(GemmParams), class Smem>
+static int gemm_configure() {
   static bool configured = false;
   if (!configured) {
-    CUDA_TRY(cudaFuncSetAttribute(gemm_tcgen05_kernel<BN, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    CUDA_TRY(cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem::bytes()));
     configured = true;
   }
-  dim3 grid(ceil_div(prm.N, BN), ceil_div(prm.M, BM));
-  gemm_tcgen05_kernel<BN, STAGES><<<grid, GEMM_THREADS, smem, stream>>>(prm);
-  CUDA_TRY(cudaGetLastError());
+  return 0;
+}
+
+template <void (*KERNEL)(GemmParams), class Smem>
+static int gemm_launch(cudaStream_t stream, dim3 grid, int cluster_z, const GemmParams& prm) {
+  TRY((gemm_configure<KERNEL, Smem>()));
+  cudaLaunchAttribute attr[1];
+  const cudaLaunchConfig_t cfg = gemm_config(grid, Smem::bytes(), stream, cluster_z, attr);
+  CUDA_TRY(cudaLaunchKernelEx(&cfg, KERNEL, prm));
   ++g_launch_count;
   return 0;
+}
+
+template <int BN, int STAGES>
+static int launch_tc(cudaStream_t stream, GemmParams& prm, const GemmSeg* segs) {
+  TRY(encode_operands(prm, segs, BM, BN));
+  if (BN >= 32) TRY(choose_tma_store(prm, true, true));    // a TMA store box is 32 columns wide
+  return gemm_launch<gemm_tcgen05_kernel<BN, STAGES>, TileSmem<BN, STAGES>>(
+      stream, dim3(ceil_div(prm.N, BN), ceil_div(prm.M, BM)), 0, prm);
 }
 
 template <int BN, int STAGES>
 static int launch_tc2(cudaStream_t stream, GemmParams& prm, const GemmSeg* segs) {
-  for (int s = 0; s < prm.nseg; ++s) {
-    TRY(encode_tmap(&prm.ta[s], segs[s].A, prm.M, segs[s].K, segs[s].lda, BM));
-    TRY(encode_tmap(&prm.tb[s], segs[s].B, prm.N, segs[s].K, segs[s].ldb, BN / 2));
-  }
-  prm.tma_store = BN >= 32 && tma_store_eligible(prm);
-  if (prm.tma_store) TRY(encode_tmap_c32(&prm.tc, prm.epi.C32, prm.M, prm.N, prm.epi.ldc32, true));
-  constexpr int smem = 1024 + STAGES * (A_STAGE_BYTES + (BN / 2) * BK * 2) + 256;
-  static bool configured = false;
-  if (!configured) {
-    CUDA_TRY(cudaFuncSetAttribute(gemm_tcgen05_2cta_kernel<BN, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    configured = true;
-  }
-  dim3 grid(2 * ceil_div(prm.N, BN), ceil_div(prm.M, 2 * BM));
-  gemm_tcgen05_2cta_kernel<BN, STAGES><<<grid, GEMM_THREADS, smem, stream>>>(prm);
-  CUDA_TRY(cudaGetLastError());
-  ++g_launch_count;
-  return 0;
+  TRY(encode_operands(prm, segs, BM, BN / 2));
+  TRY(choose_tma_store(prm, true, true));
+  return gemm_launch<gemm_tcgen05_2cta_kernel<BN, STAGES>, PairTileSmem<BN, STAGES>>(
+      stream, dim3(2 * ceil_div(prm.N, BN), ceil_div(prm.M, 2 * BM)), 0, prm);
 }
 
 // max co-resident clusters of the pair kernel for a K split of S (cluster = 2*S CTAs); 0 if the query fails
 template <int STAGES>
-static int pair_max_clusters(int S, int smem) {
+static int pair_max_clusters(int S) {
   static int cache[5] = {-1, -1, -1, -1, -1};
   if (cache[S] >= 0) return cache[S];
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * 64, 1, S);
-  cfg.blockDim = dim3(GEMM_THREADS, 1, 1);
-  cfg.dynamicSmemBytes = smem;
   cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = S;
-  cfg.attrs = attr; cfg.numAttrs = 1;
+  const cudaLaunchConfig_t cfg = gemm_config(dim3(2 * 64, 1, S), SwappedSmem<STAGES>::bytes(), 0, S, attr);
   int n = 0;
   if (cudaOccupancyMaxActiveClusters(&n, gemm_tcgen05_swapped_pair_kernel<STAGES>, &cfg) != cudaSuccess) {
     cudaGetLastError();
@@ -923,12 +907,7 @@ static int pair_max_clusters(int S, int smem) {
 
 template <int STAGES>
 static int launch_swapped_pair(cudaStream_t stream, GemmParams& prm, const GemmSeg* segs, int forced_S) {
-  constexpr int smem = 1024 + STAGES * (128 + 128) * BK * 2 + 256;
-  static bool configured = false;
-  if (!configured) {
-    CUDA_TRY(cudaFuncSetAttribute(gemm_tcgen05_swapped_pair_kernel<STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    configured = true;
-  }
+  TRY((gemm_configure<gemm_tcgen05_swapped_pair_kernel<STAGES>, SwappedSmem<STAGES>>()));
   int total_kb = 0;
   for (int s = 0; s < prm.nseg; ++s) total_kb += prm.kblocks[s];
   const int pairs = ceil_div(prm.N, 256);
@@ -937,31 +916,14 @@ static int launch_swapped_pair(cudaStream_t stream, GemmParams& prm, const GemmS
   if (forced_S > 0) S = forced_S;
   else
     for (int c = 4; c > 1; --c)
-      if (total_kb >= 4 * c && pairs <= pair_max_clusters<STAGES>(c, smem)) { S = c; break; }
+      if (total_kb >= 4 * c && pairs <= pair_max_clusters<STAGES>(c)) { S = c; break; }
   while (S > 1 && total_kb < S) --S;
   prm.kb_per_split = ceil_div(total_kb, S);
   S = ceil_div(total_kb, prm.kb_per_split);             // no empty trailing split
   prm.splits = S;
-  for (int s = 0; s < prm.nseg; ++s) {
-    TRY(encode_tmap(&prm.ta[s], segs[s].A, prm.M, segs[s].K, segs[s].lda, 128));
-    TRY(encode_tmap(&prm.tb[s], segs[s].B, prm.N, segs[s].K, segs[s].ldb, 128));
-  }
-  const GemmEpi& e = prm.epi;
-  prm.tma_store = e.C32 && !e.C16 && !e.act && !e.dtanh && !e.accumulate && !e.add1 && !e.add2 &&
-                  aligned16(e.C32) && (e.ldc32 % 4) == 0 && (prm.N % 4) == 0;
-  if (prm.tma_store) TRY(encode_tmap_c32(&prm.tc, e.C32, prm.M, prm.N, e.ldc32, false));
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * pairs, 1, S);
-  cfg.blockDim = dim3(GEMM_THREADS, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = S;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  CUDA_TRY(cudaLaunchKernelEx(&cfg, gemm_tcgen05_swapped_pair_kernel<STAGES>, prm));
-  ++g_launch_count;
-  return 0;
+  TRY(encode_operands(prm, segs, 128, 128));
+  TRY(choose_tma_store(prm, false, false));
+  return gemm_launch<gemm_tcgen05_swapped_pair_kernel<STAGES>, SwappedSmem<STAGES>>(stream, dim3(2 * pairs, 1, S), S, prm);
 }
 
 int gemm_bf16_tn(cudaStream_t stream, int M, int N, int nseg, const GemmSeg* segs, const GemmEpi& epi) {
@@ -1000,23 +962,7 @@ int gemm_bf16_tn(cudaStream_t stream, int M, int N, int nseg, const GemmSeg* seg
             "gemm: row statistics take a plain (alpha, bias) epilogue");
     REQUIRE(epi.rs->mode != 1 || (epi.rs->st_max && epi.rs->st_sum && epi.rs->st_arg), "gemm: row statistics need their partial buffers");
     REQUIRE(epi.rs->mode != 2 || (epi.rs->lse && epi.rs->gcoef && epi.rs->target && epi.C16), "gemm: CE gradient needs lse, gcoef, target and a bf16 output");
-    prm.tma_store = 0;
-    GemmParams& q = prm;
-    for (int s2 = 0; s2 < q.nseg; ++s2) {
-      TRY(encode_tmap(&q.ta[s2], segs[s2].A, q.M, segs[s2].K, segs[s2].lda, BM));
-      TRY(encode_tmap(&q.tb[s2], segs[s2].B, q.N, segs[s2].K, segs[s2].ldb, 128));
-    }
-    constexpr int smem_rs = 1024 + 3 * (A_STAGE_BYTES + 128 * BK * 2) + 256;
-    static bool configured_rs = false;
-    if (!configured_rs) {
-      CUDA_TRY(cudaFuncSetAttribute(gemm_tcgen05_kernel<128, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_rs));
-      configured_rs = true;
-    }
-    dim3 grid(ceil_div(q.N, 128), ceil_div(q.M, BM));
-    gemm_tcgen05_kernel<128, 3><<<grid, GEMM_THREADS, smem_rs, stream>>>(q);
-    CUDA_TRY(cudaGetLastError());
-    ++g_launch_count;
-    return 0;
+    return launch_tc<128, 3>(stream, prm, segs);          // a thread sees 128 logits of its row per tile
   }
   // Skinny GEMMs with enough weight rows (the per-timestep LSTM and BPTT GEMMs, short K included: the attention-LSTM
   // recurrence, K = 2Hp) run on the swapped-operand CTA-pair kernel (see the kernel); narrow N (256x768x960) stays on

@@ -118,16 +118,6 @@ struct PkSmem {
   }
 };
 
-// position of the producer / the MMA issuer in the ring
-template <int STAGES>
-struct RingPos {
-  int stage = 0;
-  uint32_t phase = 0;
-  __device__ __forceinline__ void advance() {
-    if (++stage == STAGES) { stage = 0; phase ^= 1; }
-  }
-};
-
 // TMA producer, one K segment of a job. The weight tiles do not depend on any flag: they are pulled into L2 while the
 // activations they multiply are still being produced (the ring alone keeps only STAGES tiles in flight, which left the
 // weight stream HBM-latency bound: ~0.4 us per k-block). `ready()` waits for the activations. Then per k-block: the
@@ -187,10 +177,6 @@ __device__ __forceinline__ void pk_teardown(int warp, uint32_t tmem_base) {
 // ---------------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
 // activation (k, batch row, t) of a time-major bf16 tensor with row stride ld: box 64 x 128 x 1, 128B swizzle
 static int encode_act3d(CUtensorMap* out, const bf16* base, int K, int B, int T, int ld) {
   EncodeTiledFn fn = reinterpret_cast<EncodeTiledFn>(tma_encode_fn());
@@ -205,19 +191,9 @@ static int encode_act3d(CUtensorMap* out, const bf16* base, int K, int B, int T,
   if (r != CUDA_SUCCESS) { set_error(PK_NAME ": activation tensor map failed (%d) K=%d B=%d T=%d ld=%d", (int)r, K, B, T, ld); return SSCVAE_ERR_DRIVER; }
   return 0;
 }
-// weight (k, row): box 64 x box_rows, 128B swizzle
+// weight (k, row): box 64 x box_rows, 128B swizzle; encoded on every launch, like the activation maps
 static int encode_w2d(CUtensorMap* out, const bf16* base, int K, int rows, int ld, int box_rows) {
-  EncodeTiledFn fn = reinterpret_cast<EncodeTiledFn>(tma_encode_fn());
-  if (!fn) { set_error("cuTensorMapEncodeTiled not available from the driver"); return SSCVAE_ERR_DRIVER; }
-  cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
-  cuuint32_t box[2] = {64, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<bf16*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_error(PK_NAME ": weight tensor map failed (%d) K=%d rows=%d ld=%d box=%d", (int)r, K, rows, ld, box_rows); return SSCVAE_ERR_DRIVER; }
-  return 0;
+  return encode_tmap_2d_uncached(out, base, rows, K, ld, box_rows);
 }
 
 // CTA pairs of `kernel` that can be co-resident with `smem` bytes of dynamic shared memory (0 on failure); cached

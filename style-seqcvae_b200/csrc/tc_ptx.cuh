@@ -1,5 +1,5 @@
-// tcgen05 / TMEM / TMA / mbarrier PTX wrappers shared by the sm_100a GEMM kernels (gemm_sm100.cu) and the persistent
-// recurrent kernels (persistent.cuh, recurrent_fwd.cu, recurrent_bwd.cu).
+// tcgen05 / TMEM / TMA / mbarrier PTX wrappers, the operand ring position and the tensor-map encoder shared by the sm_100a
+// GEMM kernels (gemm_sm100.cu) and the persistent recurrent kernels (persistent.cuh, recurrent_fwd.cu, recurrent_bwd.cu).
 #pragma once
 #include <cuda.h>
 #include <cstdint>
@@ -129,12 +129,13 @@ template <int NCOLS>
 __device__ __forceinline__ void tmem_dealloc_2sm(uint32_t taddr) {
   asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "n"(NCOLS) : "memory");
 }
-// arrives (once the MMAs issued so far have completed) on the barrier at this shared-memory offset in BOTH CTAs
-__device__ __forceinline__ void umma_commit_2sm(uint64_t* bar) {
+// arrives (once the MMAs issued so far have completed) on the barrier at this shared-memory offset in the CTAs of `mask`
+// (cluster ranks; default: both CTAs of the pair)
+__device__ __forceinline__ void umma_commit_2sm(uint64_t* bar, uint16_t mask = 3) {
   asm volatile(
       "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
           smem_u32(bar)),
-      "h"(static_cast<uint16_t>(3))
+      "h"(mask)
       : "memory");
 }
 __device__ __forceinline__ void umma_bf16_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
@@ -236,5 +237,24 @@ __host__ __device__ constexpr uint32_t make_idesc(int m, int n) {
   return (1u << 4) | (1u << 7) | (1u << 10) | (static_cast<uint32_t>(n >> 3) << 17) |
          (static_cast<uint32_t>(m >> 4) << 24);
 }
+
+// position of the TMA producer / the MMA issuer in an operand ring of STAGES stages
+template <int STAGES>
+struct RingPos {
+  int stage = 0;
+  uint32_t phase = 0;
+  __device__ __forceinline__ void advance() {
+    if (++stage == STAGES) { stage = 0; phase ^= 1; }
+  }
+};
+
+// ---- host side: tensor maps ---------------------------------------------------------------------------------
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+// bf16 (k, row) operand of `rows` rows x K, row stride ld: box 64 x box_rows, 128B swizzle, 256-byte L2 promotion.
+// Defined in gemm_sm100.cu, whose GEMM launches memoise the result; returns 0 or an error code.
+int encode_tmap_2d_uncached(CUtensorMap* out, const bf16* base, int rows, int K, int ld, int box_rows);
 
 }  // namespace sscvae
