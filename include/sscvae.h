@@ -230,6 +230,38 @@ int sscvae_decode_samples(SscvaeHandle* h, int batch, int samples, int num_boxes
                           int32_t* n_steps,                   /* out device int32: valid leading steps */
                           void* stream);
 
+/* ---- diverse sampling under constrained beam search: the reference's inference loop
+ * `for k in range(N_Z_SAMPLES): model(image_features, ..., fsm=..., num_constraints=...)` (var_updown/scripts/inference.py:138-167)
+ * with USE_CBS, one constrained beam search per (image, sample), in ONE call. Search group g = b*samples + j owns the S*K rows
+ * r = ((b*samples + j)*S + s)*K + k; all rows of an image share its region features, projections and mean-feature block.
+ * Every search stops on its own, exactly as the reference's batch-1 call stops when all of ITS rows have emitted the boundary
+ * token (updown-baseline/updown/modules/cbs.py:167): n_steps[b,j] is that call's step count, predictions / best of the search
+ * hold the boundary token after it.
+ *   fsm_per_sample 0: `fsm` is (B,S,S,V) uint8 (or, with option "fsm_packed", the (B,S,V) bit table) and num_constraints (B):
+ *                     the samples of an image share its machine.
+ *                  1: (B*samples,S,S,V) / (B*samples,S,V) and (B*samples): row b*samples + j is sample j's own machine.
+ *   eps: (max_steps, B*samples*S*K, Z) or NULL -> Philox(seed); step 0 reads row (b*samples + j)*S*K.
+ * Shapes: 1 <= S <= 32, 1 <= per_node <= beam <= 8, samples >= 1, an FSM whenever S > 1; otherwise SSCVAE_ERR_BAD_ARG
+ * before any device work. The (B*samples*S*K, V) fp32 logits are part of the workspace. Options "fsm_packed",
+ * "features_bf16" and "reuse_image_state" apply. */
+size_t sscvae_decode_samples_search_workspace_bytes(const SscvaeHandle* h, int batch, int samples, int num_boxes,
+                                                    int states, int beam, int fsm_per_sample);
+int sscvae_decode_samples_search(SscvaeHandle* h, int batch, int samples, int num_boxes, int states, int beam, int per_node,
+                                 const void* packed, const void* const* weights_f32,
+                                 const float* image_features, const float* sentiment, const float* obj_means,
+                                 const uint8_t* fsm, int fsm_per_sample,
+                                 const int64_t* num_constraints, int min_constraints_to_satisfy,
+                                 const float* eps, uint64_t seed,
+                                 void* workspace, size_t workspace_bytes,
+                                 int64_t* predictions,               /* out (B,samples,S,K,L) */
+                                 float* log_probs,                   /* out (B,samples,S,K) */
+                                 int64_t* best,                      /* out (B,samples,L) */
+                                 int32_t* n_steps,                   /* out device int32 (B,samples) */
+                                 void* stream);
+/* Named view into the workspace of sscvae_decode_samples_search ("tok_hist", "bp_hist", "score_hist" (L,B*samples*S*K), ...). */
+int sscvae_decode_samples_search_region(const SscvaeHandle* h, int batch, int samples, int num_boxes, int states, int beam,
+                                        int fsm_per_sample, const char* name, size_t* offset, size_t* bytes);
+
 /* Named view into the decode workspace for tests ("tok_hist", "bp_hist", "score_hist" (L,B*S*K), "logits", ...). */
 int sscvae_decode_region(const SscvaeHandle* h, int batch, int num_boxes, int states, int beam, const char* name,
                          size_t* offset, size_t* bytes);

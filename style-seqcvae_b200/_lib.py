@@ -43,7 +43,8 @@ SYMBOLS = [
     "sscvae_train_backward", "sscvae_train_region", "sscvae_fsm_pack", "sscvae_fsm_build", "sscvae_select_best_beam", "sscvae_search_first_step",
     "sscvae_search_step", "sscvae_search_scratch_bytes", "sscvae_search_finish",
     "sscvae_decode_workspace_bytes", "sscvae_decode", "sscvae_decode_region", "sscvae_decode_samples_workspace_bytes",
-    "sscvae_decode_samples", "sscvae_grad_sqnorm", "sscvae_sgd_step", "sscvae_test_gemm",
+    "sscvae_decode_samples", "sscvae_decode_samples_search_workspace_bytes", "sscvae_decode_samples_search",
+    "sscvae_decode_samples_search_region", "sscvae_grad_sqnorm", "sscvae_sgd_step", "sscvae_test_gemm",
     "sscvae_profile_enable", "sscvae_profile_report",
 ]
 
@@ -101,6 +102,11 @@ def lib():
     L.sscvae_decode_samples_workspace_bytes.argtypes = [vp, i32, i32, i32]
     L.sscvae_decode_samples_workspace_bytes.restype = sz
     L.sscvae_decode_samples.argtypes = [vp, i32, i32, i32, vp, C.POINTER(vp), vp, vp, vp, vp, u64, vp, sz, vp, vp, vp, vp]
+    L.sscvae_decode_samples_search_workspace_bytes.argtypes = [vp, i32, i32, i32, i32, i32, i32]
+    L.sscvae_decode_samples_search_workspace_bytes.restype = sz
+    L.sscvae_decode_samples_search.argtypes = [vp, i32, i32, i32, i32, i32, i32, vp, C.POINTER(vp), vp, vp, vp, vp, i32, vp, i32,
+                                               vp, u64, vp, sz, vp, vp, vp, vp, vp]
+    L.sscvae_decode_samples_search_region.argtypes = [vp, i32, i32, i32, i32, i32, i32, C.c_char_p, C.POINTER(sz), C.POINTER(sz)]
     L.sscvae_test_gemm_splitk.argtypes = [vp, i32, vp, i32, i32, i32, i32, vp, i32, i32, vp, vp]
     L.sscvae_sgd_step_multi.argtypes = [i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(u64), C.POINTER(i32),
                                         C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, vp, sz, vp]

@@ -513,17 +513,27 @@ class UpDownCaptioner(nn.Module):
         return obj_atts
 
     @torch.no_grad()
-    def sample(self, image_features: torch.Tensor, sentiment=None, n_samples: int = 100, obj_atts=None):
-        """Diverse sampling: `n_samples` greedy captions per image with independent latent draws, in one call.
+    def sample(self, image_features: torch.Tensor, sentiment=None, n_samples: int = 100, obj_atts=None, fsm=None,
+               num_constraints=None, constraints=None, constraint2states=None):
+        """Diverse sampling: `n_samples` captions per image with independent latent draws, in one call.
 
         Replaces the reference's inference loop `for k in range(N_Z_SAMPLES): model(image_features, ...)`
-        (var_updown/scripts/inference.py:138-167) over the eval branch with beam_size 1: same per-sample computation
-        (`_decode_step` with z ~ N(prior_mean, prior_var), updown_cell.py:200-208; beam-1 search), but the
-        n_samples sequences of an image share its region features and run as rows of one batch.
-        Returns {"predictions": (B, n_samples, steps) int64, "log_probs": (B, n_samples)}."""
+        (var_updown/scripts/inference.py:138-167) over the eval branch: same per-sample computation
+        (`_decode_step` with z ~ N(prior_mean, prior_var), updown_cell.py:200-208), but the n_samples sequences of an
+        image share its region features and run as rows of one batch.
+
+        use_cbs=False: beam-1 search. Returns {"predictions": (B, n_samples, steps) int64, "log_probs": (B, n_samples)};
+        `fsm` must be None.
+
+        use_cbs=True: one constrained beam search (beam_size, per_node_beam_size) per (image, sample), exactly what
+        n_samples calls of forward() on single images would run; see `_sample_search`. Returns
+        {"predictions": (B, n_samples, n) int64, "n_steps": (B, n_samples) int64}."""
         self._require_cuda(image_features)
         if self._use_cbs:
-            raise ValueError("sample() is the unconstrained beam-1 path; use forward() for constrained beam search")
+            return self._sample_search(image_features, sentiment, n_samples, obj_atts, fsm, num_constraints, constraints,
+                                       constraint2states)
+        if fsm is not None:
+            raise ValueError("fsm is only used with use_cbs=True; sample() without it is the unconstrained beam-1 path")
         L = _lib.lib()
         image_features = self._features(image_features)
         dev = image_features.device
@@ -566,6 +576,125 @@ class UpDownCaptioner(nn.Module):
             _lib.ptr(ws), nbytes, _lib.ptr(preds), _lib.ptr(scores), _lib.ptr(n_steps), stream))
         n = int(n_steps.item())
         return {"predictions": preds[..., :n].clone(), "log_probs": scores.clone()}
+
+    def _sample_search(self, image_features, sentiment, n_samples, obj_atts, fsm, num_constraints, constraints,
+                       constraint2states):
+        """sample() with use_cbs=True: the reference's loop `for k in range(N_Z_SAMPLES): model(image_features, ...,
+        fsm=..., num_constraints=...)` (inference.py:138-167) in one call (sscvae_decode_samples_search).
+
+        Every (image b, sample j) is one constrained beam search with its own latent draws, and it stops when its own
+        beams have all emitted the boundary token, as the reference's batch-1 call does (cbs.py:167).
+        - `fsm`: the reference's (B,S,S,V) uint8 tensor or an `FsmBits` (B,S,V) table, shared by the samples of an image;
+          or (B*n_samples, ...), row b*n_samples + j being sample j's own machine. `num_constraints` has as many rows.
+        - cbs_simple=False: `constraints` / `constraint2states` hold one entry per FSM row (valid_states_with_attributes).
+        - `_eps_override`: (steps, B*n_samples*S*K, Z) normals, step 0 reading row (b*n_samples + j)*S*K. Otherwise the
+          device Philox stream; rng_mode "reference" does not apply here (as in the beam-1 sample()).
+        - Workspace: the fp32 logits of all R = B*n_samples*S*K rows are materialised, R*V*4 bytes (16 images x 20
+          samples x S 8 x K 5 at V 10 000: 512 MB); sscvae_decode_samples_search_workspace_bytes gives the total.
+        Returns {"predictions": (B, n_samples, n), "n_steps": (B, n_samples)} int64 with n = the largest n_steps; a
+        sample's entries after its own n_steps are the boundary token. `last_search` holds every beam:
+        {"predictions": (B,J,S,K,n), "log_probs": (B,J,S,K), "n_steps": (B,J)}."""
+        from .fsm import FsmBits, valid_states_with_attributes
+        L = _lib.lib()
+        image_features = self._features(image_features)
+        dev = image_features.device
+        B, N, F = image_features.shape
+        if F != self.image_feature_size:
+            raise ValueError(f"image_features last dim {F} != image_feature_size {self.image_feature_size}")
+        J, K, P, steps, V = int(n_samples), self.beam_size, self.per_node_beam_size, self._max_caption_length, self._vocab_size
+        if J < 1:
+            raise ValueError("n_samples must be >= 1")
+        if self.sentiment_vae == 1:
+            if sentiment is None:
+                raise ValueError("sentiment is required when sentiment_vae == 1")
+            sentiment = sentiment.to(dev).contiguous().float().view(B, 1)
+        else:
+            sentiment = None
+        obj_means = self._obj_means(obj_atts, B, N, dev)
+        if fsm is None:
+            raise ValueError("fsm is required when use_cbs=True")
+        fsm_packed = isinstance(fsm, FsmBits)
+        if fsm_packed:                                               # bit table built on the device (fsm.build_fsm_bits)
+            fsm = fsm.bits
+            T, S = fsm.shape[0], fsm.shape[1]
+            if fsm.shape != (T, S, V) or T not in (B, B * J) or fsm.device != dev or not fsm.is_contiguous():
+                raise ValueError(f"FsmBits must be a contiguous (B or B*n_samples, S, V) table on {dev}, got {tuple(fsm.shape)}")
+        else:
+            fsm = fsm.to(dev).to(torch.uint8).contiguous()
+            T, S = fsm.shape[0], fsm.shape[1]
+            if fsm.dim() != 4 or fsm.shape != (T, S, S, V) or T not in (B, B * J):
+                raise ValueError(f"fsm must be (B or B*n_samples, S, S, V), got {tuple(fsm.shape)}")
+        per_sample = int(T != B)
+        if num_constraints is None:
+            nc = torch.zeros(T, dtype=torch.long, device=dev)
+        else:
+            nc = num_constraints.to(dev).long().contiguous().view(-1)
+            if nc.numel() != T:
+                raise ValueError(f"num_constraints must have one entry per FSM ({T}), got {nc.numel()}")
+        valid = None
+        if not self.cbs_simple:
+            # object / attribute rule (decoding.py:87-123), per machine, then per search
+            if constraints is None or constraint2states is None:
+                raise ValueError("cbs_simple=False needs `constraints` and `constraint2states`")
+            counts = [int(n) for n in nc.cpu()]
+            mask = torch.zeros(T, S, dtype=torch.uint8)
+            for i in range(T):
+                states = valid_states_with_attributes(counts[i], constraints[i], constraint2states[i],
+                                                      self._min_constraints_to_satisfy)
+                if not states:
+                    raise ValueError(f"FSM {i}: no state satisfies the constraints")
+                mask[i, states] = 1
+            valid = (mask if per_sample else mask.repeat_interleave(J, dim=0)).contiguous().to(dev)
+        R = B * J * S * K
+        eps = self._eps_override
+        if eps is not None:
+            eps = eps.to(dev).contiguous().float()
+            assert eps.shape == (steps, R, self.z_space)
+        nbytes = L.sscvae_decode_samples_search_workspace_bytes(self._handle, B, J, N, S, K, per_sample)
+        if nbytes == 0:
+            raise ValueError(f"unsupported search shape: states {S}, beam {K} (1..32 states, beam 1..8)")
+        key = ("decode", B, N, S, K, dev, J, per_sample)
+        ws = self._ws_cache.get(key)
+        if ws is None:
+            self._ws_cache = {k: v for k, v in self._ws_cache.items() if k[0] != "decode"}
+            ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+            self._ws_cache[key] = ws
+        okey = ("decode_out", B, S, K, steps, dev, J)               # persistent outputs: stable pointers for graph replay
+        outs = self._ws_cache.get(okey)
+        if outs is None:
+            outs = (torch.empty(B, J, S, K, steps, dtype=torch.long, device=dev),
+                    torch.empty(B, J, S, K, dtype=torch.float32, device=dev),
+                    torch.empty(B, J, steps, dtype=torch.long, device=dev), torch.zeros(B, J, dtype=torch.int32, device=dev))
+            self._ws_cache[okey] = outs
+        preds, scores, best, n_steps = outs
+        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        self._reuse_image_state(key, image_features)
+        _lib.check(L.sscvae_set_option(self._handle, b"fsm_packed", int(fsm_packed)))
+        _lib.check(L.sscvae_decode_samples_search(
+            self._handle, B, J, N, S, K, P, _lib.ptr(self._packed_weights()), _lib.ptr_array(self._weight_tensors()),
+            _lib.ptr(image_features), _lib.ptr(sentiment), _lib.ptr(obj_means), _lib.ptr(fsm), per_sample, _lib.ptr(nc),
+            int(self._min_constraints_to_satisfy), _lib.ptr(eps), C.c_uint64(self._next_seed()), _lib.ptr(ws), nbytes,
+            _lib.ptr(preds), _lib.ptr(scores), _lib.ptr(best), _lib.ptr(n_steps), stream))
+        if valid is not None:
+            _lib.check(L.sscvae_select_best_beam(_lib.ptr(preds), _lib.ptr(scores), _lib.ptr(valid), B * J, S, K, steps,
+                                                 _lib.ptr(best), stream))
+        ns = n_steps.long()
+        n = int(ns.max().item())                                    # each search's own early exit (cbs.py:167)
+        self.last_search = {"predictions": preds[..., :n].clone(), "log_probs": scores.clone(), "n_steps": ns.clone()}
+        return {"predictions": best[..., :n].clone(), "n_steps": ns.clone()}
+
+    def sample_search_region(self, B, N, J, S, K, fsm_per_sample, name, dtype, shape):
+        """Typed view of a named region of the last sample() workspace with use_cbs=True (tests / debugging)."""
+        off, nb = C.c_size_t(), C.c_size_t()
+        _lib.check(_lib.lib().sscvae_decode_samples_search_region(self._handle, B, J, N, S, K, int(fsm_per_sample),
+                                                                  name.encode(), C.byref(off), C.byref(nb)))
+        ws = self._ws_cache[("decode", B, N, S, K, self._embedding_layer.weight.device, J, int(fsm_per_sample))]
+        n = 1
+        for s in shape:
+            n *= s
+        itemsize = torch.empty(0, dtype=dtype).element_size()
+        assert n * itemsize <= nb.value, (name, n * itemsize, nb.value)
+        return ws[off.value: off.value + n * itemsize].view(dtype).view(*shape)
 
     @torch.no_grad()
     def _decode(self, image_features, sentiment, fsm, num_constraints, obj_means=None, constraints=None,

@@ -13,7 +13,9 @@ namespace sscvae {
 // image is decoded J times with independent latent draws in ONE call. The search sees Bv = B*J independent sequences
 // (virtual images); everything image-sized (features, projections, mean-feature gate block) stays at B and is shared
 // through the row -> image map, so the per-step GEMMs run with M = B*J rows instead of J launches with M = B.
-static void plan_decode(const Dims& d, int B, int N, int S, int K, int J, Plan& p) {
+// With S > 1 or K > 1 every virtual image is one constrained beam search of S*K rows; its FSM table is the image's (the J
+// samples share it) or its own (one machine per sample): `fsm_tables` = B or B*J (S,V) tables are packed.
+static void plan_decode(const Dims& d, int B, int N, int S, int K, int J, int fsm_tables, Plan& p) {
   const size_t b = sizeof(bf16), f = 4;
   const size_t Bv = (size_t)B * J, R = Bv * S * K, BN = (size_t)B * N;
   const int Pmax = K;
@@ -48,7 +50,7 @@ static void plan_decode(const Dims& d, int B, int N, int S, int K, int J, Plan& 
   p.add("rs_max", R * nst * f);
   p.add("rs_sum", R * nst * f);
   p.add("rs_arg", R * nst * 4);
-  p.add("fsm_bits", Bv * S * d.V * 4);
+  p.add("fsm_bits", (size_t)fsm_tables * S * d.V * 4);
   p.add("cand_val", R * S * Pmax * f);
   p.add("cand_tok", R * S * Pmax * 4);
   p.add("tok_hist", (size_t)d.L * R * 4);
@@ -57,11 +59,11 @@ static void plan_decode(const Dims& d, int B, int N, int S, int K, int J, Plan& 
   p.add("best_samples", Bv * d.L * 8);                 // sscvae_decode_samples: the "best beam" copy of its predictions
 }
 
-const Plan& Handle::decode_plan(int B, int N, int S, int K, int J) {
-  if (dp_B != B || dp_N != N || dp_S != S || dp_K != K || dp_J != J) {
+const Plan& Handle::decode_plan(int B, int N, int S, int K, int J, int fsm_tables) {
+  if (dp_B != B || dp_N != N || dp_S != S || dp_K != K || dp_J != J || dp_T != fsm_tables) {
     dp = Plan();
-    plan_decode(d, B, N, S, K, J, dp);
-    dp_B = B; dp_N = N; dp_S = S; dp_K = K; dp_J = J;
+    plan_decode(d, B, N, S, K, J, fsm_tables, dp);
+    dp_B = B; dp_N = N; dp_S = S; dp_K = K; dp_J = J; dp_T = fsm_tables;
   }
   return dp;
 }
@@ -70,7 +72,10 @@ static inline GemmSeg seg(const bf16* A, int lda, const bf16* B, int ldb, int K)
   GemmSeg s; s.A = A; s.lda = lda; s.B = B; s.ldb = ldb; s.K = K; return s;
 }
 
-static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, const char* pk, const void* const* wv,
+// gpf: search groups (virtual images) per FSM table and per num_constraints entry (1, or J when the samples of an image share
+// its machine). exit_per_search: every group stops on its own (n_steps has B*J entries) instead of the batch together.
+static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, int gpf, bool exit_per_search,
+                       const char* pk, const void* const* wv,
                        const void* feats, const float* sent, const float* obj, const uint8_t* fsm, const long long* num_constraints,
                        int min_sat, const float* eps, unsigned long long seed, char* ws, size_t ws_bytes,
                        long long* predictions, float* log_probs, long long* best, int32_t* n_steps, cudaStream_t s) {
@@ -80,9 +85,9 @@ static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, cons
   REQUIRE(!csent || sent != nullptr, "sentiment is required when sentiment_vae == 1");
   REQUIRE(!d.cvar || obj != nullptr, "obj_means is required when sentiment_vae == 2");
   REQUIRE(S == 1 || fsm != nullptr, "an FSM is required for more than one state");
-  REQUIRE(J >= 1 && (J == 1 || (S == 1 && fsm == nullptr)), "samples per image > 1 needs the unconstrained search (S == 1)");
-  const Plan& dp = h->decode_plan(B, N, S, K, J);
+  REQUIRE(J >= 1 && (gpf == 1 || gpf == J), "bad sample grouping J=%d groups per FSM=%d", J, gpf);
   const int Bv = B * J;
+  const Plan& dp = h->decode_plan(B, N, S, K, J, Bv / gpf);
   if (ws_bytes < dp.total) { set_error("workspace too small: %zu < %zu", ws_bytes, dp.total); return SSCVAE_ERR_WORKSPACE; }
   REQUIRE((reinterpret_cast<uintptr_t>(ws) & 255) == 0 && (reinterpret_cast<uintptr_t>(pk) & 255) == 0,
           "workspace and packed weights must be 256-byte aligned");
@@ -114,10 +119,10 @@ static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, cons
   TRY(iota_div_i32(s, Wi("rowmap0"), Bv, J));
   TRY(fill_i32(s, Wi("start_tok"), d.boundary, Bv));                       // updown_captioner.py:326
   const uint32_t* fsm_bits = nullptr;
-  if (fsm && h->opt_fsm_packed) {                      // already the (B,S,V) uint32 bit table (sscvae_fsm_build / sscvae_fsm_pack)
+  if (fsm && h->opt_fsm_packed) {                      // already the (tables,S,V) uint32 bit table (sscvae_fsm_build / sscvae_fsm_pack)
     fsm_bits = reinterpret_cast<const uint32_t*>(fsm);
   } else if (fsm) {
-    TRY(fsm_pack(s, fsm, Bv, S, d.V, reinterpret_cast<uint32_t*>(Wi("fsm_bits"))));
+    TRY(fsm_pack(s, fsm, Bv / gpf, S, d.V, reinterpret_cast<uint32_t*>(Wi("fsm_bits"))));
     fsm_bits = reinterpret_cast<uint32_t*>(Wi("fsm_bits"));
   }
   if (!reuse) {  // once per image (the reference recomputes both every step in decode)
@@ -211,7 +216,7 @@ static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, cons
   } else {
     SearchRowsArgs a = {};
     a.logp = Wf("logits"); a.ld = d.V; a.V = d.V; a.normalized = 0; a.fsm_bits = fsm_bits; a.R = Bv; a.S = S; a.K = K;
-    a.rows_per_image = 1; a.P = K; a.end_index = d.boundary; a.neg_value = -INFINITY;
+    a.rows_per_image = 1; a.groups_per_fsm = gpf; a.P = K; a.end_index = d.boundary; a.neg_value = -INFINITY;
     a.cand_val = score_hist; a.cand_tok = tok_hist;
     TRY(search_rows(s, a));
   }
@@ -229,7 +234,7 @@ static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, cons
     }
     SearchRowsArgs a = {};
     a.logp = Wf("logits"); a.ld = d.V; a.V = d.V; a.normalized = 0; a.fsm_bits = fsm_bits; a.R = R; a.S = S; a.K = K;
-    a.rows_per_image = SK; a.P = P; a.end_index = d.boundary; a.neg_value = -1e20f;
+    a.rows_per_image = SK; a.groups_per_fsm = gpf; a.P = P; a.end_index = d.boundary; a.neg_value = -1e20f;
     a.last_tokens = tok_hist + (size_t)(t - 1) * R; a.last_scores = score_hist + (size_t)(t - 1) * R;
     a.cand_val = Wf("cand_val"); a.cand_tok = Wi("cand_tok");
     TRY(search_rows(s, a));
@@ -237,8 +242,8 @@ static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, cons
                      score_hist + (size_t)t * R));
     TRY(state_gather(s, bp_hist + (size_t)t * R, R, SK, XA[1], XA[0], 2 * Hp, c1[1], c1[0], cd[1], cd[0], H));
   }
-  TRY(search_finish(s, tok_hist, bp_hist, score_hist, L, Bv, S, K, d.boundary, num_constraints, min_sat, predictions,
-                    log_probs, best, n_steps));
+  TRY(search_finish(s, tok_hist, bp_hist, score_hist, L, Bv, S, K, d.boundary, num_constraints, min_sat, gpf,
+                    exit_per_search ? 1 : 0, predictions, log_probs, best, n_steps));
   return 0;
 }
 
@@ -307,27 +312,27 @@ int sscvae_search_finish(const int32_t* tokens_hist, const int32_t* backptr_hist
   REQUIRE(tokens_hist && backptr_hist && scores_hist && predictions && final_scores && best && n_steps, "NULL argument");
   return search_finish(reinterpret_cast<cudaStream_t>(stream), tokens_hist, backptr_hist, scores_hist, steps_run, batch,
                        states, beam, end_index, reinterpret_cast<const long long*>(num_constraints),
-                       min_constraints_to_satisfy, reinterpret_cast<long long*>(predictions), final_scores,
+                       min_constraints_to_satisfy, 1, 0, reinterpret_cast<long long*>(predictions), final_scores,
                        reinterpret_cast<long long*>(best), n_steps);
 }
 
 size_t sscvae_decode_workspace_bytes(const SscvaeHandle* hh, int batch, int num_boxes, int states, int beam) {
   Handle* h = const_cast<Handle*>(reinterpret_cast<const Handle*>(hh));
   if (!h || batch <= 0 || num_boxes <= 0 || states <= 0 || beam <= 0) return 0;
-  return h->decode_plan(batch, num_boxes, states, beam, 1).total;
+  return h->decode_plan(batch, num_boxes, states, beam, 1, batch).total;
 }
 
 size_t sscvae_decode_samples_workspace_bytes(const SscvaeHandle* hh, int batch, int samples, int num_boxes) {
   Handle* h = const_cast<Handle*>(reinterpret_cast<const Handle*>(hh));
   if (!h || batch <= 0 || num_boxes <= 0 || samples <= 0) return 0;
-  return h->decode_plan(batch, num_boxes, 1, 1, samples).total;
+  return h->decode_plan(batch, num_boxes, 1, 1, samples, batch * samples).total;
 }
 
 int sscvae_decode_region(const SscvaeHandle* hh, int batch, int num_boxes, int states, int beam, const char* name,
                          size_t* offset, size_t* bytes) {
   Handle* h = const_cast<Handle*>(reinterpret_cast<const Handle*>(hh));
   REQUIRE(h && name && offset && bytes, "NULL argument");
-  const Region* r = h->decode_plan(batch, num_boxes, states, beam, 1).find(name);
+  const Region* r = h->decode_plan(batch, num_boxes, states, beam, 1, batch).find(name);
   REQUIRE(r != nullptr, "unknown workspace region '%s'", name);
   *offset = r->off; *bytes = r->bytes;
   return 0;
@@ -342,7 +347,7 @@ int sscvae_decode(SscvaeHandle* hh, int batch, int num_boxes, int states, int be
   REQUIRE(h && packed && weights && image_features && workspace && predictions && log_probs && best && n_steps, "NULL argument");
   REQUIRE(batch > 0 && num_boxes > 0 && states >= 1 && beam >= 1, "bad decode shape");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const Plan& dp = h->decode_plan(batch, num_boxes, states, beam, 1);
+  const Plan& dp = h->decode_plan(batch, num_boxes, states, beam, 1, batch);
   if (workspace_bytes < dp.total) { set_error("workspace too small: %zu < %zu", workspace_bytes, dp.total); return SSCVAE_ERR_WORKSPACE; }
   const unsigned long long seed_host = seed;
   CUDA_TRY(cudaMemcpyAsync(reinterpret_cast<char*>(workspace) + dp.find("seed")->off, &seed_host, sizeof(seed_host),
@@ -358,7 +363,7 @@ int sscvae_decode(SscvaeHandle* hh, int batch, int num_boxes, int states, int be
     key_add(key, q);
   for (int i = 0; i < SSCVAE_W_COUNT; ++i) key_add(key, weights[i]);
   return run_with_graph(h->dec_graphs, key, st, true, [&](cudaStream_t s) {
-    return decode_impl(h, batch, 1, num_boxes, states, beam, per_node, reinterpret_cast<const char*>(packed), weights,
+    return decode_impl(h, batch, 1, num_boxes, states, beam, per_node, 1, false, reinterpret_cast<const char*>(packed), weights,
                        image_features, sentiment, obj_means, fsm, reinterpret_cast<const long long*>(num_constraints),
                        min_constraints_to_satisfy, eps, seed, reinterpret_cast<char*>(workspace), workspace_bytes,
                        reinterpret_cast<long long*>(predictions), log_probs, reinterpret_cast<long long*>(best), n_steps, s);
@@ -373,7 +378,7 @@ int sscvae_decode_samples(SscvaeHandle* hh, int batch, int samples, int num_boxe
   REQUIRE(h && packed && weights && image_features && workspace && predictions && log_probs && n_steps, "NULL argument");
   REQUIRE(batch > 0 && num_boxes > 0 && samples >= 1, "bad decode shape");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const Plan& dp = h->decode_plan(batch, num_boxes, 1, 1, samples);
+  const Plan& dp = h->decode_plan(batch, num_boxes, 1, 1, samples, batch * samples);
   if (workspace_bytes < dp.total) { set_error("workspace too small: %zu < %zu", workspace_bytes, dp.total); return SSCVAE_ERR_WORKSPACE; }
   const unsigned long long seed_host = seed;
   CUDA_TRY(cudaMemcpyAsync(reinterpret_cast<char*>(workspace) + dp.find("seed")->off, &seed_host, sizeof(seed_host),
@@ -389,9 +394,74 @@ int sscvae_decode_samples(SscvaeHandle* hh, int batch, int samples, int num_boxe
   char* wsb = reinterpret_cast<char*>(workspace);
   long long* best = reinterpret_cast<long long*>(wsb + dp.find("best_samples")->off);
   return run_with_graph(h->dec_graphs, key, st, true, [&](cudaStream_t s) {
-    return decode_impl(h, batch, samples, num_boxes, 1, 1, 1, reinterpret_cast<const char*>(packed), weights, image_features,
+    return decode_impl(h, batch, samples, num_boxes, 1, 1, 1, 1, false, reinterpret_cast<const char*>(packed), weights, image_features,
                        sentiment, obj_means, nullptr, nullptr, 0, eps, seed, wsb, workspace_bytes, reinterpret_cast<long long*>(predictions),
                        log_probs, best, n_steps, s);
+  });
+}
+
+// Constrained beam search per latent sample (the reference's loop over N_Z_SAMPLES, inference.py:138-167, with USE_CBS): every
+// (image, sample) pair is one search of S*K rows, group g = b*J + j. Each search stops on its own, as the reference's batch-1
+// call does (cbs.py:167 over that call's rows only).
+static bool samples_search_shape_ok(int batch, int samples, int num_boxes, int states, int beam, int per_node, int fsm_per_sample) {
+  return batch > 0 && samples >= 1 && num_boxes > 0 && states >= 1 && states <= 32 && per_node >= 1 && per_node <= beam &&
+         beam <= 8 && (fsm_per_sample == 0 || fsm_per_sample == 1);
+}
+
+size_t sscvae_decode_samples_search_workspace_bytes(const SscvaeHandle* hh, int batch, int samples, int num_boxes, int states,
+                                                    int beam, int fsm_per_sample) {
+  Handle* h = const_cast<Handle*>(reinterpret_cast<const Handle*>(hh));
+  if (!h || !samples_search_shape_ok(batch, samples, num_boxes, states, beam, 1, fsm_per_sample)) return 0;
+  return h->decode_plan(batch, num_boxes, states, beam, samples, fsm_per_sample ? batch * samples : batch).total;
+}
+
+int sscvae_decode_samples_search_region(const SscvaeHandle* hh, int batch, int samples, int num_boxes, int states, int beam,
+                                        int fsm_per_sample, const char* name, size_t* offset, size_t* bytes) {
+  Handle* h = const_cast<Handle*>(reinterpret_cast<const Handle*>(hh));
+  REQUIRE(h && name && offset && bytes, "NULL argument");
+  REQUIRE(samples_search_shape_ok(batch, samples, num_boxes, states, beam, 1, fsm_per_sample),
+          "bad decode shape B=%d J=%d N=%d S=%d K=%d", batch, samples, num_boxes, states, beam);
+  const Region* r = h->decode_plan(batch, num_boxes, states, beam, samples, fsm_per_sample ? batch * samples : batch).find(name);
+  REQUIRE(r != nullptr, "unknown workspace region '%s'", name);
+  *offset = r->off; *bytes = r->bytes;
+  return 0;
+}
+
+int sscvae_decode_samples_search(SscvaeHandle* hh, int batch, int samples, int num_boxes, int states, int beam, int per_node,
+                                 const void* packed, const void* const* weights, const float* image_features,
+                                 const float* sentiment, const float* obj_means, const uint8_t* fsm, int fsm_per_sample,
+                                 const int64_t* num_constraints, int min_constraints_to_satisfy, const float* eps,
+                                 uint64_t seed, void* workspace, size_t workspace_bytes, int64_t* predictions,
+                                 float* log_probs, int64_t* best, int32_t* n_steps, void* stream) {
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  REQUIRE(h && packed && weights && image_features && workspace && predictions && log_probs && best && n_steps, "NULL argument");
+  REQUIRE(samples_search_shape_ok(batch, samples, num_boxes, states, beam, per_node, fsm_per_sample),
+          "bad decode shape B=%d J=%d N=%d S=%d K=%d P=%d fsm_per_sample=%d (1 <= S <= 32, 1 <= P <= K <= 8)", batch, samples,
+          num_boxes, states, beam, per_node, fsm_per_sample);
+  REQUIRE(states == 1 || fsm != nullptr, "an FSM is required for more than one state");
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const Plan& dp = h->decode_plan(batch, num_boxes, states, beam, samples, fsm_per_sample ? batch * samples : batch);
+  if (workspace_bytes < dp.total) { set_error("workspace too small: %zu < %zu", workspace_bytes, dp.total); return SSCVAE_ERR_WORKSPACE; }
+  const unsigned long long seed_host = seed;
+  CUDA_TRY(cudaMemcpyAsync(reinterpret_cast<char*>(workspace) + dp.find("seed")->off, &seed_host, sizeof(seed_host),
+                           cudaMemcpyHostToDevice, st));
+  std::vector<uint64_t> key;
+  for (uint64_t v : {(uint64_t)batch, (uint64_t)num_boxes, (uint64_t)samples, (uint64_t)states, (uint64_t)beam,
+                     (uint64_t)per_node, (uint64_t)fsm_per_sample, (uint64_t)min_constraints_to_satisfy, (uint64_t)0x5c5c,
+                     (uint64_t)workspace_bytes,
+                     (uint64_t)(h->opt_fsm_packed * 4 + h->opt_features_bf16 * 2 + h->opt_reuse_image_state)})
+    key_add(key, v);
+  for (const void* q : {packed, (const void*)image_features, (const void*)sentiment, (const void*)obj_means, (const void*)fsm,
+                        (const void*)num_constraints, (const void*)eps, (const void*)workspace, (const void*)predictions,
+                        (const void*)log_probs, (const void*)best, (const void*)n_steps})
+    key_add(key, q);
+  for (int i = 0; i < SSCVAE_W_COUNT; ++i) key_add(key, weights[i]);
+  return run_with_graph(h->dec_graphs, key, st, true, [&](cudaStream_t s) {
+    return decode_impl(h, batch, samples, num_boxes, states, beam, per_node, fsm_per_sample ? 1 : samples, true,
+                       reinterpret_cast<const char*>(packed), weights, image_features, sentiment, obj_means, fsm,
+                       reinterpret_cast<const long long*>(num_constraints), min_constraints_to_satisfy, eps, seed,
+                       reinterpret_cast<char*>(workspace), workspace_bytes, reinterpret_cast<long long*>(predictions),
+                       log_probs, reinterpret_cast<long long*>(best), n_steps, s);
   });
 }
 

@@ -41,7 +41,7 @@ struct Handle {
   Dims d;
   Plan pp;                 // packed weights
   Plan tp; int tp_B = -1, tp_N = -1;   // training workspace for the last (B,N)
-  Plan dp; int dp_B = -1, dp_N = -1, dp_S = -1, dp_K = -1, dp_J = -1;   // decode workspace
+  Plan dp; int dp_B = -1, dp_N = -1, dp_S = -1, dp_K = -1, dp_J = -1, dp_T = -1;   // decode workspace
   GraphCache fwd_graphs, bwd_graphs, dec_graphs;
   // per-handle options (sscvae_set_option), consumed by the following calls
   int opt_features_bf16 = 0;           // image_features pointers are bf16 (B,N,F) instead of fp32
@@ -49,7 +49,7 @@ struct Handle {
   int opt_persistent_bwd = 1;          // training: run the BPTT loop as the persistent kernel (recurrent_bwd.cu) when the shape fits
   int opt_fsm_packed = 0;              // decode: `fsm` is the (B,S,V) uint32 bit table, not the (B,S,S,V) uint8 tensor
   const Plan& train_plan(int B, int N);
-  const Plan& decode_plan(int B, int N, int S, int K, int J);
+  const Plan& decode_plan(int B, int N, int S, int K, int J, int fsm_tables);   // fsm_tables: (S,V) bit tables packed per call
 };
 
 }  // namespace sscvae

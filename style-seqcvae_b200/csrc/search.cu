@@ -10,6 +10,7 @@
 // log-probs. Algorithmic bytes per row-step: V*4 (log-probs) + V*4 (FSM word), streamed coalesced.
 #include "search.cuh"
 #include "prof.cuh"
+#include <algorithm>
 #include <climits>
 
 namespace sscvae {
@@ -116,7 +117,7 @@ __global__ void __launch_bounds__(128) search_rows_kernel(SearchRowsArgs a) {
   const int r = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (r >= a.R) return;
   const int lane = threadIdx.x & 31;
-  const int img = r / a.rows_per_image;
+  const int tab = r / (a.rows_per_image * (a.groups_per_fsm > 1 ? a.groups_per_fsm : 1));   // FSM table of the row's group
   const int s_from = (a.rows_per_image == 1) ? 0 : (r % a.rows_per_image) / a.K;
   const float* __restrict__ x = a.logp + (size_t)r * a.ld;
   const bool forced = a.last_tokens != nullptr && a.last_tokens[r] == a.end_index;   // cbs.py:177-181
@@ -146,7 +147,7 @@ __global__ void __launch_bounds__(128) search_rows_kernel(SearchRowsArgs a) {
     s = warp_sum(s);
     mx = m; lsum = logf(s);
   }
-  const uint32_t* __restrict__ bits = a.fsm_bits ? a.fsm_bits + ((size_t)img * a.S + s_from) * a.V : nullptr;
+  const uint32_t* __restrict__ bits = a.fsm_bits ? a.fsm_bits + ((size_t)tab * a.S + s_from) * a.V : nullptr;
   for (int c0 = 0; c0 < a.S; c0 += SC) {
     float val[SC][P]; int idx[SC][P];
 #pragma unroll
@@ -214,7 +215,7 @@ __global__ void __launch_bounds__(256) search_rows_block_kernel(SearchRowsArgs a
   __shared__ int ci[8][SC][P];
   const int r = blockIdx.x;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int img = r / a.rows_per_image;
+  const int tab = r / (a.rows_per_image * (a.groups_per_fsm > 1 ? a.groups_per_fsm : 1));   // FSM table of the row's group
   const int s_from = (a.rows_per_image == 1) ? 0 : (r % a.rows_per_image) / a.K;
   const float4* __restrict__ x4 = reinterpret_cast<const float4*>(a.logp + (size_t)r * a.ld);
   float4* s4 = reinterpret_cast<float4*>(srow);
@@ -250,7 +251,7 @@ __global__ void __launch_bounds__(256) search_rows_block_kernel(SearchRowsArgs a
   }
   __syncthreads();
   const uint4* __restrict__ b4 = a.fsm_bits
-      ? reinterpret_cast<const uint4*>(a.fsm_bits + ((size_t)img * a.S + s_from) * a.V) : nullptr;
+      ? reinterpret_cast<const uint4*>(a.fsm_bits + ((size_t)tab * a.S + s_from) * a.V) : nullptr;
   const float add = a.last_scores ? a.last_scores[r] : 0.f;
   for (int c0 = 0; c0 < a.S; c0 += SC) {
     float val[SC][P]; int idx[SC][P];
@@ -418,34 +419,37 @@ int search_merge(cudaStream_t st, const float* cand_val, const int32_t* cand_tok
 }
 
 // n_steps = the number of steps the reference's loop would have produced (cbs.py:161-168): it stops
-// before step t when every token of step t-1 is the boundary token.
-__global__ void search_nsteps_kernel(const int32_t* __restrict__ tokens_hist, int steps_run, int R, int end_index,
-                                     int32_t* __restrict__ n_steps) {
+// before step t when every token of step t-1 is the boundary token. Block x decides for rows [x*rows, (x+1)*rows): one
+// block over all rows is the batch-wide exit, one block per search group the exit of each search on its own.
+__global__ void search_nsteps_kernel(const int32_t* __restrict__ tokens_hist, int steps_run, int R, int rows,
+                                     int end_index, int32_t* __restrict__ n_steps) {
   __shared__ int not_end;
+  const int r0 = blockIdx.x * rows;
   int n = steps_run;
   for (int t = 1; t < steps_run; ++t) {
     if (threadIdx.x == 0) not_end = 0;
     __syncthreads();
     int local = 0;
-    for (int r = threadIdx.x; r < R; r += blockDim.x) local |= (tokens_hist[(size_t)(t - 1) * R + r] != end_index);
+    for (int r = threadIdx.x; r < rows; r += blockDim.x) local |= (tokens_hist[(size_t)(t - 1) * R + r0 + r] != end_index);
     if (local) atomicOr(&not_end, 1);
     __syncthreads();
     const int ne = not_end;
     __syncthreads();
     if (!ne) { n = t; break; }
   }
-  if (threadIdx.x == 0) *n_steps = n;
+  if (threadIdx.x == 0) n_steps[blockIdx.x] = n;
 }
 
 __global__ void search_finish_kernel(const int32_t* __restrict__ tokens_hist, const int32_t* __restrict__ backptr_hist,
                                      const float* __restrict__ scores_hist, int steps_run, int B, int S, int K,
                                      int end_index, const long long* __restrict__ num_constraints, int min_sat,
-                                     long long* __restrict__ predictions, float* __restrict__ final_scores,
-                                     long long* __restrict__ best, const int32_t* __restrict__ n_steps) {
+                                     int groups_per_table, int groups_per_exit, long long* __restrict__ predictions,
+                                     float* __restrict__ final_scores, long long* __restrict__ best,
+                                     const int32_t* __restrict__ n_steps) {
   extern __shared__ float s_score[];                        // S*K
   const int b = blockIdx.x;
   const int SK = S * K, R = B * SK;
-  const int n = *n_steps;
+  const int n = n_steps[groups_per_exit > 0 ? b / groups_per_exit : 0];
   for (int w = threadIdx.x; w < SK; w += blockDim.x) {
     long long* out = predictions + ((size_t)b * SK + w) * steps_run;
     const size_t base = (size_t)b * SK;
@@ -467,7 +471,7 @@ __global__ void search_finish_kernel(const int32_t* __restrict__ tokens_hist, co
   if (threadIdx.x == 0) {
     int best_state = 0;
     if (num_constraints) {                                  // decoding.py:82-86,128-134 (cbs_simple)
-      const int nc = (int)num_constraints[b];
+      const int nc = (int)num_constraints[groups_per_table > 1 ? b / groups_per_table : b];
       const int need = nc < min_sat ? nc : min_sat;
       float bv = 0.f; bool have = false;
       for (int s = 0; s < (1 << nc) && s < S; ++s) {
@@ -483,13 +487,23 @@ __global__ void search_finish_kernel(const int32_t* __restrict__ tokens_hist, co
 
 int search_finish(cudaStream_t st, const int32_t* tokens_hist, const int32_t* backptr_hist, const float* scores_hist,
                   int steps_run, int B, int S, int K, int end_index, const long long* num_constraints, int min_sat,
-                  long long* predictions, float* final_scores, long long* best, int32_t* n_steps) {
+                  int groups_per_table, int groups_per_exit, long long* predictions, float* final_scores, long long* best,
+                  int32_t* n_steps) {
   REQUIRE(steps_run >= 1, "no search steps");
-  search_nsteps_kernel<<<1, 1024, 0, st>>>(tokens_hist, steps_run, B * S * K, end_index, n_steps);
+  REQUIRE(groups_per_exit >= 0 && (groups_per_exit == 0 || B % groups_per_exit == 0), "bad exit grouping %d of %d groups",
+          groups_per_exit, B);
+  const int R = B * S * K;
+  if (groups_per_exit == 0) {
+    search_nsteps_kernel<<<1, 1024, 0, st>>>(tokens_hist, steps_run, R, R, end_index, n_steps);
+  } else {
+    const int rows = groups_per_exit * S * K;
+    search_nsteps_kernel<<<B / groups_per_exit, std::min(1024, ceil_div(rows, 32) * 32), 0, st>>>(tokens_hist, steps_run, R,
+                                                                                                  rows, end_index, n_steps);
+  }
   LAUNCHED();
   search_finish_kernel<<<B, 128, S * K * sizeof(float), st>>>(tokens_hist, backptr_hist, scores_hist, steps_run, B, S, K,
-                                                            end_index, num_constraints, min_sat, predictions,
-                                                            final_scores, best, n_steps);
+                                                            end_index, num_constraints, min_sat, groups_per_table,
+                                                            groups_per_exit, predictions, final_scores, best, n_steps);
   LAUNCHED();
   return 0;
 }

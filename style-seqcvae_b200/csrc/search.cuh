@@ -16,12 +16,14 @@ int select_best_masked(cudaStream_t st, const long long* predictions, const floa
 // Per row r and to-state i: the P best words by (value desc, word index asc), where
 //   value(w) = allowed(from_state(r), i, w) ? logp[r,w] : neg_value        (+ last_scores[r] afterwards)
 // and rows whose previous token is `end_index` are forced to the one-hot row (0 at end, -inf elsewhere).
-// rows_per_image = S*K (1 at the first step: every row is state 0). Output (R,S,P).
+// rows_per_image = S*K (1 at the first step: every row is state 0): row r belongs to search group r / rows_per_image, whose
+// FSM table is group / groups_per_fsm (0 or 1: one table per group; J: the J samples of an image share one). Output (R,S,P).
 struct SearchRowsArgs {
   const float* logp; int ld; int V;
   int normalized;                 // 0: raw logits, log-softmax fused
-  const uint32_t* fsm_bits;       // (B,S,V) or null (everything allowed)
+  const uint32_t* fsm_bits;       // (tables,S,V) or null (everything allowed)
   int R, S, K, rows_per_image, P;
+  int groups_per_fsm;             // search groups per FSM table; 0 = 1
   int end_index;
   const int32_t* last_tokens;     // (R) or null
   const float* last_scores;       // (R) or null
@@ -35,9 +37,13 @@ int search_rows(cudaStream_t st, const SearchRowsArgs& a);
 int search_merge(cudaStream_t st, const float* cand_val, const int32_t* cand_tok, int B, int S, int K, int P,
                  int32_t* tokens, int32_t* backptr, float* scores);
 
+// Back-trace, early exit and best beam of B search groups of S*K rows. Group b reads num_constraints[b / groups_per_table].
+// groups_per_exit = 0: one exit for the whole batch (n_steps[0], the reference's batched loop, cbs.py:167); g > 0: one exit
+// per set of g consecutive groups (n_steps[b / g]); 1 = every search stops on its own, as a batch-1 call would.
 int search_finish(cudaStream_t st, const int32_t* tokens_hist, const int32_t* backptr_hist, const float* scores_hist,
                   int steps_run, int B, int S, int K, int end_index, const long long* num_constraints, int min_sat,
-                  long long* predictions, float* final_scores, long long* best, int32_t* n_steps);
+                  int groups_per_table, int groups_per_exit, long long* predictions, float* final_scores, long long* best,
+                  int32_t* n_steps);
 
 // new_state[r] = old_state[img(r)*SK + bp[r]] for the four recurrent tensors of the eval cell
 int state_gather(cudaStream_t st, const int32_t* bp, int R, int SK, const bf16* xa_src, bf16* xa_dst, int ld_xa,
