@@ -318,6 +318,16 @@ int sscvae_test_gemm(const void* A, int lda, const void* B, int ldb, int M, int 
 int sscvae_test_gemm_splitk(const void* A, int lda, const void* B, int ldb, int M, int N, int K, float* C32, int ldc,
                             int splits, const float* bias, void* stream);
 
+/* the grouped weight-gradient GEMM: nprob (1..8) problems C32_i[M_i, N_i] = A_i[M_i, K_i] * B_i[N_i, K_i]^T (bf16, plain
+ * fp32 store with row pitch ldc_i) in one launch of the CTA-pair kernel, for unit tests and tools/wgrad_bench.py */
+int sscvae_test_gemm_grouped(int nprob, const void* const* A, const int* lda, const void* const* B, const int* ldb,
+                             const int* M, const int* N, const int* K, float* const* C32, const int* ldc, void* stream);
+
+/* the job-table bf16 transpose of the weight-gradient phase: for each of njobs (1..8) jobs, out[c, r] = in[r, c] for
+ * c < cols, r < ld_out, zero for r >= rows; one launch. ld_in, ld_out multiples of 8, bases 16-byte aligned. */
+int sscvae_test_transpose_bf16(int njobs, const void* const* in, const int* rows, const int* cols, const int* ld_in,
+                               void* const* out, const int* ld_out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -45,7 +45,7 @@ SYMBOLS = [
     "sscvae_decode_workspace_bytes", "sscvae_decode", "sscvae_decode_region", "sscvae_decode_samples_workspace_bytes",
     "sscvae_decode_samples", "sscvae_decode_samples_search_workspace_bytes", "sscvae_decode_samples_search",
     "sscvae_decode_samples_search_region", "sscvae_grad_sqnorm", "sscvae_sgd_step", "sscvae_test_gemm",
-    "sscvae_profile_enable", "sscvae_profile_report",
+    "sscvae_profile_enable", "sscvae_profile_report", "sscvae_test_gemm_grouped", "sscvae_test_transpose_bf16",
 ]
 
 
@@ -113,6 +113,10 @@ def lib():
     L.sscvae_grad_sqnorm.argtypes = [vp, sz, vp, vp, vp]
     L.sscvae_sgd_step.argtypes = [vp, vp, vp, sz, vp, f32, f32, f32, f32, i32, vp]
     L.sscvae_test_gemm.argtypes = [vp, i32, vp, i32, i32, i32, i32, vp, i32, vp, i32, i32, vp]
+    L.sscvae_test_gemm_grouped.argtypes = [i32, C.POINTER(vp), C.POINTER(i32), C.POINTER(vp), C.POINTER(i32),
+                                           C.POINTER(i32), C.POINTER(i32), C.POINTER(i32), C.POINTER(vp), C.POINTER(i32), vp]
+    L.sscvae_test_transpose_bf16.argtypes = [i32, C.POINTER(vp), C.POINTER(i32), C.POINTER(i32), C.POINTER(i32),
+                                             C.POINTER(vp), C.POINTER(i32), vp]
     L.sscvae_set_option.argtypes = [vp, C.c_char_p, i32]
     L.sscvae_train_backward_is_persistent.argtypes = [vp, i32, i32]
     L.sscvae_debug_bptt_tiling.argtypes = [vp, i32, i32, i32, C.POINTER(i32)]

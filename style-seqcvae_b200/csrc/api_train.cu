@@ -621,9 +621,14 @@ static int train_backward_impl(Handle* h, int B, int N, const char* pk, const vo
     TRY(gemm_bf16_tn(s, TB, H, 1, &sg, e));
   }
   // head weight gradients are final before the time loop starts
-  TRY(transpose_bf16(s, hdec_all, TB, H, 2 * Hp, Wb("hdecTc"), TBp));
+  TransposeJobList tj;
+  TRY(tj.add(hdec_all, TB, H, 2 * Hp, Wb("hdecTc"), TBp));
+  if (Gr(SSCVAE_W_OUT_PROJ_W) || Gr(SSCVAE_W_OUT_PROJ_B)) {
+    if (d.tied) TRY(tj.add(Wb("dpreo"), TB, E, d.Ep, Wb("dpreoT"), TBp));
+    else TRY(tj.add(Wb("dlogits"), TB, V, d.Vp, Wb("dlogitsT"), TBp));
+  }
+  TRY(transpose_bf16_jobs(s, tj));
   if (d.tied) {
-    if (Gr(SSCVAE_W_OUT_PROJ_W) || Gr(SSCVAE_W_OUT_PROJ_B)) TRY(transpose_bf16(s, Wb("dpreo"), TB, E, d.Ep, Wb("dpreoT"), TBp));
     if (Gr(SSCVAE_W_OUT_PROJ_W)) {
       GemmSeg sg = seg(Wb("dpreoT"), TBp, Wb("hdecTc"), TBp, TB);
       GemmEpi e; e.tag = "gemm.head_bwd"; e.C32 = Gr(SSCVAE_W_OUT_PROJ_W); e.ldc32 = H;
@@ -631,7 +636,6 @@ static int train_backward_impl(Handle* h, int B, int N, const char* pk, const vo
     }
     if (Gr(SSCVAE_W_OUT_PROJ_B)) TRY(rowsum_bf16(s, Wb("dpreoT"), E, TB, TBp, Gr(SSCVAE_W_OUT_PROJ_B), 0));
   } else {
-    if (Gr(SSCVAE_W_OUT_PROJ_W) || Gr(SSCVAE_W_OUT_PROJ_B)) TRY(transpose_bf16(s, Wb("dlogits"), TB, V, d.Vp, Wb("dlogitsT"), TBp));
     if (Gr(SSCVAE_W_OUT_PROJ_W)) {
       GemmSeg sg = seg(Wb("dlogitsT"), TBp, Wb("hdecTc"), TBp, TB);
       GemmEpi e; e.tag = "gemm.head_bwd"; e.C32 = Gr(SSCVAE_W_OUT_PROJ_W); e.ldc32 = H;
@@ -748,13 +752,22 @@ static int train_backward_impl(Handle* h, int B, int N, const char* pk, const vo
     }
   }
 
-  // ---- weight gradients: one GEMM per weight block over all T*B rows (K = T*B). The GEMMs of one LSTM share the
-  //      transposed gate-gradient operand dGT.
-  auto wgrad = [&](const bf16* AT, int M, const bf16* BT, int Ncols, int K, int ldk, float* C, int ldc) -> int {
+  // ---- weight gradients: one GEMM problem per weight block over all T*B rows (K = T*B). Per gradient group: one
+  //      launch transposes the group's operands, one grouped GEMM launch computes all its weight blocks (the blocks of
+  //      one LSTM share the transposed gate-gradient operand dGT), then the bias sums and the W_hh copy.
+  bf16* dGT = Wb("dGT");
+  GemmProblem pb[kMaxGemmProblems];
+  int np = 0;
+  auto wgrad_add = [&](const bf16* AT, int M, const bf16* BT, int Ncols, int K, int ldk, float* C, int ldc) -> int {
     if (!C) return 0;
-    GemmSeg sg = seg(AT, ldk, BT, ldk, K);
-    GemmEpi e; e.tag = "gemm.wgrad"; e.C32 = C; e.ldc32 = ldc;
-    return gemm_bf16_tn(s, M, Ncols, 1, &sg, e);
+    REQUIRE(np < kMaxGemmProblems, "weight-gradient group exceeds %d GEMM problems", kMaxGemmProblems);
+    pb[np++] = GemmProblem{AT, ldk, BT, ldk, K, M, Ncols, C, ldc};
+    return 0;
+  };
+  auto wgrad_launch = [&]() -> int {
+    const int n = np;
+    np = 0;
+    return gemm_bf16_tn_grouped(s, n, pb, "gemm.wgrad");
   };
   // b_ih and b_hh get the same gradient (both are added to the gates): one row sum, copied
   auto bias_pair = [&](const bf16* dGT_, int ib, int ih) -> int {
@@ -764,85 +777,109 @@ static int train_backward_impl(Handle* h, int B, int N, const char* pk, const vo
     if (g1 && g2) CUDA_TRY(cudaMemcpyAsync(g2, g1, (size_t)G * sizeof(float), cudaMemcpyDeviceToDevice, s));
     return 0;
   };
+  // The forward folds W_hh onto the W_ih column block that multiplies the same operand (packed weights), so the two
+  // gradients are one product: computed into W_ih's block when both are wanted and copied to W_hh afterwards (hh_copy:
+  // column `col` of W_ih, row pitch ld_ih), otherwise straight into the one that is wanted.
+  auto hh_pair = [&](const bf16* BT, int ih, int hh) -> int {
+    if (Gr(ih)) return 0;                               // W_ih's block is a problem of the group already
+    return wgrad_add(dGT, G, BT, H, TB, TBp, Gr(hh), H);
+  };
+  auto hh_copy = [&](int ih, int col, int ld_ih, int hh) -> int {
+    if (Gr(ih) && Gr(hh))
+      CUDA_TRY(cudaMemcpy2DAsync(Gr(hh), (size_t)H * sizeof(float), Gr(ih) + col, (size_t)ld_ih * sizeof(float),
+                                 (size_t)H * sizeof(float), G, cudaMemcpyDeviceToDevice, s));
+    return 0;
+  };
   auto any = [&](std::initializer_list<int> ids) { for (int i : ids) if (gv[i]) return true; return false; };
-  bf16* dGT = Wb("dGT");
-  TRY(transpose_bf16(s, Wb("XE"), TB, KX, KX, Wb("XET"), TBp));                   // xhat_t, h1_t, h_dec_{t-1}
-  const bf16* xhatT = Wb("XET");
+  const bf16* xhatT = Wb("XET");                                                  // xhat_t, h1_t, h_dec_{t-1}
   const bf16* h1T = Wb("XET") + (size_t)Fp * TBp;
   const bf16* hdecpT = Wb("XET") + (size_t)(Fp + Hp) * TBp;
+  const bf16* condT = Wb("ZBT") + (size_t)d.Zp * TBp;   // z_t (and, sentiment_vae == 2, the conditioning block c_t behind it)
   const float* sentv = Wf("sent");
   const int ldE = F + 2 * H + c, ldD = F + 2 * H + c + Z, ldA = E + F + 2 * H;
 
-  // z_t (and, sentiment_vae == 2, the conditioning block c_t behind it) transposed
-  if (Gr(SSCVAE_W_DEC_IH) || (d.cvar && Gr(SSCVAE_W_ENC_IH))) TRY(transpose_bf16(s, Wb("ZB"), TB, d.ZC, d.ZC, Wb("ZBT"), TBp));
-  const bf16* condT = Wb("ZBT") + (size_t)d.Zp * TBp;
   // group 1: decoder LSTM. W_ih column blocks [xhat | h1 | h_dec | cond | z]; W_hh shares the h_dec operand.
-  if (any({SSCVAE_W_DEC_IH, SSCVAE_W_DEC_HH, SSCVAE_W_DEC_BIH, SSCVAE_W_DEC_BHH})) {
-    TRY(transpose_bf16(s, Wb("dG_dec"), TB, G, Gp, dGT, TBp));
+  TRY(tj.add(Wb("XE"), TB, KX, KX, Wb("XET"), TBp));
+  if (Gr(SSCVAE_W_DEC_IH) || (d.cvar && Gr(SSCVAE_W_ENC_IH))) TRY(tj.add(Wb("ZB"), TB, d.ZC, d.ZC, Wb("ZBT"), TBp));
+  const bool dec = any({SSCVAE_W_DEC_IH, SSCVAE_W_DEC_HH, SSCVAE_W_DEC_BIH, SSCVAE_W_DEC_BHH});
+  if (dec) TRY(tj.add(Wb("dG_dec"), TB, G, Gp, dGT, TBp));
+  TRY(transpose_bf16_jobs(s, tj));
+  if (dec) {
     float* g = Gr(SSCVAE_W_DEC_IH);
     if (g) {
-      TRY(wgrad(dGT, G, xhatT, F, TB, TBp, g, ldD));
-      TRY(wgrad(dGT, G, h1T, H, TB, TBp, g + F, ldD));
-      TRY(wgrad(dGT, G, hdecpT, H, TB, TBp, g + F + H, ldD));
-      TRY(wgrad(dGT, G, Wb("ZBT"), Z, TB, TBp, g + F + 2 * H + c, ldD));
-      if (c && !d.cvar) TRY(rowdot_bf16(s, dGT, G, TB, TBp, sentv, B, g + F + 2 * H, ldD));
-      if (d.cvar) TRY(wgrad(dGT, G, condT, c, TB, TBp, g + F + 2 * H, ldD));
+      TRY(wgrad_add(dGT, G, xhatT, F, TB, TBp, g, ldD));
+      TRY(wgrad_add(dGT, G, h1T, H, TB, TBp, g + F, ldD));
+      TRY(wgrad_add(dGT, G, hdecpT, H, TB, TBp, g + F + H, ldD));
+      TRY(wgrad_add(dGT, G, Wb("ZBT"), Z, TB, TBp, g + F + 2 * H + c, ldD));
+      if (d.cvar) TRY(wgrad_add(dGT, G, condT, c, TB, TBp, g + F + 2 * H, ldD));
     }
-    TRY(wgrad(dGT, G, hdecpT, H, TB, TBp, Gr(SSCVAE_W_DEC_HH), H));
+    TRY(hh_pair(hdecpT, SSCVAE_W_DEC_IH, SSCVAE_W_DEC_HH));
+    TRY(wgrad_launch());
+    if (g && c && !d.cvar) TRY(rowdot_bf16(s, dGT, G, TB, TBp, sentv, B, g + F + 2 * H, ldD));
     TRY(bias_pair(dGT, SSCVAE_W_DEC_BIH, SSCVAE_W_DEC_BHH));
+    TRY(hh_copy(SSCVAE_W_DEC_IH, F + H, ldD, SSCVAE_W_DEC_HH));
   }
   TRY(event(1));
 
   // group 2: encoder LSTM + latent heads
-  if (any({SSCVAE_W_ENC_IH, SSCVAE_W_ENC_HH, SSCVAE_W_ENC_BIH, SSCVAE_W_ENC_BHH})) {
-    TRY(transpose_bf16(s, Wb("dG_enc"), TB, G, Gp, dGT, TBp));
-    if (Gr(SSCVAE_W_ENC_HH)) TRY(transpose_bf16(s, Wb("HE"), TB, Hp, Hp, Wb("HETp"), TBp));   // h_enc_{t-1}
-    float* g = Gr(SSCVAE_W_ENC_IH);
-    if (g) {
-      TRY(wgrad(dGT, G, xhatT, F, TB, TBp, g, ldE));
-      TRY(wgrad(dGT, G, h1T, H, TB, TBp, g + F, ldE));
-      TRY(wgrad(dGT, G, hdecpT, H, TB, TBp, g + F + H, ldE));
-      if (c && !d.cvar) TRY(rowdot_bf16(s, dGT, G, TB, TBp, sentv, B, g + F + 2 * H, ldE));
-      if (d.cvar) TRY(wgrad(dGT, G, condT, c, TB, TBp, g + F + 2 * H, ldE));
-    }
-    TRY(wgrad(dGT, G, Wb("HETp"), H, TB, TBp, Gr(SSCVAE_W_ENC_HH), H));
-    TRY(bias_pair(dGT, SSCVAE_W_ENC_BIH, SSCVAE_W_ENC_BHH));
+  const bool enc = any({SSCVAE_W_ENC_IH, SSCVAE_W_ENC_HH, SSCVAE_W_ENC_BIH, SSCVAE_W_ENC_BHH});
+  const bool fc = any({SSCVAE_W_FC_MEAN_W, SSCVAE_W_FC_MEAN_B, SSCVAE_W_FC_LOGVAR_W, SSCVAE_W_FC_LOGVAR_B});
+  if (enc) {
+    TRY(tj.add(Wb("dG_enc"), TB, G, Gp, dGT, TBp));
+    if (Gr(SSCVAE_W_ENC_HH)) TRY(tj.add(Wb("HE"), TB, Hp, Hp, Wb("HETp"), TBp));             // h_enc_{t-1}
   }
-  if (any({SSCVAE_W_FC_MEAN_W, SSCVAE_W_FC_MEAN_B, SSCVAE_W_FC_LOGVAR_W, SSCVAE_W_FC_LOGVAR_B})) {
-    TRY(transpose_bf16(s, Wb("dml"), TB, d.Z2p, d.Z2p, Wb("dmlT"), TBp));
-    TRY(transpose_bf16(s, Wb("HE") + (size_t)B * Hp, TB, Hp, Hp, Wb("HETc"), TBp));   // h_enc_t
-    const bf16* dmT = Wb("dmlT");
-    const bf16* dlT = Wb("dmlT") + (size_t)Z * TBp;
-    TRY(wgrad(dmT, Z, Wb("HETc"), H, TB, TBp, Gr(SSCVAE_W_FC_MEAN_W), H));
-    TRY(wgrad(dlT, Z, Wb("HETc"), H, TB, TBp, Gr(SSCVAE_W_FC_LOGVAR_W), H));
-    if (Gr(SSCVAE_W_FC_MEAN_B)) TRY(rowsum_bf16(s, dmT, Z, TB, TBp, Gr(SSCVAE_W_FC_MEAN_B), 0));
-    if (Gr(SSCVAE_W_FC_LOGVAR_B)) TRY(rowsum_bf16(s, dlT, Z, TB, TBp, Gr(SSCVAE_W_FC_LOGVAR_B), 0));
+  if (fc) {
+    TRY(tj.add(Wb("dml"), TB, d.Z2p, d.Z2p, Wb("dmlT"), TBp));
+    TRY(tj.add(Wb("HE") + (size_t)B * Hp, TB, Hp, Hp, Wb("HETc"), TBp));                     // h_enc_t
   }
+  TRY(transpose_bf16_jobs(s, tj));
+  const bf16* dmT = Wb("dmlT");
+  const bf16* dlT = Wb("dmlT") + (size_t)Z * TBp;
+  float* ge = enc ? Gr(SSCVAE_W_ENC_IH) : nullptr;
+  if (ge) {
+    TRY(wgrad_add(dGT, G, xhatT, F, TB, TBp, ge, ldE));
+    TRY(wgrad_add(dGT, G, h1T, H, TB, TBp, ge + F, ldE));
+    TRY(wgrad_add(dGT, G, hdecpT, H, TB, TBp, ge + F + H, ldE));
+    if (d.cvar) TRY(wgrad_add(dGT, G, condT, c, TB, TBp, ge + F + 2 * H, ldE));
+  }
+  if (enc) TRY(wgrad_add(dGT, G, Wb("HETp"), H, TB, TBp, Gr(SSCVAE_W_ENC_HH), H));
+  if (fc) {
+    TRY(wgrad_add(dmT, Z, Wb("HETc"), H, TB, TBp, Gr(SSCVAE_W_FC_MEAN_W), H));
+    TRY(wgrad_add(dlT, Z, Wb("HETc"), H, TB, TBp, Gr(SSCVAE_W_FC_LOGVAR_W), H));
+  }
+  TRY(wgrad_launch());
+  if (ge && c && !d.cvar) TRY(rowdot_bf16(s, dGT, G, TB, TBp, sentv, B, ge + F + 2 * H, ldE));
+  if (enc) TRY(bias_pair(dGT, SSCVAE_W_ENC_BIH, SSCVAE_W_ENC_BHH));
+  if (fc && Gr(SSCVAE_W_FC_MEAN_B)) TRY(rowsum_bf16(s, dmT, Z, TB, TBp, Gr(SSCVAE_W_FC_MEAN_B), 0));
+  if (fc && Gr(SSCVAE_W_FC_LOGVAR_B)) TRY(rowsum_bf16(s, dlT, Z, TB, TBp, Gr(SSCVAE_W_FC_LOGVAR_B), 0));
   TRY(event(2));
 
   // group 3: attention LSTM. W_ih column blocks [emb | avg | h1 | h_dec]; W_hh shares the h1 operand.
   const bool need_demb = !d.tied && Gr(SSCVAE_W_EMBEDDING);
   if (need_demb || any({SSCVAE_W_ATT_IH, SSCVAE_W_ATT_HH, SSCVAE_W_ATT_BIH, SSCVAE_W_ATT_BHH})) {
-    TRY(transpose_bf16(s, Wb("dG_att"), TB, G, Gp, dGT, TBp));
-    TRY(transpose_bf16(s, Wb("XA"), TB, 2 * Hp, 2 * Hp, Wb("XAT"), TBp));           // h1_{t-1}, h_dec_{t-1}
-    const bf16* h1pT = Wb("XAT");
+    const bf16* h1pT = Wb("XAT");                                                 // h1_{t-1}, h_dec_{t-1}
     const bf16* hdecp2T = Wb("XAT") + (size_t)Hp * TBp;
     float* g = Gr(SSCVAE_W_ATT_IH);
+    // mean-feature block: the operand is constant over time, so sum the gate gradients over t first
+    if (g) TRY(timesum_bf16(s, Wb("dG_att"), T, B, G, Gp, Wb("dGsum"), Gp));
+    TRY(tj.add(Wb("dG_att"), TB, G, Gp, dGT, TBp));
+    TRY(tj.add(Wb("XA"), TB, 2 * Hp, 2 * Hp, Wb("XAT"), TBp));
     if (g) {
-      TRY(transpose_bf16(s, Wb("embb_t"), TB, d.Ep, d.Ep, Wb("embT_t"), TBp));
-      // mean-feature block: the operand is constant over time, so sum the gate gradients over t first
-      TRY(timesum_bf16(s, Wb("dG_att"), T, B, G, Gp, Wb("dGsum"), Gp));
-      TRY(transpose_bf16(s, Wb("dGsum"), B, G, Gp, Wb("dGsumT"), Bp));
-      TRY(transpose_bf16(s, Wb("avgb"), B, Fp, Fp, Wb("avgT"), Bp));
+      TRY(tj.add(Wb("embb_t"), TB, d.Ep, d.Ep, Wb("embT_t"), TBp));
+      TRY(tj.add(Wb("dGsum"), B, G, Gp, Wb("dGsumT"), Bp));
+      TRY(tj.add(Wb("avgb"), B, Fp, Fp, Wb("avgT"), Bp));
     }
+    TRY(transpose_bf16_jobs(s, tj));
     if (g) {
-      TRY(wgrad(dGT, G, Wb("embT_t"), E, TB, TBp, g, ldA));
-      TRY(wgrad(Wb("dGsumT"), G, Wb("avgT"), F, B, Bp, g + E, ldA));
-      TRY(wgrad(dGT, G, h1pT, H, TB, TBp, g + E + F, ldA));
-      TRY(wgrad(dGT, G, hdecp2T, H, TB, TBp, g + E + F + H, ldA));
+      TRY(wgrad_add(dGT, G, Wb("embT_t"), E, TB, TBp, g, ldA));
+      TRY(wgrad_add(Wb("dGsumT"), G, Wb("avgT"), F, B, Bp, g + E, ldA));
+      TRY(wgrad_add(dGT, G, h1pT, H, TB, TBp, g + E + F, ldA));
+      TRY(wgrad_add(dGT, G, hdecp2T, H, TB, TBp, g + E + F + H, ldA));
     }
-    TRY(wgrad(dGT, G, h1pT, H, TB, TBp, Gr(SSCVAE_W_ATT_HH), H));
+    TRY(hh_pair(h1pT, SSCVAE_W_ATT_IH, SSCVAE_W_ATT_HH));
+    TRY(wgrad_launch());
     TRY(bias_pair(dGT, SSCVAE_W_ATT_BIH, SSCVAE_W_ATT_BHH));
+    TRY(hh_copy(SSCVAE_W_ATT_IH, E + F, ldA, SSCVAE_W_ATT_HH));
     if (need_demb) {  // learned embedding (untied): d emb rows = dG_att W_att_ih[:, :E], scattered by token id
       GemmSeg sg = seg(Wb("dG_att"), Gp, Pb("w_att_eT"), Gp, G);
       GemmEpi e; e.tag = "gemm.wgrad"; e.C32 = Wf("dxemb"); e.ldc32 = E;
@@ -854,20 +891,20 @@ static int train_backward_impl(Handle* h, int B, int N, const char* pk, const vo
   TRY(event(3));
 
   // group 4: attention module
-  if (Gr(SSCVAE_W_QUERY_PROJ)) {
-    TRY(transpose_bf16(s, Wb("dqb"), TB, d.Ap, d.Ap, Wb("dqT"), TBp));
-    TRY(wgrad(Wb("dqT"), A, h1T, H, TB, TBp, Gr(SSCVAE_W_QUERY_PROJ), H));
-  }
   if (Gr(SSCVAE_W_IMAGE_PROJ) || Gr(SSCVAE_W_ATT_VEC)) {
     // d P and d w_a for all timesteps at once (the per-step kernel only kept the score gradients d u)
     aa.q = Wf("q");
     TRY(attention_backward_deferred(s, aa, T, Wf("q"), Wf("du"), Wf("dproj_acc"), Wf("dwa_acc")));
   }
+  if (Gr(SSCVAE_W_QUERY_PROJ)) TRY(tj.add(Wb("dqb"), TB, d.Ap, d.Ap, Wb("dqT"), TBp));
   if (Gr(SSCVAE_W_IMAGE_PROJ)) {
+    TRY(tj.add(Wb("featsb"), BN, Fp, Fp, Wb("featsT"), BNp));
     TRY(transpose_f32_to_bf16(s, Wf("dproj_acc"), BN, A, A, Wb("dPT"), BNp));
-    TRY(transpose_bf16(s, Wb("featsb"), BN, Fp, Fp, Wb("featsT"), BNp));
-    TRY(wgrad(Wb("dPT"), A, Wb("featsT"), F, BN, BNp, Gr(SSCVAE_W_IMAGE_PROJ), F));
   }
+  TRY(transpose_bf16_jobs(s, tj));
+  TRY(wgrad_add(Wb("dqT"), A, h1T, H, TB, TBp, Gr(SSCVAE_W_QUERY_PROJ), H));
+  TRY(wgrad_add(Wb("dPT"), A, Wb("featsT"), F, BN, BNp, Gr(SSCVAE_W_IMAGE_PROJ), F));
+  TRY(wgrad_launch());
   if (Gr(SSCVAE_W_ATT_VEC)) TRY(colsum_f32(s, Wf("dwa_acc"), B, A, A, Gr(SSCVAE_W_ATT_VEC)));
   TRY(event(4));
   return 0;
@@ -1014,6 +1051,33 @@ int sscvae_test_gemm_splitk(const void* A, int lda, const void* B, int ldb, int 
   int repeat = 1;
   if (const char* r = getenv("SSCVAE_TEST_GEMM_REPEAT")) repeat = std::max(1, atoi(r));
   for (int i = 0; i < repeat; ++i) TRY(gemm_bf16_tn(st, M, N, 1, &sg, e));
+  return 0;
+}
+
+int sscvae_test_gemm_grouped(int nprob, const void* const* A, const int* lda, const void* const* B, const int* ldb,
+                             const int* M, const int* N, const int* K, float* const* C32, const int* ldc, void* stream) {
+  REQUIRE(nprob >= 1 && nprob <= kMaxGemmProblems && A && lda && B && ldb && M && N && K && C32 && ldc, "bad argument");
+  GemmProblem pb[kMaxGemmProblems];
+  for (int i = 0; i < nprob; ++i)
+    pb[i] = GemmProblem{reinterpret_cast<const bf16*>(A[i]), lda[i], reinterpret_cast<const bf16*>(B[i]), ldb[i], K[i], M[i],
+                        N[i], C32[i], ldc[i]};
+  int repeat = 1;
+  if (const char* r = getenv("SSCVAE_TEST_GEMM_REPEAT")) repeat = std::max(1, atoi(r));
+  for (int i = 0; i < repeat; ++i) TRY(gemm_bf16_tn_grouped(reinterpret_cast<cudaStream_t>(stream), nprob, pb, "gemm.wgrad"));
+  return 0;
+}
+
+int sscvae_test_transpose_bf16(int njobs, const void* const* in, const int* rows, const int* cols, const int* ld_in,
+                               void* const* out, const int* ld_out, void* stream) {
+  REQUIRE(njobs >= 1 && njobs <= kMaxTransposeJobs && in && rows && cols && ld_in && out && ld_out, "bad argument");
+  int repeat = 1;
+  if (const char* r = getenv("SSCVAE_TEST_GEMM_REPEAT")) repeat = std::max(1, atoi(r));
+  for (int k = 0; k < repeat; ++k) {
+    TransposeJobList tj;
+    for (int i = 0; i < njobs; ++i)
+      TRY(tj.add(reinterpret_cast<const bf16*>(in[i]), rows[i], cols[i], ld_in[i], reinterpret_cast<bf16*>(out[i]), ld_out[i]));
+    TRY(transpose_bf16_jobs(reinterpret_cast<cudaStream_t>(stream), tj));
+  }
   return 0;
 }
 

@@ -49,6 +49,19 @@ struct GemmEpi {
 // Launches on `stream`; returns 0 or an error code (message via get_error()).
 int gemm_bf16_tn(cudaStream_t stream, int M, int N, int nseg, const GemmSeg* segs, const GemmEpi& epi);
 
+// One problem of a grouped launch: C32[M,N] = A[M,K] * B[N,K]^T, a plain fp32 store (ldc32 in floats, any value).
+struct GemmProblem {
+  const bf16* A; int lda;
+  const bf16* B; int ldb;
+  int K, M, N;
+  float* C32; int ldc32;
+};
+constexpr int kMaxGemmProblems = 8;
+
+// Up to kMaxGemmProblems independent problems in ONE launch of the CTA-pair tile kernel (256 x 128 tiles), the tiles of
+// the longest-K problem first; reported to the profiler under `tag`. nprob == 0 launches nothing.
+int gemm_bf16_tn_grouped(cudaStream_t stream, int nprob, const GemmProblem* probs, const char* tag);
+
 // cuTensorMapEncodeTiled resolved through the runtime (null if the driver does not export it)
 void* tma_encode_fn();
 

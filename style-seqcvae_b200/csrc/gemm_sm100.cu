@@ -15,6 +15,7 @@
 #include "ptx.cuh"
 #include "tc_ptx.cuh"
 #include <cuda.h>
+#include <algorithm>
 #include <cstring>
 #include <mutex>
 #include <unordered_map>
@@ -289,9 +290,10 @@ __device__ __forceinline__ int total_kblocks(const GemmParams& p) {
 // Thread 0 prefetches the operand maps and initialises the barriers, warp 1 allocates the accumulator; returns its TMEM
 // address once the CTA (PAIR: both CTAs, so that no remote arrival precedes the peer's barriers) has got this far.
 template <bool PAIR, int TMEM_COLS, class Smem>
-__device__ __forceinline__ uint32_t gemm_setup(const GemmParams& p, const Smem& sm, int warp) {
+__device__ __forceinline__ uint32_t gemm_setup(const CUtensorMap* ta, const CUtensorMap* tb, int nseg, const Smem& sm,
+                                               int warp) {
   if (threadIdx.x == 0) {
-    for (int s = 0; s < p.nseg; ++s) { prefetch_tmap(&p.ta[s]); prefetch_tmap(&p.tb[s]); }
+    for (int s = 0; s < nseg; ++s) { prefetch_tmap(&ta[s]); prefetch_tmap(&tb[s]); }
     sm.init_barriers();
   }
   if (warp == 1) {
@@ -306,11 +308,12 @@ __device__ __forceinline__ uint32_t gemm_setup(const GemmParams& p, const Smem& 
 }
 
 // TMA producer (one elected thread of warp 0) for k-blocks [kb_begin, kb_end) of the concatenated K segments: per
-// k-block the slot-0 tile (map0[s], rows from row0) and the slot-1 tile (map1[s], rows from row1) of its segment s.
+// k-block the slot-0 tile (map0[s], rows from row0) and the slot-1 tile (map1[s], rows from row1) of its segment s,
+// which spans kblocks[s] k-blocks.
 // PAIR: both CTAs load and the bytes land on the leader's `full` barrier, which alone expects them.
 // EVICT_FIRST0: the slot-0 tiles are loaded with an L2 evict_first hint.
 template <bool PAIR, bool EVICT_FIRST0, class Smem>
-__device__ __forceinline__ void gemm_produce(const GemmParams& p, const Smem& sm, const CUtensorMap* map0, int row0,
+__device__ __forceinline__ void gemm_produce(const int* kblocks, const Smem& sm, const CUtensorMap* map0, int row0,
                                              const CUtensorMap* map1, int row1, int kb_begin, int kb_end, bool leader) {
   static_assert(PAIR || !EVICT_FIRST0, "the hinted load exists in the CTA-pair form only");
   constexpr uint32_t TX = (PAIR ? 2 : 1) * (Smem::kBytes0 + Smem::kBytes1);
@@ -325,7 +328,7 @@ __device__ __forceinline__ void gemm_produce(const GemmParams& p, const Smem& sm
   const CUtensorMap* t1 = map1;
   asm volatile("" : "+l"(t0), "+l"(t1));
   for (int g = kb_begin; g < kb_end; ++g) {
-    while (g >= base + p.kblocks[s]) { base += p.kblocks[s]; ++s; ++t0; ++t1; }
+    while (g >= base + kblocks[s]) { base += kblocks[s]; ++s; ++t0; ++t1; }
     const int kc = (g - base) * BK;
     uint64_t* bar = &sm.full[pos.stage];
     uint8_t* d0 = sm.s0 + pos.stage * Smem::kBytes0;
@@ -375,8 +378,8 @@ __device__ __forceinline__ void gemm_mma(const Smem& sm, uint32_t tmem_acc, uint
 // End of the kernel: the epilogue's TMA stores are complete, and nobody deallocates while MMAs, loads or (PAIR) the
 // peer's reads of its half of the accumulator are in flight.
 template <bool PAIR, int TMEM_COLS>
-__device__ __forceinline__ void gemm_teardown(const GemmParams& p, uint32_t tmem_acc, int warp) {
-  if (p.tma_store && warp >= 2 && (threadIdx.x & 31) == 0) tma_store_wait_all();
+__device__ __forceinline__ void gemm_teardown(bool tma_store, uint32_t tmem_acc, int warp) {
+  if (tma_store && warp >= 2 && (threadIdx.x & 31) == 0) tma_store_wait_all();
   tc_fence_before();
   if constexpr (PAIR) cluster_sync_all();
   else __syncthreads();
@@ -389,9 +392,11 @@ __device__ __forceinline__ void gemm_teardown(const GemmParams& p, uint32_t tmem
 
 // Epilogue warps 2..5 of the two tile kernels; a warp may only touch TMEM lanes [32*(warp%4), +32): the tile rows from
 // m0 + 32*(warp%4). It walks the tile's columns 32 at a time; each block leaves through TMA stores or epilogue_row32.
-// ROW_STATS: the tile kernel's vocabulary-head branch (RowStatsEpi). smem0: the dead stage buffers.
+// The output is (M, N) through `epi`; tc: the fp32 map of the TMA-store epilogue, null for the other paths (vec: see
+// GemmParams). ROW_STATS: the tile kernel's vocabulary-head branch (`rs_p`). smem0: the dead stage buffers.
 template <int BN, bool ROW_STATS>
-__device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t tmem_acc, uint64_t* accum, uint32_t smem0,
+__device__ __forceinline__ void epilogue_tile(const GemmEpi& epi, const RowStatsEpi& rs_p, int M, int N, int vec,
+                                              const CUtensorMap* tc, uint32_t tmem_acc, uint64_t* accum, uint32_t smem0,
                                               int m0, int n0) {
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -400,16 +405,16 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t tmem
   tc_fence_after();
   const int row = m0 + q * 32 + lane;
   // vocabulary head (RowStatsEpi): running softmax statistics of this thread's row over the tile's columns
-  const RowStatsEpi rs = ROW_STATS ? p.rs : RowStatsEpi();
+  const RowStatsEpi rs = ROW_STATS ? rs_p : RowStatsEpi();
   float rs_m = -INFINITY, rs_s = 0.f, rs_t = 0.f; int rs_a = 0x7fffffff;
   int rs_target = -1; float rs_lse = 0.f, rs_g = 0.f;
-  if (rs.mode && row < p.M) {
+  if (rs.mode && row < M) {
     if (rs.target) rs_target = rs.target[row];
     if (rs.mode == 2) { rs_lse = rs.lse[row]; rs_g = rs.gcoef[row]; }
   }
 #pragma unroll 1
   for (int c0 = 0; c0 < BN; c0 += 32) {
-    if (n0 + c0 >= p.N) break;                 // warp-uniform
+    if (n0 + c0 >= N) break;                 // warp-uniform
     uint32_t acc[32];
     tmem_ld_32x32(tmem_acc + (static_cast<uint32_t>(q * 32) << 16) + c0, acc);
     tmem_ld_wait();
@@ -417,19 +422,19 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t tmem
       // One warp per SM sub-partition runs this with nothing to hide latency behind: everything is written as
       // independent operations + tree reductions (a running  s += exp(..)  chain cost ~120 cycles per element).
       const int nb = n0 + c0;
-      const bool full = nb + 32 <= p.N;                     // warp-uniform: only the last tile has a ragged edge
+      const bool full = nb + 32 <= N;                     // warp-uniform: only the last tile has a ragged edge
       float v[32];
 #pragma unroll
-      for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(acc[j]) * p.epi.alpha;
-      if (p.epi.bias) {
+      for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(acc[j]) * epi.alpha;
+      if (epi.bias) {
 #pragma unroll
         for (int j = 0; j < 32; ++j)
-          if (full || nb + j < p.N) v[j] += p.epi.bias[nb + j];
+          if (full || nb + j < N) v[j] += epi.bias[nb + j];
       }
       if (!full) {
 #pragma unroll
         for (int j = 0; j < 32; ++j)
-          if (nb + j >= p.N) v[j] = -INFINITY;              // exp -> 0, never the max
+          if (nb + j >= N) v[j] = -INFINITY;              // exp -> 0, never the max
       }
       if (rs.mode == 1) {
         float t[16];
@@ -461,7 +466,7 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t tmem
           for (int j = 0; j < 32; ++j)
             if (nb + j == rs_target) rs_t = v[j];
         }
-        if (!p.epi.C32 && !p.epi.C16) continue;      // statistics only: the logits are never written
+        if (!epi.C32 && !epi.C16) continue;      // statistics only: the logits are never written
       } else {
         const float lb = rs_lse * 1.4426950408889634f;
 #pragma unroll
@@ -471,22 +476,22 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t tmem
           for (int j = 0; j < 32; ++j)
             if (nb + j == rs_target) acc[j] = __float_as_uint(__uint_as_float(acc[j]) - rs_g);
         }
-        GemmEpi e2 = p.epi;
+        GemmEpi e2 = epi;
         e2.alpha = 1.f; e2.bias = nullptr;
-        epilogue_row32(e2, p.vec, p.M, p.N, m0 + q * 32, n0 + c0, BN - c0 < 32 ? BN - c0 : 32, acc,
+        epilogue_row32(e2, vec, M, N, m0 + q * 32, n0 + c0, BN - c0 < 32 ? BN - c0 : 32, acc,
                        smem0 + (warp - 2) * 32 * 36 * 4);
         continue;
       }
     }
-    if (BN >= 32 && p.tma_store) {
-      epilogue_tma_row32(p.epi, &p.tc, p.N, m0 + q * 32, n0 + c0, acc, smem0 + (warp - 2) * 4096);
+    if (BN >= 32 && tc) {
+      epilogue_tma_row32(epi, tc, N, m0 + q * 32, n0 + c0, acc, smem0 + (warp - 2) * 4096);
     } else {
-      epilogue_row32(p.epi, p.vec, p.M, p.N, m0 + q * 32, n0 + c0, BN - c0 < 32 ? BN - c0 : 32, acc,
+      epilogue_row32(epi, vec, M, N, m0 + q * 32, n0 + c0, BN - c0 < 32 ? BN - c0 : 32, acc,
                      smem0 + (warp - 2) * 32 * 36 * 4);
     }
   }
-  if (rs.mode == 1 && row < p.M) {             // partial statistics of (row, this 128-column tile): lanes = consecutive rows
-    const size_t o = (size_t)blockIdx.x * p.M + row;
+  if (rs.mode == 1 && row < M) {             // partial statistics of (row, this 128-column tile): lanes = consecutive rows
+    const size_t o = (size_t)blockIdx.x * M + row;
     rs.st_max[o] = rs_m; rs.st_sum[o] = rs_s; rs.st_arg[o] = rs_a;
     if (rs.tgt_logit && rs_target >= n0 && rs_target < n0 + BN) rs.tgt_logit[row] = rs_t;
   }
@@ -505,18 +510,19 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_tcgen05_kernel(const __g
   const int m0 = blockIdx.y * BM;
   const int n0 = blockIdx.x * BN;
   const int total_kb = total_kblocks(p);
-  const uint32_t tmem_acc = gemm_setup<false, TMEM_COLS>(p, sm, warp);
+  const uint32_t tmem_acc = gemm_setup<false, TMEM_COLS>(p.ta, p.tb, p.nseg, sm, warp);
 
   if (warp == 0) {
-    if (elect_one_sync()) gemm_produce<false, false>(p, sm, p.ta, m0, p.tb, n0, 0, total_kb, true);
+    if (elect_one_sync()) gemm_produce<false, false>(p.kblocks, sm, p.ta, m0, p.tb, n0, 0, total_kb, true);
     __syncwarp();
   } else if (warp == 1) {
     if (elect_one_sync()) gemm_mma<false>(sm, tmem_acc, make_idesc(BM, BN), 0, total_kb);
     __syncwarp();
   } else {
-    epilogue_tile<BN, true>(p, tmem_acc, sm.accum, smem_u32(smem_raw), m0, n0);
+    epilogue_tile<BN, true>(p.epi, p.rs, p.M, p.N, p.vec, p.tma_store ? &p.tc : nullptr, tmem_acc, sm.accum,
+                            smem_u32(smem_raw), m0, n0);
   }
-  gemm_teardown<false, TMEM_COLS>(p, tmem_acc, warp);
+  gemm_teardown<false, TMEM_COLS>(p.tma_store, tmem_acc, warp);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -538,18 +544,72 @@ gemm_tcgen05_2cta_kernel(const __grid_constant__ GemmParams p) {
   const int m0 = blockIdx.y * (2 * BM) + (int)rank * BM;
   const int n0 = (blockIdx.x >> 1) * BN;
   const int total_kb = total_kblocks(p);
-  const uint32_t tmem_acc = gemm_setup<true, TMEM_COLS>(p, sm, warp);
+  const uint32_t tmem_acc = gemm_setup<true, TMEM_COLS>(p.ta, p.tb, p.nseg, sm, warp);
 
   if (warp == 0) {
-    if (elect_one_sync()) gemm_produce<true, false>(p, sm, p.ta, m0, p.tb, n0 + (int)rank * (BN / 2), 0, total_kb, rank == 0);
+    if (elect_one_sync()) gemm_produce<true, false>(p.kblocks, sm, p.ta, m0, p.tb, n0 + (int)rank * (BN / 2), 0, total_kb, rank == 0);
     __syncwarp();
   } else if (warp == 1) {
     if (rank == 0 && elect_one_sync()) gemm_mma<true>(sm, tmem_acc, make_idesc(2 * BM, BN), 0, total_kb);
     __syncwarp();
   } else {
-    epilogue_tile<BN, false>(p, tmem_acc, sm.accum, smem_u32(smem_raw), m0, n0);
+    epilogue_tile<BN, false>(p.epi, p.rs, p.M, p.N, p.vec, p.tma_store ? &p.tc : nullptr, tmem_acc, sm.accum,
+                             smem_u32(smem_raw), m0, n0);
   }
-  gemm_teardown<true, TMEM_COLS>(p, tmem_acc, warp);
+  gemm_teardown<true, TMEM_COLS>(p.tma_store, tmem_acc, warp);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Grouped CTA-pair kernel (gemm_bf16_tn_grouped): the 256 x BN pair tiles of up to kMaxGemmProblems independent
+// single-segment GEMMs with plain fp32 outputs in one grid. The grid is the concatenation of the problems' tile lists
+// (x = 2 * tile + rank); a pair finds its problem through the prefix table tile0 and runs the pipeline of the CTA-pair
+// tile kernel on that problem's maps. TMA stores are decided per problem.
+// ---------------------------------------------------------------------------------------------
+struct GroupedProblem {
+  CUtensorMap ta, tb;                             // A (M rows, boxes of BM), B (N rows, boxes of BN / 2)
+  CUtensorMap tc;                                 // fp32 output when tma_store (see choose_tma_store)
+  float* C; int ldc;
+  int M, N, kblocks;
+  int tile0, tiles_n;                             // first pair tile of the problem in the grid, pair tiles along N
+  int tma_store, vec;
+};
+struct GroupedParams {
+  GroupedProblem prob[kMaxGemmProblems];
+  int n;
+};
+
+template <int BN, int STAGES>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GEMM_THREADS, 1)
+gemm_tcgen05_2cta_grouped_kernel(const __grid_constant__ GroupedParams g) {
+  constexpr int TMEM_COLS = BN;
+  extern __shared__ __align__(1024) uint8_t smem_raw[];
+  const auto sm = PairTileSmem<BN, STAGES>::carve(smem_raw);
+
+  const int warp = threadIdx.x >> 5;
+  const uint32_t rank = cluster_ctarank();
+  const int tile = blockIdx.x >> 1;
+  int pi = 0;
+  while (pi + 1 < g.n && tile >= g.prob[pi + 1].tile0) ++pi;
+  const GroupedProblem& pr = g.prob[pi];
+  const int local = tile - pr.tile0;
+  const int m0 = (local / pr.tiles_n) * (2 * BM) + (int)rank * BM;
+  const int n0 = (local % pr.tiles_n) * BN;
+  const uint32_t tmem_acc = gemm_setup<true, TMEM_COLS>(&pr.ta, &pr.tb, 1, sm, warp);
+
+  if (warp == 0) {
+    if (elect_one_sync())
+      gemm_produce<true, false>(&pr.kblocks, sm, &pr.ta, m0, &pr.tb, n0 + (int)rank * (BN / 2), 0, pr.kblocks, rank == 0);
+    __syncwarp();
+  } else if (warp == 1) {
+    if (rank == 0 && elect_one_sync()) gemm_mma<true>(sm, tmem_acc, make_idesc(2 * BM, BN), 0, pr.kblocks);
+    __syncwarp();
+  } else {
+    GemmEpi e;
+    e.C32 = pr.C; e.ldc32 = pr.ldc;
+    epilogue_tile<BN, false>(e, RowStatsEpi(), pr.M, pr.N, pr.vec, pr.tma_store ? &pr.tc : nullptr, tmem_acc, sm.accum,
+                             smem_u32(smem_raw), m0, n0);
+  }
+  gemm_teardown<true, TMEM_COLS>(pr.tma_store, tmem_acc, warp);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -638,14 +698,14 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_pair_ker
   const int total_kb = total_kblocks(p);
   const int kb_begin = rank * p.kb_per_split;
   const int kb_end = min(total_kb, kb_begin + p.kb_per_split);
-  const uint32_t tmem_acc = gemm_setup<true, TCOLS>(p, sm, warp);
+  const uint32_t tmem_acc = gemm_setup<true, TCOLS>(p.ta, p.tb, p.nseg, sm, warp);
   const int CW = S == 1 ? 256 : S == 2 ? 128 : S == 3 ? 96 : 64;   // batch columns owned by each K split
 
   if (warp == 0) {
     // The weights of the skinny GEMMs (76 MB per timestep) are streamed once per launch; marking them evict_first
     // leaves L2 to the 52 MB of region features + projections the attention kernels re-read every step (measured:
     // step 8.21 -> 8.08 ms, attention_fwd 25.1 -> 23.1 us).
-    if (elect_one_sync()) gemm_produce<true, true>(p, sm, p.tb, n0, p.ta, xr * BXH, kb_begin, kb_end, xr == 0);
+    if (elect_one_sync()) gemm_produce<true, true>(p.kblocks, sm, p.tb, n0, p.ta, xr * BXH, kb_begin, kb_end, xr == 0);
     __syncwarp();
   } else if (warp == 1) {
     if (xr == 0 && elect_one_sync())
@@ -718,7 +778,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tcgen05_swapped_pair_ker
       }
     }
   }
-  gemm_teardown<true, TCOLS>(p, tmem_acc, warp);
+  gemm_teardown<true, TCOLS>(p.tma_store, tmem_acc, warp);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -826,12 +886,14 @@ static int encode_tmap_c32(CUtensorMap* out, const float* base, int rows, int co
 // Sets prm.tma_store, and encodes prm.tc when it is set: a plain fp32 tile (+ bias) leaves the epilogue through TMA
 // stores. Never with row statistics, whose epilogue writes through epilogue_row32. bias_vec4: the epilogue reads the bias
 // as float4 (the tile kernels; the swapped-pair kernel reads one bias per lane). swizzle128: the layout of the staged tile.
+static bool tma_store_ok(const float* C32, int ldc32, int N) {
+  // N % 4: the TMA unit clips stores at 16-byte granularity (measured: with N = 77 the columns 77..79 were written)
+  return aligned16(C32) && (ldc32 % 4) == 0 && (N % 4) == 0;
+}
 static int choose_tma_store(GemmParams& prm, bool bias_vec4, bool swizzle128) {
   const GemmEpi& e = prm.epi;
   prm.tma_store = !prm.rs.mode && e.C32 && !e.C16 && !e.act && !e.dtanh && !e.accumulate && !e.add1 && !e.add2 &&
-                  aligned16(e.C32) && (e.ldc32 % 4) == 0 && (prm.N % 4) == 0 &&
-                  (!bias_vec4 || !e.bias || aligned16(e.bias));
-  // N % 4: the TMA unit clips stores at 16-byte granularity (measured: with N = 77 the columns 77..79 were written)
+                  tma_store_ok(e.C32, e.ldc32, prm.N) && (!bias_vec4 || !e.bias || aligned16(e.bias));
   if (prm.tma_store) TRY(encode_tmap_c32(&prm.tc, e.C32, prm.M, prm.N, e.ldc32, swizzle128));
   return 0;
 }
@@ -853,7 +915,7 @@ static cudaLaunchConfig_t gemm_config(dim3 grid, int smem, cudaStream_t stream, 
 }
 
 // raises KERNEL's dynamic shared-memory limit to Smem::bytes(), once, before its first launch or occupancy query
-template <void (*KERNEL)(GemmParams), class Smem>
+template <auto KERNEL, class Smem>
 static int gemm_configure() {
   static bool configured = false;
   if (!configured) {
@@ -863,8 +925,8 @@ static int gemm_configure() {
   return 0;
 }
 
-template <void (*KERNEL)(GemmParams), class Smem>
-static int gemm_launch(cudaStream_t stream, dim3 grid, int cluster_z, const GemmParams& prm) {
+template <auto KERNEL, class Smem, class Params>
+static int gemm_launch(cudaStream_t stream, dim3 grid, int cluster_z, const Params& prm) {
   TRY((gemm_configure<KERNEL, Smem>()));
   cudaLaunchAttribute attr[1];
   const cudaLaunchConfig_t cfg = gemm_config(grid, Smem::bytes(), stream, cluster_z, attr);
@@ -982,6 +1044,40 @@ int gemm_bf16_tn(cudaStream_t stream, int M, int N, int nseg, const GemmSeg* seg
   if (N > 32) return launch_tc<64, 4>(stream, prm, segs);
   if (N > 16) return launch_tc<32, 5>(stream, prm, segs);
   return launch_tc<16, 6>(stream, prm, segs);
+}
+
+int gemm_bf16_tn_grouped(cudaStream_t stream, int nprob, const GemmProblem* probs, const char* tag) {
+  REQUIRE(nprob >= 0 && nprob <= kMaxGemmProblems, "gemm grouped: %d problems (0..%d)", nprob, kMaxGemmProblems);
+  if (nprob == 0) return 0;
+  constexpr int TBN = 128, STAGES = 4;
+  // longest K first: the short problems' tiles fill the tail of the grid
+  int order[kMaxGemmProblems];
+  for (int i = 0; i < nprob; ++i) order[i] = i;
+  std::stable_sort(order, order + nprob, [&](int a, int b) { return probs[a].K > probs[b].K; });
+  GroupedParams g;
+  memset(&g, 0, sizeof(g));
+  g.n = nprob;
+  double flops = 0, bytes = 0;
+  int tiles = 0;
+  for (int i = 0; i < nprob; ++i) {
+    const GemmProblem& q = probs[order[i]];
+    REQUIRE(q.M > 0 && q.N > 0 && q.K > 0 && q.C32, "gemm grouped: problem %d: M=%d N=%d K=%d C32=%p", order[i], q.M, q.N,
+            q.K, (const void*)q.C32);
+    GroupedProblem& pr = g.prob[i];
+    TRY(encode_tmap(&pr.ta, q.A, q.M, q.K, q.lda, BM));
+    TRY(encode_tmap(&pr.tb, q.B, q.N, q.K, q.ldb, TBN / 2));
+    pr.C = q.C32; pr.ldc = q.ldc32; pr.M = q.M; pr.N = q.N; pr.kblocks = ceil_div(q.K, BK);
+    pr.tiles_n = ceil_div(q.N, TBN);
+    pr.tile0 = tiles;
+    tiles += pr.tiles_n * ceil_div(q.M, 2 * BM);
+    pr.vec = aligned16(q.C32) && (q.ldc32 % 4) == 0;
+    pr.tma_store = tma_store_ok(q.C32, q.ldc32, q.N);
+    if (pr.tma_store) TRY(encode_tmap_c32(&pr.tc, q.C32, q.M, q.N, q.ldc32, true));
+    flops += 2.0 * q.M * q.N * q.K;
+    bytes += 2.0 * ((double)q.M + q.N) * q.K + 4.0 * q.M * q.N;
+  }
+  PROF_SCOPE(stream, tag, flops, bytes);
+  return gemm_launch<gemm_tcgen05_2cta_grouped_kernel<TBN, STAGES>, PairTileSmem<TBN, STAGES>>(stream, dim3(2 * tiles), 0, g);
 }
 
 }  // namespace sscvae

@@ -105,7 +105,20 @@ int greedy_merge(cudaStream_t s, const float* st_max, const float* st_sum, const
                  const int* last_tokens, const float* last_scores, int end_index, int* tok, int* bp, float* score);
 
 // ---- layout helpers -------------------------------------------------------------------------------
-int transpose_bf16(cudaStream_t s, const bf16* in, int rows, int cols, int ld_in, bf16* out, int ld_out);
+// out[c, r] = in[r, c] (bf16, c < cols, r < ld_out; zero for r >= rows, so the padded out is a GEMM operand) for a
+// list of operands in ONE launch. ld_in, ld_out multiples of 8, bases 16-byte aligned.
+struct TransposeJob {
+  const bf16* src; bf16* dst;
+  int rows, cols, ld_in, ld_out;
+  int tile0, tiles_x;                  // filled by transpose_bf16_jobs: first tile index, tiles along the output rows
+};
+constexpr int kMaxTransposeJobs = 8;
+struct TransposeJobList {
+  TransposeJob job[kMaxTransposeJobs];
+  int n = 0;
+  int add(const bf16* src, int rows, int cols, int ld_in, bf16* dst, int ld_out);
+};
+int transpose_bf16_jobs(cudaStream_t s, TransposeJobList& jobs);
 int transpose_f32_to_bf16(cudaStream_t s, const float* in, int rows, int cols, int ld_in, bf16* out, int ld_out);
 // out[r] = sum_c in[r, c]  (bf16 in, fp32 accumulate; one warp per row; deterministic)
 int rowsum_bf16(cudaStream_t s, const bf16* in, int rows, int cols, int ld, float* out, int accumulate);

@@ -735,14 +735,13 @@ template <> __device__ __forceinline__ float to_f<float>(float v) { return v; }
 template <> __device__ __forceinline__ float to_f<bf16>(bf16 v) { return __bfloat162float(v); }
 
 // out[c, r] = in[r, c]; columns of `out` in [rows, ld_out) are zero-filled so it can be a GEMM operand
-template <typename TIn>
-__global__ void transpose_kernel(const TIn* __restrict__ in, int rows, int cols, int ld_in, bf16* __restrict__ out,
-                                 int ld_out) {
+__global__ void transpose_f32_kernel(const float* __restrict__ in, int rows, int cols, int ld_in, bf16* __restrict__ out,
+                                     int ld_out) {
   __shared__ float tile[32][33];
   const int r0 = blockIdx.x * 32, c0 = blockIdx.y * 32;
   for (int i = threadIdx.y; i < 32; i += blockDim.y) {
     const int r = r0 + i, c = c0 + threadIdx.x;
-    tile[i][threadIdx.x] = (r < rows && c < cols) ? to_f<TIn>(in[(size_t)r * ld_in + c]) : 0.f;
+    tile[i][threadIdx.x] = (r < rows && c < cols) ? in[(size_t)r * ld_in + c] : 0.f;
   }
   __syncthreads();
   for (int i = threadIdx.y; i < 32; i += blockDim.y) {
@@ -751,53 +750,95 @@ __global__ void transpose_kernel(const TIn* __restrict__ in, int rows, int cols,
   }
 }
 
-// bf16 fast path: 64 x 64 tiles, 16-byte loads along the input rows and 16-byte stores along the output rows
-// (the 2-byte-per-thread form above moves 64-byte segments and ran at 1.5 TB/s)
-__global__ void __launch_bounds__(256) transpose_bf16_v8_kernel(const bf16* __restrict__ in, int rows, int cols, int ld_in,
-                                                                bf16* __restrict__ out, int ld_out) {
-  __shared__ bf16 tile[64][64 + 8];
-  const int r0 = blockIdx.x * 64, c0 = blockIdx.y * 64;
-  for (int v = threadIdx.x; v < 512; v += 256) {
-    const int i = v >> 3, cv = (v & 7) * 8;
-    const int r = r0 + i, c = c0 + cv;
-    bf16x8 x;
-    if (r < rows && c < cols) x = ld_bf16x8(in + (size_t)r * ld_in + c);      // cols % 8 == 0
-    else
+// ---- bf16 transposes of a whole list of operands in ONE launch; a CTA transposes one 64 x 64 tile -----------------
+// The tile crosses shared memory as 64 rows of eight 16-byte chunks, chunk c of row i stored at chunk c ^ ((i >> 3) & 7):
+// the 16-byte row writes and the 4-byte column reads (thread = 8 consecutive rows x 2 columns, 8 row groups per warp) are
+// both free of bank conflicts. (2-byte column reads of an unswizzled tile are an 8-way bank conflict: shared memory, not
+// HBM, then bounds the transpose at ~2 TB/s.)
+int TransposeJobList::add(const bf16* src, int rows, int cols, int ld_in, bf16* dst, int ld_out) {
+  REQUIRE(n < kMaxTransposeJobs, "transpose job list full");
+  REQUIRE(rows > 0 && cols > 0 && ld_in >= cols && ld_out >= rows && ld_in % 8 == 0 && ld_out % 8 == 0 &&
+              (reinterpret_cast<uintptr_t>(src) & 15) == 0 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0,
+          "transpose: rows %d cols %d ld_in %d ld_out %d (need ld %% 8 == 0 and 16-byte aligned bases)", rows, cols, ld_in,
+          ld_out);
+  TransposeJob& j = job[n++];
+  j.src = src; j.dst = dst; j.rows = rows; j.cols = cols; j.ld_in = ld_in; j.ld_out = ld_out; j.tile0 = 0; j.tiles_x = 0;
+  return 0;
+}
+
+struct TransposeJobTable { TransposeJob job[kMaxTransposeJobs]; int n; };
+
+__global__ void __launch_bounds__(256) transpose_bf16_jobs_kernel(const __grid_constant__ TransposeJobTable t) {
+  __shared__ __align__(16) uint8_t tile[64 * 128];
+  int ji = 0;
+  while (ji + 1 < t.n && (int)blockIdx.x >= t.job[ji + 1].tile0) ++ji;
+  const TransposeJob& j = t.job[ji];
+  const int local = blockIdx.x - j.tile0;
+  const int r0 = (local % j.tiles_x) * 64, c0 = (local / j.tiles_x) * 64;   // input rows (output columns), input columns
+  const int rows = j.rows, cols = j.cols;
 #pragma unroll
-      for (int k = 0; k < 4; ++k) x.v[k] = __floats2bfloat162_rn(0.f, 0.f);
-    *reinterpret_cast<bf16x8*>(&tile[i][cv]) = x;
+  for (int it = 0; it < 2; ++it) {
+    const int v = threadIdx.x + it * 256;
+    const int i = v >> 3, cv = v & 7;
+    const int r = r0 + i, c = c0 + cv * 8;
+    uint4 x = make_uint4(0u, 0u, 0u, 0u);
+    if (r < rows && c < cols) {
+      const bf16* p = j.src + (size_t)r * j.ld_in + c;
+      if (c + 8 <= cols) {
+        x = *reinterpret_cast<const uint4*>(p);
+      } else {                                                              // ragged right edge (cols % 8 != 0)
+        bf16 e[8];
+#pragma unroll
+        for (int k = 0; k < 8; ++k) e[k] = c + k < cols ? p[k] : __float2bfloat16_rn(0.f);
+        x = *reinterpret_cast<const uint4*>(e);
+      }
+    }
+    *reinterpret_cast<uint4*>(tile + i * 128 + ((cv ^ ((i >> 3) & 7)) << 4)) = x;
   }
   __syncthreads();
-  for (int v = threadIdx.x; v < 512; v += 256) {
-    const int i = v >> 3, rv = (v & 7) * 8;                                   // output row c0 + i, columns r0 + rv ..
-    const int c = c0 + i, r = r0 + rv;
-    if (c < cols && r < ld_out) {
-      bf16x8 x;
+  const int lane = threadIdx.x & 31, rv = lane & 7;
+  const int jw = (threadIdx.x >> 5) * 4 + (lane >> 3);                      // 4-byte word = input columns 2jw, 2jw + 1
+  uint32_t w[8];
 #pragma unroll
-      for (int k = 0; k < 4; ++k) x.v[k] = __halves2bfloat162(tile[rv + 2 * k][i], tile[rv + 2 * k + 1][i]);
-      st_bf16x8(out + (size_t)c * ld_out + r, x);                             // ld_out % 8 == 0
-    }
+  for (int k = 0; k < 8; ++k)
+    w[k] = *reinterpret_cast<const uint32_t*>(tile + (8 * rv + k) * 128 + (((jw >> 2) ^ rv) << 4) + ((jw & 3) << 2));
+  uint4 lo, hi;                                                             // column 2jw / 2jw + 1, input rows 8rv .. 8rv + 7
+  lo.x = __byte_perm(w[0], w[1], 0x5410); hi.x = __byte_perm(w[0], w[1], 0x7632);
+  lo.y = __byte_perm(w[2], w[3], 0x5410); hi.y = __byte_perm(w[2], w[3], 0x7632);
+  lo.z = __byte_perm(w[4], w[5], 0x5410); hi.z = __byte_perm(w[4], w[5], 0x7632);
+  lo.w = __byte_perm(w[6], w[7], 0x5410); hi.w = __byte_perm(w[6], w[7], 0x7632);
+  const int c = c0 + 2 * jw, r = r0 + 8 * rv;
+  if (r < j.ld_out) {                                                       // ld_out % 8 == 0: all 8 rows or none
+    if (c < cols) *reinterpret_cast<uint4*>(j.dst + (size_t)c * j.ld_out + r) = lo;
+    if (c + 1 < cols) *reinterpret_cast<uint4*>(j.dst + (size_t)(c + 1) * j.ld_out + r) = hi;
   }
 }
 
-int transpose_bf16(cudaStream_t s, const bf16* in, int rows, int cols, int ld_in, bf16* out, int ld_out) {
-  PROF_SCOPE(s, "transpose", 0, (double)rows*cols*4.0);
-  if ((cols % 8) == 0 && (ld_in % 8) == 0 && (ld_out % 8) == 0 && (reinterpret_cast<uintptr_t>(in) & 15) == 0 &&
-      (reinterpret_cast<uintptr_t>(out) & 15) == 0) {
-    dim3 grid(ceil_div(ld_out, 64), ceil_div(cols, 64));
-    transpose_bf16_v8_kernel<<<grid, 256, 0, s>>>(in, rows, cols, ld_in, out, ld_out);
-    LAUNCHED();
-    return 0;
+int transpose_bf16_jobs(cudaStream_t s, TransposeJobList& jobs) {
+  if (jobs.n == 0) return 0;
+  TransposeJobTable t;
+  double bytes = 0;
+  int tiles = 0;
+  for (int i = 0; i < jobs.n; ++i) {
+    TransposeJob& j = jobs.job[i];
+    j.tiles_x = ceil_div(j.ld_out, 64);
+    j.tile0 = tiles;
+    tiles += j.tiles_x * ceil_div(j.cols, 64);
+    bytes += (double)j.rows * j.cols * 4.0;
+    t.job[i] = j;
   }
-  dim3 grid(ceil_div(ld_out, 32), ceil_div(cols, 32));
-  transpose_kernel<bf16><<<grid, dim3(32, 8), 0, s>>>(in, rows, cols, ld_in, out, ld_out);
+  t.n = jobs.n;
+  PROF_SCOPE(s, "transpose", 0, bytes);
+  transpose_bf16_jobs_kernel<<<tiles, 256, 0, s>>>(t);
   LAUNCHED();
+  jobs.n = 0;
   return 0;
 }
+
 int transpose_f32_to_bf16(cudaStream_t s, const float* in, int rows, int cols, int ld_in, bf16* out, int ld_out) {
   PROF_SCOPE(s, "transpose", 0, (double)rows*cols*6.0);
   dim3 grid(ceil_div(ld_out, 32), ceil_div(cols, 32));
-  transpose_kernel<float><<<grid, dim3(32, 8), 0, s>>>(in, rows, cols, ld_in, out, ld_out);
+  transpose_f32_kernel<<<grid, dim3(32, 8), 0, s>>>(in, rows, cols, ld_in, out, ld_out);
   LAUNCHED();
   return 0;
 }
