@@ -281,6 +281,19 @@ int sscvae_sgd_step_multi(int count, void* const* params, const void* const* gra
                           const uint64_t* sizes, const int32_t* first_step, float max_norm, float lr, float momentum,
                           float weight_decay, float grad_scale, float* scratch, size_t scratch_floats, void* stream);
 
+/* The same update for `count` weights of this handle's model, fused with the re-pack of their images in `packed` (a
+ * buffer sscvae_pack_weights has filled from the current `weights`): afterwards `packed` equals a pack of the updated
+ * weights, and no re-pack is needed before the next forward. Three launches: the two norm launches of
+ * sscvae_sgd_step_multi and one update + pack launch. `weights` = SSCVAE_W_COUNT device pointers as for
+ * sscvae_pack_weights; grads / momentum_bufs / first_step are indexed by weight id like them and read only for the
+ * weights listed in order[0..count) (a NULL gradient = a zero gradient). `order` also fixes the summation order of the
+ * norm: given the same tensors in the same order, results are bit-identical to sscvae_sgd_step_multi followed by
+ * sscvae_pack_weights. Weights not listed are read (fold partners, bias sums), never written. */
+int sscvae_sgd_step_packed(SscvaeHandle* h, const void* const* weights, const void* const* grads,
+                           void* const* momentum_bufs, const int32_t* first_step, int count, const int32_t* order,
+                           float max_norm, float lr, float momentum, float weight_decay, float grad_scale, void* packed,
+                           size_t packed_bytes, float* scratch, size_t scratch_floats, void* stream);
+
 /* Per-handle options consumed by the following calls (0 = default):
  *   "features_bf16"     1: every `image_features` pointer is bf16 (B,N,F) instead of fp32 - the bf16 feature cache of SURVEY
  *                       8(f)-3 (updown-baseline/updown/data/readers.py:21-139 reads fp32 from HDF5). Results are bit-identical
@@ -301,6 +314,13 @@ int sscvae_train_backward_is_persistent(const SscvaeHandle* h, int batch, int nu
  * out12 = {big pairs, small pairs, S6A tiles, S6A K parts, S6B tiles, parts, S10 tiles, parts, d z tiles, parts, S4 / S8 tiles,
  * their width}; returns 1, or 0 if the shape does not fit (the per-launch path is used). For the CPU tests of the tiling. */
 int sscvae_debug_bptt_tiling(const SscvaeHandle* h, int batch, int num_boxes, int pairs, int32_t* out12);
+
+/* Host-only (no device needed): the source blocks that sscvae_pack_weights and sscvae_sgd_step_packed build their jobs
+ * from, 16 values per block: {weight id, fold partner id or -1, first column, rows, columns, row length of the weight, row
+ * length of the partner, outputs, then per output (two slots): kind (0 plain bf16, 1 transposed bf16, 2 fp32; -1 unused),
+ * byte offset in the packed buffer, leading dimension, gate_H (> 0: plain rows gate-interleaved)}. Returns the number of
+ * blocks (<= max_jobs) or an error. For the CPU tests of the packed layout. */
+int sscvae_debug_sgd_pack_jobs(const SscvaeHandle* h, int64_t* out, int max_jobs);
 
 /* Optional instrumentation (off by default): CUDA events around every kernel launch of the library,
  * aggregated per kernel class. report() synchronises the device and writes a JSON object

@@ -46,6 +46,7 @@ SYMBOLS = [
     "sscvae_decode_samples", "sscvae_decode_samples_search_workspace_bytes", "sscvae_decode_samples_search",
     "sscvae_decode_samples_search_region", "sscvae_grad_sqnorm", "sscvae_sgd_step", "sscvae_test_gemm",
     "sscvae_profile_enable", "sscvae_profile_report", "sscvae_test_gemm_grouped", "sscvae_test_transpose_bf16",
+    "sscvae_sgd_step_packed", "sscvae_debug_sgd_pack_jobs",
 ]
 
 
@@ -110,6 +111,9 @@ def lib():
     L.sscvae_test_gemm_splitk.argtypes = [vp, i32, vp, i32, i32, i32, i32, vp, i32, i32, vp, vp]
     L.sscvae_sgd_step_multi.argtypes = [i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(u64), C.POINTER(i32),
                                         C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, vp, sz, vp]
+    L.sscvae_sgd_step_packed.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(i32), i32,
+                                         C.POINTER(i32), f32, f32, f32, f32, f32, vp, sz, vp, sz, vp]
+    L.sscvae_debug_sgd_pack_jobs.argtypes = [vp, C.POINTER(C.c_int64), i32]
     L.sscvae_grad_sqnorm.argtypes = [vp, sz, vp, vp, vp]
     L.sscvae_sgd_step.argtypes = [vp, vp, vp, sz, vp, f32, f32, f32, f32, i32, vp]
     L.sscvae_test_gemm.argtypes = [vp, i32, vp, i32, i32, i32, i32, vp, i32, vp, i32, i32, vp]

@@ -11,12 +11,18 @@ BPTT, beam/CBS search) happens in hand-written sm_100a kernels behind the C ABI;
 CPU fallback — without a CUDA device and the built library this module raises.
 """
 import ctypes as C
+import weakref
 from typing import Dict, Optional
 
 import torch
 from torch import nn
+from torch.utils.weak import WeakIdKeyDictionary
 
 from . import _lib
+
+# weight tensor -> weak reference to the captioner whose packed operands were last built from it: FusedClipSGD finds the
+# captioner of its parameters here and updates the packed operands together with the weights
+PACKED_OWNERS = WeakIdKeyDictionary()
 
 
 class _ButdAttentionParams(nn.Module):
@@ -324,7 +330,7 @@ class UpDownCaptioner(nn.Module):
         ws = self._weight_tensors()
         # one key per weight: a weight is re-packed when its storage or its version counter changed (torch's own
         # optimizers bump the counter; FusedClipSGD, which writes through raw pointers, does so explicitly)
-        key = tuple((p.data_ptr(), p._version) for p in ws)
+        key = self._weights_key(ws)
         if self._packed is None or key != self._packed_key or self._packed.device != ws[0].device:
             L = _lib.lib()
             nbytes = L.sscvae_packed_bytes(self._handle)
@@ -337,7 +343,45 @@ class UpDownCaptioner(nn.Module):
             _lib.check(L.sscvae_pack_weights(self._handle, _lib.ptr_array(ws), _lib.ptr(self._packed), nbytes, dirty,
                                              stream))
             self._packed_key = key
+            me = weakref.ref(self)
+            for p in ws:
+                PACKED_OWNERS[p] = me
         return self._packed
+
+    @staticmethod
+    def _weights_key(ws) -> tuple:
+        return tuple((p.data_ptr(), p._version) for p in ws)
+
+    def _sgd_step_packed(self, ps, grads, bufs, firsts, hyper, scratch) -> bool:
+        """FusedClipSGD.step() for parameters `ps` of this module: the update and the re-pack of their bf16 / fp32
+        images in the packed operands in one pass (sscvae_sgd_step_packed), so the next forward re-packs nothing.
+        Returns False, having done nothing, unless the packed operands are current (built from exactly these
+        weights, none changed since), every tensor of `ps` is one of the weights, and the weights are contiguous fp32
+        tensors on the device of the packed operands. `hyper`: max_norm, lr, momentum, weight_decay, grad_scale."""
+        ws = self._weight_tensors()
+        if self._packed is None or self._packed_key != self._weights_key(ws):
+            return False
+        dev = self._packed.device
+        if any(w.device != dev or w.dtype != torch.float32 or not w.is_contiguous() for w in ws):
+            return False
+        slot = {id(w): i for i, w in enumerate(ws)}
+        order = [slot.get(id(p)) for p in ps]
+        if None in order or len(set(order)) != len(order):
+            return False
+        n = len(ws)
+        g_by_id, b_by_id, f_by_id = [None] * n, [None] * n, [0] * n
+        for i, g, b, f in zip(order, grads, bufs, firsts):
+            g_by_id[i], b_by_id[i], f_by_id[i] = g, b, f
+        L = _lib.lib()
+        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _lib.check(L.sscvae_sgd_step_packed(
+            self._handle, _lib.ptr_array(ws), _lib.ptr_array(g_by_id), _lib.ptr_array(b_by_id),
+            (C.c_int32 * n)(*f_by_id), len(order), (C.c_int32 * len(order))(*order), *[float(h) for h in hyper],
+            _lib.ptr(self._packed), self._packed.numel(), _lib.ptr(scratch), scratch.numel(), stream))
+        for p in ps:
+            torch.autograd.graph.increment_version(p)
+        self._packed_key = self._weights_key(ws)      # the packed operands already hold the updated weights
+        return True
 
     def _grad_views(self):
         """Per weight tensor (SSCVAE_W_* order): a view, shaped like the parameter, into the flat gradient buffer of its

@@ -234,113 +234,141 @@ const Plan& Handle::train_plan(int B, int N) {
 }
 
 // ---- weight packing ----------------------------------------------------------------------------
+// The packed blob as ONE list of source blocks (kernels.cuh: SgdPackJob): every column block of every weight with the
+// images it has in the blob. The plain pack (sscvae_pack_weights) and the fused clip + SGD + pack of the optimizer
+// (sscvae_sgd_step_packed) both run jobs built from this list, and the source blocks of each weight split its columns
+// with no overlap, so every element is updated by exactly one job.
+struct SrcOut { int kind; const char* region; size_t at; int ld, gate_H; };   // `at`: element offset in the region
+struct SrcBlock { int w, w2, c0, cols; int nout; SrcOut out[2]; };
+
+// rows, columns of each weight in reference layout (include/sscvae.h); a bias is one row
+static void weight_shapes(const Dims& d, int rows[SSCVAE_W_COUNT], int cols[SSCVAE_W_COUNT]) {
+  const int G = d.G, H = d.H, c = d.cond, NO = d.tied ? d.E : d.V;
+  auto set = [&](int w, int r, int k) { rows[w] = r; cols[w] = k; };
+  set(SSCVAE_W_EMBEDDING, d.V, d.E);
+  set(SSCVAE_W_ATT_IH, G, d.E + d.F + 2 * H); set(SSCVAE_W_ATT_HH, G, H);
+  set(SSCVAE_W_ATT_BIH, 1, G); set(SSCVAE_W_ATT_BHH, 1, G);
+  set(SSCVAE_W_QUERY_PROJ, d.A, H); set(SSCVAE_W_IMAGE_PROJ, d.A, d.F); set(SSCVAE_W_ATT_VEC, 1, d.A);
+  set(SSCVAE_W_ENC_IH, G, d.F + 2 * H + c); set(SSCVAE_W_ENC_HH, G, H);
+  set(SSCVAE_W_ENC_BIH, 1, G); set(SSCVAE_W_ENC_BHH, 1, G);
+  set(SSCVAE_W_DEC_IH, G, d.F + 2 * H + c + d.Z); set(SSCVAE_W_DEC_HH, G, H);
+  set(SSCVAE_W_DEC_BIH, 1, G); set(SSCVAE_W_DEC_BHH, 1, G);
+  set(SSCVAE_W_FC_MEAN_W, d.Z, H); set(SSCVAE_W_FC_MEAN_B, 1, d.Z);
+  set(SSCVAE_W_FC_LOGVAR_W, d.Z, H); set(SSCVAE_W_FC_LOGVAR_B, 1, d.Z);
+  set(SSCVAE_W_OUT_PROJ_W, NO, H); set(SSCVAE_W_OUT_PROJ_B, 1, NO);
+}
+
+static int source_blocks(const Dims& d, std::vector<SrcBlock>& bl) {
+  const int E = d.E, F = d.F, H = d.H, Z = d.Z, c = d.cond, NOp = d.tied ? d.Ep : d.Vp;
+  bl.clear();
+  auto add = [&](int w, int c0, int cols, int w2, std::initializer_list<SrcOut> outs) {
+    if (cols <= 0) return;
+    SrcBlock b = {w, w2, c0, cols, (int)outs.size(), {}};
+    int k = 0;
+    for (const SrcOut& o : outs) b.out[k++] = o;
+    bl.push_back(b);
+  };
+  auto plain = [](const char* r, size_t at, int ld, int gate_H = 0) { return SrcOut{kPackPlain, r, at, ld, gate_H}; };
+  auto trans = [](const char* r, size_t at, int ld) { return SrcOut{kPackTransposed, r, at, ld, 0}; };
+  auto f32 = [](const char* r, size_t at, int ld) { return SrcOut{kPackF32, r, at, ld, 0}; };
+  const size_t Gp = d.Gp;
+  // embedding (gather source and, tied, the vocabulary GEMM operand)
+  if (d.tied) add(SSCVAE_W_EMBEDDING, 0, E, -1, {plain("embb", 0, d.Ep), trans("embT", 0, d.Vp)});
+  else add(SSCVAE_W_EMBEDDING, 0, E, -1, {plain("embb", 0, d.Ep)});
+  // attention LSTM: W_ih columns [emb E | avg F | h1 H | h_dec H] (updown_cell.py:143-145); W_hh folded onto h1
+  add(SSCVAE_W_ATT_IH, 0, E, -1, {plain("w_att_e", 0, d.Ep, H), trans("w_att_eT", 0, d.Gp)});
+  add(SSCVAE_W_ATT_IH, E, F, -1, {plain("w_att_f", 0, d.Fp, H)});
+  add(SSCVAE_W_ATT_IH, E + F, H, SSCVAE_W_ATT_HH, {plain("w_att_rec", 0, 2 * d.Hp, H), trans("w_att_recT", 0, d.Gp)});
+  add(SSCVAE_W_ATT_IH, E + F + H, H, -1, {plain("w_att_rec", d.Hp, 2 * d.Hp, H), trans("w_att_recT", d.Hp * Gp, d.Gp)});
+  add(SSCVAE_W_ATT_BIH, 0, d.G, SSCVAE_W_ATT_BHH, {f32("b_att", 0, d.G)});
+  // attention
+  add(SSCVAE_W_QUERY_PROJ, 0, H, -1, {plain("wq", 0, d.Hp), trans("wqT", 0, d.Ap)});
+  add(SSCVAE_W_IMAGE_PROJ, 0, F, -1, {plain("wv", 0, d.Fp)});
+  add(SSCVAE_W_ATT_VEC, 0, d.A, -1, {});                              // read by the kernels in fp32
+  // encoder / decoder LSTMs: W_ih columns [xhat F | h1 H | h_dec H | cond c (| z Z)] (updown_cell.py:178-190, 211-224);
+  // the decoder's W_hh is folded onto h_dec; sentiment_vae 1: the conditioning column stays fp32
+  const int offs_src[3] = {0, F, F + H};
+  const size_t offs_dst[3] = {0, (size_t)d.Fp, (size_t)d.Fp + d.Hp};
+  const int widths[3] = {F, H, H};
+  for (int k = 0; k < 3; ++k)
+    add(SSCVAE_W_ENC_IH, offs_src[k], widths[k], -1, {plain("w_enc_x", offs_dst[k], d.KX, H), trans("w_enc_xhT", offs_dst[k] * Gp, d.Gp)});
+  if (d.cvar) add(SSCVAE_W_ENC_IH, F + 2 * H, c, -1, {plain("w_enc_c", 0, d.Cp, H), trans("w_enc_xhT", (size_t)(d.KX + d.Hp) * Gp, d.Gp)});
+  else add(SSCVAE_W_ENC_IH, F + 2 * H, c, -1, {f32("scol_enc", 0, 1)});
+  add(SSCVAE_W_ENC_HH, 0, H, -1, {plain("w_enc_hh", 0, d.Hp, H), trans("w_enc_xhT", (size_t)d.KX * Gp, d.Gp)});
+  add(SSCVAE_W_ENC_BIH, 0, d.G, SSCVAE_W_ENC_BHH, {f32("b_enc", 0, d.G)});
+  for (int k = 0; k < 3; ++k)
+    add(SSCVAE_W_DEC_IH, offs_src[k], widths[k], k == 2 ? SSCVAE_W_DEC_HH : -1,
+        {plain("w_dec_x", offs_dst[k], d.KX, H), trans("w_dec_xzT", offs_dst[k] * Gp, d.Gp)});
+  if (d.cvar) add(SSCVAE_W_DEC_IH, F + 2 * H, c, -1, {plain("w_dec_z", d.Zp, d.ZC, H), trans("w_dec_xzT", (size_t)(d.KX + d.Zp) * Gp, d.Gp)});
+  else add(SSCVAE_W_DEC_IH, F + 2 * H, c, -1, {f32("scol_dec", 0, 1)});
+  add(SSCVAE_W_DEC_IH, F + 2 * H + c, Z, -1, {plain("w_dec_z", 0, d.ZC, H), trans("w_dec_xzT", (size_t)d.KX * Gp, d.Gp)});
+  add(SSCVAE_W_DEC_BIH, 0, d.G, SSCVAE_W_DEC_BHH, {f32("b_dec", 0, d.G)});
+  // latent heads stacked [fc_mean ; fc_log_var]
+  add(SSCVAE_W_FC_MEAN_W, 0, H, -1, {plain("w_fc", 0, d.Hp), trans("w_fcT", 0, d.Z2p)});
+  add(SSCVAE_W_FC_LOGVAR_W, 0, H, -1, {plain("w_fc", (size_t)Z * d.Hp, d.Hp), trans("w_fcT", Z, d.Z2p)});
+  add(SSCVAE_W_FC_MEAN_B, 0, Z, -1, {f32("b_fc", 0, Z)});
+  add(SSCVAE_W_FC_LOGVAR_B, 0, Z, -1, {f32("b_fc", Z, Z)});
+  // output head
+  add(SSCVAE_W_OUT_PROJ_W, 0, H, -1, {plain("w_out", 0, d.Hp), trans("w_outT", 0, NOp)});
+  add(SSCVAE_W_OUT_PROJ_B, 0, d.tied ? E : d.V, -1, {});             // read by the kernels in fp32
+  // the blocks of each weight (its own column blocks, and the whole weight as a fold partner) split its columns
+  int rows[SSCVAE_W_COUNT], cols[SSCVAE_W_COUNT];
+  weight_shapes(d, rows, cols);
+  REQUIRE((int)bl.size() <= kMaxSgdPackJobs, "%d source blocks > %d", (int)bl.size(), kMaxSgdPackJobs);
+  for (int w = 0; w < SSCVAE_W_COUNT; ++w) {
+    int next = 0;                                      // blocks are listed in column order per weight
+    for (const SrcBlock& b : bl) {
+      if (b.w == w) { REQUIRE(b.c0 == next, "weight %d: source block at column %d, expected %d", w, b.c0, next); next += b.cols; }
+      if (b.w2 == w) {
+        REQUIRE(next == 0 && rows[w] == rows[b.w] && cols[w] == b.cols, "weight %d: fold partner does not match its block", w);
+        next = cols[w];
+      }
+    }
+    REQUIRE(next == cols[w], "weight %d: source blocks cover %d of %d columns", w, next, cols[w]);
+  }
+  return 0;
+}
+
+static size_t out_offset(const Plan& pp, const SrcOut& o) { return pp.find(o.region)->off + o.at * (o.kind == kPackF32 ? 4 : 2); }
+
+static void fill_job(const Dims& d, const Plan& pp, const SrcBlock& b, char* pk, SgdPackJob& j) {
+  int rows[SSCVAE_W_COUNT], cols[SSCVAE_W_COUNT];
+  weight_shapes(d, rows, cols);
+  j = SgdPackJob();
+  j.w = b.w; j.w2 = b.w2; j.c0 = b.c0; j.cols = b.cols; j.rows = rows[b.w]; j.ld = cols[b.w];
+  j.ld2 = b.w2 >= 0 ? cols[b.w2] : 0;
+  j.nout = b.nout;
+  for (int k = 0; k < b.nout; ++k) {
+    const SrcOut& o = b.out[k];
+    j.out[k].dst = pk + out_offset(pp, o);
+    j.out[k].kind = o.kind; j.out[k].ld = o.ld; j.out[k].gate_H = o.gate_H;
+  }
+}
+
+static void fill_tensors(const Dims& d, const void* const* wv, SgdPackTable& t) {
+  static_assert(kMaxSgdPackTensors == SSCVAE_W_COUNT, "one tensor slot per weight");
+  int rows[SSCVAE_W_COUNT], cols[SSCVAE_W_COUNT];
+  weight_shapes(d, rows, cols);
+  for (int i = 0; i < SSCVAE_W_COUNT; ++i) {
+    t.t[i] = SgdPackTensor();
+    t.t[i].p = const_cast<float*>(reinterpret_cast<const float*>(wv[i]));
+    t.t[i].n = (unsigned long long)rows[i] * cols[i];
+  }
+}
+
 static int pack_weights_impl(Handle* h, const void* const* wv, char* pk, const uint8_t* dirty, cudaStream_t s) {
   const Dims& d = h->d;
-  const Plan& pp = h->pp;
-  auto W = [&](int i) { return reinterpret_cast<const float*>(wv[i]); };
-  auto Pb = [&](const char* n) { return reinterpret_cast<bf16*>(pk + pp.find(n)->off); };
-  auto Pf = [&](const char* n) { return reinterpret_cast<float*>(pk + pp.find(n)->off); };
   // dirty == NULL: first pack of this buffer (zero the K/N padding, pack everything); otherwise only the blocks
   // whose fp32 source changed are re-packed (the padding stays zero, frozen weights are skipped)
-  auto need = [&](std::initializer_list<int> ids) {
-    if (!dirty) return true;
-    for (int i : ids) if (dirty[i]) return true;
-    return false;
-  };
   for (int i = 0; i < SSCVAE_W_COUNT; ++i) REQUIRE(wv[i] != nullptr, "weight pointer %d is NULL", i);
-  if (!dirty) CUDA_TRY(cudaMemsetAsync(pk, 0, pp.total, s));
-  PackJobList jobs;                                   // every bf16 block below is converted by ONE kernel launch
-  const int E = d.E, F = d.F, H = d.H, A = d.A, Z = d.Z, V = d.V, G = d.G, c = d.cond;
-  // embedding (gather source and, tied, the vocabulary GEMM operand)
-  if (need({SSCVAE_W_EMBEDDING})) {
-    TRY(jobs.add(Pb("embb"), d.Ep, 0, W(SSCVAE_W_EMBEDDING), E, V, E, nullptr, 0));
-    if (d.tied) TRY(jobs.add(Pb("embT"), d.Vp, 1, W(SSCVAE_W_EMBEDDING), E, V, E, nullptr, 0));
-  }
-  // attention LSTM: W_ih columns [emb E | avg F | h1 H | h_dec H] (updown_cell.py:143-145); W_hh folded onto h1
-  const int ldi = E + F + 2 * H;
-  const float* wih = W(SSCVAE_W_ATT_IH);
-  if (need({SSCVAE_W_ATT_IH, SSCVAE_W_ATT_HH})) {
-    TRY(jobs.add(Pb("w_att_rec"), 2 * d.Hp, 0, wih + E + F, ldi, G, H, W(SSCVAE_W_ATT_HH), H, H));
-    TRY(jobs.add(Pb("w_att_recT"), d.Gp, 1, wih + E + F, ldi, G, H, W(SSCVAE_W_ATT_HH), H));
-  }
-  if (need({SSCVAE_W_ATT_IH})) {
-    TRY(jobs.add(Pb("w_att_e"), d.Ep, 0, wih, ldi, G, E, nullptr, 0, H));
-    TRY(jobs.add(Pb("w_att_eT"), d.Gp, 1, wih, ldi, G, E, nullptr, 0));
-    TRY(jobs.add(Pb("w_att_f"), d.Fp, 0, wih + E, ldi, G, F, nullptr, 0, H));
-    TRY(jobs.add(Pb("w_att_rec") + d.Hp, 2 * d.Hp, 0, wih + E + F + H, ldi, G, H, nullptr, 0, H));
-    TRY(jobs.add(Pb("w_att_recT") + (size_t)d.Hp * d.Gp, d.Gp, 1, wih + E + F + H, ldi, G, H, nullptr, 0));
-  }
-  if (need({SSCVAE_W_ATT_BIH, SSCVAE_W_ATT_BHH})) TRY(vec_add_f32(s, W(SSCVAE_W_ATT_BIH), W(SSCVAE_W_ATT_BHH), Pf("b_att"), G));
-  // attention
-  if (need({SSCVAE_W_QUERY_PROJ})) {
-    TRY(jobs.add(Pb("wq"), d.Hp, 0, W(SSCVAE_W_QUERY_PROJ), H, A, H, nullptr, 0));
-    TRY(jobs.add(Pb("wqT"), d.Ap, 1, W(SSCVAE_W_QUERY_PROJ), H, A, H, nullptr, 0));
-  }
-  if (need({SSCVAE_W_IMAGE_PROJ})) TRY(jobs.add(Pb("wv"), d.Fp, 0, W(SSCVAE_W_IMAGE_PROJ), F, A, F, nullptr, 0));
-  // encoder LSTM: W_ih columns [xhat F | h1 H | h_dec H | cond c] (updown_cell.py:178-190)
-  const int lde = F + 2 * H + c;
-  const float* we = W(SSCVAE_W_ENC_IH);
-  bf16* wex = Pb("w_enc_x"); bf16* wexT = Pb("w_enc_xhT");
-  const int offs_src[3] = {0, F, F + H};
-  const int offs_dst[3] = {0, d.Fp, d.Fp + d.Hp};
-  const int widths[3] = {F, H, H};
-  if (need({SSCVAE_W_ENC_IH})) {
-    for (int k = 0; k < 3; ++k) {
-      TRY(jobs.add(wex + offs_dst[k], d.KX, 0, we + offs_src[k], lde, G, widths[k], nullptr, 0, H));
-      TRY(jobs.add(wexT + (size_t)offs_dst[k] * d.Gp, d.Gp, 1, we + offs_src[k], lde, G, widths[k], nullptr, 0));
-    }
-    if (c && !d.cvar) TRY(copy_block_f32(s, we + F + 2 * H, lde, Pf("scol_enc"), 1, G, 1));
-    if (d.cvar) {
-      TRY(jobs.add(Pb("w_enc_c"), d.Cp, 0, we + F + 2 * H, lde, G, c, nullptr, 0, H));
-      TRY(jobs.add(wexT + (size_t)(d.KX + d.Hp) * d.Gp, d.Gp, 1, we + F + 2 * H, lde, G, c, nullptr, 0));
-    }
-  }
-  if (need({SSCVAE_W_ENC_HH})) {
-    TRY(jobs.add(Pb("w_enc_hh"), d.Hp, 0, W(SSCVAE_W_ENC_HH), H, G, H, nullptr, 0, H));
-    TRY(jobs.add(Pb("w_enc_xhT") + (size_t)d.KX * d.Gp, d.Gp, 1, W(SSCVAE_W_ENC_HH), H, G, H, nullptr, 0));
-  }
-  if (need({SSCVAE_W_ENC_BIH, SSCVAE_W_ENC_BHH})) TRY(vec_add_f32(s, W(SSCVAE_W_ENC_BIH), W(SSCVAE_W_ENC_BHH), Pf("b_enc"), G));
-  // decoder LSTM: W_ih columns [xhat F | h1 H | h_dec H | cond c | z Z] (updown_cell.py:211-224); W_hh folded onto h_dec
-  const int ldd = F + 2 * H + c + Z;
-  const float* wd = W(SSCVAE_W_DEC_IH);
-  bf16* wdx = Pb("w_dec_x"); bf16* wdxT = Pb("w_dec_xzT");
-  if (need({SSCVAE_W_DEC_IH, SSCVAE_W_DEC_HH})) {
-    for (int k = 0; k < 3; ++k) {
-      if (k < 2 && !need({SSCVAE_W_DEC_IH})) continue;
-      const float* fold = (k == 2) ? W(SSCVAE_W_DEC_HH) : nullptr;
-      TRY(jobs.add(wdx + offs_dst[k], d.KX, 0, wd + offs_src[k], ldd, G, widths[k], fold, H, H));
-      TRY(jobs.add(wdxT + (size_t)offs_dst[k] * d.Gp, d.Gp, 1, wd + offs_src[k], ldd, G, widths[k], fold, H));
-    }
-  }
-  if (need({SSCVAE_W_DEC_IH})) {
-    TRY(jobs.add(Pb("w_dec_z"), d.ZC, 0, wd + F + 2 * H + c, ldd, G, Z, nullptr, 0, H));
-    TRY(jobs.add(Pb("w_dec_xzT") + (size_t)d.KX * d.Gp, d.Gp, 1, wd + F + 2 * H + c, ldd, G, Z, nullptr, 0));
-    if (c && !d.cvar) TRY(copy_block_f32(s, wd + F + 2 * H, ldd, Pf("scol_dec"), 1, G, 1));
-    if (d.cvar) {
-      TRY(jobs.add(Pb("w_dec_z") + d.Zp, d.ZC, 0, wd + F + 2 * H, ldd, G, c, nullptr, 0, H));
-      TRY(jobs.add(Pb("w_dec_xzT") + (size_t)(d.KX + d.Zp) * d.Gp, d.Gp, 1, wd + F + 2 * H, ldd, G, c, nullptr, 0));
-    }
-  }
-  if (need({SSCVAE_W_DEC_BIH, SSCVAE_W_DEC_BHH})) TRY(vec_add_f32(s, W(SSCVAE_W_DEC_BIH), W(SSCVAE_W_DEC_BHH), Pf("b_dec"), G));
-  // latent heads stacked [fc_mean ; fc_log_var]
-  if (need({SSCVAE_W_FC_MEAN_W})) {
-    TRY(jobs.add(Pb("w_fc"), d.Hp, 0, W(SSCVAE_W_FC_MEAN_W), H, Z, H, nullptr, 0));
-    TRY(jobs.add(Pb("w_fcT"), d.Z2p, 1, W(SSCVAE_W_FC_MEAN_W), H, Z, H, nullptr, 0));
-  }
-  if (need({SSCVAE_W_FC_LOGVAR_W})) {
-    TRY(jobs.add(Pb("w_fc") + (size_t)Z * d.Hp, d.Hp, 0, W(SSCVAE_W_FC_LOGVAR_W), H, Z, H, nullptr, 0));
-    TRY(jobs.add(Pb("w_fcT") + Z, d.Z2p, 1, W(SSCVAE_W_FC_LOGVAR_W), H, Z, H, nullptr, 0));
-  }
-  if (need({SSCVAE_W_FC_MEAN_B})) TRY(copy_block_f32(s, W(SSCVAE_W_FC_MEAN_B), 1, Pf("b_fc"), 1, Z, 1));
-  if (need({SSCVAE_W_FC_LOGVAR_B})) TRY(copy_block_f32(s, W(SSCVAE_W_FC_LOGVAR_B), 1, Pf("b_fc") + Z, 1, Z, 1));
-  // output head
-  const int NO = d.tied ? E : V, NOp = d.tied ? d.Ep : d.Vp;
-  if (need({SSCVAE_W_OUT_PROJ_W})) {
-    TRY(jobs.add(Pb("w_out"), d.Hp, 0, W(SSCVAE_W_OUT_PROJ_W), H, NO, H, nullptr, 0));
-    TRY(jobs.add(Pb("w_outT"), NOp, 1, W(SSCVAE_W_OUT_PROJ_W), H, NO, H, nullptr, 0));
-  }
-  TRY(pack_blocks(s, jobs));
-  return 0;
+  std::vector<SrcBlock> bl;
+  TRY(source_blocks(d, bl));
+  if (!dirty) CUDA_TRY(cudaMemsetAsync(pk, 0, h->pp.total, s));
+  SgdPackTable t;                                      // every block below is converted by ONE kernel launch
+  fill_tensors(d, wv, t);
+  for (const SrcBlock& b : bl)
+    if (b.nout > 0 && (!dirty || dirty[b.w] || (b.w2 >= 0 && dirty[b.w2]))) fill_job(d, h->pp, b, pk, t.job[t.n++]);
+  return sgd_pack(s, t);
 }
 
 
@@ -970,6 +998,61 @@ int sscvae_pack_weights(SscvaeHandle* hh, const void* const* weights, void* pack
   if (packed_bytes < h->pp.total) { set_error("packed buffer too small: %zu < %zu", packed_bytes, h->pp.total); return SSCVAE_ERR_WORKSPACE; }
   REQUIRE((reinterpret_cast<uintptr_t>(packed) & 255) == 0, "packed buffer must be 256-byte aligned");
   return pack_weights_impl(h, weights, reinterpret_cast<char*>(packed), dirty, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int sscvae_sgd_step_packed(SscvaeHandle* hh, const void* const* weights, const void* const* grads,
+                           void* const* momentum_bufs, const int32_t* first_step, int count, const int32_t* order,
+                           float max_norm, float lr, float momentum, float weight_decay, float grad_scale, void* packed,
+                           size_t packed_bytes, float* scratch, size_t scratch_floats, void* stream) {
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  REQUIRE(h && weights && grads && first_step && order && packed && scratch, "NULL argument");
+  REQUIRE(count > 0 && count <= SSCVAE_W_COUNT, "count %d not in 1..%d", count, SSCVAE_W_COUNT);
+  if (packed_bytes < h->pp.total) { set_error("packed buffer too small: %zu < %zu", packed_bytes, h->pp.total); return SSCVAE_ERR_WORKSPACE; }
+  REQUIRE((reinterpret_cast<uintptr_t>(packed) & 255) == 0, "packed buffer must be 256-byte aligned");
+  for (int i = 0; i < SSCVAE_W_COUNT; ++i) REQUIRE(weights[i] != nullptr, "weight pointer %d is NULL", i);
+  const Dims& d = h->d;
+  std::vector<SrcBlock> bl;
+  TRY(source_blocks(d, bl));
+  SgdPackTable t;
+  fill_tensors(d, weights, t);
+  for (int i = 0; i < count; ++i) {
+    const int w = order[i];
+    REQUIRE(w >= 0 && w < SSCVAE_W_COUNT && !t.t[w].upd, "order[%d] = %d: not a weight id, or repeated", i, w);
+    REQUIRE(momentum == 0.f || (momentum_bufs && momentum_bufs[w]), "NULL momentum buffer of weight %d", w);
+    SgdPackTensor& x = t.t[w];
+    x.upd = 1; x.first = first_step[w] != 0;
+    x.g = reinterpret_cast<const float*>(grads[w]);   // NULL: a zero gradient, as in sscvae_sgd_step_multi
+    x.m = momentum_bufs ? reinterpret_cast<float*>(momentum_bufs[w]) : nullptr;
+  }
+  char* pk = reinterpret_cast<char*>(packed);
+  for (const SrcBlock& b : bl)
+    if (t.t[b.w].upd || (b.w2 >= 0 && t.t[b.w2].upd)) fill_job(d, h->pp, b, pk, t.job[t.n++]);
+  return sgd_pack_step(reinterpret_cast<cudaStream_t>(stream), t, order, count,
+                       SgdParams{max_norm, lr, momentum, weight_decay, grad_scale}, scratch, scratch_floats);
+}
+
+int sscvae_debug_sgd_pack_jobs(const SscvaeHandle* hh, int64_t* out, int max_jobs) {
+  const Handle* h = reinterpret_cast<const Handle*>(hh);
+  REQUIRE(h && out && max_jobs > 0, "bad argument");
+  std::vector<SrcBlock> bl;
+  TRY(source_blocks(h->d, bl));
+  REQUIRE((int)bl.size() <= max_jobs, "%d jobs > max_jobs %d", (int)bl.size(), max_jobs);
+  int rows[SSCVAE_W_COUNT], cols[SSCVAE_W_COUNT];
+  weight_shapes(h->d, rows, cols);
+  for (size_t i = 0; i < bl.size(); ++i) {
+    const SrcBlock& b = bl[i];
+    int64_t* o = out + 16 * i;
+    const int64_t v[8] = {b.w, b.w2, b.c0, rows[b.w], b.cols, cols[b.w], b.w2 >= 0 ? cols[b.w2] : 0, b.nout};
+    for (int k = 0; k < 8; ++k) o[k] = v[k];
+    for (int k = 0; k < 2; ++k) {
+      const bool on = k < b.nout;
+      o[8 + 4 * k] = on ? b.out[k].kind : -1;
+      o[9 + 4 * k] = on ? (int64_t)out_offset(h->pp, b.out[k]) : -1;
+      o[10 + 4 * k] = on ? b.out[k].ld : 0;
+      o[11 + 4 * k] = on ? b.out[k].gate_H : 0;
+    }
+  }
+  return (int)bl.size();
 }
 
 size_t sscvae_train_workspace_bytes(const SscvaeHandle* hh, int batch, int num_boxes) {

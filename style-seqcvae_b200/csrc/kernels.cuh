@@ -133,27 +133,44 @@ int colsum_f32(cudaStream_t s, const float* in, int rows, int cols, int ld, floa
 // out[r * out_stride] = sum_c in[r, c] * vec[c % period]   (bf16 matrix row . periodic fp32 vector)
 int rowdot_bf16(cudaStream_t s, const bf16* in, int rows, int cols, int ld, const float* vec, int period, float* out,
                 int out_stride);
-// strided fp32 block copy: dst[r*ld_dst + c] = src[r*ld_src + c]
-int copy_block_f32(cudaStream_t s, const float* src, int ld_src, float* dst, int ld_dst, int rows, int cols);
-// weight packing: dst (bf16) <- src (+ src2) fp32, optionally transposed
-int pack_block(cudaStream_t s, bf16* dst, int ld_dst, int transposed, const float* src, int ld_src, int rows, int cols,
-               const float* src2, int ld_src2);
-// the same for a whole list of blocks in ONE launch (the per-step weight re-pack is ~30 blocks)
-struct PackJob {
-  const float* src; const float* src2; bf16* dst;
-  int ld_src, ld_src2, ld_dst, rows, cols, transposed;
-  int gate_H;                          // > 0: rows are (gate k, unit j) = r / gate_H, r % gate_H and go to row lstm_gate_row(k, j)
-  int tile0, tiles_x;                  // filled by pack_blocks: first tile index, tiles along the columns
+// ---- weight packing, optionally fused with the clip + SGD update (optim.cu) ------------------------------------------
+// A job owns one SOURCE BLOCK: all rows of weight `w`, columns [c0, c0 + cols), plus optionally the same rows of a fold
+// partner `w2` (columns [0, cols)), and writes every packed image of that block from v = w (+ w2): a plain bf16 copy
+// (optionally with gate-interleaved rows), a transposed bf16 copy, or an fp32 copy. A CTA owns one 64 x 64 tile of one
+// job. Tensors flagged `upd` are first updated in place (clip + SGD, the expressions of mt_sgd_kernel) and the images are
+// written from the updated values; the others are only read. With no tensor flagged this is the plain weight pack.
+enum { kPackPlain = 0, kPackTransposed = 1, kPackF32 = 2 };
+struct SgdPackOut {
+  void* dst;                           // bf16 or fp32 element (0, 0) of the image of the block
+  int kind, ld;
+  int gate_H;                          // kPackPlain, > 0: rows are (gate k, unit j) = r / gate_H, r % gate_H and go to row lstm_gate_row(k, j)
 };
-constexpr int kMaxPackJobs = 40;
-struct PackJobList {
-  PackJob job[kMaxPackJobs];
+struct SgdPackJob {
+  int w, w2;                           // tensor slots; w2 = -1: no fold partner
+  int c0, rows, cols, ld, ld2;         // column block of w (row length ld); w2 has row length ld2
+  int nout;
+  SgdPackOut out[2];
+  int tile0, tiles_x, vec;             // filled at launch: first tile index, tiles along the columns, 16-byte fp32 accesses
+};
+struct SgdPackTensor {
+  float* p; const float* g; float* m;  // g == NULL: zero gradient; m unused when momentum == 0
+  unsigned long long n;                // elements
+  int upd, first;                      // upd: updated by this launch; first: first step (momentum buffer written, not read)
+};
+constexpr int kMaxSgdPackTensors = 22, kMaxSgdPackJobs = 32;
+struct SgdPackTable {
+  SgdPackTensor t[kMaxSgdPackTensors];
+  SgdPackJob job[kMaxSgdPackJobs];
   int n = 0;
-  int add(bf16* dst, int ld_dst, int transposed, const float* src, int ld_src, int rows, int cols, const float* src2,
-          int ld_src2, int gate_H = 0);
 };
-int pack_blocks(cudaStream_t s, PackJobList& jobs);
-int vec_add_f32(cudaStream_t s, const float* a, const float* b, float* out, int n);
+struct SgdParams { float max_norm, lr, momentum, wd, gscale; };
+// The plain pack: one launch for every job of the table (no-op without jobs); no tensor may have `upd` set.
+int sgd_pack(cudaStream_t s, SgdPackTable& t);
+// Clip + SGD + pack: the squared gradient norm of the `count` tensors t.t[order[i]] (all flagged `upd`) over the chunking
+// and in the summation order of sscvae_sgd_step_multi given the same tensors in the same order (so the clip coefficient
+// is bit-identical), then one launch for every job. scratch: sscvae_sgd_step_multi's.
+int sgd_pack_step(cudaStream_t s, SgdPackTable& t, const int* order, int count, const SgdParams& sp, float* scratch,
+                  size_t scratch_floats);
 // dst (rows, cols; ld_dst) = sum of `nparts` split-K partial tiles parts + z*stride (rows, cols; ld); dst may be parts
 int sum_partials_f32(cudaStream_t s, float* dst, int ld_dst, const float* parts, size_t stride, int nparts, int rows,
                      int cols, int ld);

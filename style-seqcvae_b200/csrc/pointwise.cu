@@ -964,62 +964,6 @@ int rowdot_bf16(cudaStream_t s, const bf16* in, int rows, int cols, int ld, cons
   return 0;
 }
 
-__global__ void copy_block_kernel(const float* __restrict__ src, int ld_src, float* __restrict__ dst, int ld_dst,
-                                  int cols) {
-  const int r = blockIdx.y;
-  for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < cols; c += gridDim.x * blockDim.x)
-    dst[(size_t)r * ld_dst + c] = src[(size_t)r * ld_src + c];
-}
-int copy_block_f32(cudaStream_t s, const float* src, int ld_src, float* dst, int ld_dst, int rows, int cols) {
-  dim3 grid(min(8, ceil_div(cols, 256)), rows);
-  copy_block_kernel<<<grid, 256, 0, s>>>(src, ld_src, dst, ld_dst, cols);
-  LAUNCHED();
-  return 0;
-}
-
-__global__ void pack_block_kernel(bf16* __restrict__ dst, int ld_dst, const float* __restrict__ src, int ld_src,
-                                  int rows, int cols, const float* __restrict__ src2, int ld_src2) {
-  const int r = blockIdx.y;
-  for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < cols; c += gridDim.x * blockDim.x) {
-    float v = src[(size_t)r * ld_src + c];
-    if (src2) v += src2[(size_t)r * ld_src2 + c];
-    dst[(size_t)r * ld_dst + c] = __float2bfloat16_rn(v);
-  }
-}
-// transposed variant through a shared-memory tile: dst[c, r] = src[r, c] (+ src2[r, c])
-__global__ void pack_block_t_kernel(bf16* __restrict__ dst, int ld_dst, const float* __restrict__ src, int ld_src,
-                                    int rows, int cols, const float* __restrict__ src2, int ld_src2) {
-  __shared__ float tile[32][33];
-  const int r0 = blockIdx.x * 32, c0 = blockIdx.y * 32;
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int r = r0 + i, c = c0 + threadIdx.x;
-    float v = 0.f;
-    if (r < rows && c < cols) {
-      v = src[(size_t)r * ld_src + c];
-      if (src2) v += src2[(size_t)r * ld_src2 + c];
-    }
-    tile[i][threadIdx.x] = v;
-  }
-  __syncthreads();
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int c = c0 + i, r = r0 + threadIdx.x;
-    if (c < cols && r < rows) dst[(size_t)c * ld_dst + r] = __float2bfloat16_rn(tile[threadIdx.x][i]);
-  }
-}
-int pack_block(cudaStream_t s, bf16* dst, int ld_dst, int transposed, const float* src, int ld_src, int rows, int cols,
-               const float* src2, int ld_src2) {
-  PROF_SCOPE(s, "pack_weights", 0, (double)rows*cols*6.0);
-  if (!transposed) {
-    dim3 grid(min(16, ceil_div(cols, 256)), rows);
-    pack_block_kernel<<<grid, 256, 0, s>>>(dst, ld_dst, src, ld_src, rows, cols, src2, ld_src2);
-  } else {
-    dim3 grid(ceil_div(rows, 32), ceil_div(cols, 32));
-    pack_block_t_kernel<<<grid, dim3(32, 8), 0, s>>>(dst, ld_dst, src, ld_src, rows, cols, src2, ld_src2);
-  }
-  LAUNCHED();
-  return 0;
-}
-
 // dst[r, c] = sum_z parts[z * stride + r * ld + c]   (split-K partial tiles -> result; dst may alias parts[0])
 __global__ void sum_partials_kernel(float* __restrict__ dst, int ld_dst, const float* __restrict__ parts, size_t stride,
                                     int nparts, int rows, int cols4, int ld) {
@@ -1043,85 +987,6 @@ int sum_partials_f32(cudaStream_t s, float* dst, int ld_dst, const float* parts,
   return 0;
 }
 
-// ---- batched weight packing: one launch for every block; a CTA converts one 64 x 64 tile ------------------
-int PackJobList::add(bf16* dst, int ld_dst, int transposed, const float* src, int ld_src, int rows, int cols,
-                     const float* src2, int ld_src2, int gate_H) {
-  REQUIRE(n < kMaxPackJobs, "pack job list full");
-  REQUIRE(gate_H == 0 || (!transposed && rows == 4 * gate_H), "pack: gate interleaving needs a (4H, cols) row-major block");
-  PackJob& j = job[n++];
-  j.src = src; j.src2 = src2; j.dst = dst; j.ld_src = ld_src; j.ld_src2 = ld_src2; j.ld_dst = ld_dst;
-  j.rows = rows; j.cols = cols; j.transposed = transposed; j.gate_H = gate_H; j.tile0 = 0; j.tiles_x = 0;
-  return 0;
-}
-
-struct PackJobTable { PackJob job[kMaxPackJobs]; int n; };
-
-__global__ void __launch_bounds__(256) pack_blocks_kernel(const __grid_constant__ PackJobTable t) {
-  __shared__ float tile[64][65];
-  int ji = 0;
-  while (ji + 1 < t.n && (int)blockIdx.x >= t.job[ji + 1].tile0) ++ji;
-  const PackJob& j = t.job[ji];
-  const int local = blockIdx.x - j.tile0;
-  const int r0 = (local / j.tiles_x) * 64, c0 = (local % j.tiles_x) * 64;
-  const int tx = threadIdx.x & 63, ty = threadIdx.x >> 6;          // 64 x 4
-  if (!j.transposed) {
-    for (int i = ty; i < 64; i += 4) {
-      const int r = r0 + i, c = c0 + tx;
-      if (r < j.rows && c < j.cols) {
-        float v = j.src[(size_t)r * j.ld_src + c];
-        if (j.src2) v += j.src2[(size_t)r * j.ld_src2 + c];
-        const int rd = j.gate_H ? lstm_gate_row(r / j.gate_H, r % j.gate_H) : r;
-        j.dst[(size_t)rd * j.ld_dst + c] = __float2bfloat16_rn(v);
-      }
-    }
-    return;
-  }
-  for (int i = ty; i < 64; i += 4) {
-    const int r = r0 + i, c = c0 + tx;
-    float v = 0.f;
-    if (r < j.rows && c < j.cols) {
-      v = j.src[(size_t)r * j.ld_src + c];
-      if (j.src2) v += j.src2[(size_t)r * j.ld_src2 + c];
-    }
-    tile[i][tx] = v;
-  }
-  __syncthreads();
-  for (int i = ty; i < 64; i += 4) {
-    const int c = c0 + i, r = r0 + tx;                                // dst[c, r] = src[r, c]
-    if (c < j.cols && r < j.rows) j.dst[(size_t)c * j.ld_dst + r] = __float2bfloat16_rn(tile[tx][i]);
-  }
-}
-
-int pack_blocks(cudaStream_t s, PackJobList& jobs) {
-  if (jobs.n == 0) return 0;
-  PackJobTable t;
-  double bytes = 0;
-  int tiles = 0;
-  for (int i = 0; i < jobs.n; ++i) {
-    PackJob& j = jobs.job[i];
-    j.tiles_x = ceil_div(j.cols, 64);
-    j.tile0 = tiles;
-    tiles += j.tiles_x * ceil_div(j.rows, 64);
-    bytes += (double)j.rows * j.cols * 6.0;
-    t.job[i] = j;
-  }
-  t.n = jobs.n;
-  PROF_SCOPE(s, "pack_weights", 0, bytes);
-  pack_blocks_kernel<<<tiles, 256, 0, s>>>(t);
-  LAUNCHED();
-  jobs.n = 0;
-  return 0;
-}
-
-__global__ void vec_add_kernel(const float* a, const float* b, float* out, int n) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) out[i] = a[i] + (b ? b[i] : 0.f);
-}
-int vec_add_f32(cudaStream_t s, const float* a, const float* b, float* out, int n) {
-  vec_add_kernel<<<ceil_div(n, 256), 256, 0, s>>>(a, b, out, n);
-  LAUNCHED();
-  return 0;
-}
 __global__ void scale_kernel(const float* in, float scale, float* out, int n) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) out[i] = in ? in[i] * scale : 0.f;

@@ -7,6 +7,7 @@ from typing import Iterable
 import torch
 
 from . import _lib
+from .captioner import PACKED_OWNERS
 
 
 class FusedClipSGD(torch.optim.Optimizer):
@@ -26,10 +27,15 @@ class FusedClipSGD(torch.optim.Optimizer):
     the reverse. Besides SGD's keys the group carries `initial_lr` (base of the linear decay, the key LambdaLR uses),
     `max_norm`, `num_iterations` and `iteration`. A dict without `iteration` (a torch.optim.SGD checkpoint) restarts the
     schedule at iteration 0 from its `initial_lr` (or its `lr`), as the reference's own resume does (train.py:142-151);
-    keys it lacks are taken from the constructor."""
+    keys it lacks are taken from the constructor.
+
+    Packed operands: when the parameters being updated all belong to one UpDownCaptioner whose packed bf16 / fp32
+    operands are current, `step()` writes the updated operands in the same pass (one launch instead of the update
+    followed by a re-pack of every updated weight at the next forward); results are bit-identical. `fuse_pack=False`
+    always takes the plain update, after which the next forward re-packs."""
 
     def __init__(self, params: Iterable[torch.nn.Parameter], lr=0.015, momentum=0.9, weight_decay=0.001,
-                 max_norm=12.5, num_iterations=70000, legacy_zero_grad=False):
+                 max_norm=12.5, num_iterations=70000, legacy_zero_grad=False, fuse_pack=True):
         defaults = dict(lr=lr, momentum=momentum, dampening=0, weight_decay=weight_decay, nesterov=False,
                         maximize=False, foreach=None, differentiable=False, fused=None,
                         max_norm=max_norm, num_iterations=num_iterations, iteration=0)
@@ -38,6 +44,7 @@ class FusedClipSGD(torch.optim.Optimizer):
             raise ValueError("FusedClipSGD takes one parameter group")
         self.param_groups[0].setdefault("initial_lr", self.param_groups[0]["lr"])
         self.legacy_zero_grad = legacy_zero_grad
+        self.fuse_pack = fuse_pack
         self._partial = None
 
     def __setstate__(self, state):
@@ -114,18 +121,21 @@ class FusedClipSGD(torch.optim.Optimizer):
         chunks = sum((p.numel() + 16383) // 16384 for p in ps)
         if self._partial is None or self._partial.numel() < chunks + 1 or self._partial.device != dev:
             self._partial = torch.empty(chunks + 1, dtype=torch.float32, device=dev)
-        vp = C.c_void_p
-        _lib.check(L.sscvae_sgd_step_multi(
-            n, (vp * n)(*[p.data_ptr() for p in ps]), (vp * n)(*[None if g is None else g.data_ptr() for g in grads]),
-            (vp * n)(*[b.data_ptr() for b in bufs]), (C.c_uint64 * n)(*[p.numel() for p in ps]),
-            (C.c_int32 * n)(*firsts), float(group["max_norm"]), float(group["lr"]), float(group["momentum"]),
-            float(group["weight_decay"]), float(grad_scale),
-            _lib.ptr(self._partial), self._partial.numel(), stream))
+        hyper = (group["max_norm"], group["lr"], group["momentum"], group["weight_decay"], grad_scale)
+        owner = PACKED_OWNERS.get(ps[0]) if self.fuse_pack else None
+        owner = owner() if owner is not None else None
+        if owner is None or not owner._sgd_step_packed(ps, grads, bufs, firsts, hyper, self._partial):
+            vp = C.c_void_p
+            _lib.check(L.sscvae_sgd_step_multi(
+                n, (vp * n)(*[p.data_ptr() for p in ps]), (vp * n)(*[None if g is None else g.data_ptr() for g in grads]),
+                (vp * n)(*[b.data_ptr() for b in bufs]), (C.c_uint64 * n)(*[p.numel() for p in ps]),
+                (C.c_int32 * n)(*firsts), *[float(h) for h in hyper], _lib.ptr(self._partial), self._partial.numel(),
+                stream))
+            for p in ps:
+                # the kernel wrote through raw pointers: tell autograd (and the captioner's packed-weight cache, which
+                # is keyed on the version counters) that the parameters changed
+                torch.autograd.graph.increment_version(p)
         for p, b in new:
             state[p]["momentum_buffer"] = b
-        for p in ps:
-            # the kernel wrote through raw pointers: tell autograd (and the captioner's packed-weight cache, which is
-            # keyed on the version counters) that the parameters changed
-            torch.autograd.graph.increment_version(p)
         group["iteration"] += 1
         group["lr"] = group["initial_lr"] * (1 - group["iteration"] / group["num_iterations"])    # train.py:132-134
