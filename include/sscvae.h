@@ -262,7 +262,25 @@ int sscvae_decode_samples_search(SscvaeHandle* h, int batch, int samples, int nu
 int sscvae_decode_samples_search_region(const SscvaeHandle* h, int batch, int samples, int num_boxes, int states, int beam,
                                         int fsm_per_sample, const char* name, size_t* offset, size_t* bytes);
 
-/* Named view into the decode workspace for tests ("tok_hist", "bp_hist", "score_hist" (L,B*S*K), "logits", ...). */
+/* ---- grounding: the attention weights over the boxes that stood behind every word (updown_captioner.py:371-455 returns
+ * them as the last element of its eval step; attention.py:68-97). Every decode call keeps the (B*samples*S*K, N) weights
+ * of each step in `workspace`; this call walks the back-pointers of each search from its exit step, as the back-trace of
+ * the predictions does, and gathers, per word, the weights of the row whose log-probabilities chose it (word 0: the
+ * search's single step-0 row). Words after a caption's first boundary token and steps at or after the search's own
+ * n_steps are 0; the boundary word keeps its weights. Masked (all-zero) boxes are 0. One kernel launch.
+ *
+ * Attention over the boxes behind every word of the searches of the LAST decode call on this handle
+ * (sscvae_decode / sscvae_decode_samples / sscvae_decode_samples_search) that filled `workspace`.
+ * valid_states: (B*samples, S) uint8 when the caller applied the object/attribute rule (sscvae_select_best_beam),
+ * else NULL (the rule search_finish applied). attention_all may be NULL.
+ * samples = 1 for sscvae_decode; S = K = 1 for sscvae_decode_samples. Returns SSCVAE_ERR_BAD_ARG before any decode call on
+ * the handle, for a NULL workspace or attention_best, and for a workspace smaller than the last call's. */
+int sscvae_decode_attention(SscvaeHandle* h, const void* workspace, size_t workspace_bytes, const uint8_t* valid_states,
+                            float* attention_all /* (B*samples,S,K,L,N) */, float* attention_best /* (B*samples,L,N) */,
+                            void* stream);
+
+/* Named view into the decode workspace for tests ("tok_hist", "bp_hist", "score_hist" (L,B*S*K), "alpha_hist" (L,B*S*K,N),
+ * "logits", ...). */
 int sscvae_decode_region(const SscvaeHandle* h, int batch, int num_boxes, int states, int beam, const char* name,
                          size_t* offset, size_t* bytes);
 

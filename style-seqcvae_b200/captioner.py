@@ -239,6 +239,9 @@ class UpDownCaptioner(nn.Module):
         self._grad_view_cache = None
         self._grad_flat = {}
         self.rng_mode = "philox"           # "reference": draw eps from the CPU generator like updown_cell.py:206
+        # True: outputs also carry "attention", the attention weights over the boxes behind every word (the last element
+        # of the reference's eval step, updown_captioner.py:371-455): fp32, new tensors, not differentiable
+        self.return_attention = False
         self._eps_override = None          # tests: explicit eps tensor
         self._call_counter = 0
         self.last_search = None
@@ -515,10 +518,32 @@ class UpDownCaptioner(nn.Module):
                 assert eps.shape == (T, B, self.z_space)
             loss, kld = _TrainStep.apply(self, image_features, caption_tokens, sentiment, obj_means, eps, self._next_seed(),
                                          *self._weight_tensors())
-            return {"loss": loss, "kld": kld}
+            out = {"loss": loss, "kld": kld}
+            if self.return_attention:
+                # the forward kernels keep alpha time-major, (T, B, N), for the backward pass: a (B, T, N) copy
+                alpha = self.train_region(B, N, "alpha", torch.float32, (T, B, N))
+                out["attention"] = alpha.detach().transpose(0, 1).clone(memory_format=torch.contiguous_format)
+            return out
 
-        return {"predictions": self._decode(image_features, sentiment, fsm, num_constraints, obj_means, constraints,
-                                            constraint2states)}
+        pred, attention = self._decode(image_features, sentiment, fsm, num_constraints, obj_means, constraints,
+                                       constraint2states)
+        out = {"predictions": pred}
+        if attention is not None:
+            out["attention"] = attention
+        return out
+
+    def _decode_attention(self, ws, valid, num_boxes, rows, all_shape=None):
+        """sscvae_decode_attention on the workspace of the decode call that just ran (one kernel launch): the attention
+        weights behind every word of the returned caption of each of its `rows` searches, (rows, steps, N), and, unless
+        `all_shape` is None, of every beam, all_shape + (steps, N). `valid`: the (rows, S) uint8 mask the caller passed to
+        sscvae_select_best_beam, or None."""
+        steps, dev = self._max_caption_length, ws.device
+        best = torch.empty(rows, steps, num_boxes, dtype=torch.float32, device=dev)
+        every = None if all_shape is None else torch.empty(*all_shape, steps, num_boxes, dtype=torch.float32, device=dev)
+        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _lib.check(_lib.lib().sscvae_decode_attention(self._handle, _lib.ptr(ws), ws.numel(), _lib.ptr(valid), _lib.ptr(every),
+                                                      _lib.ptr(best), stream))
+        return best, every
 
     # ------------------------------------------------------------------------------------------
     def translate_obj_atts2obj_means(self, obj_atts) -> torch.Tensor:
@@ -571,7 +596,10 @@ class UpDownCaptioner(nn.Module):
 
         use_cbs=True: one constrained beam search (beam_size, per_node_beam_size) per (image, sample), exactly what
         n_samples calls of forward() on single images would run; see `_sample_search`. Returns
-        {"predictions": (B, n_samples, n) int64, "n_steps": (B, n_samples) int64}."""
+        {"predictions": (B, n_samples, n) int64, "n_steps": (B, n_samples) int64}.
+
+        return_attention: both results gain "attention", (B, n_samples, n, N) fp32, the attention weights over the boxes
+        behind every word (zero after the caption's first boundary token)."""
         self._require_cuda(image_features)
         if self._use_cbs:
             return self._sample_search(image_features, sentiment, n_samples, obj_atts, fsm, num_constraints, constraints,
@@ -618,8 +646,12 @@ class UpDownCaptioner(nn.Module):
             self._handle, B, J, N, _lib.ptr(self._packed_weights()), _lib.ptr_array(self._weight_tensors()),
             _lib.ptr(image_features), _lib.ptr(sentiment), _lib.ptr(obj_means), _lib.ptr(eps), C.c_uint64(self._next_seed()),
             _lib.ptr(ws), nbytes, _lib.ptr(preds), _lib.ptr(scores), _lib.ptr(n_steps), stream))
+        att = self._decode_attention(ws, None, N, B * J)[0] if self.return_attention else None
         n = int(n_steps.item())
-        return {"predictions": preds[..., :n].clone(), "log_probs": scores.clone()}
+        out = {"predictions": preds[..., :n].clone(), "log_probs": scores.clone()}
+        if att is not None:
+            out["attention"] = att.view(B, J, steps, N)[:, :, :n].contiguous()
+        return out
 
     def _sample_search(self, image_features, sentiment, n_samples, obj_atts, fsm, num_constraints, constraints,
                        constraint2states):
@@ -637,7 +669,8 @@ class UpDownCaptioner(nn.Module):
           samples x S 8 x K 5 at V 10 000: 512 MB); sscvae_decode_samples_search_workspace_bytes gives the total.
         Returns {"predictions": (B, n_samples, n), "n_steps": (B, n_samples)} int64 with n = the largest n_steps; a
         sample's entries after its own n_steps are the boundary token. `last_search` holds every beam:
-        {"predictions": (B,J,S,K,n), "log_probs": (B,J,S,K), "n_steps": (B,J)}."""
+        {"predictions": (B,J,S,K,n), "log_probs": (B,J,S,K), "n_steps": (B,J)}, plus "attention" (B,J,S,K,n,N) with
+        return_attention."""
         from .fsm import FsmBits, valid_states_with_attributes
         L = _lib.lib()
         image_features = self._features(image_features)
@@ -722,10 +755,16 @@ class UpDownCaptioner(nn.Module):
         if valid is not None:
             _lib.check(L.sscvae_select_best_beam(_lib.ptr(preds), _lib.ptr(scores), _lib.ptr(valid), B * J, S, K, steps,
                                                  _lib.ptr(best), stream))
+        if self.return_attention:
+            att, every = self._decode_attention(ws, valid, N, B * J, (B, J, S, K))
         ns = n_steps.long()
         n = int(ns.max().item())                                    # each search's own early exit (cbs.py:167)
         self.last_search = {"predictions": preds[..., :n].clone(), "log_probs": scores.clone(), "n_steps": ns.clone()}
-        return {"predictions": best[..., :n].clone(), "n_steps": ns.clone()}
+        out = {"predictions": best[..., :n].clone(), "n_steps": ns.clone()}
+        if self.return_attention:
+            self.last_search["attention"] = every[..., :n, :].contiguous()
+            out["attention"] = att.view(B, J, steps, N)[:, :, :n].contiguous()
+        return out
 
     def sample_search_region(self, B, N, J, S, K, fsm_per_sample, name, dtype, shape):
         """Typed view of a named region of the last sample() workspace with use_cbs=True (tests / debugging)."""
@@ -817,6 +856,12 @@ class UpDownCaptioner(nn.Module):
         if valid is not None:
             _lib.check(L.sscvae_select_best_beam(_lib.ptr(preds), _lib.ptr(scores), _lib.ptr(valid), B, S, K, steps,
                                                  _lib.ptr(best), stream))
+        attention = None
+        if self.return_attention:
+            attention, every = self._decode_attention(ws, valid, N, B, (B, S, K))
         n = int(n_steps.item())                                     # the reference's data-dependent early exit (cbs.py:167)
         self.last_search = {"predictions": preds[..., :n].clone(), "log_probs": scores.clone(), "n_steps": n}
-        return best[:, :n].clone()
+        if attention is not None:
+            self.last_search["attention"] = every[..., :n, :].contiguous()
+            attention = attention[:, :n].contiguous()
+        return best[:, :n].clone(), attention

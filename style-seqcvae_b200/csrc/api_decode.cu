@@ -43,7 +43,7 @@ static void plan_decode(const Dims& d, int B, int N, int S, int K, int J, int fs
   if (d.cvar) p.add("pm", R * d.Z * f);      // per-row prior mean of the current step (updown_cell.py:160-163)
   p.add("acc", R * d.GP * f);
   p.add("q", R * d.A * f);
-  p.add("alpha", R * N * f);
+  p.add("alpha_hist", (size_t)d.L * R * N * f);          // attention weights of every row of every step (step 0: Bv rows)
   if (d.tied) p.add("ob", R * d.Ep * b);
   p.add("logits", R * d.V * f);
   const size_t nst = gemm_rowstats_tiles(d.V);            // greedy: softmax statistics of the head GEMM instead of logits
@@ -57,6 +57,13 @@ static void plan_decode(const Dims& d, int B, int N, int S, int K, int J, int fs
   p.add("bp_hist", (size_t)d.L * R * 4);
   p.add("score_hist", (size_t)d.L * R * f);
   p.add("best_samples", Bv * d.L * 8);                 // sscvae_decode_samples: the "best beam" copy of its predictions
+  p.add("best_state", Bv * 4);                         // per search: the state whose beam 0 search_finish returned
+  p.add("search_steps", Bv * 4);                       // per search: its step count (n_steps of its exit)
+}
+
+// The decode entry points record their shape, so sscvae_decode_attention finds the regions of the last call.
+static void note_decode(Handle* h, int B, int N, int S, int K, int J, int fsm_tables) {
+  h->last_B = B; h->last_N = N; h->last_S = S; h->last_K = K; h->last_J = J; h->last_T = fsm_tables;
 }
 
 const Plan& Handle::decode_plan(int B, int N, int S, int K, int J, int fsm_tables) {
@@ -147,6 +154,7 @@ static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, int 
   auto cell = [&](int rows, const int* tokens, const int* rowmap, bool first, const float* eps_t, int eps_stride,
                   int step) -> int {
     // in = index 0, out = index 1
+    float* alpha_t = Wf("alpha_hist") + (size_t)step * R * N;      // kept for sscvae_decode_attention
     TRY(embed_gather_rows(s, tokens, rows, Pb("embb"), d.Ep, Wb("embb_r")));
     {
       LstmFwdArgs l = {};
@@ -167,13 +175,13 @@ static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, int 
       aa.q = Wf("q"); aa.ld_q = d.A; aa.proj = Wb("projb"); aa.feats = Wb("featsb"); aa.mask = Wf("mask");
       aa.w_a = W(SSCVAE_W_ATT_VEC);
       aa.rows_per_image = first ? J : SK * J;                  // rowmap0: r / J ; rowmap: r / (SK * J)
-      TRY(attention_forward(s, aa, Wf("alpha"), nullptr, Wb("XE"), KXe));
+      TRY(attention_forward(s, aa, alpha_t, nullptr, Wb("XE"), KXe));
     }
     {  // eval: z ~ N(prior_mean, prior_var) (updown_cell.py:200-208); no encoder LSTM
       LatentArgs la = {}; la.R = rows; la.Z = d.Z; la.Zp = d.Zp; la.sentiment_vae = d.sv; la.prior_var = d.prior_std * d.prior_std;
       la.prior_mean_row = Wf("pm_row"); la.rowmap = rowmap;
       if (d.cvar) {  // attribute-grounded prior: mean of this step from the row's attention weights; also the block c
-        TRY(prior_mean_forward(s, Wf("alpha"), obj, rowmap, rows, N, d.Z, Wf("pm"), Wb("ZB") + d.Zp, d.ZC, d.cond));
+        TRY(prior_mean_forward(s, alpha_t, obj, rowmap, rows, N, d.Z, Wf("pm"), Wb("ZB") + d.Zp, d.ZC, d.cond));
         la.prior_mean_full = Wf("pm");
       }
       TRY(latent_forward_eval(s, la, eps_t, eps_stride, seed_dev, (unsigned long long)step, Wb("ZB"), d.ZC));
@@ -243,7 +251,7 @@ static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, int 
     TRY(state_gather(s, bp_hist + (size_t)t * R, R, SK, XA[1], XA[0], 2 * Hp, c1[1], c1[0], cd[1], cd[0], H));
   }
   TRY(search_finish(s, tok_hist, bp_hist, score_hist, L, Bv, S, K, d.boundary, num_constraints, min_sat, gpf,
-                    exit_per_search ? 1 : 0, predictions, log_probs, best, n_steps));
+                    exit_per_search ? 1 : 0, predictions, log_probs, best, n_steps, Wi("best_state"), Wi("search_steps")));
   return 0;
 }
 
@@ -313,7 +321,7 @@ int sscvae_search_finish(const int32_t* tokens_hist, const int32_t* backptr_hist
   return search_finish(reinterpret_cast<cudaStream_t>(stream), tokens_hist, backptr_hist, scores_hist, steps_run, batch,
                        states, beam, end_index, reinterpret_cast<const long long*>(num_constraints),
                        min_constraints_to_satisfy, 1, 0, reinterpret_cast<long long*>(predictions), final_scores,
-                       reinterpret_cast<long long*>(best), n_steps);
+                       reinterpret_cast<long long*>(best), n_steps, nullptr, nullptr);
 }
 
 size_t sscvae_decode_workspace_bytes(const SscvaeHandle* hh, int batch, int num_boxes, int states, int beam) {
@@ -362,6 +370,7 @@ int sscvae_decode(SscvaeHandle* hh, int batch, int num_boxes, int states, int be
                         (const void*)log_probs, (const void*)best, (const void*)n_steps})
     key_add(key, q);
   for (int i = 0; i < SSCVAE_W_COUNT; ++i) key_add(key, weights[i]);
+  note_decode(h, batch, num_boxes, states, beam, 1, batch);
   return run_with_graph(h->dec_graphs, key, st, true, [&](cudaStream_t s) {
     return decode_impl(h, batch, 1, num_boxes, states, beam, per_node, 1, false, reinterpret_cast<const char*>(packed), weights,
                        image_features, sentiment, obj_means, fsm, reinterpret_cast<const long long*>(num_constraints),
@@ -393,6 +402,7 @@ int sscvae_decode_samples(SscvaeHandle* hh, int batch, int samples, int num_boxe
   for (int i = 0; i < SSCVAE_W_COUNT; ++i) key_add(key, weights[i]);
   char* wsb = reinterpret_cast<char*>(workspace);
   long long* best = reinterpret_cast<long long*>(wsb + dp.find("best_samples")->off);
+  note_decode(h, batch, num_boxes, 1, 1, samples, batch * samples);
   return run_with_graph(h->dec_graphs, key, st, true, [&](cudaStream_t s) {
     return decode_impl(h, batch, samples, num_boxes, 1, 1, 1, 1, false, reinterpret_cast<const char*>(packed), weights, image_features,
                        sentiment, obj_means, nullptr, nullptr, 0, eps, seed, wsb, workspace_bytes, reinterpret_cast<long long*>(predictions),
@@ -456,6 +466,7 @@ int sscvae_decode_samples_search(SscvaeHandle* hh, int batch, int samples, int n
                         (const void*)log_probs, (const void*)best, (const void*)n_steps})
     key_add(key, q);
   for (int i = 0; i < SSCVAE_W_COUNT; ++i) key_add(key, weights[i]);
+  note_decode(h, batch, num_boxes, states, beam, samples, fsm_per_sample ? batch * samples : batch);
   return run_with_graph(h->dec_graphs, key, st, true, [&](cudaStream_t s) {
     return decode_impl(h, batch, samples, num_boxes, states, beam, per_node, fsm_per_sample ? 1 : samples, true,
                        reinterpret_cast<const char*>(packed), weights, image_features, sentiment, obj_means, fsm,
@@ -463,6 +474,22 @@ int sscvae_decode_samples_search(SscvaeHandle* hh, int batch, int samples, int n
                        reinterpret_cast<char*>(workspace), workspace_bytes, reinterpret_cast<long long*>(predictions),
                        log_probs, reinterpret_cast<long long*>(best), n_steps, s);
   });
+}
+
+int sscvae_decode_attention(SscvaeHandle* hh, const void* workspace, size_t workspace_bytes, const uint8_t* valid_states,
+                            float* attention_all, float* attention_best, void* stream) {
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  REQUIRE(h && workspace && attention_best, "NULL argument");
+  REQUIRE(h->last_B > 0, "no decode call on this handle yet");
+  const Plan& dp = h->decode_plan(h->last_B, h->last_N, h->last_S, h->last_K, h->last_J, h->last_T);
+  REQUIRE(workspace_bytes >= dp.total, "workspace too small for the last decode call: %zu < %zu", workspace_bytes, dp.total);
+  const char* ws = reinterpret_cast<const char*>(workspace);
+  auto Wi = [&](const char* n) { return reinterpret_cast<const int32_t*>(ws + dp.find(n)->off); };
+  return search_attention(reinterpret_cast<cudaStream_t>(stream), Wi("tok_hist"), Wi("bp_hist"),
+                          reinterpret_cast<const float*>(ws + dp.find("score_hist")->off),
+                          reinterpret_cast<const float*>(ws + dp.find("alpha_hist")->off), h->d.L, h->last_B * h->last_J,
+                          h->last_S, h->last_K, h->last_N, h->d.boundary, Wi("search_steps"), Wi("best_state"), valid_states,
+                          attention_all, attention_best);
 }
 
 }  // extern "C"

@@ -42,6 +42,8 @@ struct Handle {
   Plan pp;                 // packed weights
   Plan tp; int tp_B = -1, tp_N = -1;   // training workspace for the last (B,N)
   Plan dp; int dp_B = -1, dp_N = -1, dp_S = -1, dp_K = -1, dp_J = -1, dp_T = -1;   // decode workspace
+  // shape of the last decode call (the plan above also follows workspace-size and region queries): sscvae_decode_attention
+  int last_B = -1, last_N = -1, last_S = -1, last_K = -1, last_J = -1, last_T = -1;
   GraphCache fwd_graphs, bwd_graphs, dec_graphs;
   // per-handle options (sscvae_set_option), consumed by the following calls
   int opt_features_bf16 = 0;           // image_features pointers are bf16 (B,N,F) instead of fp32

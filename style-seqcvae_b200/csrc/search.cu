@@ -70,21 +70,31 @@ int fsm_build(cudaStream_t st, const int32_t* rec, const int32_t* rec_off, const
   return 0;
 }
 
+// ---- the state whose beam 0 a finished search returns (decoding.py:82-135); score0[s * stride] = beam 0 of state s ----
+//   valid != null: the caller's valid states (decoding.py:87-135, object / attribute rule);
+//   nc >= 0:       cbs_simple, states s < 2^nc that satisfy min(nc, min_sat) constraints (decoding.py:82-86,128-134);
+//   otherwise:     state 0 (plain beam search).
+// The first maximum wins, like torch.argmax over the listed states; state 0 when no state qualifies.
+__device__ __forceinline__ int select_state(const float* __restrict__ score0, int stride, int S, const uint8_t* __restrict__ valid, int nc,
+                            int min_sat) {
+  if (valid == nullptr && nc < 0) return 0;
+  const int need = nc < min_sat ? nc : min_sat;
+  int arg = 0; float v = 0.f; bool have = false;
+  for (int s = 0; s < S; ++s) {
+    if (valid ? !valid[s] : (s >= (1 << nc) || __popc(s) < need)) continue;
+    const float x = score0[(size_t)s * stride];
+    if (!have || x > v) { arg = s; v = x; have = true; }
+  }
+  return arg;
+}
+
 // ---- best beam among an explicit set of valid states (decoding.py:125-135 with the caller's valid_states) ----
 __global__ void select_best_masked_kernel(const long long* __restrict__ predictions, const float* __restrict__ scores,
                                           const uint8_t* __restrict__ valid, int S, int K, int steps,
                                           long long* __restrict__ best) {
   const int b = blockIdx.x;
   __shared__ int s_best;
-  if (threadIdx.x == 0) {
-    int arg = -1; float v = 0.f;
-    for (int s = 0; s < S; ++s) {                     // first maximum, like torch.argmax over the listed states
-      if (!valid[(size_t)b * S + s]) continue;
-      const float x = scores[((size_t)b * S + s) * K];
-      if (arg < 0 || x > v) { arg = s; v = x; }
-    }
-    s_best = arg < 0 ? 0 : arg;
-  }
+  if (threadIdx.x == 0) s_best = select_state(scores + (size_t)b * S * K, K, S, valid + (size_t)b * S, -1, 0);
   __syncthreads();
   const long long* src = predictions + (((size_t)b * S + s_best) * K) * steps;
   for (int t = threadIdx.x; t < steps; t += blockDim.x) best[(size_t)b * steps + t] = src[t];
@@ -445,7 +455,8 @@ __global__ void search_finish_kernel(const int32_t* __restrict__ tokens_hist, co
                                      int end_index, const long long* __restrict__ num_constraints, int min_sat,
                                      int groups_per_table, int groups_per_exit, long long* __restrict__ predictions,
                                      float* __restrict__ final_scores, long long* __restrict__ best,
-                                     const int32_t* __restrict__ n_steps) {
+                                     const int32_t* __restrict__ n_steps, int32_t* __restrict__ best_state_out,
+                                     int32_t* __restrict__ steps_out) {
   extern __shared__ float s_score[];                        // S*K
   const int b = blockIdx.x;
   const int SK = S * K, R = B * SK;
@@ -469,27 +480,20 @@ __global__ void search_finish_kernel(const int32_t* __restrict__ tokens_hist, co
   }
   __syncthreads();
   if (threadIdx.x == 0) {
-    int best_state = 0;
-    if (num_constraints) {                                  // decoding.py:82-86,128-134 (cbs_simple)
-      const int nc = (int)num_constraints[groups_per_table > 1 ? b / groups_per_table : b];
-      const int need = nc < min_sat ? nc : min_sat;
-      float bv = 0.f; bool have = false;
-      for (int s = 0; s < (1 << nc) && s < S; ++s) {
-        if (__popc(s) < need) continue;
-        const float v = s_score[s * K];
-        if (!have || v > bv) { bv = v; best_state = s; have = true; }
-      }
-    }
+    const int nc = num_constraints ? (int)num_constraints[groups_per_table > 1 ? b / groups_per_table : b] : -1;
+    const int best_state = select_state(s_score, K, S, nullptr, nc, min_sat);
     const long long* src = predictions + ((size_t)b * SK + (size_t)best_state * K) * steps_run;
     for (int t = 0; t < steps_run; ++t) best[(size_t)b * steps_run + t] = src[t];
+    if (best_state_out) { best_state_out[b] = best_state; steps_out[b] = n; }
   }
 }
 
 int search_finish(cudaStream_t st, const int32_t* tokens_hist, const int32_t* backptr_hist, const float* scores_hist,
                   int steps_run, int B, int S, int K, int end_index, const long long* num_constraints, int min_sat,
                   int groups_per_table, int groups_per_exit, long long* predictions, float* final_scores, long long* best,
-                  int32_t* n_steps) {
+                  int32_t* n_steps, int32_t* best_state, int32_t* group_steps) {
   REQUIRE(steps_run >= 1, "no search steps");
+  REQUIRE((best_state == nullptr) == (group_steps == nullptr), "best_state and group_steps go together");
   REQUIRE(groups_per_exit >= 0 && (groups_per_exit == 0 || B % groups_per_exit == 0), "bad exit grouping %d of %d groups",
           groups_per_exit, B);
   const int R = B * S * K;
@@ -503,7 +507,69 @@ int search_finish(cudaStream_t st, const int32_t* tokens_hist, const int32_t* ba
   LAUNCHED();
   search_finish_kernel<<<B, 128, S * K * sizeof(float), st>>>(tokens_hist, backptr_hist, scores_hist, steps_run, B, S, K,
                                                             end_index, num_constraints, min_sat, groups_per_table,
-                                                            groups_per_exit, predictions, final_scores, best, n_steps);
+                                                            groups_per_exit, predictions, final_scores, best, n_steps,
+                                                            best_state, group_steps);
+  LAUNCHED();
+  return 0;
+}
+
+// Attention behind every word. Block (g, y) walks the back-pointers of search group g the way search_finish_kernel does,
+// from the group's exit step n - 1, for beam w = y (y < SK, all beams) or for beam 0 of the returned state (the last y).
+// Word t of the beam was chosen from the logits of one row of step t; that row's attention weights are the word's:
+//   word 0: alpha[0][g] (step 0 runs one row per group);  word t >= 1: alpha[t][base + bp[t][cur_t]] = alpha[t][base + cur_(t-1)]
+// with cur_(n-1) = w, cur_(t-1) = bp[t][cur_t]. Words after the first boundary token and steps >= n are zero.
+__global__ void __launch_bounds__(128) search_attention_kernel(
+    const int32_t* __restrict__ tokens_hist, const int32_t* __restrict__ backptr_hist, const float* __restrict__ scores_hist,
+    const float* __restrict__ alpha_hist, int L, int B, int S, int K, int N, int end_index,
+    const int32_t* __restrict__ group_steps, const int32_t* __restrict__ best_state, const uint8_t* __restrict__ valid,
+    float* __restrict__ att_all, float* __restrict__ att_best) {
+  extern __shared__ int s_mem[];
+  int* s_row = s_mem;                                       // (L) alpha row of word t within step t, -1 = zero
+  int* s_tok = s_mem + L;                                   // (L) word t
+  const int g = blockIdx.x, SK = S * K, R = B * SK, base = g * SK;
+  const bool best = att_all == nullptr || (int)blockIdx.y == SK;
+  if (threadIdx.x == 0) {
+    const int n = group_steps[g];
+    int cur = blockIdx.y;
+    if (best) {
+      const int st = valid ? select_state(scores_hist + (size_t)(n - 1) * R + base, K, S, valid + (size_t)g * S, -1, 0)
+                           : best_state[g];
+      cur = st * K;
+    }
+    // both walks stay rolled: unrolled, this thread's loads spill to local memory
+#pragma unroll 1
+    for (int t = n - 1; t >= 1; --t) {                      // cbs.py:252-271, as search_finish_kernel
+      s_tok[t] = tokens_hist[(size_t)t * R + base + cur];
+      cur = backptr_hist[(size_t)t * R + base + cur];
+      s_row[t] = base + cur;
+    }
+    s_tok[0] = tokens_hist[base + cur];
+    s_row[0] = g;
+    bool ended = false;
+#pragma unroll 1
+    for (int t = 0; t < L; ++t) {
+      if (ended || t >= n) s_row[t] = -1;
+      else ended = s_tok[t] == end_index;
+    }
+  }
+  __syncthreads();
+  float* out = best ? att_best + (size_t)g * L * N : att_all + ((size_t)g * SK + blockIdx.y) * L * N;
+  for (int i = threadIdx.x; i < L * N; i += blockDim.x) {
+    const int t = i / N, row = s_row[t];
+    out[i] = row < 0 ? 0.f : alpha_hist[((size_t)t * R + row) * N + i % N];
+  }
+}
+
+int search_attention(cudaStream_t st, const int32_t* tokens_hist, const int32_t* backptr_hist, const float* scores_hist,
+                     const float* alpha_hist, int L, int B, int S, int K, int N, int end_index, const int32_t* group_steps,
+                     const int32_t* best_state, const uint8_t* valid, float* att_all, float* att_best) {
+  REQUIRE(att_best != nullptr, "attention_best is required");
+  const int SK = S * K;
+  const unsigned ny = att_all ? SK + 1 : 1;
+  PROF_SCOPE(st, "search_attention", 0, (double)B * ny * L * N * 8.0);
+  search_attention_kernel<<<dim3(B, ny), 128, 2 * L * sizeof(int), st>>>(tokens_hist, backptr_hist, scores_hist, alpha_hist, L, B,
+                                                                    S, K, N, end_index, group_steps, best_state, valid,
+                                                                    att_all, att_best);
   LAUNCHED();
   return 0;
 }

@@ -40,10 +40,20 @@ int search_merge(cudaStream_t st, const float* cand_val, const int32_t* cand_tok
 // Back-trace, early exit and best beam of B search groups of S*K rows. Group b reads num_constraints[b / groups_per_table].
 // groups_per_exit = 0: one exit for the whole batch (n_steps[0], the reference's batched loop, cbs.py:167); g > 0: one exit
 // per set of g consecutive groups (n_steps[b / g]); 1 = every search stops on its own, as a batch-1 call would.
+// best_state / group_steps (B) int32, both or neither: the state whose beam 0 group b returned and the group's step count,
+// kept for search_attention.
 int search_finish(cudaStream_t st, const int32_t* tokens_hist, const int32_t* backptr_hist, const float* scores_hist,
                   int steps_run, int B, int S, int K, int end_index, const long long* num_constraints, int min_sat,
                   int groups_per_table, int groups_per_exit, long long* predictions, float* final_scores, long long* best,
-                  int32_t* n_steps);
+                  int32_t* n_steps, int32_t* best_state, int32_t* group_steps);
+
+// Attention over the boxes behind every word of the B finished searches (one launch): alpha_hist (L, B*S*K, N) holds the
+// attention weights of every row of every step (step 0: rows 0..B-1, one per group). att_all (B,S,K,L,N) or null: every
+// beam; att_best (B,L,N): beam 0 of the returned state, which is best_state[b], or, with valid (B,S) uint8, the state
+// select_best_masked picks. Words after a beam's first end_index token and steps >= group_steps[b] are zero.
+int search_attention(cudaStream_t st, const int32_t* tokens_hist, const int32_t* backptr_hist, const float* scores_hist,
+                     const float* alpha_hist, int L, int B, int S, int K, int N, int end_index, const int32_t* group_steps,
+                     const int32_t* best_state, const uint8_t* valid, float* att_all, float* att_best);
 
 // new_state[r] = old_state[img(r)*SK + bp[r]] for the four recurrent tensors of the eval cell
 int state_gather(cudaStream_t st, const int32_t* bp, int R, int SK, const bf16* xa_src, bf16* xa_dst, int ld_xa,
