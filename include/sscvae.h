@@ -284,6 +284,32 @@ int sscvae_decode_attention(SscvaeHandle* h, const void* workspace, size_t works
 int sscvae_decode_region(const SscvaeHandle* h, int batch, int num_boxes, int states, int beam, const char* name,
                          size_t* offset, size_t* bytes);
 
+/* ---- one decode step: the reference's `_decode_step` in eval mode (updown_captioner.py:371-455), the step function its
+ * forward hands to the search (updown_captioner.py:325-343), for callers that run their own search, rerank, or want the
+ * per-step log-probabilities and states. R = rows rows; row r belongs to image r / (R/B), the aligned layout of every decode
+ * call (the reference replicates image features with repeat_interleave but tiles sentiment / prior rows with `repeat`, which
+ * agrees with this only at B = 1 or uniform sentiment: SURVEY §7 Q1).
+ *   prior_mean, prior_var: (B,Z) per image, or NULL -> the prior forward() builds (sentiment * senti_prior_multip or 0;
+ *     prior_std^2). With sentiment_vae == 2 the attention-weighted attribute mean replaces the mean (updown_cell.py:160-163);
+ *     with simple_vae it is zero (updown_cell.py:165-166).
+ *   prev_tokens: (R) int64 device ids in [0, V) (not checked here: the kernels index the embedding unchecked).
+ *   states_in: host array of 6 device pointers (R,H) fp32 in the reference's order h1, c1, h_encoder, c_encoder, h_decoder,
+ *     c_decoder (the encoder pair is not read in eval and may be NULL), or NULL = zero states (the search's first step).
+ *   eps: (R,Z) normals, or NULL -> Philox(seed); a caller passes a new seed per call.
+ *   Outputs (device, fp32): log_probs (R,V) = log-softmax of the step's logits; states_out = host array of 4 device
+ *     pointers (R,H): h1, c1, h_decoder, c_decoder; alpha (R,N) attention weights; prior_mean_out (R,Z) the prior mean of
+ *     the step (the prior log-variance the reference also returns is log(prior_var) of the row's image).
+ * Options "features_bf16" and "reuse_image_state" (the workspace holds this batch's per-image state from an earlier step
+ * call; it stays valid across calls with another row count) apply. R % B != 0, a NULL required pointer, or a missing
+ * sentiment / obj_means return SSCVAE_ERR_BAD_ARG before any device work. Not captured as a CUDA graph. */
+size_t sscvae_decode_step_workspace_bytes(const SscvaeHandle* h, int batch, int rows, int num_boxes);
+int sscvae_decode_step(SscvaeHandle* h, int batch, int rows, int num_boxes, const void* packed, const void* const* weights_f32,
+                       const float* image_features, const float* sentiment, const float* obj_means,
+                       const float* prior_mean, const float* prior_var, const int64_t* prev_tokens,
+                       const float* const* states_in, const float* eps, uint64_t seed, void* workspace,
+                       size_t workspace_bytes, float* log_probs, float* const* states_out, float* alpha,
+                       float* prior_mean_out, void* stream);
+
 /* ---- training-step tail (SURVEY §8(f)-1): clip_grad_norm_ + SGD(momentum, weight decay) fused over
  * a flat parameter buffer; replaces var_updown/scripts/train.py:173-176. */
 int sscvae_grad_sqnorm(const float* grads, size_t n, float* partial /*>= 1024 floats*/, float* sqnorm_out, void* stream);
@@ -319,7 +345,7 @@ int sscvae_sgd_step_packed(SscvaeHandle* h, const void* const* weights, const vo
  *   "fsm_packed"        1: the `fsm` pointer of sscvae_decode is the (B,S,V) uint32 bit table (sscvae_fsm_build / sscvae_fsm_pack)
  *                       instead of the reference's (B,S,S,V) uint8 tensor.
  *   "reuse_image_state" 1: the decode workspace already holds the per-image state of THIS batch (bf16 features, mask, mean
- *                       features, W_v projection): sscvae_decode / sscvae_decode_samples skip recomputing it. The analogue
+ *                       features, W_v projection): sscvae_decode / sscvae_decode_samples / sscvae_decode_step skip recomputing it. The analogue
  *                       of the reference's lru_cache on the projected features (updown-baseline/updown/modules/attention.py:99). */
 int sscvae_set_option(SscvaeHandle* h, const char* name, int value);
 

@@ -47,6 +47,7 @@ SYMBOLS = [
     "sscvae_decode_samples_search_region", "sscvae_grad_sqnorm", "sscvae_sgd_step", "sscvae_test_gemm",
     "sscvae_profile_enable", "sscvae_profile_report", "sscvae_test_gemm_grouped", "sscvae_test_transpose_bf16",
     "sscvae_sgd_step_packed", "sscvae_debug_sgd_pack_jobs", "sscvae_decode_attention",
+    "sscvae_decode_step_workspace_bytes", "sscvae_decode_step",
 ]
 
 
@@ -108,6 +109,10 @@ def lib():
     L.sscvae_decode_samples_search.argtypes = [vp, i32, i32, i32, i32, i32, i32, vp, C.POINTER(vp), vp, vp, vp, vp, i32, vp, i32,
                                                vp, u64, vp, sz, vp, vp, vp, vp, vp]
     L.sscvae_decode_attention.argtypes = [vp, vp, sz, vp, vp, vp, vp]
+    L.sscvae_decode_step_workspace_bytes.argtypes = [vp, i32, i32, i32]
+    L.sscvae_decode_step_workspace_bytes.restype = sz
+    L.sscvae_decode_step.argtypes = [vp, i32, i32, i32, vp, C.POINTER(vp), vp, vp, vp, vp, vp, vp, C.POINTER(vp), vp, u64,
+                                     vp, sz, vp, C.POINTER(vp), vp, vp, vp]
     L.sscvae_decode_samples_search_region.argtypes = [vp, i32, i32, i32, i32, i32, i32, C.c_char_p, C.POINTER(sz), C.POINTER(sz)]
     L.sscvae_test_gemm_splitk.argtypes = [vp, i32, vp, i32, i32, i32, i32, vp, i32, i32, vp, vp]
     L.sscvae_sgd_step_multi.argtypes = [i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(u64), C.POINTER(i32),

@@ -546,6 +546,100 @@ class UpDownCaptioner(nn.Module):
         return best, every
 
     # ------------------------------------------------------------------------------------------
+    _STATE_KEYS = ("h1", "c1", "h_encoder", "c_encoder", "h_decoder", "c_decoder")
+
+    @torch.no_grad()
+    def _decode_step(self, image_features, obj_atts, previous_predictions, states, sentiment=None, prior_mean=None,
+                     prior_var=None):
+        """The reference's eval-mode step function (updown_captioner.py:371-455), which its forward hands to the search as
+        `partial(self._decode_step, image_features, obj_atts, sentiment=..., prior_mean=..., prior_var=...)`
+        (updown_captioner.py:325-343); `sscvae.ConstrainedBeamSearch` / `BeamSearch` take it the same way.
+
+        previous_predictions: (R,) token ids, R a multiple of B; row r belongs to image r // (R // B). states: the six
+        (R, H) tensors of the reference's state dict, or None for zero states. prior_mean / prior_var: (B, Z), or None
+        for the prior forward() builds. Returns the reference's eval 5-tuple
+        (log_probs (R, V), states, prior_mean (R, Z), prior_log_var (R, Z), attention (R, N)): new fp32 tensors, not
+        differentiable; h_encoder / c_encoder pass through (zeros for states=None). One sscvae_decode_step call; the
+        per-image state is recomputed only when the features changed (storage, shape, dtype or an in-place edit)."""
+        if self.training:
+            raise NotImplementedError("_decode_step runs in eval mode only; the fused training forward() is the training path")
+        self._require_cuda(image_features)
+        L = _lib.lib()
+        given = image_features
+        image_features = self._features(image_features)
+        dev = image_features.device
+        B, N, F = image_features.shape
+        if F != self.image_feature_size:
+            raise ValueError(f"image_features last dim {F} != image_feature_size {self.image_feature_size}")
+        prev = previous_predictions.to(dev).long().contiguous().view(-1)
+        R, H, Z, V = prev.numel(), self.hidden_size, self.z_space, self._vocab_size
+        if R == 0 or R % B != 0:
+            raise ValueError(f"previous_predictions has {R} rows, not a positive multiple of the batch size {B}")
+        # nn.Embedding raises on an out-of-range id; the kernels index the table unchecked (asynchronous: no host sync)
+        torch._assert_async(((prev >= 0) & (prev < V)).all(), "previous_predictions contains an id outside [0, vocab_size)")
+        if self.sentiment_vae == 1:
+            if sentiment is None:
+                raise ValueError("sentiment is required when sentiment_vae == 1")
+            sentiment = sentiment.to(dev).contiguous().float().view(B, 1)
+        else:
+            sentiment = None
+        obj_means = self._obj_means(obj_atts, B, N, dev)
+
+        def per_image(x, name):
+            if x is None:
+                return None
+            x = x.to(dev).contiguous().float()
+            if x.shape != (B, Z):
+                raise ValueError(f"{name} must be (B, z_space) = {(B, Z)}, got {tuple(x.shape)}")
+            return x
+        prior_mean, prior_var = per_image(prior_mean, "prior_mean"), per_image(prior_var, "prior_var")
+        if states is None:
+            s_in, enc = None, (torch.zeros(R, H, device=dev), torch.zeros(R, H, device=dev))
+        else:
+            st = {}
+            for k in self._STATE_KEYS:
+                v = states[k]
+                if v.shape != (R, H):
+                    raise ValueError(f"states[{k!r}] must be (R, hidden_size) = {(R, H)}, got {tuple(v.shape)}")
+                st[k] = v.to(dev).contiguous().float()
+            s_in = [st[k] for k in self._STATE_KEYS]
+            enc = (states["h_encoder"], states["c_encoder"])
+        eps = self._eps_override
+        if eps is None and self.rng_mode == "reference":
+            eps = torch.randn(R, Z)                                   # one (R,Z) CPU draw per step, like updown_cell.py:206
+        if eps is not None:
+            eps = eps.to(dev).contiguous().float()
+            assert eps.shape == (R, Z)
+        nbytes = L.sscvae_decode_step_workspace_bytes(self._handle, B, R, N)
+        # one workspace, grown on demand: a search calls with R = B first and R = B*S*K afterwards
+        ws = self._ws_cache.get(("step", dev))
+        if ws is None or ws.numel() < nbytes:
+            ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+            self._ws_cache[("step", dev)] = ws
+        # Keyed on the CALLER's tensor: `image_features` is a temporary copy for inputs that are not contiguous fp32 / bf16,
+        # and the allocator may hand its block to the next call's copy of different features.
+        key = (ws.data_ptr(), given.data_ptr(), given._version, tuple(given.shape), given.dtype, given.stride(),
+               self._weights_key(self._weight_tensors()))
+        last = getattr(self, "_step_image_state", None)
+        reuse = last is not None and last[0] is given and last[1] == key
+        self._step_image_state = (given, key)       # keeps the tensor alive: a new one cannot take over its storage
+        log_probs = torch.empty(R, V, device=dev)
+        h1, c1, hd, cd = (torch.empty(R, H, device=dev) for _ in range(4))
+        alpha = torch.empty(R, N, device=dev)
+        pm = torch.empty(R, Z, device=dev)
+        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _lib.check(L.sscvae_set_option(self._handle, b"reuse_image_state", int(reuse)))
+        _lib.check(L.sscvae_decode_step(
+            self._handle, B, R, N, _lib.ptr(self._packed_weights()), _lib.ptr_array(self._weight_tensors()),
+            _lib.ptr(image_features), _lib.ptr(sentiment), _lib.ptr(obj_means), _lib.ptr(prior_mean), _lib.ptr(prior_var),
+            _lib.ptr(prev), None if s_in is None else _lib.ptr_array(s_in), _lib.ptr(eps), C.c_uint64(self._next_seed()),
+            _lib.ptr(ws), ws.numel(), _lib.ptr(log_probs), _lib.ptr_array([h1, c1, hd, cd]), _lib.ptr(alpha), _lib.ptr(pm),
+            stream))
+        var = prior_var if prior_var is not None else torch.full((B, Z), float(self.prior_std), device=dev).pow(2)
+        prior_log_var = var.log().repeat_interleave(R // B, dim=0)
+        new_states = {"h1": h1, "c1": c1, "h_encoder": enc[0], "c_encoder": enc[1], "h_decoder": hd, "c_decoder": cd}
+        return log_probs, new_states, pm, prior_log_var, alpha
+
     def translate_obj_atts2obj_means(self, obj_atts) -> torch.Tensor:
         """Per-box attribute means of sentiment_vae == 2 (updown_captioner.py:509-532): `obj_atts` holds, per image, one
         `(object, [attribute strings])` entry per box; a box's mean is the average of `mean_choice[first word]` over its

@@ -79,6 +79,112 @@ static inline GemmSeg seg(const bf16* A, int lda, const bf16* B, int ldb, int K)
   GemmSeg s; s.A = A; s.lda = lda; s.B = B; s.ldb = ldb; s.K = K; return s;
 }
 
+// Named workspace regions and packed operands, shared by the fused decode and the single step.
+struct Views {
+  const char* pk; const Plan& pp; const void* const* wv; char* ws; const Plan& wp;
+  const float* W(int i) const { return reinterpret_cast<const float*>(wv[i]); }
+  const bf16* Pb(const char* n) const { return reinterpret_cast<const bf16*>(pk + pp.find(n)->off); }
+  const float* Pf(const char* n) const { return reinterpret_cast<const float*>(pk + pp.find(n)->off); }
+  bf16* Wb(const char* n) const { return reinterpret_cast<bf16*>(ws + wp.find(n)->off); }
+  float* Wf(const char* n) const { return reinterpret_cast<float*>(ws + wp.find(n)->off); }
+  int* Wi(const char* n) const { return reinterpret_cast<int*>(ws + wp.find(n)->off); }
+};
+
+// The per-image state (bf16 features, mask, mean, W_v projection, mean-feature gate block) depends on the images only:
+// a caller that decodes the SAME batch again (the reference's loop over latent samples, inference.py:138-167; its
+// lru_cache on the projected features, attention.py:99) sets the option "reuse_image_state" and this is skipped.
+static int image_state(cudaStream_t s, const Handle* h, const Views& v, const void* feats, int B, int N) {
+  const Dims& d = h->d;
+  CUDA_TRY(cudaMemsetAsync(v.Wb("projb"), 0, v.wp.find("projb")->bytes, s));
+  TRY(image_prep(s, feats, h->opt_features_bf16, B, N, d.F, v.Wb("featsb"), d.Fp, v.Wf("mask"), v.Wb("avgb")));
+  GemmSeg sg = seg(v.Wb("featsb"), d.Fp, v.Pb("wv"), d.Fp, d.F);
+  GemmEpi e; e.tag = "gemm.decode"; e.C16 = v.Wb("projb"); e.ldc16 = d.Ap;
+  TRY(gemm_bf16_tn(s, B * N, d.A, 1, &sg, e));
+  GemmSeg sa = seg(v.Wb("avgb"), d.Fp, v.Pb("w_att_f"), d.Fp, d.F);
+  GemmEpi ea; ea.tag = "gemm.decode"; ea.C32 = v.Wf("gavg"); ea.ldc32 = d.GP;
+  return gemm_bf16_tn(s, B, d.GP, 1, &sa, ea);
+}
+
+// Per-call buffers of one step of the cell; the other operands (embb_r, XE, ZB, acc, q, ob, pm and the per-image state) are
+// named regions of the workspace.
+struct CellIO {
+  int rows, N, rows_per_image;                 // rows_per_image: consecutive rows of one image (the attention's grouping)
+  const int* tokens; const int* rowmap;        // (rows) previous token; row -> image
+  bool first;                                  // zero states: no recurrent GEMM segment, no previous cell state
+  const float* eps; int eps_stride;            // normals of row r at eps[r * eps_stride * Z], or null -> Philox
+  const unsigned long long* seed_dev; unsigned long long seed, step;   // Philox seed (device, else by value) and counter
+  const bf16* xa_in; bf16* xa_out;             // [h1 | h_dec] bf16 operand rows (2 Hp) of the previous step / of this step
+  const float* c1_in; float* c1_out; const float* cd_in; float* cd_out;
+  float* h1_out; float* hd_out;                // optional fp32 h of this step
+  float* alpha;                                // (rows, N)
+  const float* sent; const float* pm_row;      // per image: sentiment column (sentiment_vae == 1), prior mean value
+  const float* prior_mean; const float* prior_var; float* pm_out;   // optional (images,Z) prior; (rows,Z) mean used
+  float* logits; const RowStatsEpi* rs;        // vocabulary head: fp32 logits and / or softmax statistics
+};
+
+// One eval step of the UpDown cell and the output head (updown_captioner.py:430-450, updown_cell.py:143-231).
+static int decode_cell(cudaStream_t s, const Dims& d, const Views& v, const float* obj, const CellIO& c) {
+  const int rows = c.rows, GP = d.GP, H = d.H, Hp = d.Hp, Fp = d.Fp, KXe = d.Fp + d.Hp, KX = d.KX;
+  TRY(embed_gather_rows(s, c.tokens, rows, v.Pb("embb"), d.Ep, v.Wb("embb_r")));
+  {
+    LstmFwdArgs l = {};
+    l.R = rows; l.H = H; l.add2 = v.Wf("gavg"); l.ld2 = GP; l.rowmap = c.rowmap; l.bias = v.Pf("b_att");
+    l.c_prev = c.first ? nullptr : c.c1_in; l.c_out = c.c1_out;
+    l.h1_dst = v.Wb("XE") + Fp; l.ld_h1 = KXe; l.h2_dst = c.xa_out; l.ld_h2 = 2 * Hp; l.h_out = c.h1_out;
+    l.acc = v.Wf("acc"); l.ld_acc = GP; l.perm = 1;
+    GemmSeg sg[2] = {seg(v.Wb("embb_r"), d.Ep, v.Pb("w_att_e"), d.Ep, d.E), seg(c.xa_in, 2 * Hp, v.Pb("w_att_rec"), 2 * Hp, 2 * Hp)};
+    GemmEpi e; e.tag = "gemm.decode"; e.C32 = v.Wf("acc"); e.ldc32 = GP;
+    TRY(gemm_bf16_tn(s, rows, GP, c.first ? 1 : 2, sg, e));
+    TRY(lstm_forward(s, l));
+  }
+  {
+    GemmSeg sg = seg(v.Wb("XE") + Fp, KXe, v.Pb("wq"), Hp, Hp);
+    GemmEpi e; e.tag = "gemm.decode"; e.C32 = v.Wf("q"); e.ldc32 = d.A;
+    TRY(gemm_bf16_tn(s, rows, d.A, 1, &sg, e));
+    AttnArgs aa = {}; aa.R = rows; aa.N = c.N; aa.A = d.A; aa.Ap = d.Ap; aa.F = d.F; aa.Fp = Fp; aa.rowmap = c.rowmap;
+    aa.q = v.Wf("q"); aa.ld_q = d.A; aa.proj = v.Wb("projb"); aa.feats = v.Wb("featsb"); aa.mask = v.Wf("mask");
+    aa.w_a = v.W(SSCVAE_W_ATT_VEC);
+    aa.rows_per_image = c.rows_per_image;
+    TRY(attention_forward(s, aa, c.alpha, nullptr, v.Wb("XE"), KXe));
+  }
+  {  // eval: z ~ N(prior_mean, prior_var) (updown_cell.py:200-208); no encoder LSTM
+    LatentArgs la = {}; la.R = rows; la.Z = d.Z; la.Zp = d.Zp; la.sentiment_vae = d.sv; la.prior_var = d.prior_std * d.prior_std;
+    la.prior_mean_row = c.pm_row; la.rowmap = c.rowmap;
+    la.prior_mean_img = c.prior_mean; la.prior_var_img = c.prior_var; la.pm_out = c.pm_out; la.seed = c.seed;
+    if (d.cvar) {  // attribute-grounded prior: mean of this step from the row's attention weights; also the block c
+      TRY(prior_mean_forward(s, c.alpha, obj, c.rowmap, rows, c.N, d.Z, v.Wf("pm"), v.Wb("ZB") + d.Zp, d.ZC, d.cond));
+      la.prior_mean_full = v.Wf("pm");
+    }
+    TRY(latent_forward_eval(s, la, c.eps, c.eps_stride, c.seed_dev, c.step, v.Wb("ZB"), d.ZC));
+  }
+  {
+    GemmSeg sg[3] = {seg(v.Wb("XE"), KXe, v.Pb("w_dec_x"), KX, KXe),
+                     seg(v.Wb("ZB"), d.ZC, v.Pb("w_dec_z"), d.ZC, d.ZC),
+                     seg(c.xa_in + Hp, 2 * Hp, v.Pb("w_dec_x") + KXe, KX, Hp)};
+    LstmFwdArgs l = {};
+    l.R = rows; l.H = H; l.bias = v.Pf("b_dec"); l.rowmap = c.rowmap;
+    if (c.sent) { l.sent = c.sent; l.scol = v.Pf("scol_dec"); }
+    l.c_prev = c.first ? nullptr : c.cd_in; l.c_out = c.cd_out;
+    l.h1_dst = c.xa_out + Hp; l.ld_h1 = 2 * Hp; l.h_out = c.hd_out;
+    l.acc = v.Wf("acc"); l.ld_acc = GP; l.perm = 1;
+    GemmEpi e; e.tag = "gemm.decode"; e.C32 = v.Wf("acc"); e.ldc32 = GP;
+    TRY(gemm_bf16_tn(s, rows, GP, c.first ? 2 : 3, sg, e));
+    TRY(lstm_forward(s, l));
+  }
+  GemmEpi ev; ev.tag = "gemm.decode"; ev.rs = c.rs;
+  if (c.logits) { ev.C32 = c.logits; ev.ldc32 = d.V; }
+  if (d.tied) {
+    GemmSeg sg = seg(c.xa_out + Hp, 2 * Hp, v.Pb("w_out"), Hp, Hp);
+    GemmEpi e; e.tag = "gemm.decode"; e.bias = v.W(SSCVAE_W_OUT_PROJ_B); e.act = 1; e.C16 = v.Wb("ob"); e.ldc16 = d.Ep;
+    TRY(gemm_bf16_tn(s, rows, d.E, 1, &sg, e));
+    GemmSeg sv = seg(v.Wb("ob"), d.Ep, v.Pb("embb"), d.Ep, d.E);
+    return gemm_bf16_tn(s, rows, d.V, 1, &sv, ev);
+  }
+  GemmSeg sg = seg(c.xa_out + Hp, 2 * Hp, v.Pb("w_out"), Hp, Hp);
+  ev.bias = v.W(SSCVAE_W_OUT_PROJ_B);
+  return gemm_bf16_tn(s, rows, d.V, 1, &sg, ev);
+}
+
 // gpf: search groups (virtual images) per FSM table and per num_constraints entry (1, or J when the samples of an image share
 // its machine). exit_per_search: every group stops on its own (n_steps has B*J entries) instead of the batch together.
 static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, int gpf, bool exit_per_search,
@@ -98,27 +204,19 @@ static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, int 
   if (ws_bytes < dp.total) { set_error("workspace too small: %zu < %zu", ws_bytes, dp.total); return SSCVAE_ERR_WORKSPACE; }
   REQUIRE((reinterpret_cast<uintptr_t>(ws) & 255) == 0 && (reinterpret_cast<uintptr_t>(pk) & 255) == 0,
           "workspace and packed weights must be 256-byte aligned");
-  const Plan& pp = h->pp;
-  auto W = [&](int i) { return reinterpret_cast<const float*>(wv[i]); };
-  auto Pb = [&](const char* n) { return reinterpret_cast<const bf16*>(pk + pp.find(n)->off); };
-  auto Pf = [&](const char* n) { return reinterpret_cast<const float*>(pk + pp.find(n)->off); };
-  auto Wb = [&](const char* n) { return reinterpret_cast<bf16*>(ws + dp.find(n)->off); };
-  auto Wf = [&](const char* n) { return reinterpret_cast<float*>(ws + dp.find(n)->off); };
-  auto Wi = [&](const char* n) { return reinterpret_cast<int*>(ws + dp.find(n)->off); };
+  const Views v{pk, h->pp, wv, ws, dp};
+  auto Wb = [&](const char* n) { return v.Wb(n); };
+  auto Wf = [&](const char* n) { return v.Wf(n); };
+  auto Wi = [&](const char* n) { return v.Wi(n); };
   auto zero = [&](const char* n) { return cudaMemsetAsync(ws + dp.find(n)->off, 0, dp.find(n)->bytes, s); };
-  const int SK = S * K, R = Bv * SK, GP = d.GP, H = d.H, Hp = d.Hp, Fp = d.Fp, KXe = d.Fp + d.Hp, KX = d.KX, L = d.L;
+  const int SK = S * K, R = Bv * SK, H = d.H, Hp = d.Hp, L = d.L;
   const unsigned long long* seed_dev = reinterpret_cast<const unsigned long long*>(ws + dp.find("seed")->off);
   (void)seed;
 
   CUDA_TRY(zero("XA0")); CUDA_TRY(zero("XA1")); CUDA_TRY(zero("XE")); CUDA_TRY(zero("bp_hist"));
   if (d.cvar) CUDA_TRY(zero("ZB"));                    // the padding columns behind c
-  if (!h->opt_reuse_image_state) CUDA_TRY(zero("projb"));
   if (d.tied) CUDA_TRY(zero("ob"));
-  // The per-image state (bf16 features, mask, mean, W_v projection, mean-feature gate block) depends on the images only:
-  // a caller that decodes the SAME batch again (the reference's loop over latent samples, inference.py:138-167; its
-  // lru_cache on the projected features, attention.py:99) sets the option and the state in the workspace is reused.
-  const bool reuse = h->opt_reuse_image_state != 0;
-  if (!reuse) TRY(image_prep(s, feats, h->opt_features_bf16, B, N, d.F, Wb("featsb"), Fp, Wf("mask"), Wb("avgb")));
+  if (!h->opt_reuse_image_state) TRY(image_state(s, h, v, feats, B, N));
   TRY(scale_rows_f32(s, csent ? sent : nullptr, d.mult, Wf("pm_row"), B));
   TRY(scale_rows_f32(s, csent ? sent : nullptr, 1.0f, Wf("sent"), B));
   TRY(iota_div_i32(s, Wi("rowmap"), R, SK * J));
@@ -131,14 +229,6 @@ static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, int 
   } else if (fsm) {
     TRY(fsm_pack(s, fsm, Bv / gpf, S, d.V, reinterpret_cast<uint32_t*>(Wi("fsm_bits"))));
     fsm_bits = reinterpret_cast<uint32_t*>(Wi("fsm_bits"));
-  }
-  if (!reuse) {  // once per image (the reference recomputes both every step in decode)
-    GemmSeg sg = seg(Wb("featsb"), Fp, Pb("wv"), Fp, d.F);
-    GemmEpi e; e.tag = "gemm.decode"; e.C16 = Wb("projb"); e.ldc16 = d.Ap;
-    TRY(gemm_bf16_tn(s, B * N, d.A, 1, &sg, e));
-    GemmSeg sa = seg(Wb("avgb"), Fp, Pb("w_att_f"), Fp, d.F);
-    GemmEpi ea; ea.tag = "gemm.decode"; ea.C32 = Wf("gavg"); ea.ldc32 = GP;
-    TRY(gemm_bf16_tn(s, B, GP, 1, &sa, ea));
   }
   int* tok_hist = Wi("tok_hist"); int* bp_hist = Wi("bp_hist"); float* score_hist = Wf("score_hist");
   bf16* XA[2] = {Wb("XA0"), Wb("XA1")};
@@ -153,68 +243,15 @@ static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, int 
   const int nst = gemm_rowstats_tiles(d.V);
   auto cell = [&](int rows, const int* tokens, const int* rowmap, bool first, const float* eps_t, int eps_stride,
                   int step) -> int {
-    // in = index 0, out = index 1
-    float* alpha_t = Wf("alpha_hist") + (size_t)step * R * N;      // kept for sscvae_decode_attention
-    TRY(embed_gather_rows(s, tokens, rows, Pb("embb"), d.Ep, Wb("embb_r")));
-    {
-      LstmFwdArgs l = {};
-      l.R = rows; l.H = H; l.add2 = Wf("gavg"); l.ld2 = GP; l.rowmap = rowmap; l.bias = Pf("b_att");
-      l.c_prev = first ? nullptr : c1[0]; l.c_out = c1[1];
-      l.h1_dst = Wb("XE") + Fp; l.ld_h1 = KXe; l.h2_dst = XA[1]; l.ld_h2 = 2 * Hp;
-      l.acc = Wf("acc"); l.ld_acc = GP; l.perm = 1;
-      GemmSeg sg[2] = {seg(Wb("embb_r"), d.Ep, Pb("w_att_e"), d.Ep, d.E), seg(XA[0], 2 * Hp, Pb("w_att_rec"), 2 * Hp, 2 * Hp)};
-      GemmEpi e; e.tag = "gemm.decode"; e.C32 = Wf("acc"); e.ldc32 = GP;
-      TRY(gemm_bf16_tn(s, rows, GP, first ? 1 : 2, sg, e));
-      TRY(lstm_forward(s, l));
-    }
-    {
-      GemmSeg sg = seg(Wb("XE") + Fp, KXe, Pb("wq"), Hp, Hp);
-      GemmEpi e; e.tag = "gemm.decode"; e.C32 = Wf("q"); e.ldc32 = d.A;
-      TRY(gemm_bf16_tn(s, rows, d.A, 1, &sg, e));
-      AttnArgs aa = {}; aa.R = rows; aa.N = N; aa.A = d.A; aa.Ap = d.Ap; aa.F = d.F; aa.Fp = Fp; aa.rowmap = rowmap;
-      aa.q = Wf("q"); aa.ld_q = d.A; aa.proj = Wb("projb"); aa.feats = Wb("featsb"); aa.mask = Wf("mask");
-      aa.w_a = W(SSCVAE_W_ATT_VEC);
-      aa.rows_per_image = first ? J : SK * J;                  // rowmap0: r / J ; rowmap: r / (SK * J)
-      TRY(attention_forward(s, aa, alpha_t, nullptr, Wb("XE"), KXe));
-    }
-    {  // eval: z ~ N(prior_mean, prior_var) (updown_cell.py:200-208); no encoder LSTM
-      LatentArgs la = {}; la.R = rows; la.Z = d.Z; la.Zp = d.Zp; la.sentiment_vae = d.sv; la.prior_var = d.prior_std * d.prior_std;
-      la.prior_mean_row = Wf("pm_row"); la.rowmap = rowmap;
-      if (d.cvar) {  // attribute-grounded prior: mean of this step from the row's attention weights; also the block c
-        TRY(prior_mean_forward(s, alpha_t, obj, rowmap, rows, N, d.Z, Wf("pm"), Wb("ZB") + d.Zp, d.ZC, d.cond));
-        la.prior_mean_full = Wf("pm");
-      }
-      TRY(latent_forward_eval(s, la, eps_t, eps_stride, seed_dev, (unsigned long long)step, Wb("ZB"), d.ZC));
-    }
-    {
-      GemmSeg sg[3] = {seg(Wb("XE"), KXe, Pb("w_dec_x"), KX, KXe),
-                       seg(Wb("ZB"), d.ZC, Pb("w_dec_z"), d.ZC, d.ZC),
-                       seg(XA[0] + Hp, 2 * Hp, Pb("w_dec_x") + KXe, KX, Hp)};
-      LstmFwdArgs l = {};
-      l.R = rows; l.H = H; l.bias = Pf("b_dec"); l.rowmap = rowmap;
-      if (csent) { l.sent = Wf("sent"); l.scol = Pf("scol_dec"); }
-      l.c_prev = first ? nullptr : cd[0]; l.c_out = cd[1];
-      l.h1_dst = XA[1] + Hp; l.ld_h1 = 2 * Hp;
-      l.acc = Wf("acc"); l.ld_acc = GP; l.perm = 1;
-      GemmEpi e; e.tag = "gemm.decode"; e.C32 = Wf("acc"); e.ldc32 = GP;
-      TRY(gemm_bf16_tn(s, rows, GP, first ? 2 : 3, sg, e));
-      TRY(lstm_forward(s, l));
-    }
-    if (d.tied) {
-      GemmSeg sg = seg(XA[1] + Hp, 2 * Hp, Pb("w_out"), Hp, Hp);
-      GemmEpi e; e.tag = "gemm.decode"; e.bias = W(SSCVAE_W_OUT_PROJ_B); e.act = 1; e.C16 = Wb("ob"); e.ldc16 = d.Ep;
-      TRY(gemm_bf16_tn(s, rows, d.E, 1, &sg, e));
-      GemmSeg sv = seg(Wb("ob"), d.Ep, Pb("embb"), d.Ep, d.E);
-      GemmEpi ev; ev.tag = "gemm.decode";
-      if (greedy) ev.rs = &rs; else { ev.C32 = Wf("logits"); ev.ldc32 = d.V; }
-      TRY(gemm_bf16_tn(s, rows, d.V, 1, &sv, ev));
-    } else {
-      GemmSeg sg = seg(XA[1] + Hp, 2 * Hp, Pb("w_out"), Hp, Hp);
-      GemmEpi e; e.tag = "gemm.decode"; e.bias = W(SSCVAE_W_OUT_PROJ_B);
-      if (greedy) e.rs = &rs; else { e.C32 = Wf("logits"); e.ldc32 = d.V; }
-      TRY(gemm_bf16_tn(s, rows, d.V, 1, &sg, e));
-    }
-    return 0;
+    CellIO c = {};
+    c.rows = rows; c.N = N; c.rows_per_image = first ? J : SK * J;        // rowmap0: r / J ; rowmap: r / (SK * J)
+    c.tokens = tokens; c.rowmap = rowmap; c.first = first;
+    c.eps = eps_t; c.eps_stride = eps_stride; c.seed_dev = seed_dev; c.step = (unsigned long long)step;
+    c.xa_in = XA[0]; c.xa_out = XA[1]; c.c1_in = c1[0]; c.c1_out = c1[1]; c.cd_in = cd[0]; c.cd_out = cd[1];
+    c.alpha = Wf("alpha_hist") + (size_t)step * R * N;                   // kept for sscvae_decode_attention
+    c.sent = csent ? Wf("sent") : nullptr; c.pm_row = Wf("pm_row");
+    if (greedy) c.rs = &rs; else c.logits = Wf("logits");
+    return decode_cell(s, d, v, obj, c);
   };
 
   // ---- step 0: one row per image, zero states (cbs.py:127-155)
@@ -253,6 +290,43 @@ static int decode_impl(Handle* h, int B, int J, int N, int S, int K, int P, int 
   TRY(search_finish(s, tok_hist, bp_hist, score_hist, L, Bv, S, K, d.boundary, num_constraints, min_sat, gpf,
                     exit_per_search ? 1 : 0, predictions, log_probs, best, n_steps, Wi("best_state"), Wi("search_steps")));
   return 0;
+}
+
+// Single step (sscvae_decode_step). The per-image state comes first: its offsets depend on (B, N) only, so a call with
+// another row count over the same workspace finds it in place. XA1, XE, ZB and ob are adjacent: one memset zeroes the
+// K-padding of those operands (no kernel writes the padding columns, so it stays zero while the layout does not change).
+static void plan_step(const Dims& d, int B, int R, int N, Plan& p) {
+  const size_t b = sizeof(bf16), f = 4, BN = (size_t)B * N;
+  p.add("featsb", BN * d.Fp * b);
+  p.add("mask", BN * f);
+  p.add("avgb", (size_t)B * d.Fp * b);
+  p.add("projb", BN * d.Ap * b);
+  p.add("gavg", (size_t)B * d.GP * f);
+  p.add("pm_row", B * f);
+  p.add("tok", R * 4);
+  p.add("rowmap", R * 4);
+  p.add("XA0", (size_t)R * 2 * d.Hp * b);
+  p.add("XA1", (size_t)R * 2 * d.Hp * b);
+  p.add("XE", (size_t)R * (d.Fp + d.Hp) * b);
+  p.add("ZB", (size_t)R * d.ZC * b);
+  if (d.tied) p.add("ob", (size_t)R * d.Ep * b);
+  p.add("embb_r", (size_t)R * d.Ep * b);
+  if (d.cvar) p.add("pm", (size_t)R * d.Z * f);
+  p.add("acc", (size_t)R * d.GP * f);
+  p.add("q", (size_t)R * d.A * f);
+  const size_t nst = gemm_rowstats_tiles(d.V);
+  p.add("rs_max", R * nst * f);
+  p.add("rs_sum", R * nst * f);
+  p.add("rs_arg", R * nst * 4);
+}
+
+const Plan& Handle::step_plan(int B, int R, int N) {
+  if (sp_B != B || sp_R != R || sp_N != N) {
+    sp = Plan();
+    plan_step(d, B, R, N, sp);
+    sp_B = B; sp_R = R; sp_N = N;
+  }
+  return sp;
 }
 
 }  // namespace sscvae
@@ -490,6 +564,74 @@ int sscvae_decode_attention(SscvaeHandle* hh, const void* workspace, size_t work
                           reinterpret_cast<const float*>(ws + dp.find("alpha_hist")->off), h->d.L, h->last_B * h->last_J,
                           h->last_S, h->last_K, h->last_N, h->d.boundary, Wi("search_steps"), Wi("best_state"), valid_states,
                           attention_all, attention_best);
+}
+
+
+size_t sscvae_decode_step_workspace_bytes(const SscvaeHandle* hh, int batch, int rows, int num_boxes) {
+  Handle* h = const_cast<Handle*>(reinterpret_cast<const Handle*>(hh));
+  if (!h || batch <= 0 || rows <= 0 || num_boxes <= 0 || rows % batch != 0) return 0;
+  return h->step_plan(batch, rows, num_boxes).total;
+}
+
+int sscvae_decode_step(SscvaeHandle* hh, int batch, int rows, int num_boxes, const void* packed, const void* const* weights,
+                       const float* image_features, const float* sentiment, const float* obj_means, const float* prior_mean,
+                       const float* prior_var, const int64_t* prev_tokens, const float* const* states_in, const float* eps,
+                       uint64_t seed, void* workspace, size_t workspace_bytes, float* log_probs, float* const* states_out,
+                       float* alpha, float* prior_mean_out, void* stream) {
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  REQUIRE(h && packed && weights && image_features && prev_tokens && workspace && log_probs && states_out && alpha &&
+          prior_mean_out, "NULL argument");
+  REQUIRE(states_out[0] && states_out[1] && states_out[2] && states_out[3], "NULL argument: states_out needs h1, c1, h_decoder, c_decoder");
+  REQUIRE(!states_in || (states_in[0] && states_in[1] && states_in[4] && states_in[5]),
+          "NULL argument: states_in needs h1, c1, h_decoder and c_decoder (or is NULL for zero states)");
+  REQUIRE(batch > 0 && rows > 0 && num_boxes > 0 && rows % batch == 0,
+          "bad step shape B=%d R=%d N=%d (R must be a multiple of B: row r belongs to image r / (R/B))", batch, rows, num_boxes);
+  const Dims& d = h->d;
+  const bool csent = d.cond && !d.cvar;
+  REQUIRE(!csent || sentiment != nullptr, "sentiment is required when sentiment_vae == 1");
+  REQUIRE(!d.cvar || obj_means != nullptr, "obj_means is required when sentiment_vae == 2");
+  const Plan& sp = h->step_plan(batch, rows, num_boxes);
+  if (workspace_bytes < sp.total) { set_error("workspace too small: %zu < %zu", workspace_bytes, sp.total); return SSCVAE_ERR_WORKSPACE; }
+  REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0 && (reinterpret_cast<uintptr_t>(packed) & 255) == 0,
+          "workspace and packed weights must be 256-byte aligned");
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  char* ws = reinterpret_cast<char*>(workspace);
+  const Views v{reinterpret_cast<const char*>(packed), h->pp, weights, ws, sp};
+  const int R = rows, rpi = rows / batch;
+  // Launched directly, not through the graph cache: the cache keys a graph on every pointer of the call, and a search
+  // hands the step new output buffers on every step, so each call would capture (and keep) a graph of its own.
+  const bool reuse = h->opt_reuse_image_state != 0;
+  if (!reuse || h->step_ws != workspace || h->step_R != R) {
+    const Region* first = sp.find("XA1");
+    const Region* last = sp.find(d.tied ? "ob" : "ZB");
+    CUDA_TRY(cudaMemsetAsync(ws + first->off, 0, last->off + last->bytes - first->off, s));
+  }
+  if (!reuse) TRY(image_state(s, h, v, image_features, batch, num_boxes));
+  h->step_ws = workspace; h->step_R = R;
+  TRY(step_import(s, reinterpret_cast<const long long*>(prev_tokens), R, rpi, states_in ? states_in[0] : nullptr,
+                  states_in ? states_in[4] : nullptr, d.H, d.Hp, v.Wi("tok"), v.Wi("rowmap"), v.Wb("XA0")));
+  CellIO c = {};
+  c.rows = R; c.N = num_boxes; c.rows_per_image = rpi; c.tokens = v.Wi("tok"); c.rowmap = v.Wi("rowmap");
+  c.first = states_in == nullptr;
+  c.eps = eps; c.eps_stride = 1; c.seed = seed;
+  c.xa_in = v.Wb("XA0"); c.xa_out = v.Wb("XA1");
+  c.c1_in = states_in ? states_in[1] : nullptr; c.cd_in = states_in ? states_in[5] : nullptr;
+  c.h1_out = states_out[0]; c.c1_out = states_out[1]; c.hd_out = states_out[2]; c.cd_out = states_out[3];
+  c.alpha = alpha;
+  c.sent = csent ? sentiment : nullptr;
+  if (!d.simple) {                                     // simple_vae: the prior mean is zero whatever is given (updown_cell.py:165-166)
+    c.prior_mean = prior_mean;
+    if (!prior_mean && csent) {                        // the prior forward() builds (updown_captioner.py:250-261)
+      TRY(scale_rows_f32(s, sentiment, d.mult, v.Wf("pm_row"), batch));
+      c.pm_row = v.Wf("pm_row");
+    }
+  }
+  c.prior_var = prior_var; c.pm_out = prior_mean_out;
+  RowStatsEpi rs;
+  rs.mode = 1; rs.st_max = v.Wf("rs_max"); rs.st_sum = v.Wf("rs_sum"); rs.st_arg = v.Wi("rs_arg");
+  c.logits = log_probs; c.rs = &rs;
+  TRY(decode_cell(s, d, v, obj_means, c));
+  return log_softmax_rows(s, rs.st_max, rs.st_sum, rs.st_arg, gemm_rowstats_tiles(d.V), R, d.V, log_probs);
 }
 
 }  // extern "C"

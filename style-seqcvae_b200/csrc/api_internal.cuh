@@ -44,10 +44,13 @@ struct Handle {
   Plan dp; int dp_B = -1, dp_N = -1, dp_S = -1, dp_K = -1, dp_J = -1, dp_T = -1;   // decode workspace
   // shape of the last decode call (the plan above also follows workspace-size and region queries): sscvae_decode_attention
   int last_B = -1, last_N = -1, last_S = -1, last_K = -1, last_J = -1, last_T = -1;
+  Plan sp; int sp_B = -1, sp_R = -1, sp_N = -1;   // single-step workspace (sscvae_decode_step)
+  const void* step_ws = nullptr; int step_R = -1;  // workspace and row count of the last step call: its zeroed operand padding
+  const Plan& step_plan(int B, int R, int N);
   GraphCache fwd_graphs, bwd_graphs, dec_graphs;
   // per-handle options (sscvae_set_option), consumed by the following calls
   int opt_features_bf16 = 0;           // image_features pointers are bf16 (B,N,F) instead of fp32
-  int opt_reuse_image_state = 0;       // decode: the workspace already holds this batch's featsb / projb / mask / avg state
+  int opt_reuse_image_state = 0;       // decode / step: the workspace already holds this batch's featsb / projb / mask / avg state
   int opt_persistent_bwd = 1;          // training: run the BPTT loop as the persistent kernel (recurrent_bwd.cu) when the shape fits
   int opt_fsm_packed = 0;              // decode: `fsm` is the (B,S,V) uint32 bit table, not the (B,S,S,V) uint8 tensor
   const Plan& train_plan(int B, int N);

@@ -32,6 +32,7 @@ struct LstmFwdArgs {
   float* gates_out;                    // optional (R,4H) activated gates, saved for BPTT
   bf16* h1_dst; int ld_h1;             // bf16 h -> up to two operand buffers
   bf16* h2_dst; int ld_h2;
+  float* h_out;                        // optional (R,H) fp32 h (sscvae_decode_step returns it to the caller)
   // 1: the columns of the GEMM outputs `acc`, `add1`, `add2` are in the gate-interleaved order of the packed forward LSTM weights (lstm_gate_row): tile of
   // 128 columns = 32 hidden units x 4 gates, so that one GEMM CTA owns all four gates of its units
   int perm;
@@ -63,6 +64,11 @@ struct LatentArgs {
   const int* rowmap;                   // optional row -> prior_mean_row index
   const float* prior_mean_full;        // sentiment_vae == 2: (R,Z) per-row, per-component prior mean of this step (replaces prior_mean_row)
   float* dpm_out;                      // backward, with prior_mean_full: (R,Z) gradient of the KL term w.r.t. the prior mean
+  // eval only (sscvae_decode_step: the reference's _decode_step takes the prior as arguments, updown_captioner.py:371)
+  const float* prior_mean_img;         // optional (images,Z) per-component prior mean, row r reads rowmap[r] (prior_mean_full wins)
+  const float* prior_var_img;          // optional (images,Z) per-component prior variance (replaces prior_var)
+  float* pm_out;                       // optional (R,Z): the prior mean z was drawn around
+  unsigned long long seed;             // Philox seed when seed_dev is null
 };
 // sentiment_vae == 2 (updown_cell.py:160-174): pm[r,:] = sum_n alpha[r,n] * obj[img(r),n,:]; the first `cond` components
 // are also written as the bf16 conditioning block c of the encoder / decoder LSTM inputs (cond = Z: "glove", 1: "senti_word_net")
@@ -103,6 +109,13 @@ int ce_merge(cudaStream_t s, const float* st_max, const float* st_sum, const int
              const float* tgt_logit, float* lse, float* nll);
 int greedy_merge(cudaStream_t s, const float* st_max, const float* st_sum, const int* st_arg, int ntiles, int R,
                  const int* last_tokens, const float* last_scores, int end_index, int* tok, int* bp, float* score);
+// in place: logits (R,V) -= log-sum-exp of the row, merged from the head GEMM's RowStatsEpi partials (one read, one write)
+int log_softmax_rows(cudaStream_t s, const float* st_max, const float* st_sum, const int* st_arg, int ntiles, int R, int V,
+                     float* logits);
+// sscvae_decode_step's per-call input: tok[r] = prev[r] (int64 -> int32), rowmap[r] = r / rows_per_image and, unless h1 is
+// null, the bf16 operand rows xa[r] = [h1[r] | 0 | h_dec[r] | 0] (2 blocks of Hp, K-padding zeroed) from the fp32 states
+int step_import(cudaStream_t s, const long long* prev, int R, int rows_per_image, const float* h1, const float* h_dec, int H,
+                int Hp, int* tok, int* rowmap, bf16* xa);
 
 // ---- layout helpers -------------------------------------------------------------------------------
 // out[c, r] = in[r, c] (bf16, c < cols, r < ld_out; zero for r >= rows, so the padded out is a GEMM operand) for a

@@ -182,6 +182,7 @@ __global__ void lstm_fwd_kernel(LstmFwdArgs a) {
   const bf16 hb = __float2bfloat16_rn(h);
   if (a.h1_dst) a.h1_dst[(size_t)r * a.ld_h1 + j] = hb;
   if (a.h2_dst) a.h2_dst[(size_t)r * a.ld_h2 + j] = hb;
+  if (a.h_out) a.h_out[(size_t)r * H + j] = h;
 }
 
 // 4 hidden units per thread, 16-byte accesses (H % 4 == 0 and 16-byte aligned rows: every training / decode buffer)
@@ -232,6 +233,7 @@ __global__ void __launch_bounds__(128) lstm_fwd_v4_kernel(LstmFwdArgs a) {
   }
   if (a.h1_dst) st_bf16x4(a.h1_dst + (size_t)r * a.ld_h1 + j, h.x, h.y, h.z, h.w);
   if (a.h2_dst) st_bf16x4(a.h2_dst + (size_t)r * a.ld_h2 + j, h.x, h.y, h.z, h.w);
+  if (a.h_out) *reinterpret_cast<float4*>(a.h_out + (size_t)r * H + j) = h;
 }
 
 static inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
@@ -242,7 +244,7 @@ int lstm_forward(cudaStream_t s, const LstmFwdArgs& a) {
   const bool v4 = (a.H % 4) == 0 && al16(a.acc) && (a.ld_acc % 4) == 0 && (!a.add1 || (al16(a.add1) && (a.ld1 % 4) == 0)) &&
                   (!a.add2 || (al16(a.add2) && (a.ld2 % 4) == 0)) && (!a.bias || al16(a.bias)) && (!a.sent || al16(a.scol)) &&
                   (!a.c_prev || al16(a.c_prev)) && al16(a.c_out) && (!a.gates_out || al16(a.gates_out)) &&
-                  (!a.h1_dst || (al8(a.h1_dst) && (a.ld_h1 % 4) == 0)) && (!a.h2_dst || (al8(a.h2_dst) && (a.ld_h2 % 4) == 0));
+                  (!a.h1_dst || (al8(a.h1_dst) && (a.ld_h1 % 4) == 0)) && (!a.h2_dst || (al8(a.h2_dst) && (a.ld_h2 % 4) == 0)) && (!a.h_out || al16(a.h_out));
   if (v4) {
     lstm_fwd_v4_kernel<<<dim3(ceil_div(a.R * (a.H / 4), 128)), dim3(128), 0, s>>>(a);
   } else {
@@ -415,14 +417,19 @@ __global__ void latent_fwd_eval_kernel(LatentArgs a, const float* __restrict__ e
                                        const unsigned long long* __restrict__ seed_dev, unsigned long long step, bf16* __restrict__ zb,
                                        int ld_z) {
   const int r = blockIdx.x;
-  const float pm_row = a.prior_mean_row ? a.prior_mean_row[a.rowmap ? a.rowmap[r] : r] : 0.f;
-  const float sd = sqrtf(a.prior_var);
+  const int img = a.rowmap ? a.rowmap[r] : r;
+  const float pm_row = a.prior_mean_row ? a.prior_mean_row[img] : 0.f;
+  const float sd_all = sqrtf(a.prior_var);
   for (int z = threadIdx.x; z < a.Zp; z += blockDim.x) {
     float v = 0.f;
     if (z < a.Z) {
-      const float e = eps_in ? eps_in[(size_t)r * eps_row_stride * a.Z + z] : philox_normal(*seed_dev, step, r, z, a.Z);
-      const float pm = a.prior_mean_full ? a.prior_mean_full[(size_t)r * a.Z + z] : pm_row;
+      const float e = eps_in ? eps_in[(size_t)r * eps_row_stride * a.Z + z]
+                             : philox_normal(seed_dev ? *seed_dev : a.seed, step, r, z, a.Z);
+      const float pm = a.prior_mean_full ? a.prior_mean_full[(size_t)r * a.Z + z]
+                     : a.prior_mean_img  ? a.prior_mean_img[(size_t)img * a.Z + z] : pm_row;
+      const float sd = a.prior_var_img ? sqrtf(a.prior_var_img[(size_t)img * a.Z + z]) : sd_all;
       v = e * sd + pm;
+      if (a.pm_out) a.pm_out[(size_t)r * a.Z + z] = pm;
     }
     zb[(size_t)r * ld_z + z] = __float2bfloat16_rn(v);
   }
@@ -722,6 +729,63 @@ int greedy_merge(cudaStream_t s, const float* st_max, const float* st_sum, const
   PROF_SCOPE(s, "search_rows", 0, (double)R * ntiles * 12.0);
   greedy_merge_kernel<<<ceil_div(R, 8), 256, 0, s>>>(st_max, st_sum, st_arg, ntiles, R, last_tokens, last_scores, end_index, tok,
                                                     bp, score);
+  LAUNCHED();
+  return 0;
+}
+
+// log-softmax of the step's logits in place (updown_captioner.py:450): one warp per row merges the head GEMM's per-tile
+// partials (the log-sum-exp of ce_merge) and rewrites the row with 16-byte accesses; the logits are read once, written once
+__global__ void log_softmax_rows_kernel(const float* __restrict__ st_max, const float* __restrict__ st_sum,
+                                        const int* __restrict__ st_arg, int ntiles, int R, int V, int vec4,
+                                        float* __restrict__ x) {
+  const int r = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (r >= R) return;
+  const int lane = threadIdx.x & 31;
+  float M, S; int arg;
+  merge_row_stats(st_max, st_sum, st_arg, ntiles, R, r, M, S, arg);
+  const float lse = M + logf(S);
+  float* row = x + (size_t)r * V;
+  if (vec4) {
+    float4* row4 = reinterpret_cast<float4*>(row);
+    for (int i = lane; i < (V >> 2); i += 32) {
+      float4 v = row4[i];
+      v.x -= lse; v.y -= lse; v.z -= lse; v.w -= lse;
+      row4[i] = v;
+    }
+  } else {
+    for (int i = lane; i < V; i += 32) row[i] -= lse;
+  }
+}
+int log_softmax_rows(cudaStream_t s, const float* st_max, const float* st_sum, const int* st_arg, int ntiles, int R, int V,
+                     float* logits) {
+  PROF_SCOPE(s, "log_softmax", 0, (double)R * V * 8.0 + (double)R * ntiles * 12.0);
+  const int vec4 = (V % 4) == 0 && (reinterpret_cast<uintptr_t>(logits) & 15) == 0;
+  log_softmax_rows_kernel<<<ceil_div(R, 8), 256, 0, s>>>(st_max, st_sum, st_arg, ntiles, R, V, vec4, logits);
+  LAUNCHED();
+  return 0;
+}
+
+// one warp per row: the token and image index of the row, then (with states) its bf16 [h1 | h_dec] operand row
+__global__ void step_import_kernel(const long long* __restrict__ prev, int R, int rows_per_image, const float* __restrict__ h1,
+                                   const float* __restrict__ hd, int H, int Hp, int* __restrict__ tok, int* __restrict__ rowmap,
+                                   bf16* __restrict__ xa) {
+  const int r = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (r >= R) return;
+  const int lane = threadIdx.x & 31;
+  if (lane == 0) { tok[r] = (int)prev[r]; rowmap[r] = r / rows_per_image; }
+  if (!h1) return;
+  bf16* o = xa + (size_t)r * 2 * Hp;
+  for (int c = lane; c < 2 * Hp; c += 32) {
+    const int j = c < Hp ? c : c - Hp;
+    const float* src = c < Hp ? h1 : hd;
+    o[c] = __float2bfloat16_rn(j < H ? src[(size_t)r * H + j] : 0.f);
+  }
+}
+int step_import(cudaStream_t s, const long long* prev, int R, int rows_per_image, const float* h1, const float* h_dec, int H,
+                int Hp, int* tok, int* rowmap, bf16* xa) {
+  PROF_SCOPE(s, "step_import", 0, (double)R * (12.0 + (h1 ? 2.0 * H * 4.0 + 4.0 * Hp : 0.0)));
+  REQUIRE(rows_per_image > 0 && (!h1 || (h_dec && xa)), "step_import: bad arguments");
+  step_import_kernel<<<ceil_div(R, 8), 256, 0, s>>>(prev, R, rows_per_image, h1, h_dec, H, Hp, tok, rowmap, xa);
   LAUNCHED();
   return 0;
 }
