@@ -310,6 +310,58 @@ int sscvae_decode_step(SscvaeHandle* h, int batch, int rows, int num_boxes, cons
                        size_t workspace_bytes, float* log_probs, float* const* states_out, float* alpha,
                        float* prior_mean_out, void* stream);
 
+/* ---- one training step: the reference's `_decode_step` in training mode (updown_captioner.py:371-455 with the encoder branch
+ * of updown_cell.py:176-198), the body of its training loop (updown_captioner.py:282-310), with a backward, so a caller can
+ * build its own per-step objective (per-step KL weights, free bits, losses on the attention, scheduled sampling) and
+ * back-propagate it through autograd. One row per image (R = B). Three caller-owned device buffers, 256-byte aligned:
+ *   image state: the per-image operands of one batch, built by sscvae_train_step_image_state from the features, the per-box
+ *     attribute means (sentiment_vae == 2) and the current weights. Every step over that batch reads it; build a new one for
+ *     other features or after a weight update (replaces the reference's per-step re-projection, attention.py:99-125).
+ *   tape: what one step's backward reads, written by its forward; one per step, kept until its backward has run.
+ *   workspace: scratch of one call; any forward or backward of this handle may reuse it (calls on one stream).
+ * The step neither reads nor returns the prior except with sentiment_vae == 2, where the prior mean is computed from the
+ * attention (updown_cell.py:160-163): the caller forms the KL term (updown_captioner.py:295-303) from mean / log_var and
+ * its prior. Not captured as a CUDA graph; no host synchronisation. */
+size_t sscvae_train_step_image_state_bytes(const SscvaeHandle* h, int batch, int num_boxes);   /* 0 for bad arguments */
+size_t sscvae_train_step_tape_bytes(const SscvaeHandle* h, int batch, int num_boxes);
+size_t sscvae_train_step_workspace_bytes(const SscvaeHandle* h, int batch, int num_boxes);
+/* image_features (B,N,F) fp32, or bf16 with the option "features_bf16"; obj_means (B,N,Z), required with sentiment_vae == 2
+ * (NULL otherwise). */
+int sscvae_train_step_image_state(SscvaeHandle* h, int batch, int num_boxes, const void* packed, const void* const* weights_f32,
+                                  const void* image_features, const float* obj_means, void* state, size_t state_bytes,
+                                  void* stream);
+/* Forward of one step.
+ *   sentiment: (B,1), required with sentiment_vae == 1 (the conditioning column, updown_cell.py:176-190), else NULL.
+ *   prev_tokens: (B) int64 device ids in [0, V) (not checked here: the kernels index the embedding unchecked).
+ *   states_in: host array of 6 device pointers (B,H) fp32, order h1, c1, h_encoder, c_encoder, h_decoder, c_decoder, or
+ *     NULL = zero states (the first step, updown_cell.py:131-140).
+ *   eps: (B,Z) normals, or NULL -> Philox(seed); a caller passes a new seed per call.
+ *   Outputs (device, fp32, written in full): logits (B,V) raw (not log-softmax); states_out: host array of 6 device
+ *     pointers (B,H); mean, log_var (B,Z) the posterior (updown_cell.py:196-198); prior_mean_out (B,Z) the step's prior mean,
+ *     sentiment_vae == 2 only (else ignored, may be NULL); alpha (B,N) the attention weights.
+ * A NULL required pointer, an incomplete state array, a missing sentiment / prior_mean_out return SSCVAE_ERR_BAD_ARG, a
+ * buffer that is too small SSCVAE_ERR_WORKSPACE, all before any device work. */
+int sscvae_train_step_forward(SscvaeHandle* h, int batch, int num_boxes, const void* packed, const void* const* weights_f32,
+                              const void* state, size_t state_bytes, const float* sentiment, const int64_t* prev_tokens,
+                              const float* const* states_in, const float* eps, uint64_t seed, void* tape, size_t tape_bytes,
+                              void* workspace, size_t workspace_bytes, float* logits, float* const* states_out, float* mean,
+                              float* log_var, float* prior_mean_out, float* alpha, void* stream);
+/* Backward of one step (the per-launch BPTT body of sscvae_train_backward for one timestep), reading the tape and image
+ * state of its forward with the same packed weights.
+ *   d_logits (B,V) required. d_states_out: host array of 6 (B,H) upstream gradients of states_out, a NULL entry (or a NULL
+ *     array) meaning zero. d_mean, d_log_var (B,Z), d_alpha (B,N): NULL = zero. d_prior_mean (B,Z): sentiment_vae == 2 only
+ *     (the prior mean is a function of alpha there), NULL = zero.
+ *   d_states_in: host array of 6 (B,H) outputs for the input states' gradients, a NULL entry (or array) = not wanted.
+ *   grads: SSCVAE_W_COUNT device pointers in reference layout, OVERWRITTEN with this step's gradients (not accumulated);
+ *     NULL entries (frozen parameters) are skipped with their GEMMs. The tied embedding gets no gradient (frozen GloVe,
+ *     updown_captioner.py:197-216). The untied embedding's padding row stays zero (padding_idx).
+ * Refusals as for the forward, before any device work. */
+int sscvae_train_step_backward(SscvaeHandle* h, int batch, int num_boxes, const void* packed, const void* const* weights_f32,
+                               const void* state, size_t state_bytes, const void* tape, size_t tape_bytes, void* workspace,
+                               size_t workspace_bytes, const float* d_logits, const float* const* d_states_out,
+                               const float* d_mean, const float* d_log_var, const float* d_prior_mean, const float* d_alpha,
+                               float* const* d_states_in, void* const* grads, void* stream);
+
 /* ---- training-step tail (SURVEY §8(f)-1): clip_grad_norm_ + SGD(momentum, weight decay) fused over
  * a flat parameter buffer; replaces var_updown/scripts/train.py:173-176. */
 int sscvae_grad_sqnorm(const float* grads, size_t n, float* partial /*>= 1024 floats*/, float* sqnorm_out, void* stream);

@@ -48,6 +48,8 @@ SYMBOLS = [
     "sscvae_profile_enable", "sscvae_profile_report", "sscvae_test_gemm_grouped", "sscvae_test_transpose_bf16",
     "sscvae_sgd_step_packed", "sscvae_debug_sgd_pack_jobs", "sscvae_decode_attention",
     "sscvae_decode_step_workspace_bytes", "sscvae_decode_step",
+    "sscvae_train_step_image_state_bytes", "sscvae_train_step_tape_bytes", "sscvae_train_step_workspace_bytes",
+    "sscvae_train_step_image_state", "sscvae_train_step_forward", "sscvae_train_step_backward",
 ]
 
 
@@ -113,6 +115,14 @@ def lib():
     L.sscvae_decode_step_workspace_bytes.restype = sz
     L.sscvae_decode_step.argtypes = [vp, i32, i32, i32, vp, C.POINTER(vp), vp, vp, vp, vp, vp, vp, C.POINTER(vp), vp, u64,
                                      vp, sz, vp, C.POINTER(vp), vp, vp, vp]
+    for name in ("sscvae_train_step_image_state_bytes", "sscvae_train_step_tape_bytes", "sscvae_train_step_workspace_bytes"):
+        getattr(L, name).argtypes = [vp, i32, i32]
+        getattr(L, name).restype = sz
+    L.sscvae_train_step_image_state.argtypes = [vp, i32, i32, vp, C.POINTER(vp), vp, vp, vp, sz, vp]
+    L.sscvae_train_step_forward.argtypes = [vp, i32, i32, vp, C.POINTER(vp), vp, sz, vp, vp, C.POINTER(vp), vp, u64, vp, sz,
+                                            vp, sz, vp, C.POINTER(vp), vp, vp, vp, vp, vp]
+    L.sscvae_train_step_backward.argtypes = [vp, i32, i32, vp, C.POINTER(vp), vp, sz, vp, sz, vp, sz, vp, C.POINTER(vp), vp,
+                                             vp, vp, vp, C.POINTER(vp), C.POINTER(vp), vp]
     L.sscvae_decode_samples_search_region.argtypes = [vp, i32, i32, i32, i32, i32, i32, C.c_char_p, C.POINTER(sz), C.POINTER(sz)]
     L.sscvae_test_gemm_splitk.argtypes = [vp, i32, vp, i32, i32, i32, i32, vp, i32, i32, vp, vp]
     L.sscvae_sgd_step_multi.argtypes = [i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(u64), C.POINTER(i32),

@@ -136,6 +136,58 @@ class _TrainStep(torch.autograd.Function):
         return (None, None, None, None, None, None, None) + tuple(out)
 
 
+class _TrainDecodeStep(torch.autograd.Function):
+    """One training step of the cell: forward = sscvae_train_step_forward, backward = sscvae_train_step_backward.
+
+    Inputs: module, boxes N, image state (uint8), sentiment, prev tokens, eps, seed, tape (uint8), the six input states (or
+    Nones), then the parameters. Outputs: logits, the six states, mean, log_var, prior mean (sentiment_vae == 2, else
+    empty), alpha."""
+
+    @staticmethod
+    def forward(ctx, module, N, state, sentiment, prev, eps, seed, tape, *rest):
+        states, params = rest[:6], rest[6:]
+        outs = module._train_step_call(N, state, sentiment, prev, None if states[0] is None else states, eps, seed, tape)
+        ctx.module, ctx.state, ctx.tape, ctx.shape = module, state, tape, (prev.numel(), N)
+        ctx.has_states = states[0] is not None
+        # the parameters are saved so that an in-place update before backward raises autograd's version error
+        ctx.save_for_backward(*params)
+        if outs[9].numel() == 0:
+            ctx.mark_non_differentiable(outs[9])
+        ctx.set_materialize_grads(False)
+        return outs
+
+    @staticmethod
+    def backward(ctx, d_logits, *d):
+        module = ctx.module
+        params = ctx.saved_tensors                       # raises if a parameter was modified in place since forward
+        d_states, d_mean, d_log_var, d_pm, d_alpha = d[:6], d[6], d[7], d[8], d[9]
+        B, N = ctx.shape
+        dev = params[0].device
+        if d_logits is None:
+            d_logits = torch.zeros(B, module._vocab_size, device=dev)
+        f = lambda t: None if t is None or t.numel() == 0 else t.contiguous().float()
+        # held in locals until the call has been enqueued: a temporary's block could otherwise be handed to the next one
+        d_logits, d_mean, d_log_var, d_pm, d_alpha = f(d_logits), f(d_mean), f(d_log_var), f(d_pm), f(d_alpha)
+        d_states = [f(t) for t in d_states]
+        n_in = 8
+        needs = ctx.needs_input_grad
+        d_in = [torch.empty(B, module.hidden_size, device=dev) if ctx.has_states and needs[n_in + k] else None
+                for k in range(6)]
+        grads = []
+        for i, p in enumerate(params):
+            want = needs[n_in + 6 + i] and not (module._tied and i == 0)
+            grads.append(torch.empty_like(p) if want else None)
+        L = _lib.lib()
+        ws = module._train_step_workspace(B, N)
+        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _lib.check(L.sscvae_train_step_backward(
+            module._handle, B, N, _lib.ptr(module._packed_weights()), _lib.ptr_array(params), _lib.ptr(ctx.state),
+            ctx.state.numel(), _lib.ptr(ctx.tape), ctx.tape.numel(), _lib.ptr(ws), ws.numel(), _lib.ptr(d_logits),
+            _lib.ptr_array(d_states), _lib.ptr(d_mean), _lib.ptr(d_log_var), _lib.ptr(d_pm), _lib.ptr(d_alpha),
+            _lib.ptr_array(d_in), _lib.ptr_array(grads), stream))
+        return (None,) * n_in + tuple(d_in) + tuple(grads)
+
+
 class UpDownCaptioner(nn.Module):
     def __init__(
         self,
@@ -242,6 +294,9 @@ class UpDownCaptioner(nn.Module):
         # True: outputs also carry "attention", the attention weights over the boxes behind every word (the last element
         # of the reference's eval step, updown_captioner.py:371-455): fp32, new tensors, not differentiable
         self.return_attention = False
+        # True: _decode_step also runs in training mode, as the reference's training loop calls it (updown_captioner.py:282-310):
+        # a differentiable step per call, for per-step objectives; the fused training forward() stays the fast path
+        self.stepwise_training = False
         self._eps_override = None          # tests: explicit eps tensor
         self._call_counter = 0
         self.last_search = None
@@ -548,7 +603,6 @@ class UpDownCaptioner(nn.Module):
     # ------------------------------------------------------------------------------------------
     _STATE_KEYS = ("h1", "c1", "h_encoder", "c_encoder", "h_decoder", "c_decoder")
 
-    @torch.no_grad()
     def _decode_step(self, image_features, obj_atts, previous_predictions, states, sentiment=None, prior_mean=None,
                      prior_var=None):
         """The reference's eval-mode step function (updown_captioner.py:371-455), which its forward hands to the search as
@@ -560,9 +614,21 @@ class UpDownCaptioner(nn.Module):
         for the prior forward() builds. Returns the reference's eval 5-tuple
         (log_probs (R, V), states, prior_mean (R, Z), prior_log_var (R, Z), attention (R, N)): new fp32 tensors, not
         differentiable; h_encoder / c_encoder pass through (zeros for states=None). One sscvae_decode_step call; the
-        per-image state is recomputed only when the features changed (storage, shape, dtype or an in-place edit)."""
+        per-image state is recomputed only when the features changed (storage, shape, dtype or an in-place edit).
+
+        In training mode with `stepwise_training = True` it is the reference's training step instead: see
+        `_train_decode_step`. Without the switch, training mode raises NotImplementedError."""
         if self.training:
-            raise NotImplementedError("_decode_step runs in eval mode only; the fused training forward() is the training path")
+            if not self.stepwise_training:
+                raise NotImplementedError("_decode_step in training mode needs `stepwise_training = True` (one differentiable "
+                                          "step per call); the fused training forward() is the fast training path")
+            return self._train_decode_step(image_features, obj_atts, previous_predictions, states, sentiment, prior_mean,
+                                           prior_var)
+        with torch.no_grad():
+            return self._eval_decode_step(image_features, obj_atts, previous_predictions, states, sentiment, prior_mean,
+                                          prior_var)
+
+    def _eval_decode_step(self, image_features, obj_atts, previous_predictions, states, sentiment, prior_mean, prior_var):
         self._require_cuda(image_features)
         L = _lib.lib()
         given = image_features
@@ -639,6 +705,133 @@ class UpDownCaptioner(nn.Module):
         prior_log_var = var.log().repeat_interleave(R // B, dim=0)
         new_states = {"h1": h1, "c1": c1, "h_encoder": enc[0], "c_encoder": enc[1], "h_decoder": hd, "c_decoder": cd}
         return log_probs, new_states, pm, prior_log_var, alpha
+
+    def _train_decode_step(self, image_features, obj_atts, previous_predictions, states, sentiment, prior_mean, prior_var):
+        """The reference's training-mode step (updown_captioner.py:371-455, updown_cell.py:143-231), one call per timestep of
+        its training loop (updown_captioner.py:282-310). One row per image: previous_predictions (B,). states: the six
+        (B, H) tensors, or None for zero states; the encoder pair is read. prior_mean / prior_var: (B, Z) or None for the
+        prior forward() builds; they only enter the returned prior.
+
+        Returns the reference's training 7-tuple (logits (B,V) raw, states, mean (B,Z), log_var (B,Z), prior_mean (B,Z),
+        prior_log_var (B,Z), attention (B,N)), fp32. logits, the states, mean, log_var and attention are differentiable with
+        respect to every trainable parameter and the input states, so gradients chain across steps through autograd and
+        reach `.grad` by its normal accumulation; with sentiment_vae == 2 the prior mean is differentiable through the
+        attention. The prior otherwise passes through in torch (prior_log_var = prior_var.log()), zeros for simple_vae.
+        image_features, sentiment and obj_atts get no gradient. Under torch.no_grad(), or when nothing needs a gradient, no
+        tape is kept. Each step keeps its own tape, and the per-image state of each feature tensor is a buffer of its
+        own, so graphs over different batches can be alive together."""
+        self._require_cuda(image_features)
+        given = image_features
+        image_features = self._features(image_features)
+        dev = image_features.device
+        B, N, F = image_features.shape
+        if F != self.image_feature_size:
+            raise ValueError(f"image_features last dim {F} != image_feature_size {self.image_feature_size}")
+        prev = previous_predictions.to(dev).long().contiguous().view(-1)
+        H, Z, V = self.hidden_size, self.z_space, self._vocab_size
+        if prev.numel() != B:
+            raise ValueError(f"previous_predictions has {prev.numel()} rows; in training mode it needs one per image ({B})")
+        torch._assert_async(((prev >= 0) & (prev < V)).all(), "previous_predictions contains an id outside [0, vocab_size)")
+        if self.sentiment_vae == 1:
+            if sentiment is None:
+                raise ValueError("sentiment is required when sentiment_vae == 1")
+            sentiment = sentiment.to(dev).contiguous().float().view(B, 1)
+        else:
+            sentiment = None
+        obj_means = self._obj_means(obj_atts, B, N, dev)
+        if states is None:
+            st = [None] * 6
+        else:
+            st = []
+            for k in self._STATE_KEYS:
+                v = states[k]
+                if v.shape != (B, H):
+                    raise ValueError(f"states[{k!r}] must be (B, hidden_size) = {(B, H)}, got {tuple(v.shape)}")
+                st.append(v.to(dev).contiguous().float())
+        eps = self._eps_override
+        if eps is None and self.rng_mode == "reference":
+            eps = torch.randn(B, Z)                                   # one (B,Z) CPU draw per step, like updown_cell.py:206
+        if eps is not None:
+            eps = eps.to(dev).contiguous().float()
+            assert eps.shape == (B, Z)
+        params = self._weight_tensors()
+        state = self._train_step_image_state(given, image_features, obj_atts if torch.is_tensor(obj_atts) else obj_means,
+                                             obj_means)
+        seed = self._next_seed()
+        grad = torch.is_grad_enabled() and (any(p.requires_grad for p in params) or
+                                            any(t is not None and t.requires_grad for t in st))
+        if grad:
+            tape = torch.empty(_lib.lib().sscvae_train_step_tape_bytes(self._handle, B, N), dtype=torch.uint8, device=dev)
+            outs = _TrainDecodeStep.apply(self, N, state, sentiment, prev, eps, seed, tape, *st, *params)
+        else:
+            outs = self._train_step_call(N, state, sentiment, prev, None if st[0] is None else st, eps, seed,
+                                         self._train_step_workspace(B, N, "tape"))
+        logits, s_out, mean, log_var, pm, alpha = outs[0], outs[1:7], outs[7], outs[8], outs[9], outs[10]
+        var = prior_var.to(dev).float() if prior_var is not None else torch.full((B, Z), float(self.prior_std), device=dev).pow(2)
+        if self.simple_vae:
+            pm = torch.zeros(B, Z, device=dev)                                           # updown_cell.py:165-166
+        elif self.sentiment_vae != 2:
+            if prior_mean is not None:
+                pm = prior_mean.to(dev).float()
+            elif self.sentiment_vae == 1:
+                pm = sentiment.repeat(1, Z) * self.senti_prior_multip                    # updown_captioner.py:250-253
+            else:
+                pm = torch.zeros(B, Z, device=dev)
+        new_states = dict(zip(self._STATE_KEYS, s_out))
+        return logits, new_states, mean, log_var, pm, var.log(), alpha
+
+    def _train_step_call(self, N, state, sentiment, prev, states, eps, seed, tape):
+        """sscvae_train_step_forward into new output tensors: logits, six states, mean, log_var, prior mean, alpha."""
+        B = prev.numel()
+        dev = prev.device
+        H, Z = self.hidden_size, self.z_space
+        logits = torch.empty(B, self._vocab_size, device=dev)
+        s_out = [torch.empty(B, H, device=dev) for _ in range(6)]
+        mean, log_var = torch.empty(B, Z, device=dev), torch.empty(B, Z, device=dev)
+        pm = torch.empty(B, Z, device=dev) if self.sentiment_vae == 2 and not self.simple_vae else torch.empty(0, device=dev)
+        alpha = torch.empty(B, N, device=dev)
+        ws = self._train_step_workspace(B, N)
+        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _lib.check(_lib.lib().sscvae_train_step_forward(
+            self._handle, B, N, _lib.ptr(self._packed_weights()), _lib.ptr_array(self._weight_tensors()), _lib.ptr(state),
+            state.numel(), _lib.ptr(sentiment), _lib.ptr(prev), None if states is None else _lib.ptr_array(states),
+            _lib.ptr(eps), C.c_uint64(seed), _lib.ptr(tape), tape.numel(), _lib.ptr(ws), ws.numel(), _lib.ptr(logits),
+            _lib.ptr_array(s_out), _lib.ptr(mean), _lib.ptr(log_var), _lib.ptr(pm if pm.numel() else None), _lib.ptr(alpha),
+            stream))
+        return (logits, *s_out, mean, log_var, pm, alpha)
+
+    def _train_step_workspace(self, B, N, kind="workspace") -> torch.Tensor:
+        """The training step's shared scratch (kind "workspace"), or a scratch tape for steps without autograd ("tape")."""
+        dev = self._embedding_layer.weight.device
+        key = ("step_" + kind, B, N, dev)
+        ws = self._ws_cache.get(key)
+        if ws is None:
+            fn = _lib.lib().sscvae_train_step_workspace_bytes if kind == "workspace" else _lib.lib().sscvae_train_step_tape_bytes
+            ws = torch.empty(fn(self._handle, B, N), dtype=torch.uint8, device=dev)
+            self._ws_cache = {k: v for k, v in self._ws_cache.items() if k[0] != key[0]}
+            self._ws_cache[key] = ws
+        return ws
+
+    def _train_step_image_state(self, given, image_features, given_obj, obj_means) -> torch.Tensor:
+        """The per-image state of the training step for these features (and obj_means, and the current weights): rebuilt
+        into a NEW buffer whenever any of them changed, never in place, because the tapes of earlier steps keep the old
+        one. Keyed on the caller's tensors (`given`, `given_obj`), like the eval step's state."""
+        B, N, _ = image_features.shape
+        ws = self._weight_tensors()
+        tkey = lambda t: None if t is None else (t.data_ptr(), t._version, tuple(t.shape), t.dtype, t.stride())
+        key = (tkey(given), tkey(given_obj), self._weights_key(ws))
+        last = getattr(self, "_train_step_state", None)
+        if last is not None and last[0] is given and last[1] is given_obj and last[2] == key:
+            return last[3]
+        L = _lib.lib()
+        dev = image_features.device
+        state = torch.empty(L.sscvae_train_step_image_state_bytes(self._handle, B, N), dtype=torch.uint8, device=dev)
+        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _lib.check(L.sscvae_train_step_image_state(self._handle, B, N, _lib.ptr(self._packed_weights()), _lib.ptr_array(ws),
+                                                   _lib.ptr(image_features), _lib.ptr(obj_means), _lib.ptr(state),
+                                                   state.numel(), stream))
+        self._train_step_state = (given, given_obj, key, state)    # keeps the tensors alive: no new one takes their storage
+        return state
 
     def translate_obj_atts2obj_means(self, obj_atts) -> torch.Tensor:
         """Per-box attribute means of sentiment_vae == 2 (updown_captioner.py:509-532): `obj_atts` holds, per image, one

@@ -69,6 +69,10 @@ struct LatentArgs {
   const float* prior_var_img;          // optional (images,Z) per-component prior variance (replaces prior_var)
   float* pm_out;                       // optional (R,Z): the prior mean z was drawn around
   unsigned long long seed;             // Philox seed when seed_dev is null
+  // backward of sscvae_train_step_backward: upstream gradients of the step's mean / log_var outputs (null = zero) replace
+  // the built-in KL term (gkld, tmask_t unused): the caller computes the KL (updown_captioner.py:295-303) itself
+  int upstream;
+  const float* dmean_up; const float* dlogvar_up;
 };
 // sentiment_vae == 2 (updown_cell.py:160-174): pm[r,:] = sum_n alpha[r,n] * obj[img(r),n,:]; the first `cond` components
 // are also written as the bf16 conditioning block c of the encoder / decoder LSTM inputs (cond = Z: "glove", 1: "senti_word_net")
@@ -113,9 +117,23 @@ int greedy_merge(cudaStream_t s, const float* st_max, const float* st_sum, const
 int log_softmax_rows(cudaStream_t s, const float* st_max, const float* st_sum, const int* st_arg, int ntiles, int R, int V,
                      float* logits);
 // sscvae_decode_step's per-call input: tok[r] = prev[r] (int64 -> int32), rowmap[r] = r / rows_per_image and, unless h1 is
-// null, the bf16 operand rows xa[r] = [h1[r] | 0 | h_dec[r] | 0] (2 blocks of Hp, K-padding zeroed) from the fp32 states
+// null, the bf16 operand rows xa[r] = [h1[r] | 0 | h_dec[r] | 0] (2 blocks of Hp, K-padding zeroed) from the fp32 states.
+// The training step (sscvae_train_step_forward) also builds the encoder operand rows: unless null, he[r] = [h_enc[r] | 0]
+// (Hp) and xe_hd[r * ld_xe + :Hp] = [h_dec[r] | 0], the h_dec_{t-1} block of [xhat | h1 | h_dec_{t-1}]
 int step_import(cudaStream_t s, const long long* prev, int R, int rows_per_image, const float* h1, const float* h_dec, int H,
-                int Hp, int* tok, int* rowmap, bf16* xa);
+                int Hp, int* tok, int* rowmap, bf16* xa, const float* h_enc = nullptr, bf16* he = nullptr,
+                bf16* xe_hd = nullptr, int ld_xe = 0);
+// sscvae_train_step_backward: the gradients of the step's six input states in fp32 (R,H), the reference's order h1, c1,
+// h_encoder, c_encoder, h_decoder, c_decoder (null entries skipped). d h_dec_{t-1} sums its two operand blocks: the encoder /
+// decoder input dxe[:, off_hd] and the attention-LSTM input dxa[:, Hp]
+struct StepGradExport {
+  int R, H, Hp;
+  const float* dxa; int ld_xa;         // d [h1_{t-1} | h_dec_{t-1}]
+  const float* dxe; int ld_xe; int off_hd, off_he;   // d [xhat | h1 | h_dec_{t-1} | h_enc_{t-1} ..]: column blocks
+  const float* dc[3];                  // d c1_{t-1}, d c_enc_{t-1}, d c_dec_{t-1}  (R,H)
+  float* out[6];
+};
+int step_export_grads(cudaStream_t s, const StepGradExport& a);
 
 // ---- layout helpers -------------------------------------------------------------------------------
 // out[c, r] = in[r, c] (bf16, c < cols, r < ld_out; zero for r >= rows, so the padded out is a GEMM operand) for a
@@ -190,6 +208,8 @@ int sum_partials_f32(cudaStream_t s, float* dst, int ld_dst, const float* parts,
 int scale_rows_f32(cudaStream_t s, const float* in, float scale, float* out, int n);
 // dEmb[tok[b,t], :] += dx[(t*B+b), :] skipping the padding index (nn.Embedding padding_idx)
 int embed_scatter_add(cudaStream_t s, const int* tok, int B, int L, int pad, const float* dx, int ld_dx, int E, float* demb);
+// the same for R rows of one step: dEmb[tok[r], :] += dx[r, :]
+int embed_scatter_add_rows(cudaStream_t s, const int* tok, int R, int pad, const float* dx, int ld_dx, int E, float* demb);
 int gather_rows_f32(cudaStream_t s, const float* src, const int* idx, int R, int n, float* dst);
 int gather_rows_bf16(cudaStream_t s, const bf16* src, const int* idx, int R, int n, int ld, bf16* dst);
 

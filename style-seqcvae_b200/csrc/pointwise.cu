@@ -380,7 +380,7 @@ __global__ void latent_fwd_train_kernel(LatentArgs a, const float* __restrict__ 
       const float mu = ml[(size_t)r * ld_ml + z] + bias_ml[z];
       const float lv = ml[(size_t)r * ld_ml + Z + z] + bias_ml[Z + z];
       const float var = __expf(lv);
-      const float e = eps_in ? eps_in[(size_t)r * Z + z] : philox_normal(*seed_dev, step, r, z, Z);
+      const float e = eps_in ? eps_in[(size_t)r * Z + z] : philox_normal(seed_dev ? *seed_dev : a.seed, step, r, z, Z);
       const float zz = e * sqrtf(var) + mu;
       mean_out[(size_t)r * Z + z] = mu;
       logvar_out[(size_t)r * Z + z] = lv;
@@ -451,7 +451,7 @@ __global__ void latent_bwd_kernel(LatentArgs a, const float* __restrict__ dz, in
   const int r = blockIdx.x;
   const int Z = a.Z;
   const float pm_row = a.prior_mean_row ? a.prior_mean_row[a.rowmap ? a.rowmap[r] : r] : 0.f;
-  const float w = gkld[r] * tmask_t[r];
+  const float w = a.upstream ? 0.f : gkld[r] * tmask_t[r];
   const float inv_pv = 1.0f / (a.prior_var + 0.00001f);
   for (int z = threadIdx.x; z < ld_dml; z += blockDim.x) {
     float out = 0.f;
@@ -463,11 +463,14 @@ __global__ void latent_bwd_kernel(LatentArgs a, const float* __restrict__ dz, in
       if (z < Z) {
         const float pm = a.prior_mean_full ? a.prior_mean_full[(size_t)r * Z + zi] : pm_row;
         const float dkl = (a.sentiment_vae == 0) ? mu : (mu - pm) * inv_pv;
-        out = g + w * dkl;
+        if (a.upstream) out = g + (a.dmean_up ? a.dmean_up[(size_t)r * Z + zi] : 0.f);
+        else out = g + w * dkl;
         if (a.dpm_out) a.dpm_out[(size_t)r * Z + zi] = -w * dkl;      // d kld / d prior_mean = -d kld / d mean
       } else {
         const float dkl = (a.sentiment_vae == 0) ? -0.5f * (1.f - var) : -0.5f * (1.f - var * inv_pv);
-        out = g * eps[(size_t)r * Z + zi] * 0.5f * sqrtf(var) + w * dkl;
+        const float dz_lv = g * eps[(size_t)r * Z + zi] * 0.5f * sqrtf(var);
+        if (a.upstream) out = dz_lv + (a.dlogvar_up ? a.dlogvar_up[(size_t)r * Z + zi] : 0.f);
+        else out = dz_lv + w * dkl;
       }
     }
     dml[(size_t)r * ld_dml + z] = __float2bfloat16_rn(out);
@@ -768,11 +771,12 @@ int log_softmax_rows(cudaStream_t s, const float* st_max, const float* st_sum, c
 // one warp per row: the token and image index of the row, then (with states) its bf16 [h1 | h_dec] operand row
 __global__ void step_import_kernel(const long long* __restrict__ prev, int R, int rows_per_image, const float* __restrict__ h1,
                                    const float* __restrict__ hd, int H, int Hp, int* __restrict__ tok, int* __restrict__ rowmap,
-                                   bf16* __restrict__ xa) {
+                                   bf16* __restrict__ xa, const float* __restrict__ he_in, bf16* __restrict__ he,
+                                   bf16* __restrict__ xe_hd, int ld_xe) {
   const int r = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (r >= R) return;
   const int lane = threadIdx.x & 31;
-  if (lane == 0) { tok[r] = (int)prev[r]; rowmap[r] = r / rows_per_image; }
+  if (lane == 0) { tok[r] = (int)prev[r]; if (rowmap) rowmap[r] = r / rows_per_image; }
   if (!h1) return;
   bf16* o = xa + (size_t)r * 2 * Hp;
   for (int c = lane; c < 2 * Hp; c += 32) {
@@ -780,12 +784,37 @@ __global__ void step_import_kernel(const long long* __restrict__ prev, int R, in
     const float* src = c < Hp ? h1 : hd;
     o[c] = __float2bfloat16_rn(j < H ? src[(size_t)r * H + j] : 0.f);
   }
+  if (he)
+    for (int j = lane; j < Hp; j += 32) he[(size_t)r * Hp + j] = __float2bfloat16_rn(j < H ? he_in[(size_t)r * H + j] : 0.f);
+  if (xe_hd)
+    for (int j = lane; j < Hp; j += 32) xe_hd[(size_t)r * ld_xe + j] = __float2bfloat16_rn(j < H ? hd[(size_t)r * H + j] : 0.f);
 }
 int step_import(cudaStream_t s, const long long* prev, int R, int rows_per_image, const float* h1, const float* h_dec, int H,
-                int Hp, int* tok, int* rowmap, bf16* xa) {
+                int Hp, int* tok, int* rowmap, bf16* xa, const float* h_enc, bf16* he, bf16* xe_hd, int ld_xe) {
   PROF_SCOPE(s, "step_import", 0, (double)R * (12.0 + (h1 ? 2.0 * H * 4.0 + 4.0 * Hp : 0.0)));
-  REQUIRE(rows_per_image > 0 && (!h1 || (h_dec && xa)), "step_import: bad arguments");
-  step_import_kernel<<<ceil_div(R, 8), 256, 0, s>>>(prev, R, rows_per_image, h1, h_dec, H, Hp, tok, rowmap, xa);
+  REQUIRE(rows_per_image > 0 && (!h1 || (h_dec && xa)) && (!he || (h1 && h_enc)) && (!xe_hd || h1),
+          "step_import: bad arguments");
+  step_import_kernel<<<ceil_div(R, 8), 256, 0, s>>>(prev, R, rows_per_image, h1, h_dec, H, Hp, tok, rowmap, xa, h_enc, he,
+                                                    xe_hd, ld_xe);
+  LAUNCHED();
+  return 0;
+}
+
+__global__ void step_export_grads_kernel(const StepGradExport a) {
+  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= a.R * a.H) return;
+  const int r = idx / a.H, j = idx - r * a.H;
+  const float* xa = a.dxa + (size_t)r * a.ld_xa;
+  const float* xe = a.dxe + (size_t)r * a.ld_xe;
+  if (a.out[0]) a.out[0][idx] = xa[j];
+  if (a.out[2]) a.out[2][idx] = xe[a.off_he + j];
+  if (a.out[4]) a.out[4][idx] = xe[a.off_hd + j] + xa[a.Hp + j];
+  for (int k = 0; k < 3; ++k)
+    if (a.out[2 * k + 1]) a.out[2 * k + 1][idx] = a.dc[k][idx];
+}
+int step_export_grads(cudaStream_t s, const StepGradExport& a) {
+  PROF_SCOPE(s, "step_export", 0, (double)a.R * a.H * 4.0 * 10.0);
+  step_export_grads_kernel<<<ceil_div(a.R * a.H, 256), 256, 0, s>>>(a);
   LAUNCHED();
   return 0;
 }
@@ -1061,17 +1090,23 @@ int scale_rows_f32(cudaStream_t s, const float* in, float scale, float* out, int
   return 0;
 }
 
-__global__ void embed_scatter_kernel(const int* __restrict__ tok, int B, int L, int pad, const float* __restrict__ dx,
+// row r = t * B + b of dx takes token tok[b * tok_stride_b + t]
+__global__ void embed_scatter_kernel(const int* __restrict__ tok, int B, int tok_stride_b, int pad, const float* __restrict__ dx,
                                      int ld_dx, int E, float* __restrict__ demb) {
   const int r = blockIdx.x;
   const int t = r / B, b = r % B;
-  const int id = tok[(size_t)b * (L + 2) + t];
+  const int id = tok[(size_t)b * tok_stride_b + t];
   if (id == pad) return;
   for (int e = threadIdx.x; e < E; e += blockDim.x) atomicAdd(&demb[(size_t)id * E + e], dx[(size_t)r * ld_dx + e]);
 }
 int embed_scatter_add(cudaStream_t s, const int* tok, int B, int L, int pad, const float* dx, int ld_dx, int E,
                       float* demb) {
-  embed_scatter_kernel<<<(L + 1) * B, 128, 0, s>>>(tok, B, L, pad, dx, ld_dx, E, demb);
+  embed_scatter_kernel<<<(L + 1) * B, 128, 0, s>>>(tok, B, L + 2, pad, dx, ld_dx, E, demb);
+  LAUNCHED();
+  return 0;
+}
+int embed_scatter_add_rows(cudaStream_t s, const int* tok, int R, int pad, const float* dx, int ld_dx, int E, float* demb) {
+  embed_scatter_kernel<<<R, 128, 0, s>>>(tok, R, 1, pad, dx, ld_dx, E, demb);
   LAUNCHED();
   return 0;
 }
